@@ -12,6 +12,10 @@ device calls, not the same batch K times.  ``value`` is measured with the batche
 ``e2e`` through ``GpuCaller.call()`` + the device HP / LowC pass from pinned host buffers (H2D + kernels + D2H inside the timed
 region, every step).  The panel is sharded across GPUs by BED interval (weak scaling: every rank gets its own slice); loci are
 independent, so there is no data-path collective -- torch.distributed is used for the barrier and the max-over-ranks only.
+
+The reads are a function of the arguments alone (not of the host's core count), so ``--dump-outputs DIR`` lets two builds be
+compared output for output: after the timed steps it writes what the resident runs of the last step returned (see
+``dump_outputs``) as float64 ``DIR/<name>.npy`` files.
 """
 from __future__ import annotations
 
@@ -32,6 +36,10 @@ METRIC = "target_loci_called_per_sec"
 UNIT = "loci/s"
 ALGO_BYTES_PER_EVENT = 35.0     # SURVEY.md 8(d): reads in once (2.7 B/event) + every 16-byte event written once and read once
 UMIS_PER_LOCUS, RPB = 3000, 4.0
+SYNTH_GROUPS = 16               # make_panel_mp groups per batch: fixed, so that the reads do not depend on the host's core count
+# --dump-outputs: a seeded sample of at most DUMP_LOCI loci (130 values each with the index and the non-finite codes) and DUMP_DYN
+# of their dynamic-allele rows (20 values each), all float64: at most ~58 MB in all, under the DUMP_BYTES cap
+DUMP_LOCI, DUMP_DYN, DUMP_BYTES = 40000, 100000, 64 * 10**6
 
 # BASELINE.json configs as bench workloads: (description, SynthSpec keywords, VcParams keywords, default intervals per batch)
 WORKLOADS = {
@@ -68,7 +76,13 @@ def parse_args(argv=None):
     ap.add_argument("--pipeline-intervals", type=int, default=96,
                     help="intervals of the rank-0 batch run through the whole CLI path (BAM decode -> files); 0 = skip")
     ap.add_argument("--pipeline-repeats", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed resident runs of the last step returned to DIR/<name>.npy (float64)")
     a = ap.parse_args(argv)
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm returns text rows)")
     if a.intervals <= 0:
         a.intervals = WORKLOADS[a.workload][3]
     return a
@@ -107,7 +121,7 @@ def _gen_batch(job):
     (ivs, spec_kw, seed, whole, no_compact, workers, keep_full) = job
     from smcounter_b200.synth import SynthSpec, make_panel_mp
     from smcounter_b200.targets import build_loci
-    soa, refs, truth = make_panel_mp(ivs, SynthSpec(**spec_kw), seed=seed, workers=workers)
+    soa, refs, truth = make_panel_mp(ivs, SynthSpec(**spec_kw), seed=seed, workers=workers, n_groups=SYNTH_GROUPS)
     full = soa
     if not whole:
         soa = soa.trim_to_targets(ivs)
@@ -163,6 +177,47 @@ def config_dict(args, world):
             "params": " ".join("%s %s" % kv for kv in p.items()), "seed": args.seed,
             "l2": "every step streams %d distinct batches (hundreds of MB each): inputs larger than L2, no flush needed" % args.batches,
             "parallelism": "panel sharded by BED interval (balanced by estimated events), no collective"}
+
+
+def dump_outputs(path, outs, prefix="", share=1):
+    """--dump-outputs: the LocusResults the resident runs of the last timed step downloaded, the rank's batches concatenated in
+    batch order, as float64 ``path/<prefix><name>.npy``.  Per-locus arrays keep their layout (locus axis last) for a seeded sample
+    of at most DUMP_LOCI / share loci, whose indices into the concatenation are ``locus``; the dynamic-allele rows of those loci
+    (at most DUMP_DYN / share, a seeded sample beyond that) carry the same index in ``dyn_locus``.  Left out: dyn_rep_read /
+    dyn_rep_qpos, which point at whichever read carrying the allele reached the device table first, so they vary from run to run.
+    Every file holds finite numbers only: the floating-point results (PI, Fisher p and odds ratio; NaN where a test was not
+    evaluated or an odds ratio is 0/0, +inf where it divides by zero) hold 0 in place of a non-finite value, and beside each
+    ``<name>`` a ``<name>_nonfinite`` array of the same shape says which value it was: 0 finite, 1 +inf, -1 -inf, 2 NaN."""
+    import numpy as np
+    per_locus = ("loc", "cnt", "pi", "max_allele", "second_allele", "alt_allele", "alt_pi", "second_pi", "fl1", "fl2", "biallelic",
+                 "fisher_p", "fisher_or")
+    per_dyn = ("dyn_kind", "dyn_site", "dyn_len", "dyn_iskey", "dyn_cnt", "dyn_pi")
+    base = np.cumsum([0] + [o.n_loci for o in outs])
+    n, max_loci, max_dyn = int(base[-1]), DUMP_LOCI // share, DUMP_DYN // share
+    rng = np.random.default_rng(0)
+    locus = np.arange(n) if n <= max_loci else np.sort(rng.choice(n, size=max_loci, replace=False))
+    arrays = {"locus": locus}
+    for f in per_locus:
+        arrays[f] = np.concatenate([getattr(o, f)[..., :o.n_loci] for o in outs], axis=-1)[..., locus]
+    dyn_locus = np.concatenate([o.dyn_locus[:o.n_dyn].astype(np.int64) + b for o, b in zip(outs, base)])
+    rows = np.flatnonzero(np.isin(dyn_locus, locus))
+    if len(rows) > max_dyn:
+        rows = np.sort(rng.choice(rows, size=max_dyn, replace=False))
+    arrays["dyn_locus"] = dyn_locus[rows]
+    for f in per_dyn:
+        arrays[f] = np.concatenate([getattr(o, f)[:o.n_dyn] for o in outs])[rows]
+    for k in [k for k, v in arrays.items() if v.dtype.kind == "f"]:
+        v = arrays[k]
+        code = np.where(np.isnan(v), 2.0, np.where(np.isinf(v), np.sign(v), 0.0))
+        arrays[k], arrays[k + "_nonfinite"] = np.where(code == 0, v, 0.0), code
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    assert all(np.isfinite(a).all() for a in arrays.values())
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BYTES // share, total
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, prefix + k + ".npy"), a)
+    return total
 
 
 class ClockSampler(threading.Thread):
@@ -536,6 +591,8 @@ def main():
         outs.append(c.download(LocusResults(loci.n, max(int(tm["n_dyn"]), 16), pinned=True)))
         c.close()
     n_dyn = sum(o.n_dyn for o in outs)
+    if args.dump_outputs:           # before the end-to-end leg reuses these buffers
+        dump_outputs(args.dump_outputs, outs, prefix="rank%d." % rank if world > 1 else "", share=world)
 
     # ---------------- end to end: host buffers in, host buffers out, every step: smc_call_batch (pipelined upload, kernels,
     # download) and the device HP / LowC pass over the candidates of the batch (smc_hp_lowcomp)
@@ -578,7 +635,8 @@ def main():
     for i in range(len(callers)):
         for k in range(NB):
             callers[i].call(batches[k][1], batches[k][3], out=outs[k])
-    e2e_pass(min(args.warmup, 2))
+    if args.warmup:
+        e2e_pass(min(args.warmup, 2))
     barrier()
     t1 = time.perf_counter()
     h2d_b, d2h_b, e2e_tm = e2e_pass(args.steps)

@@ -368,9 +368,10 @@ def _mp_job(args):
     return make_panel(intervals, spec, seed=seed, chroms=chroms, lengths=lengths, umi_base=umi_base)
 
 
-def make_panel_mp(intervals, spec: SynthSpec | None = None, seed: int = 1, workers: int | None = None):
+def make_panel_mp(intervals, spec: SynthSpec | None = None, seed: int = 1, workers: int | None = None, n_groups: int | None = None):
     """make_panel() over groups of intervals in worker processes (bench-scale inputs).  Deterministic for a given
-    (intervals, spec, seed, number of groups)."""
+    (intervals, spec, seed, number of groups); ``n_groups`` defaults to 4 per worker, so pass it to get the same reads
+    whatever the number of workers."""
     import multiprocessing as mp
     import os
 
@@ -384,7 +385,7 @@ def make_panel_mp(intervals, spec: SynthSpec | None = None, seed: int = 1, worke
     lengths = {c: 0 for c in chroms}
     for (c, s, e) in intervals:
         lengths[c] = max(lengths[c], e + 2 * margin)
-    ngroups = max(1, min(len(intervals), workers * 4))
+    ngroups = max(1, min(len(intervals), n_groups or workers * 4))
     groups = [intervals[i::ngroups] for i in range(ngroups)]
     jobs = [(g, spec, seed * 1000003 + i, chroms, lengths, i << 24) for i, g in enumerate(groups)]
     if workers > 1 and ngroups > 1:

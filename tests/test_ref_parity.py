@@ -17,7 +17,12 @@ What is asserted here:
     oracle's ``run()``;
   * the committed fixture tests/golden/ref_rows.json (made by tests/golden/make_ref_rows.py from the reference's code)
     is what the oracle produces -- this one also runs where /root/reference and oracle/_ref are absent.
+
+The reference is not distributed with this project.  Where it is absent, the vc() comparisons on the cases, the fuzz corpus
+and at benchmark depth take the reference's rows from tests/golden/ref_rows.json (every case, the deep cases and the fuzz
+seeds stored there); the other comparisons call the reference's functions on fresh inputs and skip.
 """
+import functools
 import json
 import math
 import multiprocessing
@@ -28,7 +33,7 @@ import pytest
 
 from oracle import ref_build, ref_shims
 from oracle import smcounter_oracle as orc
-from fuzz import CASES, case_inputs, fuzz_case
+from fuzz import CASES, DEEP_CASES, case_inputs, fuzz_case
 from smcounter_b200.soa import soa_to_records
 from smcounter_b200.caller import VcParams
 from smcounter_b200.synth import SynthSpec, make_panel
@@ -45,18 +50,32 @@ def _vc_args(prm):
     return (prm.minBQ, prm.minMQ, prm.mtDepth, prm.rpb, prm.hpLen, prm.mismatchThr, prm.mtDrop, prm.maxMT, prm.primerDist)
 
 
-def both_rows(intervals, spec, prm, seed, order="py2"):
-    """[(oracle row, reference-code row, oracle detail)] for every locus of the case."""
-    ref = ref_build.load(order)
+@functools.lru_cache(maxsize=None)
+def stored_ref_rows():
+    """{case name: rows} of tests/golden/ref_rows.json: what the reference's vc() printed (Python-2 container order)."""
+    with open(os.path.join(GOLD, "ref_rows.json")) as fh:
+        return json.load(fh)["cases"]
+
+
+def both_rows(intervals, spec, prm, seed, order="py2", stored=None):
+    """[(oracle row, reference-code row, oracle detail)] for every locus of the case.  The reference's rows come from its own
+    vc() where the reference is present, else from case ``stored`` of tests/golden/ref_rows.json."""
+    live = ref_build.available()
+    assert live or (stored is not None and order == "py2")
     soa, refs, _ = make_panel(intervals, spec, seed=seed)
     index = orc.ReadIndex(soa_to_records(soa, orc.Read))
-    bam = ref_shims.register_bam("mem:%d.bam" % seed, index)
-    fa = ref_shims.register_fasta("mem:%d.fa" % seed, refs)
+    if live:
+        ref = ref_build.load(order)
+        bam = ref_shims.register_bam("mem:%d.bam" % seed, index)
+        fa = ref_shims.register_fasta("mem:%d.fa" % seed, refs)
+    else:
+        want = stored_ref_rows()[stored]
+        assert len(want) == len(loc_list(intervals)), stored
     out = []
-    for (chrom, pos) in loc_list(intervals):
+    for k, (chrom, pos) in enumerate(loc_list(intervals)):
         d = {}
         a = orc.vc(index, chrom, pos, *_vc_args(prm), refs, detail=d)
-        b = ref.vc(bam, chrom, pos, *_vc_args(prm), fa)
+        b = ref.vc(bam, chrom, pos, *_vc_args(prm), fa) if live else want[k]
         out.append((a, b, d))
     ref_shims.clear_registries()
     return out
@@ -81,7 +100,7 @@ def classify(a, b, d):
 def _fuzz_worker(seed):
     ivs, spec, prm = fuzz_case(seed)
     n, diffs = 0, []
-    for (a, b, d) in both_rows(ivs, spec, prm, seed):
+    for (a, b, d) in both_rows(ivs, spec, prm, seed, stored="fuzz%d" % seed):
         n += 1
         c = classify(a, b, d)
         if c is not None:
@@ -107,11 +126,10 @@ def test_recipe_leaves_the_hot_path_untouched():
 
 
 # ---------------------------------------------------------------------------------------------- vc(): cases + fuzz
-@needs_ref
 @pytest.mark.parametrize("name", sorted(CASES))
 def test_reference_vc_equals_oracle_on_cases(name):
     ivs, spec, prm, seed = case_inputs(name)
-    rows = both_rows(ivs, spec, prm, seed)
+    rows = both_rows(ivs, spec, prm, seed, stored=name)
     assert len(rows) == sum(e - s for (_, s, e) in ivs)
     bad = [classify(a, b, d) for (a, b, d) in rows if a != b]
     assert not bad, bad[:5]
@@ -122,11 +140,13 @@ def test_reference_vc_equals_oracle_on_cases(name):
 FUZZ_SEEDS = list(range(101, 301))
 
 
-@needs_ref
 def test_reference_vc_equals_oracle_on_fuzz_corpus():
-    ref_build.load("py2")
-    lo, hi = os.environ.get("SMC_REF_FUZZ_SEEDS", "%d:%d" % (FUZZ_SEEDS[0], FUZZ_SEEDS[-1] + 1)).split(":")
-    seeds = list(range(int(lo), int(hi)))
+    if ref_build.available():
+        ref_build.load("py2")
+        lo, hi = os.environ.get("SMC_REF_FUZZ_SEEDS", "%d:%d" % (FUZZ_SEEDS[0], FUZZ_SEEDS[-1] + 1)).split(":")
+        seeds = list(range(int(lo), int(hi)))
+    else:
+        seeds = sorted(int(k[4:]) for k in stored_ref_rows() if k.startswith("fuzz"))
     ctx = multiprocessing.get_context("fork")
     with ctx.Pool(min(os.cpu_count() or 1, 16)) as pool:
         res = pool.map(_fuzz_worker, seeds, chunksize=1)
@@ -353,24 +373,28 @@ DEEP_TASKS = [  # (name, SynthSpec keywords, VcParams keywords, interval, seed)
 
 
 def _deep_worker(task):
-    name, spec_kw, prm_kw, iv, seed = task
-    rows = both_rows([iv], SynthSpec(**spec_kw), VcParams(**prm_kw), seed)
+    name, spec_kw, prm_kw, iv, seed, stored = task
+    rows = both_rows([iv], SynthSpec(**spec_kw), VcParams(**prm_kw), seed, stored=stored)
     return name, len(rows), [(name, seed) + c for c in (classify(a, b, d) for (a, b, d) in rows) if c is not None], \
         max(d.get("nBC", 0) for (_, _, d) in rows)
 
 
-@needs_ref
 def test_reference_vc_equals_oracle_at_benchmark_depth():
     """The same comparison at the depths the BASELINE.json configurations run at (3 000 / 4 000 / 20 000 barcodes per locus,
     rpb 4 / 9.8): thousands of barcodes go through the Python-2 dict models and calProb per locus, PI sums run over thousands
-    of terms in dict order on the reference side and exactly here."""
-    ref_build.load("py2")
+    of terms in dict order on the reference side and exactly here.  Without the reference: the deep cases of fuzz.DEEP_CASES,
+    whose reference rows tests/golden/ref_rows.json keeps."""
+    if ref_build.available():
+        ref_build.load("py2")
+        tasks = [t + (None,) for t in DEEP_TASKS]
+    else:
+        tasks = [(name[len("deep_"):], spec_kw, prm_kw, ivs[0], seed, name) for name, (spec_kw, prm_kw, ivs, seed) in sorted(DEEP_CASES.items())]
     ctx = multiprocessing.get_context("fork")
-    with ctx.Pool(min(os.cpu_count() or 1, len(DEEP_TASKS))) as pool:
-        res = pool.map(_deep_worker, DEEP_TASKS, chunksize=1)
+    with ctx.Pool(min(os.cpu_count() or 1, len(tasks))) as pool:
+        res = pool.map(_deep_worker, tasks, chunksize=1)
     n = sum(r[1] for r in res)
     diffs = [d for r in res for d in r[2]]
     print("reference vc() vs oracle at depth: %d loci, deepest %s barcodes, differences: %s" % (n, max(r[3] for r in res), diffs))
-    assert n == sum(t[3][2] - t[3][1] for t in DEEP_TASKS)
+    assert n == sum(t[3][2] - t[3][1] for t in tasks)
     assert not [d for d in diffs if d[2] == "BAD"], diffs[:5]
     assert max(r[3] for r in res if r[0] == "cfg3") > 12000 and max(r[3] for r in res if r[0] == "cfg2") > 2000
