@@ -424,7 +424,7 @@ __device__ __noinline__ uint32_t dyn_lookup(DynTab T, unsigned long long key, ui
 }
 
 // Insertions longer than 8 bases do not fit the 64-bit key: the key carries a 32-bit hash of the inserted bases and every hit is
-// verified base by base against the entry's representative read (drep_read / drep_qpos); two different insertions with
+// verified by length (dlen) and base by base against the entry's representative read (drep_read / drep_qpos); two different insertions with
 // equal hashes chain to separate entries, so alleles are never merged (collision free, like the short ones).
 // `my_seq0`: offset of this read's query position 0 in seq[]; the representative's comes from seq_off[] (reads with an
 // insertion are always stored whole).  drep_read doubles as the "entry published" flag (0xffffffff until the creator is done).
@@ -450,7 +450,9 @@ __device__ __noinline__ uint32_t dyn_lookup_long_ins(DynTab T, unsigned long lon
             __threadfence();
             const int rq = *reinterpret_cast<volatile int32_t*>(&T.drep_qpos[h]);
             const uint32_t rs0 = (uint32_t)T.seq_off[rr];
-            bool eq = true;
+            // the key carries no length (only the hash seed does): an insertion that is a prefix of the entry's, or the entry's
+            // plus more bases, must not match; with equal lengths the comparison also stays inside the representative's insertion
+            bool eq = *reinterpret_cast<volatile int32_t*>(&T.dlen[h]) == len;
             for (int t = 1; t <= len && eq; ++t) {
                 const int qa = rep_qpos + t, qb = rq + t;
                 const uint32_t ba = __ldg(T.seq + (uint32_t)(my_seq0 + (uint32_t)(qa >> 1))), bb = __ldg(T.seq + (uint32_t)(rs0 + (uint32_t)(qb >> 1)));
