@@ -10,8 +10,14 @@
  * BGZF blocks are inflated by `threads` host threads (zlib) and every pass of the record decode runs on the same number of
  * threads (record boundaries per byte range with a verified speculative start, fields + identity hashes, fragment numbering by
  * hash partition, prefix sums, payload copy); results are identical for any thread count.
+ *
+ * Two ways in.  smc_bam_open reads and inflates the whole file.  smc_bam_open_indexed takes the file's BAM index (.bai, SAMv1
+ * section 5.2) as well and inflates only the blocks of the header; smc_bam_decode then works out from the index which chunks its
+ * target intervals need (the standard bin + linear-index query), reads only their compressed byte ranges and inflates only
+ * their blocks, so time and memory follow the reads used rather than the file size.  Both give identical arrays.
+ *
  * All returned pointers stay valid until smc_bam_close().  Functions return 0 or a negative code; message via
- * smc_bam_last_error().
+ * smc_bam_last_error().  -3: the index is malformed or does not fit the BAM (the message names the index file).
  */
 #ifndef SMC_BAMIO_H
 #define SMC_BAMIO_H
@@ -52,6 +58,10 @@ typedef struct smc_bam_reads {
 } smc_bam_reads;
 
 int         smc_bam_open(const char *path, int threads, smc_bam **out);   /* read + inflate + parse the header */
+/* Inflate the header blocks only and parse the index (magic, n_ref == the header's reference count, bins with their chunks,
+ * linear index, optional n_no_coor).  smc_bam_decode with n_intervals > 0 reads the chunks the intervals need; with
+ * n_intervals == 0 it reads the whole file. */
+int         smc_bam_open_indexed(const char *path, const char *index_path, int threads, smc_bam **out);
 void        smc_bam_close(smc_bam *h);
 /* trim != 0: smc_bam_decode keeps, for every read that is one plain aligned run, only the query bases between its first and
  * its last target position (store_lo / store_len of include/smc_b200.h); needs n_intervals > 0.  Default off. */

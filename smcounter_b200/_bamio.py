@@ -10,7 +10,7 @@ from .soa import ReadsSoA
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libsmc_bamio.so")
-EXPORTS = ("smc_bam_set_trim", "smc_bam_open", "smc_bam_close", "smc_bam_last_error", "smc_bam_n_refs", "smc_bam_ref_name", "smc_bam_ref_length",
+EXPORTS = ("smc_bam_set_trim", "smc_bam_open", "smc_bam_open_indexed", "smc_bam_close", "smc_bam_last_error", "smc_bam_n_refs", "smc_bam_ref_name", "smc_bam_ref_length",
            "smc_bam_decode", "smc_bam_dict_umi", "smc_bam_inflate_raw", "smc_rows_emit", "smc_rows_free", "smc_soa_qual_hist", "smc_soa_ref_end", "smc_soa_order_stats", "smc_soa_pack_begin", "smc_soa_pack_fill",
            "smc_soa_pack_end")
 _vp = C.c_void_p
@@ -73,6 +73,8 @@ def load():
     lib = C.CDLL(LIB_PATH)
     lib.smc_bam_open.argtypes = [C.c_char_p, C.c_int, C.POINTER(_vp)]
     lib.smc_bam_open.restype = C.c_int
+    lib.smc_bam_open_indexed.argtypes = [C.c_char_p, C.c_char_p, C.c_int, C.POINTER(_vp)]
+    lib.smc_bam_open_indexed.restype = C.c_int
     lib.smc_bam_close.argtypes = [_vp]
     lib.smc_bam_close.restype = None
     lib.smc_bam_set_trim.argtypes = [_vp, C.c_int]
@@ -139,12 +141,23 @@ def _arr(ptr, n, dtype, owner):
     return np.frombuffer(buf, dtype=dtype, count=n)
 
 
-def read_bam_native(path: str, intervals=None, threads: int = 0, trim: bool = False) -> ReadsSoA:
+E_INDEX = -3                       # include/smc_bamio.h: the index is malformed or does not fit the BAM
+
+
+def _raise(rc, msg):
+    raise (IOError if rc == E_INDEX else ValueError)(msg.decode())
+
+
+def read_bam_native(path: str, intervals=None, threads: int = 0, trim: bool = False, index: str | None = None) -> ReadsSoA:
+    """``index``: path of the BAM's .bai; with intervals, only the index chunks they need are read and inflated."""
     lib = load()
     h = _vp()
-    rc = lib.smc_bam_open(os.fsencode(path), int(threads), C.byref(h))
+    if index is not None:
+        rc = lib.smc_bam_open_indexed(os.fsencode(path), os.fsencode(index), int(threads), C.byref(h))
+    else:
+        rc = lib.smc_bam_open(os.fsencode(path), int(threads), C.byref(h))
     if rc != 0:
-        raise ValueError(lib.smc_bam_last_error(None).decode())
+        _raise(rc, lib.smc_bam_last_error(None))
     owner = _Handle(lib, h)
     ok = False
     try:
@@ -162,7 +175,7 @@ def read_bam_native(path: str, intervals=None, threads: int = 0, trim: bool = Fa
         lib.smc_bam_set_trim(h, 1 if (trim and ivs) else 0)
         rc = lib.smc_bam_decode(h, n_iv, args[0].ctypes.data, args[1].ctypes.data, args[2].ctypes.data, C.byref(out))
         if rc != 0:
-            raise ValueError(lib.smc_bam_last_error(h).decode())
+            _raise(rc, lib.smc_bam_last_error(h))
         n = out.n_reads
         A = lambda ptr, count, dtype: _arr(ptr, count, dtype, owner)
         umi = A(out.umi, n, np.uint64)

@@ -1,9 +1,12 @@
 // libsmc_bamio.so -- BAM (BGZF) -> flat SoA read buffers (include/smc_bamio.h).  Host-side input decoding only.
-// Container format restated from the SAM/BAM specification (SAMv1 sections 4.1-4.2); zlib does the inflating.
+// Container format restated from the SAM/BAM specification (SAMv1 sections 4.1-4.2, the .bai index 5.2); zlib does the inflating.
+#include <fcntl.h>
+#include <sys/stat.h>
 #include <unistd.h>
 #include <zlib.h>
 
 #include <algorithm>
+#include <array>
 #include <chrono>
 #include <atomic>
 #include <cstdio>
@@ -36,7 +39,15 @@ inline uint16_t rd16(const uint8_t* p) { uint16_t v; memcpy(&v, p, 2); return v;
 inline uint32_t rd32(const uint8_t* p) { uint32_t v; memcpy(&v, p, 4); return v; }
 inline int32_t rdi32(const uint8_t* p) { int32_t v; memcpy(&v, p, 4); return v; }
 
-struct Block { size_t coff, clen; size_t uoff; uint32_t isize; };
+// one BGZF block: its deflate payload at coff, and the bytes [lo, hi) of its isize inflated ones that go to uoff of the stream
+struct Block { size_t coff, clen; size_t uoff; uint32_t isize, lo, hi; };
+
+// .bai contents of one reference (SAMv1 5.2): chunks per bin (virtual offsets, [beg, end)) and the 16 kbp linear index
+struct BaiChunk { uint64_t beg, end; };
+struct BaiRef {
+    std::unordered_map<uint32_t, std::vector<BaiChunk>> bins;
+    std::vector<uint64_t> linear;
+};
 
 // output arrays: malloc'ed and NOT zero-filled (std::vector::resize would touch every page once more, serially)
 template <class T> struct PodBuf {
@@ -88,54 +99,62 @@ struct smc_bam {
     uint64_t qual_hist[256] = {0};              // how often every phred value occurs among the stored qualities
     int trim = 0;
     bool decoded = false;
+    // opened through an index (smc_bam_open_indexed): raw holds only the header until smc_bam_decode reads the chunks it needs
+    bool indexed = false;
+    std::string path, index_path;
+    size_t file_size = 0;
+    std::vector<BaiRef> bai;
 };
 
-static int inflate_all(const RawBuf& file, int threads, RawBuf& out, std::string& err) {
-    std::vector<Block> blocks;
-    size_t off = 0, uoff = 0;
-    const size_t n = file.size();
-    while (off < n) {
-        if (off + 18 > n || file[off] != 0x1f || file[off + 1] != 0x8b || file[off + 2] != 8 || !(file[off + 3] & 4)) {
-            err = "not a BGZF block at offset " + std::to_string(off); return -1;
-        }
-        const uint16_t xlen = rd16(&file[off + 10]);
-        size_t p = off + 12, end = p + xlen;
-        int64_t bsize = -1;
-        while (p + 4 <= end && end <= n) {
-            const uint16_t slen = rd16(&file[p + 2]);
-            if (file[p] == 66 && file[p + 1] == 67 && slen == 2) bsize = rd16(&file[p + 4]);
-            p += 4 + slen;
-        }
-        if (bsize < 0 || off + (size_t)bsize + 1 > n) { err = "truncated or malformed BGZF block at offset " + std::to_string(off); return -1; }
-        Block b;
-        b.coff = off + 12 + xlen;
-        b.clen = (size_t)bsize + 1 - 12 - xlen - 8;
-        b.isize = rd32(&file[off + bsize + 1 - 4]);
-        b.uoff = uoff;
-        uoff += b.isize;
-        blocks.push_back(b);
-        off += (size_t)bsize + 1;
+// the BGZF block at seg[off] (seg has n bytes): 0 and the block (coff relative to seg) and the offset of the next one;
+// 1 not a BGZF block, 2 truncated or malformed
+static int bgzf_block(const uint8_t* seg, size_t n, size_t off, Block& b, size_t& next) {
+    if (off + 18 > n || seg[off] != 0x1f || seg[off + 1] != 0x8b || seg[off + 2] != 8 || !(seg[off + 3] & 4)) return 1;
+    const uint16_t xlen = rd16(&seg[off + 10]);
+    size_t p = off + 12, end = p + xlen;
+    int64_t bsize = -1;
+    while (p + 4 <= end && end <= n) {
+        const uint16_t slen = rd16(&seg[p + 2]);
+        if (seg[p] == 66 && seg[p + 1] == 67 && slen == 2) bsize = rd16(&seg[p + 4]);
+        p += 4 + slen;
     }
-    if (!out.alloc(uoff)) { err = "out of memory for the inflated BAM"; return -1; }
+    if (bsize < 0 || off + (size_t)bsize + 1 > n || (size_t)bsize + 1 < 12 + (size_t)xlen + 8) return 2;
+    b.coff = off + 12 + xlen;
+    b.clen = (size_t)bsize + 1 - 12 - xlen - 8;
+    b.isize = rd32(&seg[off + bsize + 1 - 4]);
+    b.lo = 0; b.hi = b.isize;
+    next = off + (size_t)bsize + 1;
+    return 0;
+}
+
+// inflate every block of src (which is readable 64 bytes past its last block) and store its bytes [lo, hi) at out[uoff];
+// a block cut by a chunk boundary is inflated into a scratch buffer first
+static int inflate_blocks(const uint8_t* src, const std::vector<Block>& blocks, int threads, RawBuf& out, std::string& err) {
     std::atomic<size_t> next(0);
     std::atomic<int> bad(0);
     // the blocks go through the decoder of smc_inflate.h; a block it rejects is given to zlib (SMC_INFLATE=zlib: zlib for all)
     static const bool own_inflate = [] { const char* ev = getenv("SMC_INFLATE"); return !(ev && strcmp(ev, "zlib") == 0); }();
     auto work = [&]() {
         z_stream zs;
+        std::vector<uint8_t> scratch;
         for (;;) {
             const size_t i = next.fetch_add(1);
             if (i >= blocks.size() || bad.load()) break;
             const Block& b = blocks[i];
-            if (b.isize == 0) continue;
-            if (own_inflate && smc_inflate_raw(&file[b.coff], b.clen, &out[b.uoff], b.isize) == 0) continue;
-            memset(&zs, 0, sizeof(zs));
-            if (inflateInit2(&zs, -15) != Z_OK) { bad = 1; break; }
-            zs.next_in = const_cast<Bytef*>(&file[b.coff]); zs.avail_in = (uInt)b.clen;
-            zs.next_out = &out[b.uoff]; zs.avail_out = b.isize;
-            const int rc = inflate(&zs, Z_FINISH);
-            inflateEnd(&zs);
-            if (rc != Z_STREAM_END || zs.avail_out != 0) { bad = 1; break; }
+            if (b.hi == b.lo) continue;
+            const bool whole = b.lo == 0 && b.hi == b.isize;
+            if (!whole && scratch.size() < b.isize) scratch.resize(b.isize);
+            uint8_t* dst = whole ? &out[b.uoff] : scratch.data();
+            if (!(own_inflate && smc_inflate_raw(&src[b.coff], b.clen, dst, b.isize) == 0)) {
+                memset(&zs, 0, sizeof(zs));
+                if (inflateInit2(&zs, -15) != Z_OK) { bad = 1; break; }
+                zs.next_in = const_cast<Bytef*>(&src[b.coff]); zs.avail_in = (uInt)b.clen;
+                zs.next_out = dst; zs.avail_out = b.isize;
+                const int rc = inflate(&zs, Z_FINISH);
+                inflateEnd(&zs);
+                if (rc != Z_STREAM_END || zs.avail_out != 0) { bad = 1; break; }
+            }
+            if (!whole) memcpy(&out[b.uoff], dst + b.lo, b.hi - b.lo);
         }
     };
     const int nt = std::max(1, std::min<int>(threads, (int)blocks.size()));
@@ -147,62 +166,344 @@ static int inflate_all(const RawBuf& file, int threads, RawBuf& out, std::string
     return 0;
 }
 
-extern "C" int smc_bam_open(const char* path, int threads, smc_bam** out) {
-    if (!path || !out) { g_open_error = "smc_bam_open: null argument"; return -2; }
-    FILE* fh = fopen(path, "rb");
-    if (!fh) { g_open_error = std::string("smc_bam_open: cannot open ") + path; return -1; }
-    PhaseTimer pt;
-    RawBuf file;
-    fseek(fh, 0, SEEK_END);
-    const long sz = ftell(fh);
-    fseek(fh, 0, SEEK_SET);
-    // 64 bytes of slack: the block decoder reads its input eight bytes at a time
-    if (!file.alloc((sz > 0 ? (size_t)sz : 0) + 64)) { fclose(fh); g_open_error = "smc_bam_open: out of memory"; return -1; }
-    memset(file.p + (sz > 0 ? (size_t)sz : 0), 0, 64);
-    file.n = sz > 0 ? (size_t)sz : 0;
-    if (threads <= 0) threads = (int)std::max(1u, std::thread::hardware_concurrency());
-    {   // the file (usually in the page cache) is read by all threads, each its own range (pread)
-        const int fd = fileno(fh);
-        const size_t total = file.size();
-        const int nt = (int)std::max<size_t>(1, std::min<size_t>((size_t)threads, total / (size_t(4) << 20) + 1));
-        std::atomic<int> short_read(0);
-        auto rd = [&](int t) {
-            size_t a = total * (size_t)t / (size_t)nt;
-            const size_t e = total * (size_t)(t + 1) / (size_t)nt;
-            while (a < e) {
-                const ssize_t k = pread(fd, file.p + a, e - a, (off_t)a);
+static int inflate_all(const RawBuf& file, int threads, RawBuf& out, std::string& err) {
+    std::vector<Block> blocks;
+    size_t off = 0, uoff = 0;
+    const size_t n = file.size();
+    while (off < n) {
+        Block b;
+        size_t nxt = 0;
+        const int rc = bgzf_block(file.data(), n, off, b, nxt);
+        if (rc == 1) { err = "not a BGZF block at offset " + std::to_string(off); return -1; }
+        if (rc == 2) { err = "truncated or malformed BGZF block at offset " + std::to_string(off); return -1; }
+        b.uoff = uoff;
+        uoff += b.isize;
+        blocks.push_back(b);
+        off = nxt;
+    }
+    if (!out.alloc(uoff)) { err = "out of memory for the inflated BAM"; return -1; }
+    return inflate_blocks(file.data(), blocks, threads, out, err);
+}
+
+// pread the pieces (file offset, buffer offset, length) on up to `threads` threads; false on a short read
+static bool pread_pieces(int fd, uint8_t* buf, const std::vector<std::array<size_t, 3>>& pieces, int threads) {
+    std::atomic<size_t> next(0);
+    std::atomic<int> short_read(0);
+    auto rd = [&]() {
+        for (size_t i; (i = next.fetch_add(1)) < pieces.size() && !short_read.load();) {
+            size_t a = 0;
+            const size_t off = pieces[i][0], len = pieces[i][2];
+            uint8_t* dst = buf + pieces[i][1];
+            while (a < len) {
+                const ssize_t k = pread(fd, dst + a, len - a, (off_t)(off + a));
                 if (k <= 0) { short_read = 1; return; }
                 a += (size_t)k;
             }
-        };
-        std::vector<std::thread> ts;
-        for (int t = 1; t < nt; ++t) ts.emplace_back(rd, t);
-        rd(0);
-        for (auto& t : ts) t.join();
-        fclose(fh);
-        if (short_read.load()) { g_open_error = "smc_bam_open: short read"; return -1; }
-    }
-    pt.lap("read file");
-    smc_bam* h = new smc_bam();
-    h->threads = threads;
-    if (inflate_all(file, threads, h->raw, g_open_error) != 0) { delete h; return -1; }
-    pt.lap("inflate");
-    const RawBuf& r = h->raw;
-    if (r.size() < 12 || memcmp(r.data(), "BAM\1", 4) != 0) { g_open_error = "not a BAM file (bad magic)"; delete h; return -1; }
-    size_t p = 8 + (size_t)rdi32(&r[4]);
-    if (p + 4 > r.size()) { g_open_error = "truncated BAM header"; delete h; return -1; }
+        }
+    };
+    const int nt = (int)std::max<size_t>(1, std::min<size_t>((size_t)threads, pieces.size()));
+    std::vector<std::thread> ts;
+    for (int t = 1; t < nt; ++t) ts.emplace_back(rd);
+    rd();
+    for (auto& t : ts) t.join();
+    return !short_read.load();
+}
+
+// [off, off + len) of the file cut into pieces of at most 4 MiB, stored from buf_off on
+static void add_pieces(std::vector<std::array<size_t, 3>>& pieces, size_t off, size_t buf_off, size_t len) {
+    const size_t piece = size_t(4) << 20;
+    for (size_t a = 0; a < len; a += piece) pieces.push_back({off + a, buf_off + a, std::min(piece, len - a)});
+}
+
+// the whole file (usually in the page cache) read by all threads, each its own ranges (pread), plus 64 zero bytes of slack:
+// the block decoder reads its input eight bytes at a time
+static int read_whole_file(const char* path, int threads, RawBuf& file, std::string& err) {
+    const int fd = open(path, O_RDONLY);
+    if (fd < 0) { err = std::string("smc_bam_open: cannot open ") + path; return -1; }
+    struct stat st;
+    const size_t sz = fstat(fd, &st) == 0 && st.st_size > 0 ? (size_t)st.st_size : 0;
+    if (!file.alloc(sz + 64)) { close(fd); err = "smc_bam_open: out of memory"; return -1; }
+    memset(file.p + sz, 0, 64);
+    file.n = sz;
+    std::vector<std::array<size_t, 3>> pieces;
+    add_pieces(pieces, 0, 0, sz);
+    const bool ok = pread_pieces(fd, file.p, pieces, threads);
+    close(fd);
+    if (!ok) { err = "smc_bam_open: short read"; return -1; }
+    return 0;
+}
+
+// magic, header text and reference list from the start of the inflated stream: 0 (h->ref_names / ref_lens / first_record set),
+// 1 the stream ends before the reference list does (err says how), -1 not a BAM stream
+static int parse_header(const uint8_t* r, size_t n, smc_bam* h, std::string& err) {
+    h->ref_names.clear(); h->ref_lens.clear();
+    if (n >= 4 && memcmp(r, "BAM\1", 4) != 0) { err = "not a BAM file (bad magic)"; return -1; }
+    if (n < 12) { err = "not a BAM file (bad magic)"; return 1; }
+    const int32_t l_text = rdi32(&r[4]);
+    if (l_text < 0) { err = "truncated BAM header"; return -1; }
+    size_t p = 8 + (size_t)l_text;
+    if (p + 4 > n) { err = "truncated BAM header"; return 1; }
     const int32_t n_ref = rdi32(&r[p]);
     p += 4;
     for (int32_t i = 0; i < n_ref; ++i) {
-        if (p + 4 > r.size()) { g_open_error = "truncated BAM reference list"; delete h; return -1; }
+        if (p + 4 > n) { err = "truncated BAM reference list"; return 1; }
         const int32_t l_name = rdi32(&r[p]);
-        if (l_name < 1 || p + 8 + (size_t)l_name > r.size()) { g_open_error = "truncated BAM reference list"; delete h; return -1; }
+        if (l_name < 1) { err = "truncated BAM reference list"; return -1; }
+        if (p + 8 + (size_t)l_name > n) { err = "truncated BAM reference list"; return 1; }
         h->ref_names.emplace_back(reinterpret_cast<const char*>(&r[p + 4]), (size_t)l_name - 1);
         h->ref_lens.push_back(rdi32(&r[p + 4 + l_name]));
         p += 8 + (size_t)l_name;
     }
     h->first_record = p;
+    return 0;
+}
+
+static void timing_bytes(const char* what, size_t compressed, size_t inflated) {
+    if (getenv("SMC_BAM_TIMING")) fprintf(stderr, "[smc_bamio] %s: compressed bytes read %zu, inflated bytes %zu\n", what, compressed, inflated);
+}
+
+extern "C" int smc_bam_open(const char* path, int threads, smc_bam** out) {
+    if (!path || !out) { g_open_error = "smc_bam_open: null argument"; return -2; }
+    PhaseTimer pt;
+    if (threads <= 0) threads = (int)std::max(1u, std::thread::hardware_concurrency());
+    RawBuf file;
+    if (read_whole_file(path, threads, file, g_open_error) != 0) return -1;
+    pt.lap("read file");
+    smc_bam* h = new smc_bam();
+    h->threads = threads;
+    if (inflate_all(file, threads, h->raw, g_open_error) != 0) { delete h; return -1; }
+    pt.lap("inflate");
+    timing_bytes("whole file", file.size(), h->raw.size());
+    if (parse_header(h->raw.data(), h->raw.size(), h, g_open_error) != 0) { delete h; return -1; }
     *out = h;
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// Region access through a .bai (SAMv1 5.2)
+// ------------------------------------------------------------------------------------------------------------
+static int parse_bai(const std::string& ipath, size_t n_ref_bam, std::vector<BaiRef>& refs, std::string& err) {
+    const std::string who = "BAM index " + ipath + ": ";
+    FILE* fh = fopen(ipath.c_str(), "rb");
+    if (!fh) { err = who + "cannot open"; return -3; }
+    std::vector<uint8_t> d;
+    uint8_t buf[1 << 16];
+    for (size_t k; (k = fread(buf, 1, sizeof(buf), fh)) > 0;) d.insert(d.end(), buf, buf + k);
+    fclose(fh);
+    const size_t n = d.size();
+    size_t p = 0;
+    auto truncated = [&]() { err = who + "truncated or malformed at byte " + std::to_string(p); return -3; };
+    if (n < 8 || memcmp(d.data(), "BAI\1", 4) != 0) { err = who + "bad magic (not a .bai file)"; return -3; }
+    const int32_t n_ref = rdi32(&d[4]);
+    p = 8;
+    if (n_ref < 0 || (size_t)n_ref != n_ref_bam) {
+        err = who + "n_ref is " + std::to_string(n_ref) + " but the BAM header has " + std::to_string(n_ref_bam) + " references";
+        return -3;
+    }
+    refs.assign((size_t)n_ref, BaiRef());
+    for (int32_t r = 0; r < n_ref; ++r) {
+        if (p + 4 > n) return truncated();
+        const int32_t n_bin = rdi32(&d[p]);
+        p += 4;
+        if (n_bin < 0) return truncated();
+        for (int32_t k = 0; k < n_bin; ++k) {
+            if (p + 8 > n) return truncated();
+            const uint32_t bin = rd32(&d[p]);
+            const int32_t n_chunk = rdi32(&d[p + 4]);
+            p += 8;
+            if (n_chunk < 0 || p + 16 * (size_t)n_chunk > n) return truncated();
+            if (bin != 37450) {                          // 37450: the metadata pseudo-bin (reference span, mapped / unmapped counts)
+                auto& v = refs[(size_t)r].bins[bin];
+                for (int32_t c = 0; c < n_chunk; ++c) {
+                    BaiChunk ch;
+                    memcpy(&ch.beg, &d[p + 16 * (size_t)c], 8); memcpy(&ch.end, &d[p + 16 * (size_t)c + 8], 8);
+                    v.push_back(ch);
+                }
+            }
+            p += 16 * (size_t)n_chunk;
+        }
+        if (p + 4 > n) return truncated();
+        const int32_t n_intv = rdi32(&d[p]);
+        p += 4;
+        if (n_intv < 0 || p + 8 * (size_t)n_intv > n) return truncated();
+        refs[(size_t)r].linear.resize((size_t)n_intv);
+        if (n_intv) memcpy(refs[(size_t)r].linear.data(), &d[p], 8 * (size_t)n_intv);
+        p += 8 * (size_t)n_intv;
+    }
+    if (p != n && p + 8 != n) return truncated();      // nothing, or the optional n_no_coor
+    return 0;
+}
+
+extern "C" int smc_bam_open_indexed(const char* path, const char* index_path, int threads, smc_bam** out) {
+    if (!path || !index_path || !out) { g_open_error = "smc_bam_open_indexed: null argument"; return -2; }
+    PhaseTimer pt;
+    if (threads <= 0) threads = (int)std::max(1u, std::thread::hardware_concurrency());
+    const int fd = open(path, O_RDONLY);
+    if (fd < 0) { g_open_error = std::string("smc_bam_open: cannot open ") + path; return -1; }
+    struct stat st;
+    const size_t size = fstat(fd, &st) == 0 && st.st_size > 0 ? (size_t)st.st_size : 0;
+    smc_bam* h = new smc_bam();
+    h->threads = threads; h->indexed = true; h->path = path; h->index_path = index_path; h->file_size = size;
+    // the header: BGZF blocks from offset 0, one at a time, until the header text and the reference list are complete
+    std::vector<uint8_t> comp((size_t(1) << 16) + 64, 0), hdr;
+    size_t off = 0, comp_read = 0;
+    int st_hdr = 1;
+    g_open_error = "not a BAM file (bad magic)";
+    while (st_hdr == 1 && off < size) {
+        const size_t len = std::min(size - off, size_t(1) << 16);           // a BGZF block is at most 64 KiB
+        std::vector<std::array<size_t, 3>> piece{{off, 0, len}};
+        if (!pread_pieces(fd, comp.data(), piece, 1)) { g_open_error = "smc_bam_open: short read"; break; }
+        memset(comp.data() + len, 0, 64);
+        Block b;
+        size_t nxt = 0;
+        const int rc = bgzf_block(comp.data(), len, 0, b, nxt);
+        if (rc) { g_open_error = (rc == 1 ? "not a BGZF block at offset " : "truncated or malformed BGZF block at offset ") + std::to_string(off); st_hdr = -1; break; }
+        comp_read += nxt;
+        RawBuf one;
+        b.uoff = 0;
+        if (!one.alloc(b.isize)) { g_open_error = "smc_bam_open: out of memory"; st_hdr = -1; break; }
+        if (inflate_blocks(comp.data(), std::vector<Block>{b}, 1, one, g_open_error) != 0) { st_hdr = -1; break; }
+        hdr.insert(hdr.end(), one.data(), one.data() + b.isize);
+        st_hdr = parse_header(hdr.data(), hdr.size(), h, g_open_error);
+        off += nxt;
+    }
+    close(fd);
+    if (st_hdr != 0) { delete h; return -1; }
+    pt.lap("header blocks");
+    timing_bytes("header", comp_read, hdr.size());
+    const int rc = parse_bai(h->index_path, h->ref_names.size(), h->bai, g_open_error);
+    if (rc != 0) { delete h; return rc; }
+    pt.lap("index parse");
+    *out = h;
+    return 0;
+}
+
+// SAMv1 5.3: the bins that may hold a record overlapping [beg, end)
+static void reg2bins(int64_t beg, int64_t end, std::vector<uint32_t>& out) {
+    out.clear();
+    --end;
+    out.push_back(0);
+    for (int64_t k = 1 + (beg >> 26); k <= 1 + (end >> 26); ++k) out.push_back((uint32_t)k);
+    for (int64_t k = 9 + (beg >> 23); k <= 9 + (end >> 23); ++k) out.push_back((uint32_t)k);
+    for (int64_t k = 73 + (beg >> 20); k <= 73 + (end >> 20); ++k) out.push_back((uint32_t)k);
+    for (int64_t k = 585 + (beg >> 17); k <= 585 + (end >> 17); ++k) out.push_back((uint32_t)k);
+    for (int64_t k = 4681 + (beg >> 14); k <= 4681 + (end >> 14); ++k) out.push_back((uint32_t)k);
+}
+
+// h->raw = the records of the index chunks that the intervals need, in file order.  A chunk [beg, end) covers whole records,
+// so the concatenated slices are a valid record chain; chunks that share a BGZF block are merged, which adds only whole records
+// in between (dropped by the interval filter like any other) and inflates every block once.
+static int load_chunks(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, const int32_t* iv_start, const int32_t* iv_end) {
+    PhaseTimer pt;
+    const std::string who = "BAM index " + h->index_path + ": ";
+    std::vector<BaiChunk> ch;
+    std::vector<uint32_t> bins;
+    for (int64_t k = 0; k < n_iv; ++k) {
+        const int32_t rid = iv_ref[k];
+        if (rid < 0 || (size_t)rid >= h->bai.size()) continue;
+        const int64_t beg = std::max<int64_t>(0, iv_start[k]), end = std::min<int64_t>(iv_end[k], int64_t(1) << 29);
+        if (end <= beg) continue;
+        const BaiRef& R = h->bai[(size_t)rid];
+        const uint64_t min_off = R.linear.empty() ? 0 : R.linear[std::min<size_t>((size_t)(beg >> 14), R.linear.size() - 1)];
+        reg2bins(beg, end, bins);
+        for (uint32_t bin : bins) {
+            auto it = R.bins.find(bin);
+            if (it == R.bins.end()) continue;
+            for (const BaiChunk& c : it->second)
+                if (c.end > min_off && c.end > c.beg) ch.push_back(c);
+        }
+    }
+    std::sort(ch.begin(), ch.end(), [](const BaiChunk& a, const BaiChunk& b) { return a.beg < b.beg || (a.beg == b.beg && a.end < b.end); });
+    std::vector<BaiChunk> merged;
+    for (const BaiChunk& c : ch) {
+        if (!merged.empty() && (c.beg >> 16) <= (merged.back().end >> 16)) merged.back().end = std::max(merged.back().end, c.end);
+        else merged.push_back(c);
+    }
+    pt.lap("index: chunk query");
+    // compressed byte range of every merged chunk: from the block of its start to the end of the block of its end (or to the start
+    // of that block when the end is at its offset 0)
+    const int fd = open(h->path.c_str(), O_RDONLY);
+    if (fd < 0) { h->err = "smc_bam_decode: cannot open " + h->path; return -1; }
+    struct Range { size_t cbeg, cend, buf; };
+    std::vector<Range> ranges;
+    size_t total = 0;
+    int rc = 0;
+    for (const BaiChunk& c : merged) {
+        const size_t cbeg = (size_t)(c.beg >> 16), cend = (size_t)(c.end >> 16);
+        size_t stop = cend;
+        if (cbeg >= h->file_size || cend > h->file_size || (cend == h->file_size && (c.end & 0xffff))) {
+            h->err = who + "chunk [" + std::to_string(c.beg) + ", " + std::to_string(c.end) + ") points past the end of " + h->path;
+            rc = -3; break;
+        }
+        if (c.end & 0xffff) {                       // the block holding the chunk's end: its size from its own header
+            uint8_t head[18 + 64];
+            const size_t len = cend < h->file_size ? std::min<size_t>(sizeof(head), h->file_size - cend) : 0;
+            std::vector<std::array<size_t, 3>> piece{{cend, 0, len}};
+            if (len < 12 || !pread_pieces(fd, head, piece, 1) || head[0] != 0x1f || head[1] != 0x8b) {
+                h->err = who + "chunk end at virtual offset " + std::to_string(c.end) + " is not in a BGZF block of " + h->path;
+                rc = -3; break;
+            }
+            const uint16_t xlen = rd16(&head[10]);
+            int64_t bsize = -1;
+            for (size_t p = 12; p + 4 <= 12 + (size_t)xlen && p + 6 <= len; p += 4 + rd16(&head[p + 2]))
+                if (head[p] == 66 && head[p + 1] == 67 && rd16(&head[p + 2]) == 2) { bsize = rd16(&head[p + 4]); break; }
+            if (bsize < 0) { h->err = who + "chunk end at virtual offset " + std::to_string(c.end) + " is not in a BGZF block of " + h->path; rc = -3; break; }
+            stop = cend + (size_t)bsize + 1;
+        }
+        if (stop > h->file_size || cbeg >= h->file_size) {
+            h->err = who + "chunk [" + std::to_string(c.beg) + ", " + std::to_string(c.end) + ") points past the end of " + h->path;
+            rc = -3; break;
+        }
+        if (cbeg >= stop) { h->err = who + "chunk [" + std::to_string(c.beg) + ", " + std::to_string(c.end) + ") is malformed"; rc = -3; break; }
+        ranges.push_back({cbeg, stop, total});
+        total += stop - cbeg;
+    }
+    RawBuf comp;
+    if (rc == 0 && !comp.alloc(total + 64)) { h->err = "out of memory for the compressed chunks"; rc = -1; }
+    if (rc == 0) {
+        memset(comp.p + total, 0, 64);
+        std::vector<std::array<size_t, 3>> pieces;
+        for (const Range& g : ranges) add_pieces(pieces, g.cbeg, g.buf, g.cend - g.cbeg);
+        if (!pread_pieces(fd, comp.p, pieces, h->threads)) { h->err = "smc_bam_decode: short read of " + h->path; rc = -1; }
+    }
+    close(fd);
+    if (rc != 0) return rc;
+    pt.lap("index: chunk reads");
+    // the blocks of every range, each with the slice of its inflated bytes that the chunk covers
+    std::vector<Block> blocks;
+    size_t uoff = 0;
+    for (size_t g = 0; g < ranges.size(); ++g) {
+        const Range& R = ranges[g];
+        const BaiChunk& c = merged[g];
+        const uint8_t* seg = comp.p + R.buf;
+        const size_t n = R.cend - R.cbeg;
+        for (size_t off = 0; off < n;) {
+            Block b;
+            size_t nxt = 0;
+            const bool last = bgzf_block(seg, n, off, b, nxt) == 0 && nxt == n;
+            if (nxt == 0 || (last && (c.end & 0xffff) && off != (size_t)(c.end >> 16) - R.cbeg)) {
+                h->err = who + "chunk [" + std::to_string(c.beg) + ", " + std::to_string(c.end) + ") does not point at BGZF blocks of " + h->path +
+                         " (offset " + std::to_string(R.cbeg + off) + ")";
+                return -3;
+            }
+            if (off == 0) b.lo = (uint32_t)(c.beg & 0xffff);
+            if (last && (c.end & 0xffff)) b.hi = (uint32_t)(c.end & 0xffff);
+            if (b.lo > b.hi || b.hi > b.isize) {
+                h->err = who + "chunk [" + std::to_string(c.beg) + ", " + std::to_string(c.end) + ") points past the data of a BGZF block of " + h->path;
+                return -3;
+            }
+            b.coff += R.buf;
+            b.uoff = uoff;
+            uoff += b.hi - b.lo;
+            blocks.push_back(b);
+            off = nxt;
+        }
+    }
+    if (!h->raw.alloc(uoff)) { h->err = "out of memory for the inflated chunks"; return -1; }
+    if (inflate_blocks(comp.data(), blocks, h->threads, h->raw, h->err) != 0) return -1;
+    h->first_record = 0;
+    pt.lap("index: chunk inflate");
+    timing_bytes("index chunks", total, uoff);
     return 0;
 }
 
@@ -293,6 +594,21 @@ extern "C" int smc_bam_decode(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, c
                               smc_bam_reads* out) {
     if (!h || !out || (n_iv > 0 && (!iv_ref || !iv_start || !iv_end))) { if (h) h->err = "smc_bam_decode: null argument"; return -2; }
     if (h->decoded) { h->err = "smc_bam_decode: a handle decodes once (the inflated stream is released afterwards); open the file again"; return -2; }
+    if (h->indexed) {                      // the records come from the index chunks the intervals need, or from the whole file
+        h->indexed = false;
+        if (n_iv > 0) {
+            const int rc = load_chunks(h, n_iv, iv_ref, iv_start, iv_end);
+            if (rc != 0) { h->decoded = true; return rc; }
+        } else {
+            PhaseTimer pt;
+            RawBuf file;
+            if (read_whole_file(h->path.c_str(), h->threads, file, h->err) != 0 || inflate_all(file, h->threads, h->raw, h->err) != 0) {
+                h->decoded = true; return -1;
+            }
+            pt.lap("read + inflate whole file");
+            timing_bytes("whole file", file.size(), h->raw.size());
+        }
+    }
     // per reference: interval starts (sorted) and the running maximum of their ends
     const size_t nref = h->ref_names.size();
     std::vector<std::vector<std::pair<int64_t, int64_t>>> iv(nref);
