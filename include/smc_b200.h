@@ -277,6 +277,7 @@ int smc_call_batch(smc_ctx *ctx, const smc_reads_soa *reads, const smc_loci *loc
                    smc_out *out);
 
 /* The same three phases separately, so that the kernels can be timed with inputs resident in HBM. */
+/* When smc_upload returns an error, no copy from the caller's buffers is still in flight. */
 int smc_upload(smc_ctx *ctx, const smc_reads_soa *reads, const smc_loci *loci, const smc_umi_keep *keep /* nullable */);
 int smc_run_resident(smc_ctx *ctx);
 int smc_download(smc_ctx *ctx, smc_out *out);

@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libsmc_b200.so")
 SOURCES = ["smc_api.cu"]
-HEADERS = ["smc_common.cuh", "smc_sort.cuh", "smc_pileup.cuh", "smc_stats.cuh", os.path.join("..", "..", "include", "smc_b200.h")]
+HEADERS = ["smc_common.cuh", "smc_sort.cuh", "smc_pileup.cuh", "smc_stats.cuh", "smc_upload.cuh", os.path.join("..", "..", "include", "smc_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-fmad=false",                 # FP64 parity: no FMA contraction anywhere in the statistics
               "-shared", "-Xcompiler", "-fPIC"]

@@ -23,6 +23,7 @@
 #include "smc_sort.cuh"
 #include "smc_pileup.cuh"
 #include "smc_stats.cuh"
+#include "smc_upload.cuh"
 
 namespace {
 
@@ -45,8 +46,12 @@ static smc_ctx* g_link_owner[64] = {};
 // is raised in smc_ctx_create): growing a buffer or destroying a context hands the memory back to the pool, not to the
 // driver, so the next batch / the next context of the process does not pay cudaMalloc / cudaFree again (measured: a fresh
 // context right after another one was destroyed spent 100-900 ms in cudaMalloc for a 0.3 M read batch).
+// Every buffer joins its context's registry when it is constructed: the context gives it its stream and releases it.
 struct DevBuf {
     void* p = nullptr; size_t cap = 0; cudaStream_t st = nullptr;
+    explicit DevBuf(std::vector<DevBuf*>& registry) { registry.push_back(this); }
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
     cudaError_t ensure(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
         if (p) cudaFreeAsync(p, st);
@@ -80,80 +85,75 @@ enum SmallWord {
     SW_CHUNK_READS_SEQ = 96  // the same for the compact bases
 };
 
+// stage events of ctx->ev; the SMC_TIMELINE line prints the first seven, in this order
+enum StageEvent {
+    EV_COPY_BEGIN, EV_COPY_END,                 // host link: the upload (H2D), or smc_download (D2H)
+    EV_RUN_BEGIN, EV_PREP_DONE, EV_SORT_DONE, EV_PILEUP_DONE, EV_STATS_DONE,
+    EV_PILEUP_BEGIN, EV_GATHER_DONE, EV_MERGE_DONE,
+    EV_READ_SORT_BEGIN, EV_READ_SORT_DONE, EV_READ_PREP_BEGIN, EV_READ_PREP_DONE, EV_EVENT_SORT_BEGIN, EV_EVENT_SORT_DONE,
+    EV_COUNT
+};
+
 struct smc_ctx {
     int device = 0;
     smc_params prm{};
     std::string err;
     cudaStream_t st = nullptr;
-    cudaEvent_t ev[18]{};
+    cudaEvent_t ev[EV_COUNT]{};
+    std::vector<DevBuf*> bufs;                  // every DevBuf member below (DevBuf's constructor)
     // pipelined upload of smc_call_batch: bases / qualities arrive in chunks on st_copy while st already computes
     cudaStream_t st_copy = nullptr;
-    cudaEvent_t ev_scal = nullptr, ev_link = nullptr, ev_tmp = nullptr, ev_tmp2 = nullptr, ev_chunk[SMC_PIPE_MAX]{};
+    cudaEvent_t ev_link = nullptr, ev_tmp = nullptr, ev_tmp2 = nullptr, ev_chunk[SMC_PIPE_MAX]{};
     int pipe_n = 0;                             // > 1: the chunk events of the current batch are pending / recorded
     uint32_t pipe_seq_chunk = 0, pipe_qual_chunk = 0;   // bytes of bases / qualities per chunk
-    DevBuf d_pipe_need;
+    DevBuf d_pipe_need{bufs};
     bool packed_seq = false, packed_qual = false, packed_cigar = false;   // offsets were NULL: computed on the device
     uint32_t pipe_end[SMC_PIPE_MAX]{};          // launch c of the pileup kernels covers units [pipe_end[c-1], pipe_end[c])
     // resident inputs
     int64_t n_reads = 0, n_loci = 0, n_keep_loci = 0, n_keep_umi = 0;
     int64_t seq_bytes = 0, qual_bytes = 0, n_cigar_words = 0;
-    DevBuf d_ref_id, d_pos, d_flag, d_mapq, d_nm, d_lseq, d_seq_off, d_qual_off, d_cig_off, d_ncig, d_umi, d_frag, d_seq, d_qual,
-        d_cigar, d_store_lo, d_store_len;
+    DevBuf d_ref_id{bufs}, d_pos{bufs}, d_flag{bufs}, d_mapq{bufs}, d_nm{bufs}, d_lseq{bufs}, d_seq_off{bufs}, d_qual_off{bufs},
+        d_cig_off{bufs}, d_ncig{bufs}, d_umi{bufs}, d_frag{bufs}, d_seq{bufs}, d_qual{bufs}, d_cigar{bufs}, d_store_lo{bufs}, d_store_len{bufs};
     bool has_store = false;                     // reads carry a stored window (smc_reads_soa::store_lo / store_len)
     int qual_bits = 8;                          // 4 / 2: compact qualities were uploaded (d_qual_packed) and are expanded into d_qual
-    DevBuf d_qual_packed, d_qual_poff, d_qual_lut, d_stage16, d_stage_ids, d_spill, d_seq_packed, d_seq_poff, d_exc_read, d_exc_pos, d_exc_nib;
+    DevBuf d_qual_packed{bufs}, d_qual_poff{bufs}, d_qual_lut{bufs}, d_stage{bufs}, d_spill{bufs}, d_seq_packed{bufs}, d_seq_poff{bufs},
+        d_exc_read{bufs}, d_exc_pos{bufs}, d_exc_nib{bufs};
     int seq_bits = 4; int64_t n_seq_exc = 0;    // 2: compact bases were uploaded (d_seq_packed) and are expanded into d_seq
     uint32_t spill_cap = 0;                     // records in the k_merge spill pool (grows x4 on GF_SPILL_FULL)
     const uint32_t* inv_ptr = nullptr;          // read index -> sorted position (lives in d_v0 or d_v1 after the read sort)
-    DevBuf d_loci_ref, d_loci_pos, d_loci_base, d_loci_key;
-    DevBuf d_keep_idx, d_keep_off, d_keep_umi;
+    DevBuf d_loci_ref{bufs}, d_loci_pos{bufs}, d_loci_base{bufs}, d_loci_key{bufs};
+    DevBuf d_keep_idx{bufs}, d_keep_off{bufs}, d_keep_umi{bufs};
     bool has_keep = false, uploaded = false, ran = false;
     // tables
-    DevBuf d_bqtab, d_pcrtab;
+    DevBuf d_bqtab{bufs}, d_pcrtab{bufs};
     // scratch
-    DevBuf d_k0, d_k1, d_v0, d_v1, d_hist, d_scan, d_flags32a, d_flags32b, d_urank, d_frank, d_umi_of_urank, d_recs, d_ntiles,
-        d_evoff, d_ek0, d_ek1, d_ev0, d_ev1, d_tile_off, d_unit_cnt, d_unit_off, d_small,
-        d_grec, d_unit_eb, d_unit_ee, d_unit_tile, d_unit_nfrag, d_codes, d_frag_first, d_umi_urank, d_umi_table;
+    DevBuf d_k0{bufs}, d_k1{bufs}, d_v0{bufs}, d_v1{bufs}, d_hist{bufs}, d_scan{bufs}, d_urank{bufs}, d_frank{bufs}, d_umi_of_urank{bufs},
+        d_recs{bufs}, d_ek0{bufs}, d_ek1{bufs}, d_ev0{bufs}, d_ev1{bufs}, d_tile_off{bufs}, d_unit_cnt{bufs}, d_unit_off{bufs}, d_small{bufs},
+        d_grec{bufs}, d_unit_eb{bufs}, d_unit_ee{bufs}, d_unit_tile{bufs}, d_unit_nfrag{bufs}, d_codes{bufs}, d_frag_first{bufs},
+        d_umi_urank{bufs}, d_umi_table{bufs};
     uint32_t code_mult = 1;                     // fragment-code storage per tile event (1, or 3 = worst case after GF_CODE_FULL)
     uint32_t n_units_cap = 0;
     // per-locus accumulators / outputs
-    DevBuf d_loc, d_cnt, d_limb, d_pi, d_max, d_second, d_alt, d_altpi, d_secondpi, d_fl1, d_fl2, d_bial, d_fp, d_for;
+    DevBuf d_loc{bufs}, d_cnt{bufs}, d_limb{bufs}, d_pi{bufs}, d_max{bufs}, d_second{bufs}, d_alt{bufs}, d_altpi{bufs}, d_secondpi{bufs},
+        d_fl1{bufs}, d_fl2{bufs}, d_bial{bufs}, d_fp{bufs}, d_for{bufs};
     // dynamic allele table + sorted rows
     uint32_t dyn_cap = 0;
-    DevBuf d_dkey, d_drep_read, d_drep_qpos, d_dlen, d_dcnt, d_dlimb, d_diskey;
-    DevBuf d_lk0, d_lk1, d_lv0, d_lv1;
-    DevBuf d_s_key, d_s_cnt, d_s_limb, d_s_iskey, d_s_pi, d_s_rep_read, d_s_rep_qpos, d_s_len, d_dyn_first;
+    DevBuf d_dkey{bufs}, d_drep_read{bufs}, d_drep_qpos{bufs}, d_dlen{bufs}, d_dcnt{bufs}, d_dlimb{bufs}, d_diskey{bufs};
+    DevBuf d_lk0{bufs}, d_lv0{bufs}, d_lv1{bufs};
+    DevBuf d_s_key{bufs}, d_s_cnt{bufs}, d_s_limb{bufs}, d_s_iskey{bufs}, d_s_pi{bufs}, d_s_rep_read{bufs}, d_s_rep_qpos{bufs}, d_s_len{bufs},
+        d_dyn_first{bufs};
     int64_t n_dyn = 0;
-    DevBuf d_tasks;
+    DevBuf d_tasks{bufs};
     uint32_t task_cap = 0;
     // barcode listing
-    DevBuf d_list_idx, d_list_count, d_list_off, d_list_umi, d_list_first;
-    DevBuf d_hp_bases, d_hp_meta, d_hp_flags;     // smc_hp_lowcomp
+    DevBuf d_list_idx{bufs}, d_list_count{bufs}, d_list_off{bufs}, d_list_umi{bufs}, d_list_first{bufs};
+    DevBuf d_hp_bases{bufs}, d_hp_meta{bufs}, d_hp_flags{bufs};     // smc_hp_lowcomp
     smc_timings tm{};
     uint32_t chunk = 128;       // tile events per warp unit (A/B on B200, whole step: 96 -> 4.42 ms, 128 -> 4.39, 160 -> 4.39, 256 -> 4.47, 384 -> 4.60)
     const uint32_t* ev_read_sorted = nullptr;   // tile-sorted event -> srank map (lives in d_ev0 or d_ev1)
     uint32_t n_tiles = 0; int64_t n_tile_events = 0;
     int64_t ne_cap = 0;                         // capacity of the tile-event buffers (grow only)
 };
-
-static std::vector<DevBuf*> all_bufs(smc_ctx* ctx) {
-    return {&ctx->d_store_lo, &ctx->d_store_len, &ctx->d_ref_id, &ctx->d_pos, &ctx->d_flag, &ctx->d_mapq, &ctx->d_nm, &ctx->d_lseq, &ctx->d_seq_off, &ctx->d_qual_off,
-                      &ctx->d_cig_off, &ctx->d_ncig, &ctx->d_umi, &ctx->d_frag, &ctx->d_seq, &ctx->d_qual, &ctx->d_cigar, &ctx->d_loci_ref,
-                      &ctx->d_loci_pos, &ctx->d_loci_base, &ctx->d_loci_key, &ctx->d_keep_idx, &ctx->d_keep_off, &ctx->d_keep_umi,
-                      &ctx->d_bqtab, &ctx->d_pcrtab, &ctx->d_k0, &ctx->d_k1, &ctx->d_v0, &ctx->d_v1, &ctx->d_hist, &ctx->d_scan,
-                      &ctx->d_flags32a, &ctx->d_flags32b, &ctx->d_urank, &ctx->d_frank, &ctx->d_umi_of_urank, &ctx->d_recs, &ctx->d_ntiles,
-                      &ctx->d_evoff, &ctx->d_ek0, &ctx->d_ek1, &ctx->d_ev0, &ctx->d_ev1, &ctx->d_tile_off, &ctx->d_unit_cnt,
-                      &ctx->d_unit_off, &ctx->d_small, &ctx->d_grec, &ctx->d_unit_eb, &ctx->d_unit_ee, &ctx->d_unit_tile,
-                      &ctx->d_unit_nfrag, &ctx->d_codes, &ctx->d_frag_first, &ctx->d_umi_urank, &ctx->d_loc, &ctx->d_cnt, &ctx->d_limb, &ctx->d_pi, &ctx->d_max, &ctx->d_second,
-                      &ctx->d_alt, &ctx->d_altpi, &ctx->d_secondpi, &ctx->d_fl1, &ctx->d_fl2, &ctx->d_bial, &ctx->d_fp, &ctx->d_for,
-                      &ctx->d_dkey, &ctx->d_drep_read, &ctx->d_drep_qpos, &ctx->d_dlen, &ctx->d_dcnt, &ctx->d_dlimb, &ctx->d_diskey,
-                      &ctx->d_lk0, &ctx->d_lk1, &ctx->d_lv0, &ctx->d_lv1, &ctx->d_s_key, &ctx->d_s_cnt, &ctx->d_s_limb, &ctx->d_s_iskey,
-                      &ctx->d_s_pi, &ctx->d_s_rep_read, &ctx->d_s_rep_qpos, &ctx->d_s_len, &ctx->d_dyn_first, &ctx->d_tasks,
-                      &ctx->d_list_idx, &ctx->d_list_count, &ctx->d_list_off, &ctx->d_list_umi, &ctx->d_list_first,
-                      &ctx->d_hp_bases, &ctx->d_hp_meta, &ctx->d_hp_flags, &ctx->d_pipe_need, &ctx->d_umi_table,
-                      &ctx->d_qual_packed, &ctx->d_qual_poff, &ctx->d_qual_lut, &ctx->d_stage16, &ctx->d_stage_ids, &ctx->d_spill,
-                      &ctx->d_seq_packed, &ctx->d_seq_poff, &ctx->d_exc_read, &ctx->d_exc_pos, &ctx->d_exc_nib};
-}
 
 #define CK(call)                                                                                         \
     do {                                                                                                 \
@@ -167,10 +167,6 @@ static std::vector<DevBuf*> all_bufs(smc_ctx* ctx) {
 // ------------------------------------------------------------------------------------------------------------
 // small kernels used only by the orchestration
 // ------------------------------------------------------------------------------------------------------------
-__global__ void k_loci_keys(const int32_t* ref_id, const int32_t* pos0, int64_t n, uint64_t* key) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) key[i] = ((uint64_t)(uint32_t)ref_id[i] << 32) | (uint32_t)pos0[i];
-}
 // Barcode slots: every distinct barcode code gets one slot of an open-addressing table (linear probing, atomicCAS); the slot
 // index stands in for the barcode in the read sort key, so that ONE sort on (slot, fragment id) groups the reads by barcode and
 // fragment.  Which slot a barcode lands in may differ from run to run; nothing downstream depends on the order of barcodes
@@ -333,14 +329,6 @@ __global__ void k_tile_offsets(const uint64_t* ev_key, int64_t ne, uint32_t n_ti
     if (t < n_tiles) nev = (ne > 0 ? (uint32_t)lower_bound_u64(ev_key, ne, (uint64_t)t + 1ull) : 0u) - a;
     unit_cnt[t] = (nev + chunk - 1) / chunk;
 }
-__global__ void k_fill_i32(int32_t* p, int64_t n, int32_t v) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) p[i] = v;
-}
-__global__ void k_scatter_idx(const int64_t* locus, int64_t n, int32_t* idx) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) idx[locus[i]] = (int32_t)i;
-}
 // Dynamic-allele rows, grouped by locus and ordered by key inside a locus: count per locus, scan, place, and a tiny
 // insertion sort per locus (a locus has a handful of such alleles) -- 7 launches instead of a 6-pass radix sort of a few
 // thousand keys that was pure launch latency.
@@ -425,7 +413,7 @@ extern "C" int smc_ctx_create(int device, const smc_params* params, smc_ctx** ou
     };
     if ((e = cudaSetDevice(device)) != cudaSuccess) return fail("cudaSetDevice", e);
     if ((e = cudaStreamCreateWithFlags(&ctx->st, cudaStreamNonBlocking)) != cudaSuccess) return fail("cudaStreamCreate", e);
-    for (DevBuf* b : all_bufs(ctx)) b->st = ctx->st;
+    for (DevBuf* b : ctx->bufs) b->st = ctx->st;
     {   // keep freed scratch in the pool for the next batch / context of this process
         cudaMemPool_t pool;
         unsigned long long keep = ~0ull;
@@ -434,7 +422,6 @@ extern "C" int smc_ctx_create(int device, const smc_params* params, smc_ctx** ou
     }
     for (auto& ev : ctx->ev) if ((e = cudaEventCreate(&ev)) != cudaSuccess) return fail("cudaEventCreate", e);
     if ((e = cudaStreamCreateWithFlags(&ctx->st_copy, cudaStreamNonBlocking)) != cudaSuccess) return fail("cudaStreamCreate", e);
-    if ((e = cudaEventCreateWithFlags(&ctx->ev_scal, cudaEventDisableTiming)) != cudaSuccess) return fail("cudaEventCreate", e);
     if ((e = cudaEventCreateWithFlags(&ctx->ev_link, cudaEventDisableTiming)) != cudaSuccess) return fail("cudaEventCreate", e);
     if ((e = cudaEventCreateWithFlags(&ctx->ev_tmp, cudaEventDisableTiming)) != cudaSuccess) return fail("cudaEventCreate", e);
     if ((e = cudaEventCreateWithFlags(&ctx->ev_tmp2, cudaEventDisableTiming)) != cudaSuccess) return fail("cudaEventCreate", e);
@@ -478,11 +465,10 @@ extern "C" void smc_ctx_destroy(smc_ctx* ctx) {
     cudaSetDevice(ctx->device);
     if (ctx->st_copy) cudaStreamSynchronize(ctx->st_copy);
     cudaStreamSynchronize(ctx->st);
-    for (DevBuf* b : all_bufs(ctx)) b->release();
+    for (DevBuf* b : ctx->bufs) b->release();
     cudaStreamSynchronize(ctx->st);
     for (auto& ev : ctx->ev) if (ev) cudaEventDestroy(ev);
     for (auto& ev : ctx->ev_chunk) if (ev) cudaEventDestroy(ev);
-    if (ctx->ev_scal) cudaEventDestroy(ctx->ev_scal);
     if (ctx->ev_tmp) cudaEventDestroy(ctx->ev_tmp);
     if (ctx->ev_tmp2) cudaEventDestroy(ctx->ev_tmp2);
     if (ctx->ev_link) {
@@ -507,202 +493,217 @@ static int pipe_chunks_for(const smc_reads_soa* R) {
     return (int)(g < 2 ? 2 : g > 12 ? 12 : g);
 }
 
+static int qual_bits_of(const smc_reads_soa* R) { return (R->qual_bits == 4 || R->qual_bits == 2) ? R->qual_bits : 8; }
+static int seq_bits_of(const smc_reads_soa* R) { return R->seq_bits == 2 ? 2 : 4; }
+// expanded payloads: a read stores (len + 1) / 2 bytes of 4-bit bases for (len + 3) / 4 bytes of 2-bit ones, and never more
+// qualities than two per byte of 4-bit bases; up to 3 bytes of padding per read
+static int64_t expanded_seq_bytes(const smc_reads_soa* R) {
+    return seq_bits_of(R) == 4 ? R->seq_bytes : 2 * R->seq_bytes + 4 * R->n_reads + 16;
+}
+static int64_t expanded_qual_bytes(const smc_reads_soa* R) {
+    return qual_bits_of(R) == 8 ? R->qual_bytes : 2 * (seq_bits_of(R) == 4 ? R->seq_bytes : 2 * R->seq_bytes) + 4 * R->n_reads + 16;
+}
+
+// Every argument check of an upload.  It runs before anything is queued, so a rejected batch leaves the context as it was.
+static int check_upload(const smc_reads_soa* R, const smc_loci* Lc, std::string& err) {
+    if (!R || !Lc) { err = "smc_upload: null reads/loci"; return SMC_E_ARG; }
+    if (R->n_reads < 0 || Lc->n_loci < 0) { err = "smc_upload: negative size"; return SMC_E_ARG; }
+    if (Lc->n_loci > SMC_MAX_LOCI) { err = "smc_upload: more than 4194302 loci in one batch"; return SMC_E_LIMIT; }
+    if (R->n_reads > (1ll << 30) || R->seq_bytes >= (1ll << 32) || R->qual_bytes >= (1ll << 32) || R->n_cigar_words >= (1ll << 32)) {
+        err = "smc_upload: batch exceeds 2^30 reads or 4 GiB of bases/qualities/cigar; split the batch"; return SMC_E_LIMIT;
+    }
+    if (R->scalar_bits != 0 && R->scalar_bits != 32 && R->scalar_bits != 16 && R->scalar_bits != 8) { err = "smc_upload: scalar_bits must be 0, 8, 16 or 32"; return SMC_E_ARG; }
+    if (R->qual_bits != 0 && R->qual_bits != 8 && R->qual_bits != 4 && R->qual_bits != 2) { err = "smc_upload: qual_bits must be 0, 2, 4 or 8"; return SMC_E_ARG; }
+    if (qual_bits_of(R) != 8 && (R->qual_off || !R->qual_lut)) { err = "smc_upload: compact qualities need the packed layout (qual_off == NULL) and a qual_lut"; return SMC_E_ARG; }
+    if (R->seq_bits != 0 && R->seq_bits != 4 && R->seq_bits != 2) { err = "smc_upload: seq_bits must be 0, 2 or 4"; return SMC_E_ARG; }
+    if (seq_bits_of(R) == 2 && (R->seq_off || R->n_seq_exc < 0 || (R->n_seq_exc > 0 && (!R->seq_exc_read || !R->seq_exc_pos || !R->seq_exc_nib)))) {
+        err = "smc_upload: compact bases need the packed layout (seq_off == NULL) and consistent exception arrays"; return SMC_E_ARG;
+    }
+    if ((R->ref_id_bits != 0 && R->ref_id_bits != 32 && R->ref_id_bits != 8) || (R->umi_bits != 0 && R->umi_bits != 64 && R->umi_bits != 32)) {
+        err = "smc_upload: ref_id_bits must be 0, 8 or 32 and umi_bits 0, 32 or 64"; return SMC_E_ARG;
+    }
+    if ((R->store_lo == nullptr) != (R->store_len == nullptr)) { err = "smc_upload: store_lo and store_len must be given together"; return SMC_E_ARG; }
+    if (expanded_seq_bytes(R) >= (1ll << 32) || expanded_qual_bytes(R) >= (1ll << 32)) {
+        err = "smc_upload: the expanded bases / qualities of the batch exceed 4 GiB; split the batch"; return SMC_E_LIMIT;
+    }
+    return SMC_OK;
+}
+
+// Host -> device copies of one upload.  A chunked upload queues them on the copy stream while the compute stream runs the
+// upload's kernels: a copy must not write a buffer the compute stream (re)allocated before the copy stream has waited for
+// it, and a kernel must not read what the compute stream has not waited for (hand_over).
+struct Upload {
+    smc_ctx* ctx;
+    bool split;                 // copies go to ctx->st_copy (else to ctx->st, in order with the kernels)
+    bool grew = false;          // a buffer was (re)allocated on ctx->st since the copy stream last waited for it
+    int64_t bytes = 0;          // bytes copied (smc_timings::bytes_h2d)
+    cudaError_t ensure(DevBuf& b, size_t n) {
+        if (n <= b.cap) return cudaSuccess;
+        grew = true;
+        return b.ensure(n);
+    }
+    cudaError_t copy(void* dst, const void* src, size_t n) {
+        if (n == 0) return cudaSuccess;
+        if (split && grew) {
+            cudaError_t e = cudaEventRecord(ctx->ev_tmp, ctx->st);
+            if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->st_copy, ctx->ev_tmp, 0);
+            if (e != cudaSuccess) return e;
+            grew = false;
+        }
+        bytes += (int64_t)n;
+        return cudaMemcpyAsync(dst, src, n, cudaMemcpyHostToDevice, split ? ctx->st_copy : ctx->st);
+    }
+    // a whole array, into a buffer grown to hold it (16 bytes at least, so that an empty array has an address too)
+    cudaError_t copy(DevBuf& b, const void* src, size_t n) {
+        const cudaError_t e = ensure(b, n ? n : 16);
+        return e != cudaSuccess ? e : copy(b.p, src, n);
+    }
+    cudaError_t hand_over() {
+        if (!split) return cudaSuccess;
+        const cudaError_t e = cudaEventRecord(ctx->ev_tmp2, ctx->st_copy);
+        return e != cudaSuccess ? e : cudaStreamWaitEvent(ctx->st, ctx->ev_tmp2, 0);
+    }
+};
+
+// one k_widen launch: 8- / 16-bit values -> int32, 32-bit values -> int64
+static void widen(smc_ctx* ctx, const void* in, int in_bytes, int64_t n, void* out) {
+    if (in_bytes == 1) { auto k = k_widen<uint8_t, int32_t>; LAUNCH(k, nblk(n, 256), 256, 0, (const uint8_t*)in, n, (int32_t*)out); }
+    else if (in_bytes == 2) { auto k = k_widen<uint16_t, int32_t>; LAUNCH(k, nblk(n, 256), 256, 0, (const uint16_t*)in, n, (int32_t*)out); }
+    else { auto k = k_widen<uint32_t, int64_t>; LAUNCH(k, nblk(n, 256), 256, 0, (const uint32_t*)in, n, (int64_t*)out); }
+}
+
+// Offsets of a payload packed in read order: per-read sizes of k_pack_len `kind` scanned in place in `out`; their total goes to
+// d_small word SW_PACK_TOTALS + total_word (smc_run_resident compares it with the payload size the caller declared).
+static int pack_offsets(smc_ctx* ctx, int64_t n, int kind, int qbits, uint32_t* out, int total_word) {
+    CK(ctx->d_scan.ensure((size_t)scan_scratch_words(n + 1) * 4 + 1024));
+    LAUNCH(k_pack_len, nblk(n, 256), 256, 0, ctx->d_lseq.as<int32_t>(), ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr,
+           ctx->d_ncig.as<uint16_t>(), n, kind, qbits, out);
+    exclusive_scan_u32(out, out, n, ctx->d_scan.as<uint32_t>(), ctx->d_small.as<uint32_t>() + SW_PACK_TOTALS + total_word, ctx->st);
+    return SMC_OK;
+}
+
+// k_unpack grid (grid-stride over the reads): 8 blocks of 256 threads on each of the 148 SMs of a B200
+static constexpr unsigned UNPACK_GRID = 148u * 8u;
+
+// Compact bases / qualities -> the expanded d_seq / d_qual, for the reads of upload chunk c: d_small words
+// SW_CHUNK_READS_SEQ + c, + c + 1 (bases) and SW_CHUNK_READS + c, + c + 1 (qualities) hold its first read and its end.
+static void expand_compact(smc_ctx* ctx, int c, unsigned grid) {
+    uint32_t* small = ctx->d_small.as<uint32_t>();
+    const int32_t* store_len = ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr;
+    if (ctx->seq_bits == 2) {           // compact bases -> nibbles, then the exceptions
+        LAUNCH(k_unpack<2>, grid, 256, 0, small + SW_CHUNK_READS_SEQ + c, ctx->d_seq_poff.as<uint32_t>(), ctx->d_seq_off.as<int64_t>(),
+               ctx->d_lseq.as<int32_t>(), store_len, nullptr, ctx->d_seq_packed.as<uint8_t>(), ctx->d_seq.as<uint8_t>());
+        LAUNCH(k_patch_seq, nblk(ctx->n_seq_exc, 256), 256, 0, small + SW_CHUNK_READS_SEQ + c, ctx->n_seq_exc, ctx->d_exc_read.as<uint32_t>(),
+               ctx->d_exc_pos.as<uint32_t>(), ctx->d_exc_nib.as<uint8_t>(), ctx->d_seq_off.as<int64_t>(), ctx->d_seq.as<uint8_t>());
+    }
+    if (ctx->qual_bits != 8) {          // compact qualities -> bytes
+        auto unpack = ctx->qual_bits == 2 ? k_unpack<0> : k_unpack<1>;
+        LAUNCH(unpack, grid, 256, 0, small + SW_CHUNK_READS + c, ctx->d_qual_poff.as<uint32_t>(), ctx->d_qual_off.as<int64_t>(),
+               ctx->d_lseq.as<int32_t>(), store_len, ctx->d_qual_lut.as<uint8_t>(), ctx->d_qual_packed.as<uint8_t>(), ctx->d_qual.as<uint8_t>());
+    }
+}
+
 // pipelined = false: everything on ctx->st, synchronised on return (smc_upload).
 // pipelined = true : scalars / CIGAR / loci on ctx->st; bases and qualities in ctx->pipe_n chunks of equal byte size on
 //                    ctx->st_copy, one event per chunk; returns without waiting (smc_call_batch synchronises both streams).
-static int upload_impl(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc, const smc_umi_keep* K, bool pipelined) {
-    if (!ctx) return SMC_E_ARG;
-    NvtxRange nvtx_r("smc:upload");
-    if (!R || !Lc) { ctx->err = "smc_upload: null reads/loci"; return SMC_E_ARG; }
-    if (R->n_reads < 0 || Lc->n_loci < 0) { ctx->err = "smc_upload: negative size"; return SMC_E_ARG; }
-    if (Lc->n_loci > SMC_MAX_LOCI) { ctx->err = "smc_upload: more than 4194302 loci in one batch"; return SMC_E_LIMIT; }
-    if (R->n_reads > (1ll << 30) || R->seq_bytes >= (1ll << 32) || R->qual_bytes >= (1ll << 32) || R->n_cigar_words >= (1ll << 32)) {
-        ctx->err = "smc_upload: batch exceeds 2^30 reads or 4 GiB of bases/qualities/cigar; split the batch"; return SMC_E_LIMIT;
-    }
+static int queue_upload(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc, const smc_umi_keep* K, bool pipelined) {
     CK(cudaSetDevice(ctx->device));
     ctx->uploaded = false; ctx->ran = false;
     const int64_t n = R->n_reads, nl = Lc->n_loci;
+    const size_t nz = (size_t)(n ? n : 1);
     const int G = pipelined ? pipe_chunks_for(R) : 1;
     ctx->pipe_n = 0;
     // A chunked batch sends EVERYTHING over the copy stream, in the order the kernels need it (scalars, CIGARs, loci, then
     // the chunks of bases / qualities): no copy waits for a kernel, so the link stays busy however long this context's --
-    // or another context's -- kernels queue on the GPU.  The compute stream waits for what it consumes (SYNC_UP).
-    const bool split = pipelined && G > 1;
-    cudaStream_t up_st = split ? ctx->st_copy : ctx->st;
+    // or another context's -- kernels queue on the GPU.  The compute stream waits for what it consumes (hand_over).
+    Upload up{ctx, pipelined && G > 1};
     static const bool link_turns = [] { const char* ev = getenv("SMC_LINK_TURNS"); return !(ev && atoi(ev) == 0); }();
     std::unique_lock<std::mutex> link_lock(g_link_mu, std::defer_lock);
     const int dv = ctx->device;
-    if (split && link_turns && dv >= 0 && dv < 64) {
+    if (up.split && link_turns && dv >= 0 && dv < 64) {
         link_lock.lock();
         if (g_link_tail[dv] && g_link_owner[dv] != ctx) CK(cudaStreamWaitEvent(ctx->st_copy, g_link_tail[dv], 0));
     }
-    CK(cudaEventRecord(ctx->ev[0], up_st));
-    int64_t bytes = 0;
-    bool grew = false;                      // a buffer was (re)allocated on ctx->st since the copy stream last waited for it
-#define ALLOC_SYNC()                                                                                             \
-    do {                                                                                                         \
-        if (split && grew) { CK(cudaEventRecord(ctx->ev_tmp, ctx->st)); CK(cudaStreamWaitEvent(ctx->st_copy, ctx->ev_tmp, 0)); grew = false; } \
-    } while (0)
-#define ENSURE(buf, nbytes)                                                                                      \
-    do { void* before__ = (buf).p; CK((buf).ensure(nbytes)); if ((buf).p != before__) grew = true; } while (0)
-#define SYNC_UP()                                                                                                \
-    do {                                                                                                         \
-        if (split) { CK(cudaEventRecord(ctx->ev_tmp2, ctx->st_copy)); CK(cudaStreamWaitEvent(ctx->st, ctx->ev_tmp2, 0)); } \
-    } while (0)
-#define UP(buf, src, count, T)                                                                                   \
-    do {                                                                                                         \
-        size_t b__ = (size_t)(count) * sizeof(T);                                                                \
-        ENSURE(buf, b__ ? b__ : 16);                                                                             \
-        if (b__) { ALLOC_SYNC(); CK(cudaMemcpyAsync((buf).p, (src), b__, cudaMemcpyHostToDevice, up_st)); bytes += b__; } \
-    } while (0)
-    if (R->scalar_bits != 0 && R->scalar_bits != 32 && R->scalar_bits != 16 && R->scalar_bits != 8) { ctx->err = "smc_upload: scalar_bits must be 0, 8, 16 or 32"; return SMC_E_ARG; }
-    if (R->qual_bits != 0 && R->qual_bits != 8 && R->qual_bits != 4 && R->qual_bits != 2) { ctx->err = "smc_upload: qual_bits must be 0, 2, 4 or 8"; return SMC_E_ARG; }
-    const bool s16 = R->scalar_bits == 16 || R->scalar_bits == 8;       // narrow scalars: staged, widened on the device
-    const size_t sw = R->scalar_bits == 8 ? 1 : 2;                      // bytes per narrow scalar
-    const int qbits = (R->qual_bits == 4 || R->qual_bits == 2) ? R->qual_bits : 8;
-    if (qbits != 8 && (R->qual_off || !R->qual_lut)) { ctx->err = "smc_upload: compact qualities need the packed layout (qual_off == NULL) and a qual_lut"; return SMC_E_ARG; }
-    if (R->seq_bits != 0 && R->seq_bits != 4 && R->seq_bits != 2) { ctx->err = "smc_upload: seq_bits must be 0, 2 or 4"; return SMC_E_ARG; }
-    const int sbits = R->seq_bits == 2 ? 2 : 4;
-    if (sbits == 2 && (R->seq_off || R->n_seq_exc < 0 || (R->n_seq_exc > 0 && (!R->seq_exc_read || !R->seq_exc_pos || !R->seq_exc_nib)))) {
-        ctx->err = "smc_upload: compact bases need the packed layout (seq_off == NULL) and consistent exception arrays"; return SMC_E_ARG;
-    }
-    if ((R->ref_id_bits != 0 && R->ref_id_bits != 32 && R->ref_id_bits != 8) || (R->umi_bits != 0 && R->umi_bits != 64 && R->umi_bits != 32)) {
-        ctx->err = "smc_upload: ref_id_bits must be 0, 8 or 32 and umi_bits 0, 32 or 64"; return SMC_E_ARG;
-    }
-    const bool ref8 = R->ref_id_bits == 8, umi32 = R->umi_bits == 32;
-    if (!ref8) UP(ctx->d_ref_id, R->ref_id, n, int32_t);
-    UP(ctx->d_pos, R->pos, n, int32_t); UP(ctx->d_flag, R->flag, n, uint16_t);
-    UP(ctx->d_mapq, R->mapq, n, uint8_t);
-    UP(ctx->d_ncig, R->n_cigar, n, uint16_t); UP(ctx->d_frag, R->frag_id, n, uint32_t);
-    if (!umi32) UP(ctx->d_umi, R->umi, n, uint64_t);
-    if (ref8 || umi32) {
-        // narrow reference indices / barcode codes: staged back to back (u32 codes first), widened on the device
-        ENSURE(ctx->d_stage_ids, (size_t)(n ? n : 1) * 5);
-        uint32_t* st32 = ctx->d_stage_ids.as<uint32_t>();
-        uint8_t* st8 = ctx->d_stage_ids.as<uint8_t>() + (size_t)n * 4;
-        if (umi32) { CK(ctx->d_umi.ensure((size_t)(n ? n : 1) * 8)); if (n) { ALLOC_SYNC(); CK(cudaMemcpyAsync(st32, R->umi, (size_t)n * 4, cudaMemcpyHostToDevice, up_st)); bytes += n * 4; } }
-        if (ref8) { CK(ctx->d_ref_id.ensure((size_t)(n ? n : 1) * 4)); if (n) { ALLOC_SYNC(); CK(cudaMemcpyAsync(st8, R->ref_id, (size_t)n, cudaMemcpyHostToDevice, up_st)); bytes += n; } }
-        SYNC_UP();
-        if (umi32) LAUNCH(k_widen_u32, nblk(n, 256), 256, 0, st32, n, ctx->d_umi.as<int64_t>());
-        if (ref8) LAUNCH(k_widen_u8, nblk(n, 256), 256, 0, st8, n, ctx->d_ref_id.as<int32_t>());
-    }
-    if ((R->store_lo == nullptr) != (R->store_len == nullptr)) { ctx->err = "smc_upload: store_lo and store_len must be given together"; return SMC_E_ARG; }
+    CK(cudaEventRecord(ctx->ev[EV_COPY_BEGIN], up.split ? ctx->st_copy : ctx->st));
+    // per-read scalars; narrow ones (8- / 16-bit scalars, 8-bit reference indices, 32-bit barcode codes) are staged as they
+    // are, 16-byte aligned, and widened on the device
+    struct Narrow { const void* src; int bytes; DevBuf* dst; size_t stage_off; };
+    Narrow narrow[6];
+    int n_narrow = 0;
+    size_t stage_bytes = 0;
+    auto scalars = [&](DevBuf& dst, const void* src, int bytes, int wide_bytes) {
+        if (bytes == wide_bytes) return up.copy(dst, src, (size_t)n * bytes);
+        narrow[n_narrow++] = {src, bytes, &dst, stage_bytes};
+        stage_bytes += ((size_t)n * bytes + 15) & ~(size_t)15;
+        return dst.ensure(nz * (bytes == 4 ? 8 : 4));
+    };
+    const int sw = R->scalar_bits == 8 ? 1 : R->scalar_bits == 16 ? 2 : 4;      // bytes per nm / l_seq / store_lo / store_len
+    CK(scalars(ctx->d_ref_id, R->ref_id, R->ref_id_bits == 8 ? 1 : 4, 4));
+    CK(up.copy(ctx->d_pos, R->pos, (size_t)n * 4)); CK(up.copy(ctx->d_flag, R->flag, (size_t)n * 2));
+    CK(up.copy(ctx->d_mapq, R->mapq, (size_t)n)); CK(up.copy(ctx->d_ncig, R->n_cigar, (size_t)n * 2));
+    CK(up.copy(ctx->d_frag, R->frag_id, (size_t)n * 4));
+    CK(scalars(ctx->d_umi, R->umi, R->umi_bits == 32 ? 4 : 8, 8));
     ctx->has_store = R->store_lo != nullptr;
-    if (!s16) {
-        UP(ctx->d_nm, R->nm, n, int32_t); UP(ctx->d_lseq, R->l_seq, n, int32_t);
-        if (ctx->has_store) { UP(ctx->d_store_lo, R->store_lo, n, int32_t); UP(ctx->d_store_len, R->store_len, n, int32_t); }
-    } else {
-        // 8- / 16-bit scalars: four arrays staged back to back, widened on the device
-        const void* src16[4] = {R->nm, R->l_seq, R->store_lo, R->store_len};
-        DevBuf* dst32[4] = {&ctx->d_nm, &ctx->d_lseq, &ctx->d_store_lo, &ctx->d_store_len};
-        ENSURE(ctx->d_stage16, (size_t)(n ? n : 1) * 2 * 4);
-        for (int k = 0; k < (ctx->has_store ? 4 : 2); ++k) {
-            uint8_t* stg = ctx->d_stage16.as<uint8_t>() + (size_t)k * n * 2;
-            CK(dst32[k]->ensure((size_t)(n ? n : 1) * 4));
-            if (n) { ALLOC_SYNC(); CK(cudaMemcpyAsync(stg, src16[k], (size_t)n * sw, cudaMemcpyHostToDevice, up_st)); bytes += n * (int64_t)sw; }
-        }
-        SYNC_UP();
-        for (int k = 0; k < (ctx->has_store ? 4 : 2); ++k) {
-            uint8_t* stg = ctx->d_stage16.as<uint8_t>() + (size_t)k * n * 2;
-            if (sw == 2) LAUNCH(k_widen_u16, nblk(n, 256), 256, 0, reinterpret_cast<uint16_t*>(stg), n, dst32[k]->as<int32_t>());
-            else LAUNCH(k_widen_u8, nblk(n, 256), 256, 0, stg, n, dst32[k]->as<int32_t>());
-        }
-    }
-    SYNC_UP();                              // the offsets below are computed from the scalars
+    CK(scalars(ctx->d_nm, R->nm, sw, 4)); CK(scalars(ctx->d_lseq, R->l_seq, sw, 4));
+    if (ctx->has_store) { CK(scalars(ctx->d_store_lo, R->store_lo, sw, 4)); CK(scalars(ctx->d_store_len, R->store_len, sw, 4)); }
+    if (n_narrow) CK(up.ensure(ctx->d_stage, stage_bytes));
+    for (int k = 0; k < n_narrow; ++k) CK(up.copy(ctx->d_stage.as<uint8_t>() + narrow[k].stage_off, narrow[k].src, (size_t)n * narrow[k].bytes));
+    CK(up.hand_over());                     // the widening and the offsets below read the scalars
+    for (int k = 0; k < n_narrow; ++k) widen(ctx, ctx->d_stage.as<uint8_t>() + narrow[k].stage_off, narrow[k].bytes, n, narrow[k].dst->p);
+    const int qbits = qual_bits_of(R), sbits = seq_bits_of(R);
     ctx->qual_bits = qbits; ctx->seq_bits = sbits; ctx->n_seq_exc = sbits == 2 ? R->n_seq_exc : 0;
     // offsets: uploaded, or -- NULL = payload packed in read order -- computed here from l_seq / n_cigar (saves 24 B per read of PCIe)
     ctx->packed_seq = !R->seq_off; ctx->packed_qual = !R->qual_off; ctx->packed_cigar = !R->cigar_off;
-    {
-        uint32_t* small = ctx->d_small.as<uint32_t>();
-        const int64_t* host_off[3] = {R->seq_off, R->qual_off, R->cigar_off};
-        DevBuf* dev_off[3] = {&ctx->d_seq_off, &ctx->d_qual_off, &ctx->d_cig_off};
-        for (int kind = 0; kind < 3; ++kind) {
-            if (host_off[kind]) { UP(*dev_off[kind], host_off[kind], n, int64_t); continue; }
-            CK(dev_off[kind]->ensure((size_t)(n ? n : 1) * 8));
-            CK(ctx->d_v0.ensure((size_t)(n ? n : 1) * 4));
-            CK(ctx->d_scan.ensure((size_t)scan_scratch_words(n + 1) * 4 + 1024));
-            // compact payloads are expanded into a device-only layout with every read on a word boundary (k_unpack)
-            const int layout = (kind == 0 && sbits == 2) ? 5 : (kind == 1 && qbits != 8) ? 6 : kind;
-            LAUNCH(k_pack_len, nblk(n, 256), 256, 0, ctx->d_lseq.as<int32_t>(), ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr,
-                   ctx->d_ncig.as<uint16_t>(), n, layout, 8, ctx->d_v0.as<uint32_t>());
-            exclusive_scan_u32(ctx->d_v0.as<uint32_t>(), ctx->d_v0.as<uint32_t>(), n, ctx->d_scan.as<uint32_t>(), small + SW_PACK_TOTALS + kind, ctx->st);
-            LAUNCH(k_widen_u32, nblk(n, 256), 256, 0, ctx->d_v0.as<uint32_t>(), n, dev_off[kind]->as<int64_t>());
-        }
-        if (qbits != 8) {          // byte offsets of the compact qualities inside the uploaded array
-            CK(ctx->d_qual_poff.ensure((size_t)(n ? n : 1) * 4));
-            CK(ctx->d_scan.ensure((size_t)scan_scratch_words(n + 1) * 4 + 1024));
-            LAUNCH(k_pack_len, nblk(n, 256), 256, 0, ctx->d_lseq.as<int32_t>(), ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr,
-                   ctx->d_ncig.as<uint16_t>(), n, 3, qbits, ctx->d_qual_poff.as<uint32_t>());
-            exclusive_scan_u32(ctx->d_qual_poff.as<uint32_t>(), ctx->d_qual_poff.as<uint32_t>(), n, ctx->d_scan.as<uint32_t>(), small + SW_PACK_TOTALS + 3, ctx->st);
-            CK(ctx->d_qual_lut.ensure(16));
-            CK(cudaMemcpyAsync(ctx->d_qual_lut.p, R->qual_lut, qbits == 4 ? 16 : 4, cudaMemcpyHostToDevice, ctx->st));
-        }
-        if (sbits == 2) {          // byte offsets of the compact bases inside the uploaded array, and their exceptions
-            CK(ctx->d_seq_poff.ensure((size_t)(n ? n : 1) * 4));
-            CK(ctx->d_scan.ensure((size_t)scan_scratch_words(n + 1) * 4 + 1024));
-            LAUNCH(k_pack_len, nblk(n, 256), 256, 0, ctx->d_lseq.as<int32_t>(), ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr,
-                   ctx->d_ncig.as<uint16_t>(), n, 4, 2, ctx->d_seq_poff.as<uint32_t>());
-            exclusive_scan_u32(ctx->d_seq_poff.as<uint32_t>(), ctx->d_seq_poff.as<uint32_t>(), n, ctx->d_scan.as<uint32_t>(), small + SW_PACK_TOTALS + 4, ctx->st);
-            UP(ctx->d_exc_read, R->seq_exc_read, R->n_seq_exc, uint32_t); UP(ctx->d_exc_pos, R->seq_exc_pos, R->n_seq_exc, uint32_t);
-            UP(ctx->d_exc_nib, R->seq_exc_nib, R->n_seq_exc, uint8_t);
-        }
+    const int64_t* host_off[3] = {R->seq_off, R->qual_off, R->cigar_off};
+    DevBuf* dev_off[3] = {&ctx->d_seq_off, &ctx->d_qual_off, &ctx->d_cig_off};
+    for (int kind = 0; kind < 3; ++kind) {
+        if (host_off[kind]) { CK(up.copy(*dev_off[kind], host_off[kind], (size_t)n * 8)); continue; }
+        CK(dev_off[kind]->ensure(nz * 8));
+        CK(ctx->d_v0.ensure(nz * 4));
+        // compact payloads are expanded into a device-only layout with every read on a word boundary (k_unpack)
+        const int layout = (kind == 0 && sbits == 2) ? 5 : (kind == 1 && qbits != 8) ? 6 : kind;
+        if (const int rc = pack_offsets(ctx, n, layout, 8, ctx->d_v0.as<uint32_t>(), kind)) return rc;
+        widen(ctx, ctx->d_v0.p, 4, n, dev_off[kind]->p);
     }
-    // expanded payloads: a read stores (len + 1) / 2 bytes of 4-bit bases for (len + 3) / 4 bytes of 2-bit ones, and never more
-    // qualities than two per byte of 4-bit bases; up to 3 bytes of padding per read
-    const int64_t seq_dev_bytes = sbits == 4 ? R->seq_bytes : 2 * R->seq_bytes + 4 * n + 16;
-    const int64_t qual_dev_bytes = qbits == 8 ? R->qual_bytes : 2 * (sbits == 4 ? R->seq_bytes : 2 * R->seq_bytes) + 4 * n + 16;
-    if (seq_dev_bytes >= (1ll << 32) || qual_dev_bytes >= (1ll << 32)) {
-        ctx->err = "smc_upload: the expanded bases / qualities of the batch exceed 4 GiB; split the batch"; return SMC_E_LIMIT;
+    if (qbits != 8) {          // byte offsets of the compact qualities inside the uploaded array
+        CK(ctx->d_qual_poff.ensure(nz * 4));
+        if (const int rc = pack_offsets(ctx, n, 3, qbits, ctx->d_qual_poff.as<uint32_t>(), 3)) return rc;
+        CK(ctx->d_qual_lut.ensure(16));
+        CK(cudaMemcpyAsync(ctx->d_qual_lut.p, R->qual_lut, qbits == 4 ? 16 : 4, cudaMemcpyHostToDevice, ctx->st));
+    }
+    if (sbits == 2) {          // byte offsets of the compact bases inside the uploaded array, and their exceptions
+        CK(ctx->d_seq_poff.ensure(nz * 4));
+        if (const int rc = pack_offsets(ctx, n, 4, 2, ctx->d_seq_poff.as<uint32_t>(), 4)) return rc;
+        CK(up.copy(ctx->d_exc_read, R->seq_exc_read, (size_t)R->n_seq_exc * 4)); CK(up.copy(ctx->d_exc_pos, R->seq_exc_pos, (size_t)R->n_seq_exc * 4));
+        CK(up.copy(ctx->d_exc_nib, R->seq_exc_nib, (size_t)R->n_seq_exc));
     }
     DevBuf& seq_up = sbits == 4 ? ctx->d_seq : ctx->d_seq_packed;              // where the caller's seq[] bytes land
-    if (sbits == 2) CK(ctx->d_seq.ensure((size_t)seq_dev_bytes + 16));
+    if (sbits == 2) CK(ctx->d_seq.ensure((size_t)expanded_seq_bytes(R) + 16));
     DevBuf& qual_up = qbits == 8 ? ctx->d_qual : ctx->d_qual_packed;           // where the caller's qual[] bytes land
-    if (qbits != 8) CK(ctx->d_qual.ensure((size_t)qual_dev_bytes + 16));
+    if (qbits != 8) CK(ctx->d_qual.ensure((size_t)expanded_qual_bytes(R) + 16));
     if (G == 1) {
-        UP(seq_up, R->seq, R->seq_bytes, uint8_t); UP(qual_up, R->qual, R->qual_bytes, uint8_t);
-        if (sbits == 2) {
-            const uint32_t whole[2] = {0u, (uint32_t)n};
-            CK(cudaMemcpyAsync(ctx->d_small.as<uint32_t>() + SW_CHUNK_READS_SEQ, whole, 8, cudaMemcpyHostToDevice, ctx->st));
-            LAUNCH(k_unpack<2>, std::min<unsigned>(nblk(n, 256) + 1u, 148u * 8u), 256, 0, ctx->d_small.as<uint32_t>() + SW_CHUNK_READS_SEQ,
-                   ctx->d_seq_poff.as<uint32_t>(), ctx->d_seq_off.as<int64_t>(), ctx->d_lseq.as<int32_t>(),
-                   ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr, nullptr, ctx->d_seq_packed.as<uint8_t>(), ctx->d_seq.as<uint8_t>());
-            LAUNCH(k_patch_seq, nblk(ctx->n_seq_exc, 256), 256, 0, ctx->d_small.as<uint32_t>() + SW_CHUNK_READS_SEQ, ctx->n_seq_exc,
-                   ctx->d_exc_read.as<uint32_t>(), ctx->d_exc_pos.as<uint32_t>(), ctx->d_exc_nib.as<uint8_t>(), ctx->d_seq_off.as<int64_t>(),
-                   ctx->d_seq.as<uint8_t>());
-        }
-        if (qbits != 8) {
-            const uint32_t whole[2] = {0u, (uint32_t)n};
-            CK(cudaMemcpyAsync(ctx->d_small.as<uint32_t>() + SW_CHUNK_READS, whole, 8, cudaMemcpyHostToDevice, ctx->st));
-            const unsigned ug = std::min<unsigned>(nblk(n, 256) + 1u, 148u * 8u);
-            if (qbits == 2)
-                LAUNCH(k_unpack<0>, ug, 256, 0, ctx->d_small.as<uint32_t>() + SW_CHUNK_READS, ctx->d_qual_poff.as<uint32_t>(), ctx->d_qual_off.as<int64_t>(),
-                       ctx->d_lseq.as<int32_t>(), ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr, ctx->d_qual_lut.as<uint8_t>(),
-                       ctx->d_qual_packed.as<uint8_t>(), ctx->d_qual.as<uint8_t>());
-            else
-                LAUNCH(k_unpack<1>, ug, 256, 0, ctx->d_small.as<uint32_t>() + SW_CHUNK_READS, ctx->d_qual_poff.as<uint32_t>(), ctx->d_qual_off.as<int64_t>(),
-                       ctx->d_lseq.as<int32_t>(), ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr, ctx->d_qual_lut.as<uint8_t>(),
-                       ctx->d_qual_packed.as<uint8_t>(), ctx->d_qual.as<uint8_t>());
-        }
+        CK(up.copy(seq_up, R->seq, (size_t)R->seq_bytes)); CK(up.copy(qual_up, R->qual, (size_t)R->qual_bytes));
+        const uint32_t whole[2] = {0u, (uint32_t)n};                            // the one chunk: reads [0, n)
+        if (sbits == 2) CK(cudaMemcpyAsync(ctx->d_small.as<uint32_t>() + SW_CHUNK_READS_SEQ, whole, 8, cudaMemcpyHostToDevice, ctx->st));
+        if (qbits != 8) CK(cudaMemcpyAsync(ctx->d_small.as<uint32_t>() + SW_CHUNK_READS, whole, 8, cudaMemcpyHostToDevice, ctx->st));
+        expand_compact(ctx, 0, std::min<unsigned>(nblk(n, 256) + 1u, UNPACK_GRID));
     }
-    if (G == 1) SYNC_UP();
-    UP(ctx->d_cigar, R->cigar, R->n_cigar_words, uint32_t);
-    UP(ctx->d_loci_ref, Lc->ref_id, nl, int32_t); UP(ctx->d_loci_pos, Lc->pos0, nl, int32_t); UP(ctx->d_loci_base, Lc->ref_base, nl, uint8_t);
+    CK(up.copy(ctx->d_cigar, R->cigar, (size_t)R->n_cigar_words * 4));
+    CK(up.copy(ctx->d_loci_ref, Lc->ref_id, (size_t)nl * 4)); CK(up.copy(ctx->d_loci_pos, Lc->pos0, (size_t)nl * 4));
+    CK(up.copy(ctx->d_loci_base, Lc->ref_base, (size_t)nl));
     ctx->has_keep = K && K->n_loci > 0;
     if (ctx->has_keep) {
-        UP(ctx->d_keep_off, K->off, K->n_loci + 1, int64_t);
-        UP(ctx->d_keep_umi, K->umi, K->off[K->n_loci], uint64_t);
-        // d_k0 doubles as the staging buffer of the masked-locus list
-        ENSURE(ctx->d_k0, (size_t)K->n_loci * 8);
-        ALLOC_SYNC();
-        CK(cudaMemcpyAsync(ctx->d_k0.p, K->locus, (size_t)K->n_loci * 8, cudaMemcpyHostToDevice, up_st));
-        bytes += K->n_loci * 8;
-        SYNC_UP();
+        CK(up.copy(ctx->d_keep_off, K->off, (size_t)(K->n_loci + 1) * 8));
+        CK(up.copy(ctx->d_keep_umi, K->umi, (size_t)K->off[K->n_loci] * 8));
+        CK(up.copy(ctx->d_k0, K->locus, (size_t)K->n_loci * 8));              // d_k0 doubles as the staging buffer of the masked-locus list
+    }
+    CK(up.hand_over());
+    if (ctx->has_keep) {
         CK(ctx->d_keep_idx.ensure((size_t)(nl ? nl : 1) * 4));
         LAUNCH(k_fill_i32, nblk(nl, 256), 256, 0, ctx->d_keep_idx.as<int32_t>(), nl, -1);
         LAUNCH(k_scatter_idx, nblk(K->n_loci, 256), 256, 0, ctx->d_k0.as<int64_t>(), K->n_loci, ctx->d_keep_idx.as<int32_t>());
         ctx->n_keep_loci = K->n_loci;
     }
-    SYNC_UP();
     CK(ctx->d_loci_key.ensure((size_t)(nl ? nl : 1) * 8));
     LAUNCH(k_loci_keys, nblk(nl, 256), 256, 0, ctx->d_loci_ref.as<int32_t>(), ctx->d_loci_pos.as<int32_t>(), nl, ctx->d_loci_key.as<uint64_t>());
     ctx->n_reads = n; ctx->n_loci = nl;
@@ -710,14 +711,14 @@ static int upload_impl(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc,
     ctx->tm = smc_timings{};
     ctx->tm.n_reads = n; ctx->tm.n_loci = nl;
     if (G == 1) {
-        CK(cudaEventRecord(ctx->ev[1], ctx->st));
+        CK(cudaEventRecord(ctx->ev[EV_COPY_END], ctx->st));
         if (!pipelined) {
             CK(cudaStreamSynchronize(ctx->st));
-            cudaEventElapsedTime(&ctx->tm.ms_h2d, ctx->ev[0], ctx->ev[1]);
+            cudaEventElapsedTime(&ctx->tm.ms_h2d, ctx->ev[EV_COPY_BEGIN], ctx->ev[EV_COPY_END]);
         }
     } else {
         // the chunks follow the scalars on the link; everything up to the first pileup launch needs the scalars only
-        ENSURE(seq_up, (size_t)R->seq_bytes + 16); ENSURE(qual_up, (size_t)R->qual_bytes + 16);
+        CK(up.ensure(seq_up, (size_t)R->seq_bytes + 16)); CK(up.ensure(qual_up, (size_t)R->qual_bytes + 16));
         auto chunk_bytes = [&](int64_t total) { int64_t c = (total + G - 1) / G; c = (c + 255) & ~255ll; return (uint32_t)std::max<int64_t>(c, 256); };
         ctx->pipe_seq_chunk = chunk_bytes(R->seq_bytes); ctx->pipe_qual_chunk = chunk_bytes(R->qual_bytes);
         if (qbits != 8)            // which reads each chunk completes (the compact payload is in read order)
@@ -726,31 +727,36 @@ static int upload_impl(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc,
         if (sbits == 2)
             LAUNCH(k_chunk_reads, 1, 32, 0, ctx->d_seq_poff.as<uint32_t>(), n, (uint32_t)R->seq_bytes, ctx->pipe_seq_chunk, G,
                    ctx->d_small.as<uint32_t>() + SW_CHUNK_READS_SEQ);
-        grew = true;                        // d_seq / d_qual (the expanded payloads) may have been reallocated above as well
-        ALLOC_SYNC();
         for (int c = 0; c < G; ++c) {
             const int64_t s0 = std::min<int64_t>(R->seq_bytes, (int64_t)c * ctx->pipe_seq_chunk), s1 = std::min<int64_t>(R->seq_bytes, (int64_t)(c + 1) * ctx->pipe_seq_chunk);
             const int64_t q0 = std::min<int64_t>(R->qual_bytes, (int64_t)c * ctx->pipe_qual_chunk), q1 = std::min<int64_t>(R->qual_bytes, (int64_t)(c + 1) * ctx->pipe_qual_chunk);
-            if (s1 > s0) CK(cudaMemcpyAsync(seq_up.as<uint8_t>() + s0, R->seq + s0, (size_t)(s1 - s0), cudaMemcpyHostToDevice, ctx->st_copy));
-            if (q1 > q0) CK(cudaMemcpyAsync(qual_up.as<uint8_t>() + q0, R->qual + q0, (size_t)(q1 - q0), cudaMemcpyHostToDevice, ctx->st_copy));
+            CK(up.copy(seq_up.as<uint8_t>() + s0, R->seq + s0, (size_t)(s1 - s0)));
+            CK(up.copy(qual_up.as<uint8_t>() + q0, R->qual + q0, (size_t)(q1 - q0)));
             CK(cudaEventRecord(ctx->ev_chunk[c], ctx->st_copy));
-            bytes += (s1 - s0) + (q1 - q0);
         }
-        CK(cudaEventRecord(ctx->ev[1], ctx->st_copy));
+        CK(cudaEventRecord(ctx->ev[EV_COPY_END], ctx->st_copy));
         if (link_lock.owns_lock()) {
             CK(cudaEventRecord(ctx->ev_link, ctx->st_copy));
             g_link_tail[dv] = ctx->ev_link; g_link_owner[dv] = ctx;
         }
         ctx->pipe_n = G;
     }
-#undef UP
-#undef SYNC_UP
-#undef ENSURE
-#undef ALLOC_SYNC
     ctx->tm.pipe_chunks = pipelined ? G : 0;
-    ctx->tm.bytes_h2d = bytes;
+    ctx->tm.bytes_h2d = up.bytes;
     ctx->uploaded = true;
     return SMC_OK;
+}
+
+static int upload_impl(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc, const smc_umi_keep* K, bool pipelined) {
+    if (!ctx) return SMC_E_ARG;
+    NvtxRange nvtx_r("smc:upload");
+    if (const int rc = check_upload(R, Lc, ctx->err)) return rc;
+    const int rc = queue_upload(ctx, R, Lc, K, pipelined);
+    if (rc != SMC_OK) {                     // no copy may still read the caller's buffers when an error is returned
+        cudaStreamSynchronize(ctx->st_copy);
+        cudaStreamSynchronize(ctx->st);
+    }
+    return rc;
 }
 
 extern "C" int smc_upload(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc, const smc_umi_keep* K) {
@@ -768,7 +774,7 @@ extern "C" int smc_run_resident(smc_ctx* ctx) {
     const int64_t n = ctx->n_reads, nl = ctx->n_loci;
     const uint32_t n_tiles = (uint32_t)((nl + 31) / 32);
     uint32_t* small = ctx->d_small.as<uint32_t>();          // words: enum SmallWord
-    CK(cudaEventRecord(ctx->ev[2], ctx->st));
+    CK(cudaEventRecord(ctx->ev[EV_RUN_BEGIN], ctx->st));
     int64_t NE = 0;
     int frag_bits_used = 32;
     if (n > 0 && nl > 0) {
@@ -791,11 +797,11 @@ extern "C" int smc_run_resident(smc_ctx* ctx) {
         CK(cudaMemsetAsync(small + SW_FRAG_OR, 0, 8, ctx->st));
         LAUNCH(k_umi_slots, nblk(n, 256), 256, 0, ctx->d_umi.as<uint64_t>(), ctx->d_frag.as<uint32_t>(), n,
                ctx->d_umi_table.as<unsigned long long>(), (uint32_t)((1u << slot_bits) - 1u), frag_bits, k0, v0, (unsigned long long*)(small + SW_FRAG_OR));
-        CK(cudaEventRecord(ctx->ev[11], ctx->st));
+        CK(cudaEventRecord(ctx->ev[EV_READ_SORT_BEGIN], ctx->st));
         if (radix_sort_bits(k0, v0, k1, v1, n, 0, slot_bits + frag_bits, ctx->d_hist.as<uint32_t>(), ctx->d_scan.as<uint32_t>(), ctx->st)) {
             std::swap(k0, k1); std::swap(v0, v1);
         }
-        CK(cudaEventRecord(ctx->ev[12], ctx->st));
+        CK(cudaEventRecord(ctx->ev[EV_READ_SORT_DONE], ctx->st));
         ctx->tm.read_sort_passes = (slot_bits + frag_bits + RS_MAX_BITS - 1) / RS_MAX_BITS;
         const uint32_t* perm = v0;
         // dense barcode / fragment ranks, inverse permutation, barcode of every rank: one single-pass scan
@@ -830,9 +836,9 @@ extern "C" int smc_run_resident(smc_ctx* ctx) {
             if (ctx->qual_bits != 8) { P.qual_poff = ctx->d_qual_poff.as<uint32_t>(); P.qual_bits = ctx->qual_bits; }
             if (ctx->seq_bits == 2) P.seq_poff = ctx->d_seq_poff.as<uint32_t>();
         }
-        CK(cudaEventRecord(ctx->ev[13], ctx->st));
+        CK(cudaEventRecord(ctx->ev[EV_READ_PREP_BEGIN], ctx->st));
         LAUNCH(k_read_prep, nblk(n, 256), 256, 0, P);
-        CK(cudaEventRecord(ctx->ev[14], ctx->st));
+        CK(cudaEventRecord(ctx->ev[EV_READ_PREP_DONE], ctx->st));
         ctx->tm.read_prep_bytes = n * (int64_t)(4 + 4 + 2 + 1 + 4 + 4 + 8 + 8 + 8 + 2 + (ctx->has_store ? 8 : 0) + 4 + sizeof(ReadRec) + sizeof(GRec)) + 4 * ctx->n_cigar_words;
         // ---------------- K2b (first half): the (read x tile) events, scanned and written by one kernel into buffers sized from the
         // previous batch (or 4 per read); the exact count comes back with the checks below
@@ -869,8 +875,8 @@ extern "C" int smc_run_resident(smc_ctx* ctx) {
             ctx->ne_cap = NE + NE / 8 + 4096;                 // first batch of this shape: grow and write the events again
         }
     }
-    CK(cudaEventRecord(ctx->ev[3], ctx->st));
-    CK(cudaEventRecord(ctx->ev[15], ctx->st));
+    CK(cudaEventRecord(ctx->ev[EV_PREP_DONE], ctx->st));
+    CK(cudaEventRecord(ctx->ev[EV_EVENT_SORT_BEGIN], ctx->st));
     // ---------------- K2b: (read x tile) events, stable sort by tile
     const uint64_t* ev_key_sorted = nullptr; const uint32_t* ev_read_sorted = nullptr;
     CK(ctx->d_tile_off.ensure((size_t)(n_tiles + 2) * 4)); CK(ctx->d_unit_cnt.ensure((size_t)(n_tiles + 2) * 4));
@@ -888,7 +894,7 @@ extern "C" int smc_run_resident(smc_ctx* ctx) {
     } else {
         CK(ctx->d_scan.ensure((size_t)scan_scratch_words((int64_t)n_tiles + 2) * 4 + 1024));
     }
-    CK(cudaEventRecord(ctx->ev[16], ctx->st));
+    CK(cudaEventRecord(ctx->ev[EV_EVENT_SORT_DONE], ctx->st));
     LAUNCH(k_tile_offsets, nblk((int64_t)n_tiles + 1, 256), 256, 0, ev_key_sorted, NE, n_tiles, ctx->chunk, ctx->d_tile_off.as<uint32_t>(),
            ctx->d_unit_cnt.as<uint32_t>());
     exclusive_scan_u32(ctx->d_unit_cnt.as<uint32_t>(), ctx->d_unit_off.as<uint32_t>(), (int64_t)n_tiles + 1, ctx->d_scan.as<uint32_t>(),
@@ -924,7 +930,7 @@ extern "C" int smc_run_resident(smc_ctx* ctx) {
             ctx->pipe_end[c] = run;
         }
     }
-    CK(cudaEventRecord(ctx->ev[4], ctx->st));
+    CK(cudaEventRecord(ctx->ev[EV_SORT_DONE], ctx->st));
     return run_pileup_and_stats(ctx, n_tiles, NE);
 }
 
@@ -1023,30 +1029,14 @@ static int run_pileup_and_stats(smc_ctx* ctx, uint32_t n_tiles, int64_t NE) {
             { int rc = ensure_code_storage(ctx, false, ctx->has_keep); if (rc) return rc; }
             KAArgs A; KBArgs B;
             fill_kargs(ctx, A, B, false, ctx->has_keep);
-            CK(cudaEventRecord(ctx->ev[8], ctx->st));
+            CK(cudaEventRecord(ctx->ev[EV_PILEUP_BEGIN], ctx->st));
             if (ctx->pipe_n > 1) {
                 // pipelined upload: units [pipe_end[c-1], pipe_end[c]) start as soon as chunk c of the bases / qualities is in
                 uint32_t u0 = 0;
                 ctx->tm.pipe_launches = 0;
                 for (int c = 0; c < ctx->pipe_n; ++c) {
                     CK(cudaStreamWaitEvent(ctx->st, ctx->ev_chunk[c], 0));
-                    if (ctx->seq_bits == 2 && attempt == 0) {       // the reads completed by this chunk: compact bases -> nibbles, exceptions
-                        LAUNCH(k_unpack<2>, 148u * 8u, 256, 0, small + SW_CHUNK_READS_SEQ + c, ctx->d_seq_poff.as<uint32_t>(), ctx->d_seq_off.as<int64_t>(),
-                               ctx->d_lseq.as<int32_t>(), ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr, nullptr, ctx->d_seq_packed.as<uint8_t>(),
-                               ctx->d_seq.as<uint8_t>());
-                        LAUNCH(k_patch_seq, nblk(ctx->n_seq_exc, 256), 256, 0, small + SW_CHUNK_READS_SEQ + c, ctx->n_seq_exc, ctx->d_exc_read.as<uint32_t>(),
-                               ctx->d_exc_pos.as<uint32_t>(), ctx->d_exc_nib.as<uint8_t>(), ctx->d_seq_off.as<int64_t>(), ctx->d_seq.as<uint8_t>());
-                    }
-                    if (ctx->qual_bits != 8 && attempt == 0) {      // the reads completed by this chunk: compact qualities -> bytes
-                        if (ctx->qual_bits == 2)
-                            LAUNCH(k_unpack<0>, 148u * 8u, 256, 0, small + SW_CHUNK_READS + c, ctx->d_qual_poff.as<uint32_t>(), ctx->d_qual_off.as<int64_t>(),
-                                   ctx->d_lseq.as<int32_t>(), ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr, ctx->d_qual_lut.as<uint8_t>(),
-                                   ctx->d_qual_packed.as<uint8_t>(), ctx->d_qual.as<uint8_t>());
-                        else
-                            LAUNCH(k_unpack<1>, 148u * 8u, 256, 0, small + SW_CHUNK_READS + c, ctx->d_qual_poff.as<uint32_t>(), ctx->d_qual_off.as<int64_t>(),
-                                   ctx->d_lseq.as<int32_t>(), ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr, ctx->d_qual_lut.as<uint8_t>(),
-                                   ctx->d_qual_packed.as<uint8_t>(), ctx->d_qual.as<uint8_t>());
-                    }
+                    if (attempt == 0) expand_compact(ctx, c, UNPACK_GRID);     // the reads completed by this chunk
                     const uint32_t u1 = ctx->pipe_end[c];
                     if (u1 <= u0) continue;
                     A.unit0 = B.unit0 = u0; A.n_units = B.n_units = u1;
@@ -1054,13 +1044,13 @@ static int run_pileup_and_stats(smc_ctx* ctx, uint32_t n_tiles, int64_t NE) {
                     LAUNCH(k_merge_t<false>, nblk(u1 - u0, KB_WARPS), KB_WARPS * 32, KB_SMEM_BYTES, B);
                     u0 = u1; ++ctx->tm.pipe_launches;
                 }
-                CK(cudaEventRecord(ctx->ev[9], ctx->st));
+                CK(cudaEventRecord(ctx->ev[EV_GATHER_DONE], ctx->st));
             } else {
                 LAUNCH(k_gather_t<false>, nblk(ctx->n_units_cap, KA_WARPS), KA_WARPS * 32, KA_SMEM_BYTES(false), A);
-                CK(cudaEventRecord(ctx->ev[9], ctx->st));
+                CK(cudaEventRecord(ctx->ev[EV_GATHER_DONE], ctx->st));
                 LAUNCH(k_merge_t<false>, nblk(ctx->n_units_cap, KB_WARPS), KB_WARPS * 32, KB_SMEM_BYTES, B);
             }
-            CK(cudaEventRecord(ctx->ev[10], ctx->st));
+            CK(cudaEventRecord(ctx->ev[EV_MERGE_DONE], ctx->st));
         }
         uint32_t h[3];
         CK(cudaMemcpyAsync(h, small + SW_GFLAGS, 12, cudaMemcpyDeviceToHost, ctx->st));
@@ -1075,7 +1065,7 @@ static int run_pileup_and_stats(smc_ctx* ctx, uint32_t n_tiles, int64_t NE) {
             ctx->dyn_cap <<= 2;
         }
     }
-    CK(cudaEventRecord(ctx->ev[5], ctx->st));
+    CK(cudaEventRecord(ctx->ev[EV_PILEUP_DONE], ctx->st));
     NvtxRange nvtx_s("smc:dyn_rows+call+fisher");
     // ---------------- dynamic alleles -> sorted rows
     const int64_t nd = ctx->n_dyn;
@@ -1128,7 +1118,7 @@ static int run_pileup_and_stats(smc_ctx* ctx, uint32_t n_tiles, int64_t NE) {
         CK(cudaMemsetAsync(small + SW_CVG_SUM, 0, 8, ctx->st));
         LAUNCH(k_sum_cvg, std::min<unsigned>(nblk(nl, 256), 592u), 256, 0, ctx->d_loc.as<int32_t>() + (size_t)SMC_L_CVG * nl, nl,
                (unsigned long long*)(small + SW_CVG_SUM));
-        CK(cudaEventRecord(ctx->ev[6], ctx->st));
+        CK(cudaEventRecord(ctx->ev[EV_STATS_DONE], ctx->st));
         CK(cudaMemcpyAsync(&n_tasks_h, small + SW_N_TASKS, 4, cudaMemcpyDeviceToHost, ctx->st));
         CK(cudaMemcpyAsync(&cvgsum, small + SW_CVG_SUM, 8, cudaMemcpyDeviceToHost, ctx->st));
         CK(cudaStreamSynchronize(ctx->st));
@@ -1137,22 +1127,22 @@ static int run_pileup_and_stats(smc_ctx* ctx, uint32_t n_tiles, int64_t NE) {
         if (attempt == 1) { ctx->err = "Fisher task list overflow"; return SMC_E_OVERFLOW; }
         ctx->task_cap = n_tasks_h + n_tasks_h / 4 + 1024;      // grow and redo the (cheap) call kernel
     }
-    cudaEventElapsedTime(&ctx->tm.ms_prep, ctx->ev[2], ctx->ev[3]);
-    cudaEventElapsedTime(&ctx->tm.ms_sort, ctx->ev[3], ctx->ev[4]);
-    cudaEventElapsedTime(&ctx->tm.ms_pileup, ctx->ev[4], ctx->ev[5]);
-    cudaEventElapsedTime(&ctx->tm.ms_stats, ctx->ev[5], ctx->ev[6]);
-    cudaEventElapsedTime(&ctx->tm.ms_total_device, ctx->ev[2], ctx->ev[6]);
+    cudaEventElapsedTime(&ctx->tm.ms_prep, ctx->ev[EV_RUN_BEGIN], ctx->ev[EV_PREP_DONE]);
+    cudaEventElapsedTime(&ctx->tm.ms_sort, ctx->ev[EV_PREP_DONE], ctx->ev[EV_SORT_DONE]);
+    cudaEventElapsedTime(&ctx->tm.ms_pileup, ctx->ev[EV_SORT_DONE], ctx->ev[EV_PILEUP_DONE]);
+    cudaEventElapsedTime(&ctx->tm.ms_stats, ctx->ev[EV_PILEUP_DONE], ctx->ev[EV_STATS_DONE]);
+    cudaEventElapsedTime(&ctx->tm.ms_total_device, ctx->ev[EV_RUN_BEGIN], ctx->ev[EV_STATS_DONE]);
     ctx->tm.ms_read_sort = ctx->tm.ms_k_read_prep = ctx->tm.ms_event_sort = 0.f;
     if (ctx->n_reads > 0 && nl > 0) {
-        cudaEventElapsedTime(&ctx->tm.ms_read_sort, ctx->ev[11], ctx->ev[12]);
-        cudaEventElapsedTime(&ctx->tm.ms_k_read_prep, ctx->ev[13], ctx->ev[14]);
+        cudaEventElapsedTime(&ctx->tm.ms_read_sort, ctx->ev[EV_READ_SORT_BEGIN], ctx->ev[EV_READ_SORT_DONE]);
+        cudaEventElapsedTime(&ctx->tm.ms_k_read_prep, ctx->ev[EV_READ_PREP_BEGIN], ctx->ev[EV_READ_PREP_DONE]);
     }
-    cudaEventElapsedTime(&ctx->tm.ms_event_sort, ctx->ev[15], ctx->ev[16]);
+    cudaEventElapsedTime(&ctx->tm.ms_event_sort, ctx->ev[EV_EVENT_SORT_BEGIN], ctx->ev[EV_EVENT_SORT_DONE]);
     ctx->tm.ms_k_pileup = ctx->tm.ms_k_gather = ctx->tm.ms_k_merge = 0.f;
     if (NE > 0) {
-        cudaEventElapsedTime(&ctx->tm.ms_k_pileup, ctx->ev[8], ctx->ev[10]);
-        cudaEventElapsedTime(&ctx->tm.ms_k_gather, ctx->ev[8], ctx->ev[9]);
-        cudaEventElapsedTime(&ctx->tm.ms_k_merge, ctx->ev[9], ctx->ev[10]);
+        cudaEventElapsedTime(&ctx->tm.ms_k_pileup, ctx->ev[EV_PILEUP_BEGIN], ctx->ev[EV_MERGE_DONE]);
+        cudaEventElapsedTime(&ctx->tm.ms_k_gather, ctx->ev[EV_PILEUP_BEGIN], ctx->ev[EV_GATHER_DONE]);
+        cudaEventElapsedTime(&ctx->tm.ms_k_merge, ctx->ev[EV_GATHER_DONE], ctx->ev[EV_MERGE_DONE]);
     }
     ctx->tm.n_pileup_events = (int64_t)cvgsum;
     ctx->tm.n_dyn = nd; ctx->tm.n_fisher = n_tasks_h;
@@ -1173,7 +1163,7 @@ extern "C" int smc_download(smc_ctx* ctx, smc_out* out) {
     if (nd > out->dyn_capacity) { ctx->err = "smc_download: dyn_capacity too small (n_dyn reported in smc_out.n_dyn)"; return SMC_E_LIMIT; }
     NvtxRange nvtx_r("smc:download");
     int64_t bytes = 0;
-    CK(cudaEventRecord(ctx->ev[0], ctx->st));
+    CK(cudaEventRecord(ctx->ev[EV_COPY_BEGIN], ctx->st));
 #define DOWN(dst, buf, count, T)                                                                                \
     do {                                                                                                        \
         size_t b__ = (size_t)(count) * sizeof(T);                                                               \
@@ -1194,7 +1184,7 @@ extern "C" int smc_download(smc_ctx* ctx, smc_out* out) {
     if (nd) CK(cudaMemcpyAsync(keys.data(), ctx->d_s_key.p, (size_t)nd * 8, cudaMemcpyDeviceToHost, ctx->st));
     CK(cudaMemcpyAsync(first.data(), ctx->d_dyn_first.p, (nl + 1) * 4, cudaMemcpyDeviceToHost, ctx->st));
     bytes += nd * 8 + (int64_t)(nl + 1) * 4;
-    CK(cudaEventRecord(ctx->ev[1], ctx->st));
+    CK(cudaEventRecord(ctx->ev[EV_COPY_END], ctx->st));
     CK(cudaStreamSynchronize(ctx->st));
     for (int64_t j = 0; j < nd; ++j) {
         unsigned long long k = keys[(size_t)j];
@@ -1203,7 +1193,7 @@ extern "C" int smc_download(smc_ctx* ctx, smc_out* out) {
         if (out->dyn_site) out->dyn_site[j] = (uint8_t)((k >> 36) & 15u);
     }
     if (out->dyn_first) for (size_t i = 0; i <= nl; ++i) out->dyn_first[i] = first[i];
-    cudaEventElapsedTime(&ctx->tm.ms_d2h, ctx->ev[0], ctx->ev[1]);
+    cudaEventElapsedTime(&ctx->tm.ms_d2h, ctx->ev[EV_COPY_BEGIN], ctx->ev[EV_COPY_END]);
     ctx->tm.bytes_d2h = bytes;
     return SMC_OK;
 }
@@ -1242,9 +1232,9 @@ extern "C" int smc_call_batch(smc_ctx* ctx, const smc_reads_soa* reads, const sm
         if (rc == SMC_OK && (e1 != cudaSuccess || e2 != cudaSuccess)) {
             ctx->err = std::string("smc_call_batch: ") + cudaGetErrorString(e1 != cudaSuccess ? e1 : e2); rc = SMC_E_CUDA;
         }
-        if (rc == SMC_OK && ctx->uploaded) cudaEventElapsedTime(&ctx->tm.ms_h2d, ctx->ev[0], ctx->ev[1]);
+        if (rc == SMC_OK && ctx->uploaded) cudaEventElapsedTime(&ctx->tm.ms_h2d, ctx->ev[EV_COPY_BEGIN], ctx->ev[EV_COPY_END]);
         if (timeline && rc == SMC_OK) {
-            for (int i = 0; i < 7; ++i) if (cudaEventElapsedTime(&tl.dev[i], g_tl_base, ctx->ev[i]) != cudaSuccess) { tl.dev[i] = -1.f; cudaGetLastError(); }
+            for (int i = EV_COPY_BEGIN; i <= EV_STATS_DONE; ++i) if (cudaEventElapsedTime(&tl.dev[i], g_tl_base, ctx->ev[i]) != cudaSuccess) { tl.dev[i] = -1.f; cudaGetLastError(); }
             tl.on = true;
         }
         ctx->pipe_n = 0;                                 // the batch is resident now: later smc_run_resident calls run it in one go

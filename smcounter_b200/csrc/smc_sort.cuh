@@ -292,12 +292,3 @@ static int radix_sort_bits(uint64_t* k0, uint32_t* v0, uint64_t* k1, uint32_t* v
     }
     return cur;
 }
-
-// bitwise OR of an array of u32 into out[0] (range check of the fragment ids)
-__global__ void k_or_and_u32(const uint32_t* __restrict__ a, int64_t n, unsigned long long* __restrict__ out) {
-    unsigned long long o = 0;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) o |= a[i];
-#pragma unroll
-    for (int s = 16; s > 0; s >>= 1) o |= __shfl_xor_sync(FULL_MASK, o, s);
-    if (lane_id() == 0 && o) atomicOr(&out[0], o);
-}
