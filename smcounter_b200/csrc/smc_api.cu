@@ -71,15 +71,15 @@ struct DevBuf {
 
 // words of the small device scratch block (smc_ctx::d_small) the kernels report through
 enum SmallWord {
-    SW_FRAG_OR = 0,          // u64: OR of all fragment ids (range check)
+    SW_FRAG_OR = 0,          // u64: OR of the fragment ids k_umi_slots found out of range (0: all ids are dense)
     SW_N_TILE_EVENTS = 4,    // total of the tile-event scan
     SW_GFLAGS = 5,           // GF_* bits raised by the kernels
     SW_DYN_COUNT = 6,        // entries of the dynamic-allele table
     SW_N_TASKS = 7,          // Fisher tasks emitted by k_call
     SW_CVG_SUM = 8,          // u64: sum of cvg over the loci (= pileup read-events)
-    SW_N_UMI = 10,           // distinct barcodes
+    SW_N_UMI = 12,           // distinct barcodes (k_rank_scan; past the words k_read_prep's memset clears)
     SW_PIPE_BLOCKED = 16,    // [SMC_PIPE_MAX]: first unit that has to wait for chunk c + 1
-    SW_PACK_TOTALS = 40,     // [4]: bytes / words of packed bases, qualities, CIGARs, compact qualities
+    SW_PACK_TOTALS = 40,     // [5]: bytes / words of packed bases, qualities, CIGARs, compact qualities, compact bases
     SW_SPILL_COUNT = 48,     // k_merge spill records handed out
     SW_CHUNK_READS = 64,     // [SMC_PIPE_MAX + 2]: first read completed by each upload chunk (compact qualities)
     SW_CHUNK_READS_SEQ = 96  // the same for the compact bases
@@ -110,7 +110,7 @@ struct smc_ctx {
     bool packed_seq = false, packed_qual = false, packed_cigar = false;   // offsets were NULL: computed on the device
     uint32_t pipe_end[SMC_PIPE_MAX]{};          // launch c of the pileup kernels covers units [pipe_end[c-1], pipe_end[c])
     // resident inputs
-    int64_t n_reads = 0, n_loci = 0, n_keep_loci = 0, n_keep_umi = 0;
+    int64_t n_reads = 0, n_loci = 0;
     int64_t seq_bytes = 0, qual_bytes = 0, n_cigar_words = 0;
     DevBuf d_ref_id{bufs}, d_pos{bufs}, d_flag{bufs}, d_mapq{bufs}, d_nm{bufs}, d_lseq{bufs}, d_seq_off{bufs}, d_qual_off{bufs},
         d_cig_off{bufs}, d_ncig{bufs}, d_umi{bufs}, d_frag{bufs}, d_seq{bufs}, d_qual{bufs}, d_cigar{bufs}, d_store_lo{bufs}, d_store_len{bufs};
@@ -120,7 +120,6 @@ struct smc_ctx {
         d_exc_read{bufs}, d_exc_pos{bufs}, d_exc_nib{bufs};
     int seq_bits = 4; int64_t n_seq_exc = 0;    // 2: compact bases were uploaded (d_seq_packed) and are expanded into d_seq
     uint32_t spill_cap = 0;                     // records in the k_merge spill pool (grows x4 on GF_SPILL_FULL)
-    const uint32_t* inv_ptr = nullptr;          // read index -> sorted position (lives in d_v0 or d_v1 after the read sort)
     DevBuf d_loci_ref{bufs}, d_loci_pos{bufs}, d_loci_base{bufs}, d_loci_key{bufs};
     DevBuf d_keep_idx{bufs}, d_keep_off{bufs}, d_keep_umi{bufs};
     bool has_keep = false, uploaded = false, ran = false;
@@ -151,7 +150,7 @@ struct smc_ctx {
     smc_timings tm{};
     uint32_t chunk = 128;       // tile events per warp unit (A/B on B200, whole step: 96 -> 4.42 ms, 128 -> 4.39, 160 -> 4.39, 256 -> 4.47, 384 -> 4.60)
     const uint32_t* ev_read_sorted = nullptr;   // tile-sorted event -> srank map (lives in d_ev0 or d_ev1)
-    uint32_t n_tiles = 0; int64_t n_tile_events = 0;
+    int64_t n_tile_events = 0;
     int64_t ne_cap = 0;                         // capacity of the tile-event buffers (grow only)
 };
 
@@ -702,7 +701,6 @@ static int queue_upload(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc
         CK(ctx->d_keep_idx.ensure((size_t)(nl ? nl : 1) * 4));
         LAUNCH(k_fill_i32, nblk(nl, 256), 256, 0, ctx->d_keep_idx.as<int32_t>(), nl, -1);
         LAUNCH(k_scatter_idx, nblk(K->n_loci, 256), 256, 0, ctx->d_k0.as<int64_t>(), K->n_loci, ctx->d_keep_idx.as<int32_t>());
-        ctx->n_keep_loci = K->n_loci;
     }
     CK(ctx->d_loci_key.ensure((size_t)(nl ? nl : 1) * 8));
     LAUNCH(k_loci_keys, nblk(nl, 256), 256, 0, ctx->d_loci_ref.as<int32_t>(), ctx->d_loci_pos.as<int32_t>(), nl, ctx->d_loci_key.as<uint64_t>());
@@ -763,122 +761,140 @@ extern "C" int smc_upload(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* 
     return upload_impl(ctx, R, Lc, K, false);
 }
 
-static int run_pileup_and_stats(smc_ctx* ctx, uint32_t n_tiles, int64_t NE);
+// One host round trip: `bytes` of device memory into `dst`, behind everything queued on ctx->st.
+static int read_back(smc_ctx* ctx, void* dst, const void* src, size_t bytes) {
+    CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, ctx->st));
+    CK(cudaStreamSynchronize(ctx->st));
+    return SMC_OK;
+}
 
-extern "C" int smc_run_resident(smc_ctx* ctx) {
-    if (!ctx) return SMC_E_ARG;
-    if (!ctx->uploaded) { ctx->err = "smc_run_resident: nothing uploaded"; return SMC_E_STATE; }
-    CK(cudaSetDevice(ctx->device));
-    g_launches = 0;
-    NvtxRange nvtx_r("smc:read_sort+prep+tile_events");
-    const int64_t n = ctx->n_reads, nl = ctx->n_loci;
-    const uint32_t n_tiles = (uint32_t)((nl + 31) / 32);
-    uint32_t* small = ctx->d_small.as<uint32_t>();          // words: enum SmallWord
-    CK(cudaEventRecord(ctx->ev[EV_RUN_BEGIN], ctx->st));
-    int64_t NE = 0;
-    int frag_bits_used = 32;
-    if (n > 0 && nl > 0) {
-        // ---------------- K2a: order reads by (barcode, frag_id, BAM index): one stable sort on (barcode slot, frag_id)
-        CK(ctx->d_k0.ensure((size_t)n * 8)); CK(ctx->d_k1.ensure((size_t)n * 8));
-        CK(ctx->d_v0.ensure((size_t)n * 4)); CK(ctx->d_v1.ensure((size_t)n * 4));
-        CK(ctx->d_hist.ensure(radix_hist_words(n) * 4 + 1024));
-        CK(ctx->d_scan.ensure((size_t)std::max<int64_t>(radix_scan_words(n), scan_scratch_words(n + 1)) * 4 + 1024));
-        uint64_t* k0 = ctx->d_k0.as<uint64_t>(); uint64_t* k1 = ctx->d_k1.as<uint64_t>();
-        uint32_t* v0 = ctx->d_v0.as<uint32_t>(); uint32_t* v1 = ctx->d_v1.as<uint32_t>();
-        // barcode table of >= 1.1 n slots (a batch has far fewer distinct barcodes than reads) and dense fragment ids < n:
-        // a 2.9 M read panel batch sorts on 22 + 22 = 44 key bits = four 11-bit passes
-        int slot_bits = 4;
-        while ((double)(1ll << slot_bits) < 1.1 * (double)n) ++slot_bits;
-        int frag_bits = 1;                                             // frag_id < 2^frag_bits; checked below (the contract says
-        while ((1ll << frag_bits) < n) ++frag_bits;                    // ids are dense, first-appearance numbers, hence < n_reads)
-        frag_bits_used = frag_bits;
-        CK(ctx->d_umi_table.ensure(((size_t)1 << slot_bits) * 8));
-        CK(cudaMemsetAsync(ctx->d_umi_table.p, 0xff, ((size_t)1 << slot_bits) * 8, ctx->st));
-        CK(cudaMemsetAsync(small + SW_FRAG_OR, 0, 8, ctx->st));
-        LAUNCH(k_umi_slots, nblk(n, 256), 256, 0, ctx->d_umi.as<uint64_t>(), ctx->d_frag.as<uint32_t>(), n,
-               ctx->d_umi_table.as<unsigned long long>(), (uint32_t)((1u << slot_bits) - 1u), frag_bits, k0, v0, (unsigned long long*)(small + SW_FRAG_OR));
-        CK(cudaEventRecord(ctx->ev[EV_READ_SORT_BEGIN], ctx->st));
-        if (radix_sort_bits(k0, v0, k1, v1, n, 0, slot_bits + frag_bits, ctx->d_hist.as<uint32_t>(), ctx->d_scan.as<uint32_t>(), ctx->st)) {
-            std::swap(k0, k1); std::swap(v0, v1);
-        }
-        CK(cudaEventRecord(ctx->ev[EV_READ_SORT_DONE], ctx->st));
-        ctx->tm.read_sort_passes = (slot_bits + frag_bits + RS_MAX_BITS - 1) / RS_MAX_BITS;
-        const uint32_t* perm = v0;
-        // dense barcode / fragment ranks, inverse permutation, barcode of every rank: one single-pass scan
-        CK(ctx->d_urank.ensure((size_t)n * 4)); CK(ctx->d_frank.ensure((size_t)n * 4));
-        CK(ctx->d_umi_of_urank.ensure((size_t)n * 8));
-        uint32_t* uex = ctx->d_urank.as<uint32_t>(); uint32_t* fex = ctx->d_frank.as<uint32_t>();
-        {
-            const int64_t nbt = (n + SCAN_TILE - 1) / SCAN_TILE;
-            uint32_t* scr = ctx->d_scan.as<uint32_t>();
-            CK(cudaMemsetAsync(scr, 0, (size_t)(2 * nbt + 8) * 4, ctx->st));
-            LAUNCH(k_rank_scan, (unsigned)nbt, SCAN_THREADS, 0, k0, frag_bits, n, ctx->d_umi.as<uint64_t>(), perm, uex, fex,
-                   ctx->d_umi_of_urank.as<uint64_t>(), v1, reinterpret_cast<unsigned long long*>(scr + 2), scr, small + SW_N_UMI);
-        }
-        // ---------------- K1: per-read records, computed in BAM order (coalesced inputs) and stored at their sorted position
-        CK(ctx->d_recs.ensure((size_t)n * sizeof(ReadRec))); CK(ctx->d_grec.ensure((size_t)n * sizeof(GRec)));
-        CK(cudaMemsetAsync(small + SW_N_TILE_EVENTS, 0, 32, ctx->st));
-        PrepArgs P{};
-        ctx->inv_ptr = v1;
-        P.n_reads = n; P.inv = v1; P.urank = uex; P.frank = fex;
-        P.ref_id = ctx->d_ref_id.as<int32_t>(); P.pos = ctx->d_pos.as<int32_t>(); P.flag = ctx->d_flag.as<uint16_t>();
-        P.mapq = ctx->d_mapq.as<uint8_t>(); P.nm = ctx->d_nm.as<int32_t>(); P.l_seq = ctx->d_lseq.as<int32_t>();
-        P.seq_off = ctx->d_seq_off.as<int64_t>(); P.qual_off = ctx->d_qual_off.as<int64_t>(); P.cigar_off = ctx->d_cig_off.as<int64_t>();
-        P.n_cigar = ctx->d_ncig.as<uint16_t>(); P.cigar = ctx->d_cigar.as<uint32_t>();
-        if (ctx->has_store) { P.store_lo = ctx->d_store_lo.as<int32_t>(); P.store_len = ctx->d_store_len.as<int32_t>(); }
-        P.loci_key = ctx->d_loci_key.as<uint64_t>(); P.n_loci = nl;
-        P.minMQ = ctx->prm.minMQ; P.primerDist = ctx->prm.primerDist; P.mismatchThr = ctx->prm.mismatchThr;
-        P.recs = ctx->d_recs.as<ReadRec>(); P.grec = ctx->d_grec.as<GRec>(); P.gflags = small + SW_GFLAGS;
-        if (ctx->pipe_n > 1) {
-            CK(ctx->d_pipe_need.ensure((size_t)n));
-            P.pipe_need = ctx->d_pipe_need.as<uint8_t>(); P.pipe_n = (uint32_t)ctx->pipe_n;
-            P.pipe_seq_chunk = ctx->pipe_seq_chunk; P.pipe_qual_chunk = ctx->pipe_qual_chunk;
-            if (ctx->qual_bits != 8) { P.qual_poff = ctx->d_qual_poff.as<uint32_t>(); P.qual_bits = ctx->qual_bits; }
-            if (ctx->seq_bits == 2) P.seq_poff = ctx->d_seq_poff.as<uint32_t>();
-        }
-        CK(cudaEventRecord(ctx->ev[EV_READ_PREP_BEGIN], ctx->st));
-        LAUNCH(k_read_prep, nblk(n, 256), 256, 0, P);
-        CK(cudaEventRecord(ctx->ev[EV_READ_PREP_DONE], ctx->st));
-        ctx->tm.read_prep_bytes = n * (int64_t)(4 + 4 + 2 + 1 + 4 + 4 + 8 + 8 + 8 + 2 + (ctx->has_store ? 8 : 0) + 4 + sizeof(ReadRec) + sizeof(GRec)) + 4 * ctx->n_cigar_words;
-        // ---------------- K2b (first half): the (read x tile) events, scanned and written by one kernel into buffers sized from the
-        // previous batch (or 4 per read); the exact count comes back with the checks below
-        if (ctx->ne_cap < 4 * n + 4096) ctx->ne_cap = 4 * n + 4096;
-        for (int attempt = 0; attempt < 2; ++attempt) {
-            if (ctx->ne_cap > 0xfffffff0ll) ctx->ne_cap = 0xfffffff0ll;
-            CK(ctx->d_ek0.ensure((size_t)ctx->ne_cap * 8)); CK(ctx->d_ev0.ensure((size_t)ctx->ne_cap * 4));
-            const int64_t nbt = (n + SCAN_TILE - 1) / SCAN_TILE;
-            uint32_t* scr = ctx->d_scan.as<uint32_t>();
-            CK(cudaMemsetAsync(scr, 0, (size_t)(2 * nbt + 8) * 4, ctx->st));
-            LAUNCH(k_expand_scan, (unsigned)nbt, SCAN_THREADS, 0, ctx->d_recs.as<ReadRec>(), n, ctx->d_ek0.as<uint64_t>(), ctx->d_ev0.as<uint32_t>(),
-                   (uint32_t)ctx->ne_cap, reinterpret_cast<unsigned long long*>(scr + 2), scr, small + SW_N_TILE_EVENTS);
-            if (attempt == 1) break;
-        uint32_t h[2], tot[5];
-        unsigned long long frag_or = 0;
-        CK(cudaMemcpyAsync(&frag_or, small + SW_FRAG_OR, 8, cudaMemcpyDeviceToHost, ctx->st));
-        CK(cudaMemcpyAsync(h, small + SW_N_TILE_EVENTS, 8, cudaMemcpyDeviceToHost, ctx->st));
-        CK(cudaMemcpyAsync(tot, small + SW_PACK_TOTALS, 20, cudaMemcpyDeviceToHost, ctx->st));
-        CK(cudaStreamSynchronize(ctx->st));
-        if (h[1] & GF_BAD_READ) { ctx->err = "a read has l_seq or clip length > 65535 (unsupported)"; return SMC_E_LIMIT; }
-        if (h[1] & GF_BAD_STORE) {
-            ctx->err = "stored window: store_lo must be even and >= 0, store_lo + store_len <= l_seq, reads with indels / clips inside must be "
-                       "stored whole, and every target base of a read must lie inside its window";
-            return SMC_E_ARG;
-        }
-        if (frag_or >> frag_bits_used) { ctx->err = "frag_id must be a dense id (< n_reads), numbered by first appearance"; return SMC_E_ARG; }
-        if ((ctx->packed_seq && (int64_t)tot[ctx->seq_bits == 2 ? 4 : 0] != ctx->seq_bytes) || (ctx->packed_qual && (int64_t)tot[ctx->qual_bits != 8 ? 3 : 1] != ctx->qual_bytes) ||
-            (ctx->packed_cigar && (int64_t)tot[2] != ctx->n_cigar_words)) {
-            ctx->err = "packed payload (NULL offsets): seq_bytes / qual_bytes / n_cigar_words do not match the sums of (len+1)/2, len, n_cigar (len = store_len or l_seq)";
-            return SMC_E_ARG;
-        }
-            NE = h[0];
-            if (NE <= ctx->ne_cap) break;
-            ctx->ne_cap = NE + NE / 8 + 4096;                 // first batch of this shape: grow and write the events again
-        }
+// K2a: order reads by (barcode, frag_id, BAM index): one stable sort on (barcode slot, frag_id), then one single-pass scan for
+// the dense barcode / fragment ranks, the barcode of every rank and the inverse permutation (*inv: read index -> sorted position).
+static int read_sort(smc_ctx* ctx, const uint32_t** inv) {
+    const int64_t n = ctx->n_reads;
+    uint32_t* small = ctx->d_small.as<uint32_t>();
+    CK(ctx->d_k0.ensure((size_t)n * 8)); CK(ctx->d_k1.ensure((size_t)n * 8));
+    CK(ctx->d_v0.ensure((size_t)n * 4)); CK(ctx->d_v1.ensure((size_t)n * 4));
+    CK(ctx->d_hist.ensure(radix_hist_words(n) * 4 + 1024));
+    CK(ctx->d_scan.ensure((size_t)std::max<int64_t>(radix_scan_words(n), scan_scratch_words(n + 1)) * 4 + 1024));
+    uint64_t* k0 = ctx->d_k0.as<uint64_t>(); uint64_t* k1 = ctx->d_k1.as<uint64_t>();
+    uint32_t* v0 = ctx->d_v0.as<uint32_t>(); uint32_t* v1 = ctx->d_v1.as<uint32_t>();
+    // barcode table of >= 1.1 n slots (a batch has far fewer distinct barcodes than reads) and dense fragment ids < n:
+    // a 2.9 M read panel batch sorts on 22 + 22 = 44 key bits = four 11-bit passes
+    int slot_bits = 4;
+    while ((double)(1ll << slot_bits) < 1.1 * (double)n) ++slot_bits;
+    int frag_bits = 1;                                             // frag_id < 2^frag_bits; checked after the round trip (the
+    while ((1ll << frag_bits) < n) ++frag_bits;                    // contract says ids are dense, first-appearance numbers)
+    CK(ctx->d_umi_table.ensure(((size_t)1 << slot_bits) * 8));
+    CK(cudaMemsetAsync(ctx->d_umi_table.p, 0xff, ((size_t)1 << slot_bits) * 8, ctx->st));
+    CK(cudaMemsetAsync(small + SW_FRAG_OR, 0, 8, ctx->st));
+    LAUNCH(k_umi_slots, nblk(n, 256), 256, 0, ctx->d_umi.as<uint64_t>(), ctx->d_frag.as<uint32_t>(), n,
+           ctx->d_umi_table.as<unsigned long long>(), (uint32_t)((1u << slot_bits) - 1u), frag_bits, k0, v0, (unsigned long long*)(small + SW_FRAG_OR));
+    CK(cudaEventRecord(ctx->ev[EV_READ_SORT_BEGIN], ctx->st));
+    if (radix_sort_bits(k0, v0, k1, v1, n, 0, slot_bits + frag_bits, ctx->d_hist.as<uint32_t>(), ctx->d_scan.as<uint32_t>(), ctx->st)) {
+        std::swap(k0, k1); std::swap(v0, v1);
     }
-    CK(cudaEventRecord(ctx->ev[EV_PREP_DONE], ctx->st));
+    CK(cudaEventRecord(ctx->ev[EV_READ_SORT_DONE], ctx->st));
+    ctx->tm.read_sort_passes = (slot_bits + frag_bits + RS_MAX_BITS - 1) / RS_MAX_BITS;
+    const uint32_t* perm = v0;
+    CK(ctx->d_urank.ensure((size_t)n * 4)); CK(ctx->d_frank.ensure((size_t)n * 4));
+    CK(ctx->d_umi_of_urank.ensure((size_t)n * 8));
+    const int64_t nbt = (n + SCAN_TILE - 1) / SCAN_TILE;
+    uint32_t* scr = ctx->d_scan.as<uint32_t>();
+    CK(cudaMemsetAsync(scr, 0, (size_t)(2 * nbt + 8) * 4, ctx->st));
+    LAUNCH(k_rank_scan, (unsigned)nbt, SCAN_THREADS, 0, k0, frag_bits, n, ctx->d_umi.as<uint64_t>(), perm, ctx->d_urank.as<uint32_t>(),
+           ctx->d_frank.as<uint32_t>(), ctx->d_umi_of_urank.as<uint64_t>(), v1, reinterpret_cast<unsigned long long*>(scr + 2), scr, small + SW_N_UMI);
+    *inv = v1;
+    return SMC_OK;
+}
+
+// K1: per-read records, computed in BAM order (coalesced inputs) and stored at their sorted position
+static int read_prep(smc_ctx* ctx, const uint32_t* inv) {
+    const int64_t n = ctx->n_reads;
+    uint32_t* small = ctx->d_small.as<uint32_t>();
+    CK(ctx->d_recs.ensure((size_t)n * sizeof(ReadRec))); CK(ctx->d_grec.ensure((size_t)n * sizeof(GRec)));
+    CK(cudaMemsetAsync(small + SW_N_TILE_EVENTS, 0, 32, ctx->st));
+    PrepArgs P{};
+    P.n_reads = n; P.inv = inv; P.urank = ctx->d_urank.as<uint32_t>(); P.frank = ctx->d_frank.as<uint32_t>();
+    P.ref_id = ctx->d_ref_id.as<int32_t>(); P.pos = ctx->d_pos.as<int32_t>(); P.flag = ctx->d_flag.as<uint16_t>();
+    P.mapq = ctx->d_mapq.as<uint8_t>(); P.nm = ctx->d_nm.as<int32_t>(); P.l_seq = ctx->d_lseq.as<int32_t>();
+    P.seq_off = ctx->d_seq_off.as<int64_t>(); P.qual_off = ctx->d_qual_off.as<int64_t>(); P.cigar_off = ctx->d_cig_off.as<int64_t>();
+    P.n_cigar = ctx->d_ncig.as<uint16_t>(); P.cigar = ctx->d_cigar.as<uint32_t>();
+    if (ctx->has_store) { P.store_lo = ctx->d_store_lo.as<int32_t>(); P.store_len = ctx->d_store_len.as<int32_t>(); }
+    P.loci_key = ctx->d_loci_key.as<uint64_t>(); P.n_loci = ctx->n_loci;
+    P.minMQ = ctx->prm.minMQ; P.primerDist = ctx->prm.primerDist; P.mismatchThr = ctx->prm.mismatchThr;
+    P.recs = ctx->d_recs.as<ReadRec>(); P.grec = ctx->d_grec.as<GRec>(); P.gflags = small + SW_GFLAGS;
+    if (ctx->pipe_n > 1) {
+        CK(ctx->d_pipe_need.ensure((size_t)n));
+        P.pipe_need = ctx->d_pipe_need.as<uint8_t>(); P.pipe_n = (uint32_t)ctx->pipe_n;
+        P.pipe_seq_chunk = ctx->pipe_seq_chunk; P.pipe_qual_chunk = ctx->pipe_qual_chunk;
+        if (ctx->qual_bits != 8) { P.qual_poff = ctx->d_qual_poff.as<uint32_t>(); P.qual_bits = ctx->qual_bits; }
+        if (ctx->seq_bits == 2) P.seq_poff = ctx->d_seq_poff.as<uint32_t>();
+    }
+    CK(cudaEventRecord(ctx->ev[EV_READ_PREP_BEGIN], ctx->st));
+    LAUNCH(k_read_prep, nblk(n, 256), 256, 0, P);
+    CK(cudaEventRecord(ctx->ev[EV_READ_PREP_DONE], ctx->st));
+    ctx->tm.read_prep_bytes = n * (int64_t)(4 + 4 + 2 + 1 + 4 + 4 + 8 + 8 + 8 + 2 + (ctx->has_store ? 8 : 0) + 4 + sizeof(ReadRec) + sizeof(GRec)) + 4 * ctx->n_cigar_words;
+    return SMC_OK;
+}
+
+// The input checks only the device can make, from d_small words 0 .. SW_PACK_TOTALS + 4 as the read sort, k_read_prep and the
+// upload left them (w[i] = word i).
+static int check_device_inputs(smc_ctx* ctx, const uint32_t* w) {
+    const uint32_t gflags = w[SW_GFLAGS];
+    if (gflags & GF_BAD_READ) { ctx->err = "a read has l_seq or clip length > 65535 (unsupported)"; return SMC_E_LIMIT; }
+    if (gflags & GF_BAD_STORE) {
+        ctx->err = "stored window: store_lo must be even and >= 0, store_lo + store_len <= l_seq, reads with indels / clips inside must be "
+                   "stored whole, and every target base of a read must lie inside its window";
+        return SMC_E_ARG;
+    }
+    if (w[SW_FRAG_OR] | w[SW_FRAG_OR + 1]) { ctx->err = "frag_id must be a dense id (< n_reads), numbered by first appearance"; return SMC_E_ARG; }
+    const uint32_t* tot = w + SW_PACK_TOTALS;
+    if ((ctx->packed_seq && (int64_t)tot[ctx->seq_bits == 2 ? 4 : 0] != ctx->seq_bytes) || (ctx->packed_qual && (int64_t)tot[ctx->qual_bits != 8 ? 3 : 1] != ctx->qual_bytes) ||
+        (ctx->packed_cigar && (int64_t)tot[2] != ctx->n_cigar_words)) {
+        ctx->err = "packed payload (NULL offsets): seq_bytes / qual_bytes / n_cigar_words do not match the sums of (len+1)/2, len, n_cigar (len = store_len or l_seq)";
+        return SMC_E_ARG;
+    }
+    return SMC_OK;
+}
+
+// k_expand_scan into event buffers of ctx->ne_cap entries: events beyond them are not written, their total always is
+static int expand_tile_events(smc_ctx* ctx) {
+    const int64_t n = ctx->n_reads;
+    if (ctx->ne_cap > 0xfffffff0ll) ctx->ne_cap = 0xfffffff0ll;
+    CK(ctx->d_ek0.ensure((size_t)ctx->ne_cap * 8)); CK(ctx->d_ev0.ensure((size_t)ctx->ne_cap * 4));
+    const int64_t nbt = (n + SCAN_TILE - 1) / SCAN_TILE;
+    uint32_t* scr = ctx->d_scan.as<uint32_t>();
+    CK(cudaMemsetAsync(scr, 0, (size_t)(2 * nbt + 8) * 4, ctx->st));
+    LAUNCH(k_expand_scan, (unsigned)nbt, SCAN_THREADS, 0, ctx->d_recs.as<ReadRec>(), n, ctx->d_ek0.as<uint64_t>(), ctx->d_ev0.as<uint32_t>(),
+           (uint32_t)ctx->ne_cap, reinterpret_cast<unsigned long long*>(scr + 2), scr, ctx->d_small.as<uint32_t>() + SW_N_TILE_EVENTS);
+    return SMC_OK;
+}
+
+// K2b (first half): the (read x tile) events, written into buffers sized from the previous batch (or 4 per read).  The round
+// trip after them brings back their exact count, the barcode count and the device-side input checks; the first batch of a
+// shape whose events did not fit grows the buffers and writes them again.
+static int tile_events(smc_ctx* ctx) {
+    if (ctx->ne_cap < 4 * ctx->n_reads + 4096) ctx->ne_cap = 4 * ctx->n_reads + 4096;
+    if (const int rc = expand_tile_events(ctx)) return rc;
+    uint32_t w[SW_PACK_TOTALS + 5];
+    if (const int rc = read_back(ctx, w, ctx->d_small.p, sizeof(w))) return rc;
+    if (const int rc = check_device_inputs(ctx, w)) return rc;
+    ctx->tm.n_umi_groups = w[SW_N_UMI];
+    ctx->n_tile_events = w[SW_N_TILE_EVENTS];
+    if (ctx->n_tile_events <= ctx->ne_cap) return SMC_OK;
+    ctx->ne_cap = ctx->n_tile_events + ctx->n_tile_events / 8 + 4096;
+    return expand_tile_events(ctx);
+}
+
+// K2b: the events, stable sort by tile; first event and warp units of every tile; [eb, ee) of every unit, cut at barcode
+// boundaries
+static int sort_tiles(smc_ctx* ctx) {
+    const int64_t NE = ctx->n_tile_events;
+    const uint32_t n_tiles = (uint32_t)((ctx->n_loci + 31) / 32);
     CK(cudaEventRecord(ctx->ev[EV_EVENT_SORT_BEGIN], ctx->st));
-    // ---------------- K2b: (read x tile) events, stable sort by tile
-    const uint64_t* ev_key_sorted = nullptr; const uint32_t* ev_read_sorted = nullptr;
+    const uint64_t* ev_key_sorted = nullptr;
+    ctx->ev_read_sorted = nullptr;
     CK(ctx->d_tile_off.ensure((size_t)(n_tiles + 2) * 4)); CK(ctx->d_unit_cnt.ensure((size_t)(n_tiles + 2) * 4));
     CK(ctx->d_unit_off.ensure((size_t)(n_tiles + 2) * 4));
     if (NE > 0) {
@@ -890,7 +906,7 @@ extern "C" int smc_run_resident(smc_ctx* ctx) {
         int res = radix_sort_bits(ctx->d_ek0.as<uint64_t>(), ctx->d_ev0.as<uint32_t>(), ctx->d_ek1.as<uint64_t>(), ctx->d_ev1.as<uint32_t>(),
                                   NE, 0, tile_bits, ctx->d_hist.as<uint32_t>(), ctx->d_scan.as<uint32_t>(), ctx->st);
         ev_key_sorted = res ? ctx->d_ek1.as<uint64_t>() : ctx->d_ek0.as<uint64_t>();
-        ev_read_sorted = res ? ctx->d_ev1.as<uint32_t>() : ctx->d_ev0.as<uint32_t>();
+        ctx->ev_read_sorted = res ? ctx->d_ev1.as<uint32_t>() : ctx->d_ev0.as<uint32_t>();
     } else {
         CK(ctx->d_scan.ensure((size_t)scan_scratch_words((int64_t)n_tiles + 2) * 4 + 1024));
     }
@@ -899,41 +915,34 @@ extern "C" int smc_run_resident(smc_ctx* ctx) {
            ctx->d_unit_cnt.as<uint32_t>());
     exclusive_scan_u32(ctx->d_unit_cnt.as<uint32_t>(), ctx->d_unit_off.as<uint32_t>(), (int64_t)n_tiles + 1, ctx->d_scan.as<uint32_t>(),
                        nullptr, ctx->st);
-    {   // unit geometry: [eb, ee) of every unit, cut at barcode boundaries
-        const int64_t max_units = (int64_t)n_tiles + NE / ctx->chunk + 1;
-        ctx->n_units_cap = (uint32_t)max_units;
-        CK(ctx->d_unit_eb.ensure((size_t)max_units * 4)); CK(ctx->d_unit_ee.ensure((size_t)max_units * 4));
-        CK(ctx->d_unit_tile.ensure((size_t)max_units * 4)); CK(ctx->d_unit_nfrag.ensure((size_t)max_units * 4));
-        LAUNCH(k_unit_bounds, nblk(max_units, 256), 256, 0, ctx->d_tile_off.as<uint32_t>(), ctx->d_unit_off.as<uint32_t>(), n_tiles, ctx->chunk,
-               ev_read_sorted, ctx->d_urank.as<uint32_t>(), ctx->d_unit_eb.as<uint32_t>(), ctx->d_unit_ee.as<uint32_t>(), ctx->d_unit_tile.as<uint32_t>(),
-               ctx->n_units_cap);
-    }
-    ctx->tm.n_tile_events = NE;
-    ctx->ev_read_sorted = ev_read_sorted;
-    ctx->n_tiles = n_tiles; ctx->n_tile_events = NE;
-    (void)ev_key_sorted;
-    if (ctx->pipe_n > 1 && NE > 0) {
-        // which units may start after which chunk: a unit needs the latest chunk any of its reads needs (k_read_prep: pipe_need)
-        const int G = ctx->pipe_n;
-        uint32_t init[SMC_PIPE_MAX];
-        for (int c = 0; c < SMC_PIPE_MAX; ++c) init[c] = ctx->n_units_cap;
-        uint32_t* pd = small + SW_PIPE_BLOCKED;                      // first blocked unit per chunk
-        CK(cudaMemcpyAsync(pd, init, sizeof(init), cudaMemcpyHostToDevice, ctx->st));
-        LAUNCH(k_pipe_unit_need, nblk((int64_t)ctx->n_units_cap * 32, 256), 256, 0, ctx->d_unit_eb.as<uint32_t>(),
-               ctx->d_unit_ee.as<uint32_t>(), ev_read_sorted, ctx->d_pipe_need.as<uint8_t>(), ctx->n_units_cap, pd);
-        uint32_t h[SMC_PIPE_MAX];
-        CK(cudaMemcpyAsync(h, pd, sizeof(h), cudaMemcpyDeviceToHost, ctx->st));
-        CK(cudaStreamSynchronize(ctx->st));
-        uint32_t run = ctx->n_units_cap;
-        for (int c = G - 1; c >= 0; --c) {
-            if (c < G - 1) run = std::min(run, h[c]);
-            ctx->pipe_end[c] = run;
-        }
-    }
-    CK(cudaEventRecord(ctx->ev[EV_SORT_DONE], ctx->st));
-    return run_pileup_and_stats(ctx, n_tiles, NE);
+    const int64_t max_units = (int64_t)n_tiles + NE / ctx->chunk + 1;
+    ctx->n_units_cap = (uint32_t)max_units;
+    CK(ctx->d_unit_eb.ensure((size_t)max_units * 4)); CK(ctx->d_unit_ee.ensure((size_t)max_units * 4));
+    CK(ctx->d_unit_tile.ensure((size_t)max_units * 4)); CK(ctx->d_unit_nfrag.ensure((size_t)max_units * 4));
+    LAUNCH(k_unit_bounds, nblk(max_units, 256), 256, 0, ctx->d_tile_off.as<uint32_t>(), ctx->d_unit_off.as<uint32_t>(), n_tiles, ctx->chunk,
+           ctx->ev_read_sorted, ctx->d_urank.as<uint32_t>(), ctx->d_unit_eb.as<uint32_t>(), ctx->d_unit_ee.as<uint32_t>(),
+           ctx->d_unit_tile.as<uint32_t>(), ctx->n_units_cap);
+    return SMC_OK;
 }
 
+// Chunked upload: which units may start after which chunk.  A unit needs the latest chunk any of its reads needs (k_read_prep:
+// pipe_need); pipe_end[c] is the end of the units that chunks 0 .. c complete.
+static int plan_chunks(smc_ctx* ctx) {
+    const int G = ctx->pipe_n;
+    uint32_t init[SMC_PIPE_MAX], blocked[SMC_PIPE_MAX];
+    for (int c = 0; c < SMC_PIPE_MAX; ++c) init[c] = ctx->n_units_cap;
+    uint32_t* pd = ctx->d_small.as<uint32_t>() + SW_PIPE_BLOCKED;
+    CK(cudaMemcpyAsync(pd, init, sizeof(init), cudaMemcpyHostToDevice, ctx->st));
+    LAUNCH(k_pipe_unit_need, nblk((int64_t)ctx->n_units_cap * 32, 256), 256, 0, ctx->d_unit_eb.as<uint32_t>(),
+           ctx->d_unit_ee.as<uint32_t>(), ctx->ev_read_sorted, ctx->d_pipe_need.as<uint8_t>(), ctx->n_units_cap, pd);
+    if (const int rc = read_back(ctx, blocked, pd, sizeof(blocked))) return rc;
+    uint32_t run = ctx->n_units_cap;
+    for (int c = G - 1; c >= 0; --c) {
+        if (c < G - 1) run = std::min(run, blocked[c]);
+        ctx->pipe_end[c] = run;
+    }
+    return SMC_OK;
+}
 
 static DynTab make_dyntab(smc_ctx* ctx) {
     uint32_t* small = ctx->d_small.as<uint32_t>();
@@ -985,11 +994,38 @@ static void fill_kargs(smc_ctx* ctx, KAArgs& A, KBArgs& B, bool list, bool need_
     B.list_idx = nullptr;
 }
 
-static int run_pileup_and_stats(smc_ctx* ctx, uint32_t n_tiles, int64_t NE) {
-    NvtxRange nvtx_r("smc:pileup+stats");
-    const int64_t nl = ctx->n_loci;
+// k_gather + k_merge over units [0, n_units_cap): one pair, or for a chunked upload one pair per range [pipe_end[c-1],
+// pipe_end[c]) that starts once chunk c is in (after expanding its compact payload when `expand`).  `gather_done`, unless null,
+// is recorded between the kernels of the one pair, or after the last pair of a chunked run.
+template <bool LIST>
+static int launch_pileup(smc_ctx* ctx, KAArgs& A, KBArgs& B, bool chunked, bool expand, cudaEvent_t gather_done) {
+    if (chunked) ctx->tm.pipe_launches = 0;
+    uint32_t u0 = 0;
+    for (int c = 0; c < (chunked ? ctx->pipe_n : 1); ++c) {
+        if (chunked) {
+            CK(cudaStreamWaitEvent(ctx->st, ctx->ev_chunk[c], 0));
+            if (expand) expand_compact(ctx, c, UNPACK_GRID);
+        }
+        const uint32_t u1 = chunked ? ctx->pipe_end[c] : ctx->n_units_cap;
+        if (u1 <= u0) continue;
+        A.unit0 = B.unit0 = u0; A.n_units = B.n_units = u1;
+        LAUNCH(k_gather_t<LIST>, nblk(u1 - u0, KA_WARPS), KA_WARPS * 32, KA_SMEM_BYTES(LIST), A);
+        if (gather_done && !chunked) CK(cudaEventRecord(gather_done, ctx->st));
+        LAUNCH(k_merge_t<LIST>, nblk(u1 - u0, KB_WARPS), KB_WARPS * 32, KB_SMEM_BYTES, B);
+        u0 = u1;
+        if (chunked) ++ctx->tm.pipe_launches;
+    }
+    if (gather_done && chunked) CK(cudaEventRecord(gather_done, ctx->st));
+    return SMC_OK;
+}
+
+// K3: the pileup, into per-locus accumulators and a dynamic-allele table cleared for it.  The round trip after it brings back
+// the overflow flags: a pileup that overflowed the dynamic-allele table, the fragment-code storage or the spill pool runs again
+// with the one that overflowed grown.
+static int pileup(smc_ctx* ctx) {
+    NvtxRange nvtx_r("smc:pileup");
+    const size_t nlz = (size_t)(ctx->n_loci ? ctx->n_loci : 1);
     uint32_t* small = ctx->d_small.as<uint32_t>();
-    const size_t nlz = (size_t)(nl ? nl : 1);
     CK(ctx->d_loc.ensure(nlz * SMC_NLOC * 4)); CK(ctx->d_cnt.ensure(nlz * SMC_NFIXED * SMC_NCNT * 4));
     CK(ctx->d_limb.ensure(nlz * SMC_NFIXED * 3 * 8)); CK(ctx->d_pi.ensure(nlz * SMC_NFIXED * 8));
     CK(ctx->d_max.ensure(nlz * 4)); CK(ctx->d_second.ensure(nlz * 4)); CK(ctx->d_alt.ensure(nlz * 4));
@@ -998,14 +1034,14 @@ static int run_pileup_and_stats(smc_ctx* ctx, uint32_t n_tiles, int64_t NE) {
     CK(ctx->d_dyn_first.ensure((nlz + 2) * 4));
     if (ctx->dyn_cap == 0) {
         uint32_t want = 1u << 16;
-        while ((int64_t)want < 2 * nl && want < (1u << 28)) want <<= 1;
+        while ((int64_t)want < 2 * ctx->n_loci && want < (1u << 28)) want <<= 1;
         if (const char* ev = getenv("SMC_DYN_CAP0")) {            // test hook: start small to exercise the regrowth path
             long v = atol(ev);
             if (v >= 16 && v <= (1l << 28) && (v & (v - 1)) == 0) want = (uint32_t)v;
         }
         ctx->dyn_cap = want;
     }
-    for (int attempt = 0; attempt < 6; ++attempt) {
+    for (int attempt = 0;; ++attempt) {
         const uint32_t cap = ctx->dyn_cap;
         CK(ctx->d_dkey.ensure((size_t)cap * 8)); CK(ctx->d_drep_read.ensure((size_t)cap * 4)); CK(ctx->d_drep_qpos.ensure((size_t)cap * 4));
         CK(ctx->d_dlen.ensure((size_t)cap * 4)); CK(ctx->d_dcnt.ensure((size_t)cap * SMC_NCNT * 4)); CK(ctx->d_dlimb.ensure((size_t)cap * 24));
@@ -1025,83 +1061,71 @@ static int run_pileup_and_stats(smc_ctx* ctx, uint32_t n_tiles, int64_t NE) {
         }
         CK(ctx->d_spill.ensure((size_t)ctx->spill_cap * sizeof(SpillRec)));
         CK(cudaMemsetAsync(small + SW_SPILL_COUNT, 0, 4, ctx->st));
-        if (NE > 0) {
-            { int rc = ensure_code_storage(ctx, false, ctx->has_keep); if (rc) return rc; }
+        if (ctx->n_tile_events > 0) {
+            if (const int rc = ensure_code_storage(ctx, false, ctx->has_keep)) return rc;
             KAArgs A; KBArgs B;
             fill_kargs(ctx, A, B, false, ctx->has_keep);
             CK(cudaEventRecord(ctx->ev[EV_PILEUP_BEGIN], ctx->st));
-            if (ctx->pipe_n > 1) {
-                // pipelined upload: units [pipe_end[c-1], pipe_end[c]) start as soon as chunk c of the bases / qualities is in
-                uint32_t u0 = 0;
-                ctx->tm.pipe_launches = 0;
-                for (int c = 0; c < ctx->pipe_n; ++c) {
-                    CK(cudaStreamWaitEvent(ctx->st, ctx->ev_chunk[c], 0));
-                    if (attempt == 0) expand_compact(ctx, c, UNPACK_GRID);     // the reads completed by this chunk
-                    const uint32_t u1 = ctx->pipe_end[c];
-                    if (u1 <= u0) continue;
-                    A.unit0 = B.unit0 = u0; A.n_units = B.n_units = u1;
-                    LAUNCH(k_gather_t<false>, nblk(u1 - u0, KA_WARPS), KA_WARPS * 32, KA_SMEM_BYTES(false), A);
-                    LAUNCH(k_merge_t<false>, nblk(u1 - u0, KB_WARPS), KB_WARPS * 32, KB_SMEM_BYTES, B);
-                    u0 = u1; ++ctx->tm.pipe_launches;
-                }
-                CK(cudaEventRecord(ctx->ev[EV_GATHER_DONE], ctx->st));
-            } else {
-                LAUNCH(k_gather_t<false>, nblk(ctx->n_units_cap, KA_WARPS), KA_WARPS * 32, KA_SMEM_BYTES(false), A);
-                CK(cudaEventRecord(ctx->ev[EV_GATHER_DONE], ctx->st));
-                LAUNCH(k_merge_t<false>, nblk(ctx->n_units_cap, KB_WARPS), KB_WARPS * 32, KB_SMEM_BYTES, B);
-            }
+            if (const int rc = launch_pileup<false>(ctx, A, B, ctx->pipe_n > 1, attempt == 0, ctx->ev[EV_GATHER_DONE])) return rc;
             CK(cudaEventRecord(ctx->ev[EV_MERGE_DONE], ctx->st));
         }
-        uint32_t h[3];
-        CK(cudaMemcpyAsync(h, small + SW_GFLAGS, 12, cudaMemcpyDeviceToHost, ctx->st));
-        CK(cudaStreamSynchronize(ctx->st));
+        uint32_t w[2];                                               // d_small words SW_GFLAGS, SW_DYN_COUNT
+        if (const int rc = read_back(ctx, w, small + SW_GFLAGS, sizeof(w))) return rc;
         CK(cudaGetLastError());
-        if (!(h[0] & (GF_DYN_FULL | GF_CODE_FULL | GF_SPILL_FULL))) { ctx->n_dyn = h[1]; break; }
-        if (h[0] & GF_SPILL_FULL) ctx->spill_cap = ctx->spill_cap >= (1u << 24) ? ctx->spill_cap : ctx->spill_cap * 4;
+        const uint32_t gflags = w[0];
+        if (!(gflags & (GF_DYN_FULL | GF_CODE_FULL | GF_SPILL_FULL))) { ctx->n_dyn = w[1]; return SMC_OK; }
+        if (gflags & GF_SPILL_FULL) ctx->spill_cap = ctx->spill_cap >= (1u << 24) ? ctx->spill_cap : ctx->spill_cap * 4;
         if (attempt == 5) { ctx->err = "dynamic allele table / fragment code storage overflow"; return SMC_E_OVERFLOW; }
-        if (h[0] & GF_CODE_FULL) ctx->code_mult = 3;             // worst-case layout: always fits
-        if (h[0] & GF_DYN_FULL) {
+        if (gflags & GF_CODE_FULL) ctx->code_mult = 3;             // worst-case layout: always fits
+        if (gflags & GF_DYN_FULL) {
             if (ctx->dyn_cap >= (1u << 28)) { ctx->err = "dynamic allele table overflow"; return SMC_E_OVERFLOW; }
             ctx->dyn_cap <<= 2;
         }
     }
-    CK(cudaEventRecord(ctx->ev[EV_PILEUP_DONE], ctx->st));
-    NvtxRange nvtx_s("smc:dyn_rows+call+fisher");
-    // ---------------- dynamic alleles -> sorted rows
-    const int64_t nd = ctx->n_dyn;
-    const size_t ndz = (size_t)(nd ? nd : 1);
+}
+
+// Dynamic alleles -> rows grouped by locus, ordered by key inside a locus
+static int dyn_rows(smc_ctx* ctx) {
+    NvtxRange nvtx_r("smc:dyn_rows");
+    const int64_t nl = ctx->n_loci, nd = ctx->n_dyn;
+    const size_t nlz = (size_t)(nl ? nl : 1), ndz = (size_t)(nd ? nd : 1);
     CK(ctx->d_s_key.ensure(ndz * 8)); CK(ctx->d_s_cnt.ensure(ndz * SMC_NCNT * 4)); CK(ctx->d_s_limb.ensure(ndz * 24));
     CK(ctx->d_s_iskey.ensure(ndz)); CK(ctx->d_s_pi.ensure(ndz * 8)); CK(ctx->d_s_rep_read.ensure(ndz * 4));
     CK(ctx->d_s_rep_qpos.ensure(ndz * 4)); CK(ctx->d_s_len.ensure(ndz * 4));
     CK(cudaMemsetAsync(ctx->d_dyn_first.p, 0, (nlz + 2) * 4, ctx->st));
-    if (nd > 0) {
-        CK(ctx->d_lk0.ensure(ndz * 8)); CK(ctx->d_lv0.ensure(ndz * 4)); CK(ctx->d_lv1.ensure((nlz + 2) * 4));
-        CK(ctx->d_scan.ensure((size_t)scan_scratch_words((int64_t)nl + 2) * 4 + 1024));
-        uint32_t* first = ctx->d_dyn_first.as<uint32_t>();
-        uint32_t* cursor = ctx->d_lv1.as<uint32_t>();
-        CK(cudaMemsetAsync(cursor, 0, (nlz + 2) * 4, ctx->st));
-        LAUNCH(k_dyn_count, nblk(ctx->dyn_cap, 256), 256, 0, ctx->d_dkey.as<unsigned long long>(), ctx->dyn_cap, first);
-        exclusive_scan_u32(first, first, nl + 1, ctx->d_scan.as<uint32_t>(), nullptr, ctx->st);
-        LAUNCH(k_dyn_place, nblk(ctx->dyn_cap, 256), 256, 0, ctx->d_dkey.as<unsigned long long>(), ctx->dyn_cap, first, cursor,
-               ctx->d_lk0.as<uint64_t>(), ctx->d_lv0.as<uint32_t>());
-        LAUNCH(k_dyn_sort_local, nblk(nl, 256), 256, 0, first, nl, ctx->d_lk0.as<uint64_t>(), ctx->d_lv0.as<uint32_t>());
-        LAUNCH(k_dyn_gather, nblk(nd, 128), 128, 0, ctx->d_lk0.as<uint64_t>(), ctx->d_lv0.as<uint32_t>(), nd, ctx->d_dcnt.as<int32_t>(),
-               ctx->d_dlimb.as<unsigned long long>(),
-               ctx->d_diskey.as<uint8_t>(), ctx->d_drep_read.as<uint32_t>(), ctx->d_drep_qpos.as<int32_t>(), ctx->d_dlen.as<int32_t>(),
-               ctx->d_s_key.as<unsigned long long>(), ctx->d_s_cnt.as<int32_t>(), ctx->d_s_limb.as<unsigned long long>(),
-               ctx->d_s_iskey.as<uint8_t>(), ctx->d_s_rep_read.as<uint32_t>(), ctx->d_s_rep_qpos.as<int32_t>(), ctx->d_s_len.as<int32_t>());
-    }
-    // ---------------- K4
-    uint32_t n_tasks_h = 0;
-    unsigned long long cvgsum = 0;
-    for (int attempt = 0; attempt < 2; ++attempt) {
+    if (nd == 0) return SMC_OK;
+    CK(ctx->d_lk0.ensure(ndz * 8)); CK(ctx->d_lv0.ensure(ndz * 4)); CK(ctx->d_lv1.ensure((nlz + 2) * 4));
+    CK(ctx->d_scan.ensure((size_t)scan_scratch_words((int64_t)nl + 2) * 4 + 1024));
+    uint32_t* first = ctx->d_dyn_first.as<uint32_t>();
+    uint32_t* cursor = ctx->d_lv1.as<uint32_t>();
+    CK(cudaMemsetAsync(cursor, 0, (nlz + 2) * 4, ctx->st));
+    LAUNCH(k_dyn_count, nblk(ctx->dyn_cap, 256), 256, 0, ctx->d_dkey.as<unsigned long long>(), ctx->dyn_cap, first);
+    exclusive_scan_u32(first, first, nl + 1, ctx->d_scan.as<uint32_t>(), nullptr, ctx->st);
+    LAUNCH(k_dyn_place, nblk(ctx->dyn_cap, 256), 256, 0, ctx->d_dkey.as<unsigned long long>(), ctx->dyn_cap, first, cursor,
+           ctx->d_lk0.as<uint64_t>(), ctx->d_lv0.as<uint32_t>());
+    LAUNCH(k_dyn_sort_local, nblk(nl, 256), 256, 0, first, nl, ctx->d_lk0.as<uint64_t>(), ctx->d_lv0.as<uint32_t>());
+    LAUNCH(k_dyn_gather, nblk(nd, 128), 128, 0, ctx->d_lk0.as<uint64_t>(), ctx->d_lv0.as<uint32_t>(), nd, ctx->d_dcnt.as<int32_t>(),
+           ctx->d_dlimb.as<unsigned long long>(),
+           ctx->d_diskey.as<uint8_t>(), ctx->d_drep_read.as<uint32_t>(), ctx->d_drep_qpos.as<int32_t>(), ctx->d_dlen.as<int32_t>(),
+           ctx->d_s_key.as<unsigned long long>(), ctx->d_s_cnt.as<int32_t>(), ctx->d_s_limb.as<unsigned long long>(),
+           ctx->d_s_iskey.as<uint8_t>(), ctx->d_s_rep_read.as<uint32_t>(), ctx->d_s_rep_qpos.as<int32_t>(), ctx->d_s_len.as<int32_t>());
+    return SMC_OK;
+}
+
+// K4: k_call (PI, ALT, filters, Fisher task list), k_fisher, and the sum of cvg.  The round trip after them brings back the task
+// count: a list longer than its buffer is grown and the three kernels run once more.
+static int call_stats(smc_ctx* ctx) {
+    NvtxRange nvtx_r("smc:call+fisher");
+    const int64_t nl = ctx->n_loci;
+    uint32_t* small = ctx->d_small.as<uint32_t>();
+    for (int attempt = 0;; ++attempt) {
         if (ctx->task_cap == 0) ctx->task_cap = 1u << 13;
         CK(ctx->d_tasks.ensure((size_t)ctx->task_cap * sizeof(FisherTask)));
         CK(cudaMemsetAsync(small + SW_N_TASKS, 0, 4, ctx->st));
         K4Args B{};
         B.n_loci = nl; B.ref_base = ctx->d_loci_base.as<uint8_t>(); B.loc = ctx->d_loc.as<int32_t>(); B.cnt = ctx->d_cnt.as<int32_t>();
         B.limb = ctx->d_limb.as<unsigned long long>(); B.pi = ctx->d_pi.as<double>();
-        B.n_dyn = nd; B.dyn_key = ctx->d_s_key.as<unsigned long long>(); B.dyn_cnt = ctx->d_s_cnt.as<int32_t>();
+        B.n_dyn = ctx->n_dyn; B.dyn_key = ctx->d_s_key.as<unsigned long long>(); B.dyn_cnt = ctx->d_s_cnt.as<int32_t>();
         B.dyn_limb = ctx->d_s_limb.as<unsigned long long>(); B.dyn_iskey = ctx->d_s_iskey.as<uint8_t>(); B.dyn_pi = ctx->d_s_pi.as<double>();
         B.dyn_first = ctx->d_dyn_first.as<uint32_t>();
         B.keep_idx = ctx->has_keep ? ctx->d_keep_idx.as<int32_t>() : nullptr;
@@ -1112,45 +1136,95 @@ static int run_pileup_and_stats(smc_ctx* ctx, uint32_t n_tiles, int64_t NE) {
         B.fisher_or = ctx->d_for.as<double>(); B.tasks = ctx->d_tasks.as<FisherTask>(); B.n_tasks = small + SW_N_TASKS; B.task_cap = ctx->task_cap;
         LAUNCH(k_call, nblk(nl, 128), 128, 0, B);
         // k_fisher reads the task count on the device: launched for the whole task buffer (idle threads leave at once), so
-        // that no host round trip sits between the two kernels; an overflowing task list is noticed at the final sync
+        // that no host round trip sits between the two kernels; an overflowing task list is noticed at the round trip below
         LAUNCH(k_fisher, nblk((int64_t)ctx->task_cap * 32, 128), 128, 0, ctx->d_tasks.as<FisherTask>(), small + SW_N_TASKS, ctx->task_cap, nl, (int)ctx->prm.fisherLegacy,
                ctx->d_fp.as<double>(), ctx->d_for.as<double>(), ctx->d_fl1.as<uint32_t>(), ctx->d_fl2.as<uint32_t>());
         CK(cudaMemsetAsync(small + SW_CVG_SUM, 0, 8, ctx->st));
         LAUNCH(k_sum_cvg, std::min<unsigned>(nblk(nl, 256), 592u), 256, 0, ctx->d_loc.as<int32_t>() + (size_t)SMC_L_CVG * nl, nl,
                (unsigned long long*)(small + SW_CVG_SUM));
         CK(cudaEventRecord(ctx->ev[EV_STATS_DONE], ctx->st));
-        CK(cudaMemcpyAsync(&n_tasks_h, small + SW_N_TASKS, 4, cudaMemcpyDeviceToHost, ctx->st));
-        CK(cudaMemcpyAsync(&cvgsum, small + SW_CVG_SUM, 8, cudaMemcpyDeviceToHost, ctx->st));
-        CK(cudaStreamSynchronize(ctx->st));
+        uint32_t w[3];                                               // d_small words SW_N_TASKS, SW_CVG_SUM (u64)
+        if (const int rc = read_back(ctx, w, small + SW_N_TASKS, sizeof(w))) return rc;
         CK(cudaGetLastError());
-        if (n_tasks_h <= ctx->task_cap) break;
+        const uint32_t n_tasks = w[0];
+        if (n_tasks <= ctx->task_cap) {
+            ctx->tm.n_fisher = n_tasks;
+            ctx->tm.n_pileup_events = (int64_t)(w[1] | (uint64_t)w[2] << 32);
+            return SMC_OK;
+        }
         if (attempt == 1) { ctx->err = "Fisher task list overflow"; return SMC_E_OVERFLOW; }
-        ctx->task_cap = n_tasks_h + n_tasks_h / 4 + 1024;      // grow and redo the (cheap) call kernel
+        ctx->task_cap = n_tasks + n_tasks / 4 + 1024;                // grow and redo the (cheap) call kernel
     }
-    cudaEventElapsedTime(&ctx->tm.ms_prep, ctx->ev[EV_RUN_BEGIN], ctx->ev[EV_PREP_DONE]);
-    cudaEventElapsedTime(&ctx->tm.ms_sort, ctx->ev[EV_PREP_DONE], ctx->ev[EV_SORT_DONE]);
-    cudaEventElapsedTime(&ctx->tm.ms_pileup, ctx->ev[EV_SORT_DONE], ctx->ev[EV_PILEUP_DONE]);
-    cudaEventElapsedTime(&ctx->tm.ms_stats, ctx->ev[EV_PILEUP_DONE], ctx->ev[EV_STATS_DONE]);
-    cudaEventElapsedTime(&ctx->tm.ms_total_device, ctx->ev[EV_RUN_BEGIN], ctx->ev[EV_STATS_DONE]);
-    ctx->tm.ms_read_sort = ctx->tm.ms_k_read_prep = ctx->tm.ms_event_sort = 0.f;
-    if (ctx->n_reads > 0 && nl > 0) {
-        cudaEventElapsedTime(&ctx->tm.ms_read_sort, ctx->ev[EV_READ_SORT_BEGIN], ctx->ev[EV_READ_SORT_DONE]);
-        cudaEventElapsedTime(&ctx->tm.ms_k_read_prep, ctx->ev[EV_READ_PREP_BEGIN], ctx->ev[EV_READ_PREP_DONE]);
+}
+
+// smc_timings of the run: the stage times from the events the stages that ran recorded, and the work counts
+static void record_timings(smc_ctx* ctx) {
+    smc_timings& t = ctx->tm;
+    auto ms = [ctx](float* out, StageEvent from, StageEvent to) { cudaEventElapsedTime(out, ctx->ev[from], ctx->ev[to]); };
+    ms(&t.ms_prep, EV_RUN_BEGIN, EV_PREP_DONE);
+    ms(&t.ms_sort, EV_PREP_DONE, EV_SORT_DONE);
+    ms(&t.ms_pileup, EV_SORT_DONE, EV_PILEUP_DONE);
+    ms(&t.ms_stats, EV_PILEUP_DONE, EV_STATS_DONE);
+    ms(&t.ms_total_device, EV_RUN_BEGIN, EV_STATS_DONE);
+    ms(&t.ms_event_sort, EV_EVENT_SORT_BEGIN, EV_EVENT_SORT_DONE);
+    t.ms_read_sort = t.ms_k_read_prep = 0.f;
+    if (ctx->n_reads > 0 && ctx->n_loci > 0) {
+        ms(&t.ms_read_sort, EV_READ_SORT_BEGIN, EV_READ_SORT_DONE);
+        ms(&t.ms_k_read_prep, EV_READ_PREP_BEGIN, EV_READ_PREP_DONE);
     }
-    cudaEventElapsedTime(&ctx->tm.ms_event_sort, ctx->ev[EV_EVENT_SORT_BEGIN], ctx->ev[EV_EVENT_SORT_DONE]);
-    ctx->tm.ms_k_pileup = ctx->tm.ms_k_gather = ctx->tm.ms_k_merge = 0.f;
-    if (NE > 0) {
-        cudaEventElapsedTime(&ctx->tm.ms_k_pileup, ctx->ev[EV_PILEUP_BEGIN], ctx->ev[EV_MERGE_DONE]);
-        cudaEventElapsedTime(&ctx->tm.ms_k_gather, ctx->ev[EV_PILEUP_BEGIN], ctx->ev[EV_GATHER_DONE]);
-        cudaEventElapsedTime(&ctx->tm.ms_k_merge, ctx->ev[EV_GATHER_DONE], ctx->ev[EV_MERGE_DONE]);
+    t.ms_k_pileup = t.ms_k_gather = t.ms_k_merge = 0.f;
+    if (ctx->n_tile_events > 0) {
+        ms(&t.ms_k_pileup, EV_PILEUP_BEGIN, EV_MERGE_DONE);
+        ms(&t.ms_k_gather, EV_PILEUP_BEGIN, EV_GATHER_DONE);
+        ms(&t.ms_k_merge, EV_GATHER_DONE, EV_MERGE_DONE);
     }
-    ctx->tm.n_pileup_events = (int64_t)cvgsum;
-    ctx->tm.n_dyn = nd; ctx->tm.n_fisher = n_tasks_h;
-    ctx->tm.kernel_launches = g_launches;
-    ctx->tm.code_mult = (int32_t)ctx->code_mult; ctx->tm.dyn_capacity = (int32_t)ctx->dyn_cap;
+    t.n_tile_events = ctx->n_tile_events;
+    t.n_dyn = ctx->n_dyn;
+    t.kernel_launches = g_launches;
+    t.code_mult = (int32_t)ctx->code_mult; t.dyn_capacity = (int32_t)ctx->dyn_cap;
+}
+
+// One batch run of the resident upload, stage by stage.  Host round trips: after the tile events (their count and the
+// device-side input checks), after the chunk plan (chunked uploads only), after the pileup and after the statistics; the
+// tile events, the pileup and the statistics run once more when one of their buffers turned out too small.
+extern "C" int smc_run_resident(smc_ctx* ctx) {
+    if (!ctx) return SMC_E_ARG;
+    if (!ctx->uploaded) { ctx->err = "smc_run_resident: nothing uploaded"; return SMC_E_STATE; }
+    CK(cudaSetDevice(ctx->device));
+    g_launches = 0;
+    ctx->n_tile_events = 0;
+    CK(cudaEventRecord(ctx->ev[EV_RUN_BEGIN], ctx->st));
+    if (ctx->n_reads > 0 && ctx->n_loci > 0) {
+        NvtxRange nvtx_r("smc:read_sort+prep+tile_events");
+        const uint32_t* inv = nullptr;
+        if (const int rc = read_sort(ctx, &inv)) return rc;
+        if (const int rc = read_prep(ctx, inv)) return rc;
+        if (const int rc = tile_events(ctx)) return rc;
+    }
+    CK(cudaEventRecord(ctx->ev[EV_PREP_DONE], ctx->st));
+    if (const int rc = sort_tiles(ctx)) return rc;
+    if (ctx->pipe_n > 1 && ctx->n_tile_events > 0)
+        if (const int rc = plan_chunks(ctx)) return rc;
+    CK(cudaEventRecord(ctx->ev[EV_SORT_DONE], ctx->st));
+    if (const int rc = pileup(ctx)) return rc;
+    CK(cudaEventRecord(ctx->ev[EV_PILEUP_DONE], ctx->st));
+    if (const int rc = dyn_rows(ctx)) return rc;
+    if (const int rc = call_stats(ctx)) return rc;
+    record_timings(ctx);
     ctx->ran = true;
     return SMC_OK;
 }
+
+// Device -> host copies of one download; an output array the caller left NULL is skipped.
+struct Download {
+    smc_ctx* ctx;
+    int64_t bytes = 0;          // bytes copied (smc_timings::bytes_d2h)
+    template <class T> cudaError_t copy(T* dst, const DevBuf& src, size_t count) {
+        if (!dst || count == 0) return cudaSuccess;
+        bytes += (int64_t)(count * sizeof(T));
+        return cudaMemcpyAsync(dst, src.p, count * sizeof(T), cudaMemcpyDeviceToHost, ctx->st);
+    }
+};
 
 extern "C" int smc_download(smc_ctx* ctx, smc_out* out) {
     if (!ctx) return SMC_E_ARG;
@@ -1162,28 +1236,20 @@ extern "C" int smc_download(smc_ctx* ctx, smc_out* out) {
     out->n_dyn = nd;
     if (nd > out->dyn_capacity) { ctx->err = "smc_download: dyn_capacity too small (n_dyn reported in smc_out.n_dyn)"; return SMC_E_LIMIT; }
     NvtxRange nvtx_r("smc:download");
-    int64_t bytes = 0;
+    Download down{ctx};
     CK(cudaEventRecord(ctx->ev[EV_COPY_BEGIN], ctx->st));
-#define DOWN(dst, buf, count, T)                                                                                \
-    do {                                                                                                        \
-        size_t b__ = (size_t)(count) * sizeof(T);                                                               \
-        if (b__ && (dst)) { CK(cudaMemcpyAsync((dst), (buf).p, b__, cudaMemcpyDeviceToHost, ctx->st)); bytes += b__; } \
-    } while (0)
-    DOWN(out->loc, ctx->d_loc, nl * SMC_NLOC, int32_t); DOWN(out->cnt, ctx->d_cnt, nl * SMC_NFIXED * SMC_NCNT, int32_t);
-    DOWN(out->pi, ctx->d_pi, nl * SMC_NFIXED, double); DOWN(out->max_allele, ctx->d_max, nl, int32_t);
-    DOWN(out->second_allele, ctx->d_second, nl, int32_t); DOWN(out->alt_allele, ctx->d_alt, nl, int32_t);
-    DOWN(out->alt_pi, ctx->d_altpi, nl, double); DOWN(out->second_pi, ctx->d_secondpi, nl, double);
-    DOWN(out->fl1, ctx->d_fl1, nl, uint32_t); DOWN(out->fl2, ctx->d_fl2, nl, uint32_t); DOWN(out->biallelic, ctx->d_bial, nl, uint8_t);
-    DOWN(out->fisher_p, ctx->d_fp, nl * 8, double); DOWN(out->fisher_or, ctx->d_for, nl * 8, double);
-    DOWN(out->dyn_cnt, ctx->d_s_cnt, (size_t)nd * SMC_NCNT, int32_t); DOWN(out->dyn_pi, ctx->d_s_pi, nd, double);
-    DOWN(out->dyn_iskey, ctx->d_s_iskey, nd, uint8_t); DOWN(out->dyn_rep_read, ctx->d_s_rep_read, nd, uint32_t);
-    DOWN(out->dyn_rep_qpos, ctx->d_s_rep_qpos, nd, int32_t); DOWN(out->dyn_len, ctx->d_s_len, nd, int32_t);
-#undef DOWN
+    CK(down.copy(out->loc, ctx->d_loc, nl * SMC_NLOC)); CK(down.copy(out->cnt, ctx->d_cnt, nl * SMC_NFIXED * SMC_NCNT));
+    CK(down.copy(out->pi, ctx->d_pi, nl * SMC_NFIXED)); CK(down.copy(out->max_allele, ctx->d_max, nl));
+    CK(down.copy(out->second_allele, ctx->d_second, nl)); CK(down.copy(out->alt_allele, ctx->d_alt, nl));
+    CK(down.copy(out->alt_pi, ctx->d_altpi, nl)); CK(down.copy(out->second_pi, ctx->d_secondpi, nl));
+    CK(down.copy(out->fl1, ctx->d_fl1, nl)); CK(down.copy(out->fl2, ctx->d_fl2, nl)); CK(down.copy(out->biallelic, ctx->d_bial, nl));
+    CK(down.copy(out->fisher_p, ctx->d_fp, nl * 8)); CK(down.copy(out->fisher_or, ctx->d_for, nl * 8));
+    CK(down.copy(out->dyn_cnt, ctx->d_s_cnt, (size_t)nd * SMC_NCNT)); CK(down.copy(out->dyn_pi, ctx->d_s_pi, nd));
+    CK(down.copy(out->dyn_iskey, ctx->d_s_iskey, nd)); CK(down.copy(out->dyn_rep_read, ctx->d_s_rep_read, nd));
+    CK(down.copy(out->dyn_rep_qpos, ctx->d_s_rep_qpos, nd)); CK(down.copy(out->dyn_len, ctx->d_s_len, nd));
     std::vector<unsigned long long> keys((size_t)nd);
     std::vector<uint32_t> first(nl + 1);
-    if (nd) CK(cudaMemcpyAsync(keys.data(), ctx->d_s_key.p, (size_t)nd * 8, cudaMemcpyDeviceToHost, ctx->st));
-    CK(cudaMemcpyAsync(first.data(), ctx->d_dyn_first.p, (nl + 1) * 4, cudaMemcpyDeviceToHost, ctx->st));
-    bytes += nd * 8 + (int64_t)(nl + 1) * 4;
+    CK(down.copy(keys.data(), ctx->d_s_key, nd)); CK(down.copy(first.data(), ctx->d_dyn_first, nl + 1));
     CK(cudaEventRecord(ctx->ev[EV_COPY_END], ctx->st));
     CK(cudaStreamSynchronize(ctx->st));
     for (int64_t j = 0; j < nd; ++j) {
@@ -1194,7 +1260,7 @@ extern "C" int smc_download(smc_ctx* ctx, smc_out* out) {
     }
     if (out->dyn_first) for (size_t i = 0; i <= nl; ++i) out->dyn_first[i] = first[i];
     cudaEventElapsedTime(&ctx->tm.ms_d2h, ctx->ev[EV_COPY_BEGIN], ctx->ev[EV_COPY_END]);
-    ctx->tm.bytes_d2h = bytes;
+    ctx->tm.bytes_d2h = down.bytes;
     return SMC_OK;
 }
 
@@ -1267,7 +1333,8 @@ extern "C" int smc_list_barcodes(smc_ctx* ctx, int64_t n, const int64_t* locus, 
     CK(cudaSetDevice(ctx->device));
     const int64_t nl = ctx->n_loci;
     std::vector<int32_t> nbc((size_t)(nl ? nl : 1));
-    if (nl) CK(cudaMemcpy(nbc.data(), ctx->d_loc.as<int32_t>() + (size_t)SMC_L_NBC * nl, (size_t)nl * 4, cudaMemcpyDeviceToHost));
+    if (nl)
+        if (const int rc = read_back(ctx, nbc.data(), ctx->d_loc.as<int32_t>() + (size_t)SMC_L_NBC * nl, (size_t)nl * 4)) return rc;
     std::vector<int32_t> idx((size_t)(nl ? nl : 1), -1);
     off_out[0] = 0;
     for (int64_t k = 0; k < n; ++k) {
@@ -1290,15 +1357,14 @@ extern "C" int smc_list_barcodes(smc_ctx* ctx, int64_t n, const int64_t* locus, 
     // The listing pass re-runs the pileup kernel; it adds to the accumulators again, so the batch must be re-run
     // (with the mask) before the next download.
     ctx->ran = false;
-    { int rc = ensure_code_storage(ctx, true, true); if (rc) return rc; }
+    if (const int rc = ensure_code_storage(ctx, true, true)) return rc;
     KAArgs A; KBArgs B;
     fill_kargs(ctx, A, B, true, true);
     B.keep_idx = nullptr;
     B.list_idx = ctx->d_list_idx.as<int32_t>(); B.list_count = ctx->d_list_count.as<uint32_t>();
     B.list_off = ctx->d_list_off.as<int64_t>(); B.list_umi = ctx->d_list_umi.as<uint64_t>();
     B.list_first = ctx->d_list_first.as<uint32_t>(); B.list_cap = total;
-    LAUNCH(k_gather_t<true>, nblk(ctx->n_units_cap, KA_WARPS), KA_WARPS * 32, KA_SMEM_BYTES(true), A);
-    LAUNCH(k_merge_t<true>, nblk(ctx->n_units_cap, KB_WARPS), KB_WARPS * 32, KB_SMEM_BYTES, B);
+    if (const int rc = launch_pileup<true>(ctx, A, B, false, false, nullptr)) return rc;
     CK(cudaMemcpyAsync(umi_out, ctx->d_list_umi.p, (size_t)total * 8, cudaMemcpyDeviceToHost, ctx->st));
     CK(cudaMemcpyAsync(first_read_out, ctx->d_list_first.p, (size_t)total * 4, cudaMemcpyDeviceToHost, ctx->st));
     CK(cudaStreamSynchronize(ctx->st));

@@ -7,7 +7,7 @@ import numpy as np
 
 from oracle import smcounter_oracle as orc
 from smcounter_b200 import _ffi
-from smcounter_b200.caller import GpuCaller, UmiKeep, VcParams
+from smcounter_b200.caller import GpuCaller, LocusResults, UmiKeep, VcParams
 from smcounter_b200.rows import AlleleNamer, device_hp_flags, format_rows
 from smcounter_b200.soa import soa_to_records
 from smcounter_b200.synth import SynthSpec, make_panel
@@ -51,6 +51,23 @@ def rel_err(a, b):
     if math.isinf(a) or math.isinf(b) or math.isnan(a) or math.isnan(b):
         return float("inf")
     return abs(a - b) / max(abs(a), abs(b))
+
+
+def result_arrays(res: LocusResults) -> dict:
+    """Every output array of a call, dynamic-allele rows cut to n_dyn, for comparing two calls bit for bit."""
+    # the representative-read handles of dynamic alleles name whichever read reached the device table first
+    skip = ("dyn_rep_read", "dyn_rep_qpos")
+    out = {k: v[: res.n_dyn] if k.startswith("dyn_") and k != "dyn_first" else v
+           for k, v in res.__dict__.items() if isinstance(v, np.ndarray) and k not in skip}
+    out["n_dyn"] = np.array([res.n_dyn])
+    return out
+
+
+def assert_same_results(a: LocusResults, b: LocusResults):
+    ra, rb = result_arrays(a), result_arrays(b)
+    assert ra.keys() == rb.keys()
+    for k in ra:
+        assert np.array_equal(ra[k], rb[k], equal_nan=ra[k].dtype.kind == "f"), k
 
 
 def diff_details(res, loci, bed_order, details, soa, refs, max_report=20):

@@ -8,6 +8,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
+from helpers import assert_same_results
 from smcounter_b200 import _ffi
 from smcounter_b200.caller import GpuCaller, LocusResults, VcParams
 from smcounter_b200.synth import SynthSpec, make_panel
@@ -61,22 +62,6 @@ def panel():
     return soa.repack(), soa.trim_to_targets(IVS).compact(seq_bits_wanted=2), loci
 
 
-def _results(res: LocusResults) -> dict:
-    # the representative-read handles of dynamic alleles name whichever read reached the device table first
-    skip = ("dyn_rep_read", "dyn_rep_qpos")
-    out = {k: v[: res.n_dyn] if k.startswith("dyn_") and k != "dyn_first" else v
-           for k, v in res.__dict__.items() if isinstance(v, np.ndarray) and k not in skip}
-    out["n_dyn"] = np.array([res.n_dyn])
-    return out
-
-
-def _assert_same(a: LocusResults, b: LocusResults):
-    ra, rb = _results(a), _results(b)
-    assert ra.keys() == rb.keys()
-    for k in ra:
-        assert np.array_equal(ra[k], rb[k], equal_nan=ra[k].dtype.kind == "f"), k
-
-
 def _rejected(caller, rs, ls, entry):
     if entry == "smc_upload":
         return caller.lib.smc_upload(caller.h, C.byref(rs), C.byref(ls), None)
@@ -115,6 +100,6 @@ def test_rejected_batches_leave_the_context_usable(panel, entry, monkeypatch):
                 else:
                     got = caller.call(soa, loci)
                     assert caller.timings()["pipe_chunks"] == int(chunks)
-                _assert_same(got, want)
+                assert_same_results(got, want)
     finally:
         caller.close()
