@@ -33,7 +33,7 @@ SOA_HDR = os.path.join(HERE, "..", "include", "smc_soa.h")
 
 def build_bamio(force: bool = False) -> str:
     """Host-side BAM decoder (C++17, zlib, threads) -> libsmc_bamio.so."""
-    if not force and os.path.exists(BAMIO_OUT) and os.path.getmtime(BAMIO_OUT) >= max(os.path.getmtime(f) for f in (BAMIO_SRC, BAMIO_HDR, ROWS_SRC, ROWS_HDR, SOA_SRC, SOA_HDR, os.path.join(CSRC, "smc_inflate.h"))):
+    if not force and os.path.exists(BAMIO_OUT) and os.path.getmtime(BAMIO_OUT) >= max(os.path.getmtime(f) for f in (BAMIO_SRC, BAMIO_HDR, ROWS_SRC, ROWS_HDR, SOA_SRC, SOA_HDR, os.path.join(CSRC, "smc_inflate.h"), os.path.join(CSRC, "smc_host.h"))):
         return BAMIO_OUT
     cmd = [os.environ.get("CXX", "g++"), "-O2", "-std=c++17", "-shared", "-fPIC", "-pthread", "-o", BAMIO_OUT, BAMIO_SRC, ROWS_SRC, SOA_SRC, "-lz"]
     r = subprocess.run(cmd, capture_output=True, text=True)

@@ -9,11 +9,11 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
-#include <thread>
 #include <vector>
 
 #include "../../include/smc_b200.h"
 #include "../../include/smc_rows.h"
+#include "smc_host.h"
 
 namespace {
 
@@ -302,17 +302,9 @@ extern "C" int smc_rows_emit(const smc_rows_in* in, smc_rows_out* out) {
         C.trf.build(in->n_chroms, in->n_trf, in->trf_chrom, in->trf_lo, in->trf_hi);
         C.rm.build(in->n_chroms, in->n_rm, in->rm_chrom, in->rm_lo, in->rm_hi);
     }
-    int T = in->threads > 0 ? in->threads : (int)std::thread::hardware_concurrency();
-    if (T < 1) T = 1;
-    T = (int)std::min<int64_t>(T, std::max<int64_t>(1, in->n_rows / 2048));
+    const int T = (int)std::min<int64_t>(smc_host::n_threads(in->threads), std::max<int64_t>(1, in->n_rows / 2048));
     std::vector<Chunk> chunks((size_t)T);
-    std::vector<std::thread> th;
-    for (int t = 0; t < T; ++t) {
-        const int64_t r0 = in->n_rows * t / T, r1 = in->n_rows * (t + 1) / T;
-        if (T == 1) emit_range(C, r0, r1, chunks[0]);
-        else th.emplace_back([&C, &chunks, r0, r1, t]() { emit_range(C, r0, r1, chunks[(size_t)t]); });
-    }
-    for (auto& x : th) x.join();
+    smc_host::for_ranges((size_t)in->n_rows, T, [&](size_t r0, size_t r1, int t) { emit_range(C, (int64_t)r0, (int64_t)r1, chunks[(size_t)t]); });
     for (const Chunk& c : chunks)
         if (c.status != SMC_ROWS_OK) { out->bad_row = c.bad_row; out->bad_status = c.bad_status; return c.status; }
     auto gather = [&](std::string Chunk::*buf, std::vector<int64_t> Chunk::*lens, char*& dst, int64_t*& off) -> bool {

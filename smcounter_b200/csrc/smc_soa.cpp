@@ -3,50 +3,25 @@
 #include "../../include/smc_soa.h"
 
 #include <algorithm>
-#include <chrono>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <memory>
 #include <new>
-#include <thread>
 #include <vector>
+
+#include "smc_host.h"
+
+using smc_host::n_threads;
 
 namespace {
 
-template <class F> void par_for(size_t n, int threads, F f) {      // f(begin, end, thread)
-    if (threads <= 1 || n < 4096) { f(0, n, 0); return; }
-    std::vector<std::thread> ts;
-    const size_t per = (n + (size_t)threads - 1) / (size_t)threads;
-    for (int t = 0; t < threads; ++t) {
-        const size_t a = std::min(n, per * (size_t)t), e = std::min(n, a + per);
-        if (a >= e) break;
-        ts.emplace_back([=] { f(a, e, t); });
-    }
-    for (auto& th : ts) th.join();
+template <class F> void par_for(size_t n, int threads, F&& f) {    // f(begin, end, thread); inline below 4096 items
+    smc_host::for_ranges(n, n < 4096 ? 1 : threads, f);
 }
-
-template <class F> void par_each(int tasks, F f) {                  // f(task) for every task, one thread each
-    std::vector<std::thread> ts;
-    for (int t = 1; t < tasks; ++t) ts.emplace_back([=] { f(t); });
-    if (tasks > 0) f(0);
-    for (auto& th : ts) th.join();
-}
-
-int n_threads(int want) { return want > 0 ? want : (int)std::max(1u, std::thread::hardware_concurrency()); }
 
 struct Exc { uint32_t read, pos; uint8_t nib; };
 
-struct PhaseTimer {             // SMC_SOA_TIMING=1: phase times on stderr
-    bool on; std::chrono::steady_clock::time_point t;
-    PhaseTimer() : on(getenv("SMC_SOA_TIMING") != nullptr), t(std::chrono::steady_clock::now()) {}
-    void lap(const char* what) {
-        if (!on) return;
-        auto n = std::chrono::steady_clock::now();
-        fprintf(stderr, "[smc_soa] %-28s %.2f ms\n", what, std::chrono::duration<double, std::milli>(n - t).count());
-        t = n;
-    }
-};
+// SMC_SOA_TIMING=1: phase times on stderr
+smc_host::PhaseTimer phase_timer() { return smc_host::PhaseTimer("SMC_SOA_TIMING", "smc_soa"); }
 
 }  // namespace
 
@@ -148,7 +123,7 @@ extern "C" int smc_soa_pack_begin(const smc_soa_view* v, const int64_t* idx, int
     if (!h) return SMC_SOA_E_MEM;
     h->v = *v; h->idx = idx; h->n = idx ? n_idx : v->n_reads; h->o = *opts; h->threads = n_threads(opts->threads);
     const int64_t n = h->n;
-    PhaseTimer pt;
+    auto pt = phase_timer();
     try {
         h->seq_off.reset(new int64_t[(size_t)n + 1]); h->qual_off.reset(new int64_t[(size_t)n + 1]); h->cig_off.reset(new int64_t[(size_t)n + 1]);
         h->seq_off[0] = h->qual_off[0] = h->cig_off[0] = 0;      // the sizes pass writes every other entry
@@ -187,23 +162,20 @@ extern "C" int smc_soa_pack_begin(const smc_soa_view* v, const int64_t* idx, int
     {
         struct Tot { int64_t s, q, c; };
         std::vector<Tot> tot((size_t)T + 1, Tot{0, 0, 0});
-        const size_t per = ((size_t)n + (size_t)T - 1) / (size_t)T;
         const int tasks = (size_t)n < 65536 ? 1 : T;
-        par_each(tasks, [&](int ti) {
-            const size_t t = (size_t)ti, a = tasks == 1 ? 0 : std::min((size_t)n, per * t), e = tasks == 1 ? (size_t)n : std::min((size_t)n, a + per);
+        smc_host::for_ranges((size_t)n, tasks, [&](size_t a, size_t e, int t) {
             Tot run{0, 0, 0};
             for (size_t k = a; k < e; ++k) {
                 run.s += h->seq_off[k + 1]; run.q += h->qual_off[k + 1]; run.c += h->cig_off[k + 1];
                 h->seq_off[k + 1] = run.s; h->qual_off[k + 1] = run.q; h->cig_off[k + 1] = run.c;
             }
-            tot[t + 1] = run;
+            tot[(size_t)t + 1] = run;
         });
         for (int t = 0; t < tasks; ++t) { tot[(size_t)t + 1].s += tot[(size_t)t].s; tot[(size_t)t + 1].q += tot[(size_t)t].q; tot[(size_t)t + 1].c += tot[(size_t)t].c; }
         if (tasks > 1)
-            par_each(tasks, [&](int ti) {
-                if (ti == 0) return;
-                const size_t t = (size_t)ti, a = std::min((size_t)n, per * t), e = std::min((size_t)n, a + per);
-                const Tot b = tot[t];
+            smc_host::for_ranges((size_t)n, tasks, [&](size_t a, size_t e, int t) {
+                if (t == 0) return;
+                const Tot b = tot[(size_t)t];
                 for (size_t k = a; k < e; ++k) { h->seq_off[k + 1] += b.s; h->qual_off[k + 1] += b.q; h->cig_off[k + 1] += b.c; }
             });
     }
@@ -260,7 +232,7 @@ extern "C" int smc_soa_pack_fill(smc_soa_pack* h, const smc_soa_pack_bufs* B, sm
     code2[1] = 0; code2[2] = 1; code2[4] = 2; code2[8] = 3; plain[1] = plain[2] = plain[4] = plain[8] = 1;
     std::vector<std::vector<Exc>> excs((size_t)T);
     std::vector<int> bad((size_t)T, 0);
-    PhaseTimer pt;
+    auto pt = phase_timer();
     par_for((size_t)n, T, [&](size_t a, size_t e, int t) {
         std::vector<Exc>& ex = excs[(size_t)t];
         for (size_t k = a; k < e; ++k) {

@@ -394,6 +394,39 @@ def test_hand_built_corpus_indexed_equals_whole_file(tmp_path):
     check_indexed_equals_whole(path, ivs[::3], tmp_path, threads=(1, 4))
 
 
+# ---------------------------------------------------------------------------------------------------------------- 8: shared boundary
+def test_reads_without_reference_length_at_a_boundary_two_intervals_share(tmp_path):
+    """Mapped reads that consume no reference (CIGAR 10S, no CIGAR) around [1000, 1100) and [1100, 1200).  Such a read at p
+    touches an interval only when start < p < end, so the ones at 1000, 1100 and 1200 are dropped: the two intervals must not
+    act as one [1000, 1200).  The native decoder, whole file and indexed, equals the Python one, trimmed and untrimmed."""
+    q = lambda n: [30 + k % 7 for k in range(n)]
+    recs = []
+
+    def add(pos, cigar, n):
+        recs.append(Rec("r%d:ACGT:1" % len(recs), "chr1", pos, 0x40, 60, 0, cigar, ("ACGTTGCA" * 8)[:n], q(n)))
+    for p in (999, 1000, 1001, 1099, 1100, 1101, 1199, 1200, 1201):
+        add(p, [(4, 10)], 10)
+        add(p, [], 12)
+    add(1080, [(4, 3), (0, 40), (4, 2)], 45)                  # aligned across the shared boundary: trimmed to [1080, 1120)
+    add(1190, [(0, 30)], 30)
+    recs.sort(key=lambda r: r.pos)
+    soa = records_to_soa(recs, ["chr1"])
+    path = str(tmp_path / "edge.bam")
+    bam.write_bam(path, soa, {"chr1": 5000}, index=True, block=200)
+    whole = str(tmp_path / "edge_whole.bam")
+    shutil.copyfile(path, whole)
+    ivs = [("chr1", 1000, 1100), ("chr1", 1100, 1200)]
+    for trim in (False, True):
+        want = decode(whole, ivs, False, trim)
+        no_span = want.pos[want.ref_end() == want.pos].tolist()
+        assert no_span == [1001, 1001, 1099, 1099, 1101, 1101, 1199, 1199]
+        assert want.n == len(no_span) + 2
+        if len(_decoders()) > 1:
+            for p in (whole, path):
+                for th in (1, 3):
+                    same(decode(p, ivs, True, trim, th), want, trim)
+
+
 # ---------------------------------------------------------------------------------------------------------------- GPU
 @pytest.mark.gpu
 def test_cli_output_identical_with_and_without_the_index(tmp_path):

@@ -361,6 +361,53 @@ def test_native_decoder_counts_the_stored_qualities(tmp_path):
             assert cb["qual_bits"] == cb2["qual_bits"] and np.array_equal(cb["qual_lut"], cb2["qual_lut"]) and np.array_equal(cb["code_of"], cb2["code_of"])
 
 
+_OOM_CHILD = r"""
+import resource, sys
+from smcounter_b200 import _bamio, bam
+lib = _bamio.load()
+decode = lib.smc_bam_decode
+
+def limited(*args):
+    # from here on the process may map 1 MiB more than it has (VmData); the file is already inflated
+    with open("/proc/self/status") as fh:
+        vm_data = next(int(l.split()[1]) for l in fh if l.startswith("VmData:")) << 10
+    resource.setrlimit(resource.RLIMIT_DATA, (vm_data + (1 << 20), resource.getrlimit(resource.RLIMIT_DATA)[1]))
+    try:
+        bytearray(8 << 20)
+        print("limit not enforced")
+        sys.exit(0)
+    except MemoryError:
+        pass
+    return decode(*args)
+
+lib.smc_bam_decode = limited
+try:
+    bam.read_bam(sys.argv[1], [("chr1", 0, 1 << 20), ("chr2", 0, 1 << 20)], native=True, threads=1, trim=True)
+    print("decoded")
+except ValueError as e:
+    print("ValueError:", e)
+"""
+
+
+@pytest.mark.skipif(len(_decoders()) < 2, reason="libsmc_bamio.so not built")
+def test_native_decoder_out_of_memory_is_an_error(tmp_path):
+    """A decode whose tables and output arrays do not fit in memory (a child process, one thread, its data limit set just above
+    what it uses before smc_bam_decode runs) raises ValueError('out of memory for ...'): the decoder checks its allocations
+    instead of writing through a null pointer."""
+    import subprocess
+    import sys
+    s, refs, _ = make_panel([("chr1", 1000, 1150), ("chr2", 300, 420)], SynthSpec(umis_per_locus=3000, rpb=4.0), seed=4)
+    path = str(tmp_path / "oom.bam")
+    bam.write_bam(path, s, refs.lengths)
+    assert s.n * 56 > (2 << 20)                              # record offsets and the record table alone need more than 2 MiB
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, "-c", _OOM_CHILD, path], cwd=root, capture_output=True, text=True)
+    if "limit not enforced" in r.stdout:
+        pytest.skip("RLIMIT_DATA is not enforced here")
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert r.stdout.startswith("ValueError: out of memory for "), r.stdout + r.stderr[-2000:]
+
+
 def _random_code_lengths(rng, n_symbols_used, alphabet, must_have=(), deep=False):
     """Lengths (<= 15) of a COMPLETE prefix code over ``n_symbols_used`` random symbols of ``alphabet`` (others 0)."""
     leaves = [0]
