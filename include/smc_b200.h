@@ -76,7 +76,8 @@ typedef struct smc_reads_soa {
     const uint64_t *umi;        /* injective 64-bit code of the barcode string  (BC, smCounter.py:323) */
     const uint32_t *frag_id;    /* id of (BC, readid) (smCounter.py:321), numbered by first appearance in BAM order:
                                    ascending frag_id is the canonical fragment order inside a barcode; ids are dense
-                                   (every id < n_reads, checked: SMC_E_ARG otherwise) */
+                                   (every id < n_reads) and every read of one id carries the same barcode (both checked:
+                                   SMC_E_ARG otherwise) */
     const uint8_t  *seq;        /* BAM 4-bit bases, high nibble first, every read byte aligned */
     int64_t         seq_bytes;  /* < 4 GiB per batch */
     const uint8_t  *qual;       /* phred */
@@ -255,7 +256,7 @@ typedef struct smc_timings {
     int32_t pipe_chunks;   /* smc_call_batch: chunks the bases / qualities were uploaded in (1 = no overlap, small batch) */
     int32_t pipe_launches; /* smc_call_batch: (k_gather, k_merge) launch pairs issued as the chunks arrived */
     /* ABI v3: CUDA-event times of the kernels north_star names besides the pileup pair, and what they move */
-    float   ms_read_sort;  /* the radix passes over the reads on (barcode slot, fragment id): histogram + scan + scatter per pass */
+    float   ms_read_sort;  /* the radix passes over the fragment ids on barcode slot: histogram + scan + scatter per pass */
     float   ms_k_read_prep;/* k_read_prep alone */
     float   ms_event_sort; /* (read x tile) events: k_expand_scan + the radix pass by tile */
     int32_t read_sort_passes;

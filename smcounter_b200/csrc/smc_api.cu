@@ -1,7 +1,7 @@
 // libsmc_b200.so -- C ABI (include/smc_b200.h) and pipeline orchestration.
 //
 //   H2D (scalars first; bases / qualities in chunks on a second stream, overlapped with everything up to K3)
-//       -> K2a barcode slots (hash table) + one radix sort of the reads on (slot, fragment id)     smc_sort.cuh
+//       -> K2a barcode slots (hash table) + one radix sort of the fragment ids on barcode slot     smc_sort.cuh
 //       -> K1 read prep (CIGAR walk, QC gate, locus range, stored window)                         smc_pileup.cuh
 //       -> K2b (read x 32-locus tile) events, radix sort by tile                                  smc_sort.cuh
 //       -> K3a k_gather: lane = locus, base/quality gather, read tallies, fragment merge smc_pileup.cuh
@@ -77,7 +77,8 @@ enum SmallWord {
     SW_DYN_COUNT = 6,        // entries of the dynamic-allele table
     SW_N_TASKS = 7,          // Fisher tasks emitted by k_call
     SW_CVG_SUM = 8,          // u64: sum of cvg over the loci (= pileup read-events)
-    SW_N_UMI = 12,           // distinct barcodes (k_rank_scan; past the words k_read_prep's memset clears)
+    SW_N_MULTI = 10,         // reads of fragments of >= 3 reads (k_place_reads)
+    SW_N_UMI = 12,           // distinct barcodes (k_frag_scan)
     SW_PIPE_BLOCKED = 16,    // [SMC_PIPE_MAX]: first unit that has to wait for chunk c + 1
     SW_PACK_TOTALS = 40,     // [5]: bytes / words of packed bases, qualities, CIGARs, compact qualities, compact bases
     SW_SPILL_COUNT = 48,     // k_merge spill records handed out
@@ -129,7 +130,7 @@ struct smc_ctx {
     DevBuf d_k0{bufs}, d_k1{bufs}, d_v0{bufs}, d_v1{bufs}, d_hist{bufs}, d_scan{bufs}, d_urank{bufs}, d_frank{bufs}, d_umi_of_urank{bufs},
         d_recs{bufs}, d_ek0{bufs}, d_ek1{bufs}, d_ev0{bufs}, d_ev1{bufs}, d_tile_off{bufs}, d_unit_cnt{bufs}, d_unit_off{bufs}, d_small{bufs},
         d_grec{bufs}, d_unit_eb{bufs}, d_unit_ee{bufs}, d_unit_tile{bufs}, d_unit_nfrag{bufs}, d_codes{bufs}, d_frag_first{bufs},
-        d_umi_urank{bufs}, d_umi_table{bufs};
+        d_umi_urank{bufs}, d_umi_table{bufs}, d_frag_cnt{bufs}, d_frag_min{bufs};
     uint32_t code_mult = 1;                     // fragment-code storage per tile event (1, or 3 = worst case after GF_CODE_FULL)
     uint32_t n_units_cap = 0;
     // per-locus accumulators / outputs
@@ -166,39 +167,45 @@ struct smc_ctx {
 // ------------------------------------------------------------------------------------------------------------
 // small kernels used only by the orchestration
 // ------------------------------------------------------------------------------------------------------------
-// Barcode slots: every distinct barcode code gets one slot of an open-addressing table (linear probing, atomicCAS); the slot
-// index stands in for the barcode in the read sort key, so that ONE sort on (slot, fragment id) groups the reads by barcode and
-// fragment.  Which slot a barcode lands in may differ from run to run; nothing downstream depends on the order of barcodes
-// (the PI sums are fixed point, every other accumulation is an integer).
+// Barcode slots and per-fragment facts.  Every distinct barcode code gets one slot of an open-addressing table (linear probing,
+// atomicCAS); the slot index stands in for the barcode in the fragment sort key.  Which slot a barcode lands in may differ from
+// run to run; nothing downstream depends on the order of barcodes (the PI sums are fixed point, every other accumulation is an
+// integer).  The last slot (mask) is never handed out: FRAG_NONE, the key of fragment ids no read carries, sorts behind every
+// barcode.  Per fragment id f < n: its barcode slot (a read of another barcode raises GF_FRAG_UMI), its read count and its
+// smallest BAM index.  Ids >= n are ORed into frag_or (refused at the round trip) and left out of the tables.
 #define UMI_EMPTY 0xffffffffffffffffull
+#define FRAG_NONE 0xffffffffu
 __global__ void k_umi_slots(const uint64_t* __restrict__ umi, const uint32_t* __restrict__ frag, int64_t n, unsigned long long* __restrict__ table,
-                            uint32_t mask, int frag_bits, uint64_t* __restrict__ key, uint32_t* __restrict__ val, unsigned long long* __restrict__ frag_or) {
+                            uint32_t mask, uint32_t* __restrict__ frag_slot, uint32_t* __restrict__ frag_cnt, uint32_t* __restrict__ frag_min,
+                            uint32_t* __restrict__ frag_ids, unsigned long long* __restrict__ frag_or, uint32_t* __restrict__ gflags) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    uint32_t f = 0;
-    if (i < n) {
-        const unsigned long long u = umi[i];
-        f = frag[i];
-        uint32_t h = hash64to32(u) & mask;
-        for (;;) {
-            unsigned long long cur = table[h];
-            if (cur == UMI_EMPTY) cur = atomicCAS(&table[h], UMI_EMPTY, u);
-            if (cur == UMI_EMPTY || cur == u) break;
-            h = (h + 1) & mask;
-        }
-        key[i] = ((uint64_t)h << frag_bits) | (uint64_t)f;
-        val[i] = (uint32_t)i;
+    if (i >= n) return;
+    const unsigned long long u = umi[i];
+    const uint32_t f = frag[i];
+    uint32_t h = hash64to32(u) & mask;
+    for (;; ++h) {
+        if (h == mask) h = 0;
+        unsigned long long cur = table[h];
+        if (cur == UMI_EMPTY) cur = atomicCAS(&table[h], UMI_EMPTY, u);
+        if (cur == UMI_EMPTY || cur == u) break;
     }
-    // OR of all fragment ids (range check on the host: ids must be < 2^frag_bits)
-    f = __reduce_or_sync(FULL_MASK, f);
-    if ((threadIdx.x & 31) == 0 && (f >> frag_bits)) atomicOr(frag_or, (unsigned long long)f);
+    frag_ids[i] = (uint32_t)i;                                        // the payload of the fragment sort: every id, in id order
+    if (f >= (uint64_t)n) { atomicOr(frag_or, (unsigned long long)f); return; }
+    const uint32_t had = atomicCAS(&frag_slot[f], FRAG_NONE, h);
+    if (had != FRAG_NONE && had != h) atomicOr(gflags, GF_FRAG_UMI);
+    atomicAdd(&frag_cnt[f], 1u);
+    atomicMin(&frag_min[f], (uint32_t)i);
 }
-// Reads in sorted order: a new barcode starts where the slot part of the key changes, a new fragment where the key changes.
-// ONE single-pass scan (decoupled look-back, smc_sort.cuh) over both head flags at once (two 31-bit counts in one word) turns
-// them into the dense barcode / fragment ranks, and writes the inverse permutation and the barcode of every rank.
+// Fragment ids in barcode-slot order (stable: frag_id order inside a barcode; the ids no read carries last).  A real fragment's
+// rank is its position j in that list.  ONE single-pass scan (decoupled look-back, smc_sort.cuh) over the barcode head flags and
+// the read counts at once (two 31-bit counts in one word) gives every fragment its first sorted read position and its barcode
+// rank; it writes urank / frank of every sorted read position, the barcode of every barcode rank, and frag_start[f], with
+// FRAG_MULTI set for fragments of three or more reads (k_place_reads).
+#define FRAG_MULTI 0x80000000u
 __global__ void __launch_bounds__(SCAN_THREADS)
-k_rank_scan(const uint64_t* __restrict__ key_sorted, int frag_bits, int64_t n, const uint64_t* __restrict__ umi, const uint32_t* __restrict__ perm,
-            uint32_t* __restrict__ urank, uint32_t* __restrict__ frank, uint64_t* __restrict__ umi_of_urank, uint32_t* __restrict__ inv,
-            unsigned long long* desc, uint32_t* counter, uint32_t* n_umi_out) {
+k_frag_scan(const uint32_t* __restrict__ slot_sorted, const uint32_t* __restrict__ frag_sorted, int64_t n, const uint32_t* __restrict__ frag_cnt,
+            const uint32_t* __restrict__ frag_min, const uint64_t* __restrict__ umi, uint32_t* __restrict__ urank, uint32_t* __restrict__ frank,
+            uint64_t* __restrict__ umi_of_urank, uint32_t* __restrict__ frag_start, unsigned long long* desc, uint32_t* counter, uint32_t* n_umi_out) {
     __shared__ unsigned long long warp_tot[SCAN_THREADS / 32];
     __shared__ uint32_t s_tile;
     __shared__ unsigned long long s_prefix;
@@ -206,18 +213,15 @@ k_rank_scan(const uint64_t* __restrict__ key_sorted, int frag_bits, int64_t n, c
     __syncthreads();
     const uint32_t tile = s_tile;
     const int64_t base = (int64_t)tile * SCAN_TILE + (int64_t)threadIdx.x * SCAN_ITEMS;
-    unsigned long long v[SCAN_ITEMS], tsum = 0;
-    uint64_t prev = (base > 0 && base <= n) ? key_sorted[base - 1] : 0ull;
+    unsigned long long v[SCAN_ITEMS], tsum = 0;                        // (barcode head << 31) | reads; 0 for an id without reads
+    uint32_t prev = (base > 0 && base <= n) ? slot_sorted[base - 1] : FRAG_NONE;
 #pragma unroll
     for (int i = 0; i < SCAN_ITEMS; ++i) {
         v[i] = 0;
         if (base + i < n) {
-            const uint64_t k = key_sorted[base + i];
-            const bool first = base + i == 0;
-            const unsigned long long uh = (first || (k >> frag_bits) != (prev >> frag_bits)) ? 1ull : 0ull;
-            const unsigned long long fh = (first || k != prev) ? 1ull : 0ull;
-            v[i] = (uh << 31) | fh;
-            prev = k;
+            const uint32_t s = slot_sorted[base + i];
+            if (s != FRAG_NONE) v[i] = ((s != prev ? 1ull : 0ull) << 31) | frag_cnt[frag_sorted[base + i]];
+            prev = s;
         }
         tsum += v[i];
     }
@@ -245,17 +249,53 @@ k_rank_scan(const uint64_t* __restrict__ key_sorted, int frag_bits, int64_t n, c
         }
     }
     __syncthreads();
-    unsigned long long run = s_prefix + woff + incl - tsum;            // exclusive counts before the thread's first read
+    unsigned long long run = s_prefix + woff + incl - tsum;            // exclusive counts before the thread's first fragment
 #pragma unroll
     for (int i = 0; i < SCAN_ITEMS; ++i) {
-        if (base + i < n) {
-            run += v[i];
-            const uint32_t ur = (uint32_t)(run >> 31) - 1u, fr = (uint32_t)(run & 0x7fffffffull) - 1u;
-            urank[base + i] = ur; frank[base + i] = fr;
-            const uint32_t r = perm[base + i];
-            inv[r] = (uint32_t)(base + i);                                // sorted position of read r (k_read_prep runs in BAM order)
-            if (v[i] >> 31) umi_of_urank[ur] = umi[r];
-        }
+        if (v[i] == 0) continue;
+        const uint32_t start = (uint32_t)(run & 0x7fffffffull), cnt = (uint32_t)(v[i] & 0x7fffffffull), j = (uint32_t)(base + i);
+        run += v[i];
+        const uint32_t ur = (uint32_t)(run >> 31) - 1u, f = frag_sorted[j];
+        SMC_BOUNDS((int64_t)start + cnt <= n && (int64_t)ur < n && (int64_t)f < n);
+        for (uint32_t k = start; k < start + cnt; ++k) { urank[k] = ur; frank[k] = j; }
+        if (v[i] >> 31) umi_of_urank[ur] = umi[frag_min[f]];
+        frag_start[f] = start | (cnt > 2 ? FRAG_MULTI : 0u);
+    }
+}
+// Sorted position of every read (inv[i], k_read_prep runs in BAM order): its fragment's first position plus its rank among the
+// fragment's reads in BAM order, which for a fragment of one or two reads is whether it is not the smallest BAM index.  The reads
+// of larger fragments take the positions of their fragment's range in arrival order (multi_read) and join multi_list, for
+// k_rank_multi to rank them.
+__global__ void k_place_reads(const uint32_t* __restrict__ frag, int64_t n, const uint32_t* __restrict__ frag_min, uint32_t* __restrict__ frag_start,
+                              uint32_t* __restrict__ inv, uint32_t* __restrict__ multi_read, uint32_t* __restrict__ multi_list, uint32_t* __restrict__ n_multi) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t f = frag[i];
+    if (f >= (uint64_t)n) { inv[i] = (uint32_t)i; return; }          // refused at the round trip; until then any position in range
+    const uint32_t s = frag_start[f];
+    if (!(s & FRAG_MULTI)) {
+        inv[i] = s + ((uint32_t)i != frag_min[f] ? 1u : 0u);
+        SMC_BOUNDS((int64_t)inv[i] < n);
+        return;
+    }
+    const uint32_t p = atomicAdd(&frag_start[f], 1u) & ~FRAG_MULTI;   // FRAG_MULTI stays set: start + reads <= n < 2^31
+    const uint32_t k = atomicAdd(n_multi, 1u);
+    SMC_BOUNDS((int64_t)p < n && (int64_t)k < n);
+    multi_read[p] = (uint32_t)i;
+    multi_list[k] = (uint32_t)i;
+}
+// Reads of fragments of three or more reads (none in most batches): rank among the fragment's reads by BAM index.
+__global__ void k_rank_multi(const uint32_t* __restrict__ multi_list, const uint32_t* __restrict__ n_multi, const uint32_t* __restrict__ frag,
+                             const uint32_t* __restrict__ frag_cnt, const uint32_t* __restrict__ frag_start, const uint32_t* __restrict__ multi_read,
+                             uint32_t* __restrict__ inv) {
+    const uint32_t m = *n_multi;
+    for (uint32_t t = blockIdx.x * blockDim.x + threadIdx.x; t < m; t += gridDim.x * blockDim.x) {
+        const uint32_t i = multi_list[t], f = frag[i], cnt = frag_cnt[f];
+        const uint32_t start = (frag_start[f] & ~FRAG_MULTI) - cnt;   // k_place_reads advanced it by cnt
+        uint32_t r = 0;
+        for (uint32_t k = start; k < start + cnt; ++k) r += multi_read[k] < i ? 1u : 0u;
+        SMC_BOUNDS(r < cnt);
+        inv[i] = start + r;
     }
 }
 // (read x 32-locus tile) events: the number of tiles each read covers is scanned (single pass, look-back) and the events are
@@ -768,43 +808,56 @@ static int read_back(smc_ctx* ctx, void* dst, const void* src, size_t bytes) {
     return SMC_OK;
 }
 
-// K2a: order reads by (barcode, frag_id, BAM index): one stable sort on (barcode slot, frag_id), then one single-pass scan for
-// the dense barcode / fragment ranks, the barcode of every rank and the inverse permutation (*inv: read index -> sorted position).
+// K2a: order reads by (barcode, frag_id, BAM index).  Fragment ids are already in order inside a barcode and reads in BAM order
+// inside a fragment, so it is the fragment ids that are sorted, stably on barcode slot; one single-pass scan over them gives the
+// dense barcode / fragment ranks, the barcode of every rank and every fragment's first sorted position, from which each read
+// takes its own (*inv: read index -> sorted position).  The two key buffers and the two payload buffers ping-pong in the sort;
+// of the pair the sort does not leave its result in, the key buffer takes frag_start and the payload buffer inv, and once the
+// scan has read the sorted pair, it takes the rare path's multi_read / multi_list.
 static int read_sort(smc_ctx* ctx, const uint32_t** inv) {
     const int64_t n = ctx->n_reads;
+    const size_t n4 = (size_t)n * 4;
     uint32_t* small = ctx->d_small.as<uint32_t>();
-    CK(ctx->d_k0.ensure((size_t)n * 8)); CK(ctx->d_k1.ensure((size_t)n * 8));
-    CK(ctx->d_v0.ensure((size_t)n * 4)); CK(ctx->d_v1.ensure((size_t)n * 4));
+    CK(ctx->d_k0.ensure(n4)); CK(ctx->d_k1.ensure(n4)); CK(ctx->d_v0.ensure(n4)); CK(ctx->d_v1.ensure(n4));
+    CK(ctx->d_frag_cnt.ensure(n4)); CK(ctx->d_frag_min.ensure(n4));
     CK(ctx->d_hist.ensure(radix_hist_words(n) * 4 + 1024));
     CK(ctx->d_scan.ensure((size_t)std::max<int64_t>(radix_scan_words(n), scan_scratch_words(n + 1)) * 4 + 1024));
-    uint64_t* k0 = ctx->d_k0.as<uint64_t>(); uint64_t* k1 = ctx->d_k1.as<uint64_t>();
+    uint32_t* k0 = ctx->d_k0.as<uint32_t>(); uint32_t* k1 = ctx->d_k1.as<uint32_t>();
     uint32_t* v0 = ctx->d_v0.as<uint32_t>(); uint32_t* v1 = ctx->d_v1.as<uint32_t>();
-    // barcode table of >= 1.1 n slots (a batch has far fewer distinct barcodes than reads) and dense fragment ids < n:
-    // a 2.9 M read panel batch sorts on 22 + 22 = 44 key bits = four 11-bit passes
+    uint32_t* frag_cnt = ctx->d_frag_cnt.as<uint32_t>(); uint32_t* frag_min = ctx->d_frag_min.as<uint32_t>();
+    // barcode table of >= 1.1 n slots (a batch has far fewer distinct barcodes than reads): a 2.9 M read panel batch sorts its
+    // fragment ids on 22 key bits = two 11-bit passes
     int slot_bits = 4;
     while ((double)(1ll << slot_bits) < 1.1 * (double)n) ++slot_bits;
-    int frag_bits = 1;                                             // frag_id < 2^frag_bits; checked after the round trip (the
-    while ((1ll << frag_bits) < n) ++frag_bits;                    // contract says ids are dense, first-appearance numbers)
     CK(ctx->d_umi_table.ensure(((size_t)1 << slot_bits) * 8));
     CK(cudaMemsetAsync(ctx->d_umi_table.p, 0xff, ((size_t)1 << slot_bits) * 8, ctx->st));
+    CK(cudaMemsetAsync(k0, 0xff, n4, ctx->st));                       // frag_slot = FRAG_NONE
+    CK(cudaMemsetAsync(frag_min, 0xff, n4, ctx->st));
+    CK(cudaMemsetAsync(frag_cnt, 0, n4, ctx->st));
     CK(cudaMemsetAsync(small + SW_FRAG_OR, 0, 8, ctx->st));
+    CK(cudaMemsetAsync(small + SW_N_TILE_EVENTS, 0, 32, ctx->st));    // words 4 .. 11: tile-event total, gflags, ..., SW_N_MULTI
     LAUNCH(k_umi_slots, nblk(n, 256), 256, 0, ctx->d_umi.as<uint64_t>(), ctx->d_frag.as<uint32_t>(), n,
-           ctx->d_umi_table.as<unsigned long long>(), (uint32_t)((1u << slot_bits) - 1u), frag_bits, k0, v0, (unsigned long long*)(small + SW_FRAG_OR));
+           ctx->d_umi_table.as<unsigned long long>(), (uint32_t)((1u << slot_bits) - 1u), k0, frag_cnt, frag_min, v0,
+           (unsigned long long*)(small + SW_FRAG_OR), small + SW_GFLAGS);
     CK(cudaEventRecord(ctx->ev[EV_READ_SORT_BEGIN], ctx->st));
-    if (radix_sort_bits(k0, v0, k1, v1, n, 0, slot_bits + frag_bits, ctx->d_hist.as<uint32_t>(), ctx->d_scan.as<uint32_t>(), ctx->st)) {
-        std::swap(k0, k1); std::swap(v0, v1);
-    }
+    const int res = radix_sort_bits(k0, v0, k1, v1, n, 0, slot_bits, ctx->d_hist.as<uint32_t>(), ctx->d_scan.as<uint32_t>(), ctx->st);
     CK(cudaEventRecord(ctx->ev[EV_READ_SORT_DONE], ctx->st));
-    ctx->tm.read_sort_passes = (slot_bits + frag_bits + RS_MAX_BITS - 1) / RS_MAX_BITS;
-    const uint32_t* perm = v0;
-    CK(ctx->d_urank.ensure((size_t)n * 4)); CK(ctx->d_frank.ensure((size_t)n * 4));
+    ctx->tm.read_sort_passes = n > 1 ? (slot_bits + RS_MAX_BITS - 1) / RS_MAX_BITS : 0;
+    uint32_t* slot_sorted = res ? k1 : k0; uint32_t* frag_sorted = res ? v1 : v0;
+    uint32_t* frag_start = res ? k0 : k1; uint32_t* inv_out = res ? v0 : v1;
+    CK(ctx->d_urank.ensure(n4)); CK(ctx->d_frank.ensure(n4));
     CK(ctx->d_umi_of_urank.ensure((size_t)n * 8));
     const int64_t nbt = (n + SCAN_TILE - 1) / SCAN_TILE;
     uint32_t* scr = ctx->d_scan.as<uint32_t>();
     CK(cudaMemsetAsync(scr, 0, (size_t)(2 * nbt + 8) * 4, ctx->st));
-    LAUNCH(k_rank_scan, (unsigned)nbt, SCAN_THREADS, 0, k0, frag_bits, n, ctx->d_umi.as<uint64_t>(), perm, ctx->d_urank.as<uint32_t>(),
-           ctx->d_frank.as<uint32_t>(), ctx->d_umi_of_urank.as<uint64_t>(), v1, reinterpret_cast<unsigned long long*>(scr + 2), scr, small + SW_N_UMI);
-    *inv = v1;
+    LAUNCH(k_frag_scan, (unsigned)nbt, SCAN_THREADS, 0, slot_sorted, frag_sorted, n, frag_cnt, frag_min, ctx->d_umi.as<uint64_t>(),
+           ctx->d_urank.as<uint32_t>(), ctx->d_frank.as<uint32_t>(), ctx->d_umi_of_urank.as<uint64_t>(), frag_start,
+           reinterpret_cast<unsigned long long*>(scr + 2), scr, small + SW_N_UMI);
+    LAUNCH(k_place_reads, nblk(n, 256), 256, 0, ctx->d_frag.as<uint32_t>(), n, frag_min, frag_start, inv_out, slot_sorted, frag_sorted,
+           small + SW_N_MULTI);
+    LAUNCH(k_rank_multi, std::min<unsigned>(nblk(n, 256), 148u), 256, 0, frag_sorted, small + SW_N_MULTI, ctx->d_frag.as<uint32_t>(),
+           frag_cnt, frag_start, slot_sorted, inv_out);
+    *inv = inv_out;
     return SMC_OK;
 }
 
@@ -813,7 +866,6 @@ static int read_prep(smc_ctx* ctx, const uint32_t* inv) {
     const int64_t n = ctx->n_reads;
     uint32_t* small = ctx->d_small.as<uint32_t>();
     CK(ctx->d_recs.ensure((size_t)n * sizeof(ReadRec))); CK(ctx->d_grec.ensure((size_t)n * sizeof(GRec)));
-    CK(cudaMemsetAsync(small + SW_N_TILE_EVENTS, 0, 32, ctx->st));
     PrepArgs P{};
     P.n_reads = n; P.inv = inv; P.urank = ctx->d_urank.as<uint32_t>(); P.frank = ctx->d_frank.as<uint32_t>();
     P.ref_id = ctx->d_ref_id.as<int32_t>(); P.pos = ctx->d_pos.as<int32_t>(); P.flag = ctx->d_flag.as<uint16_t>();
@@ -849,6 +901,7 @@ static int check_device_inputs(smc_ctx* ctx, const uint32_t* w) {
         return SMC_E_ARG;
     }
     if (w[SW_FRAG_OR] | w[SW_FRAG_OR + 1]) { ctx->err = "frag_id must be a dense id (< n_reads), numbered by first appearance"; return SMC_E_ARG; }
+    if (gflags & GF_FRAG_UMI) { ctx->err = "a frag_id must belong to one barcode"; return SMC_E_ARG; }
     const uint32_t* tot = w + SW_PACK_TOTALS;
     if ((ctx->packed_seq && (int64_t)tot[ctx->seq_bits == 2 ? 4 : 0] != ctx->seq_bytes) || (ctx->packed_qual && (int64_t)tot[ctx->qual_bits != 8 ? 3 : 1] != ctx->qual_bytes) ||
         (ctx->packed_cigar && (int64_t)tot[2] != ctx->n_cigar_words)) {

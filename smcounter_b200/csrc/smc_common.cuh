@@ -58,6 +58,15 @@ __host__ __device__ inline uint64_t dyn_make_key(uint32_t locus, uint32_t kind, 
 
 __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31; }
 
+// Built with -DSMC_BOUNDS_ASSERT (SMC_NVCC_EXTRA): device asserts on the positions the read-sort kernels compute from the
+// fragment tables, which the index checks of a normal build take on trust.
+#ifdef SMC_BOUNDS_ASSERT
+#include <cassert>
+#define SMC_BOUNDS(cond) assert(cond)
+#else
+#define SMC_BOUNDS(cond) ((void)0)
+#endif
+
 __device__ __forceinline__ uint32_t hash64to32(uint64_t x) {
     x ^= x >> 33; x *= 0xff51afd7ed558ccdull; x ^= x >> 33; x *= 0xc4ceb9fe1a85ec53ull; x ^= x >> 33;
     return (uint32_t)x;

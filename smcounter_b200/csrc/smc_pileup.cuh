@@ -62,6 +62,7 @@ struct PrepArgs {
 #define GF_CODE_FULL  4u     // a unit ran out of fragment-code storage (host retries with the worst-case layout)
 #define GF_BAD_STORE  8u     // stored window (store_lo / store_len) malformed or not covering every target base of the read
 #define GF_SPILL_FULL 16u    // k_merge ran out of spill records (host retries with a larger pool)
+#define GF_FRAG_UMI   32u    // a frag_id carries reads of two barcodes (k_umi_slots)
 
 __global__ void __launch_bounds__(256) k_read_prep(PrepArgs A) {
     const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;      // BAM order in (coalesced), sorted position out

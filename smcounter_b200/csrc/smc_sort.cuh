@@ -1,10 +1,10 @@
-// Hand-written device-wide exclusive scan and stable LSD radix sort (u64 key, u32 payload).
+// Hand-written device-wide exclusive scan and stable LSD radix sort (u32 or u64 key, u32 payload).
 //
-// K2 of the pipeline ("segmented radix sort"): reads are ordered by (barcode slot, fragment, BAM index) and the
-// (read x 32-locus tile) events by tile, so that every tile's events form one segment in which barcodes and
-// fragments are contiguous runs in BAM order.  Both sorts are LSD passes over exactly the key bits in use, with a digit
-// width of 8-11 bits chosen per sort.  Each pass reads 12 B and writes 12 B per element (the working sets of a panel batch
-// fit the 126 MB L2); histogram, scan and scatter are separate kernels.
+// K2 of the pipeline ("segmented radix sort"): fragment ids are ordered by barcode slot (u32 key) and the (read x 32-locus
+// tile) events by tile (u64 key), so that every tile's events form one segment in which barcodes and fragments are
+// contiguous runs in BAM order.  Both sorts are LSD passes over exactly the key bits in use, with a digit width of 8-11 bits
+// chosen per sort.  Each pass reads and writes key + payload once per element (the working sets of a panel batch fit the
+// 126 MB L2); histogram, scan and scatter are separate kernels.
 #pragma once
 #include "smc_common.cuh"
 
@@ -158,8 +158,8 @@ static void exclusive_scan_u32(const uint32_t* in, uint32_t* out, int64_t n, uin
 
 // ---------------------------------------------------------------- radix sort --------------------------------
 // LSD passes over a bit field of the key: digit = (key >> shift) & (2^BITS - 1), BITS = 8 ... 11 chosen per sort so that
-// the varying bits are covered in as few passes as possible (e.g. a 9-bit tile index is ONE pass, a 45-bit
-// (barcode slot, fragment) key is five 9-bit passes).
+// the varying bits are covered in as few passes as possible (e.g. a 9-bit tile index is ONE pass, a 22-bit barcode slot two
+// 11-bit passes).
 #define RS_WARPS   8
 #define RS_THREADS (RS_WARPS * 32)
 #define RS_ITEMS   8
@@ -171,9 +171,9 @@ __device__ __forceinline__ int64_t rs_index(int64_t tile_base, int w, int it, in
     return tile_base + (int64_t)w * (32 * RS_ITEMS) + it * 32 + lane;
 }
 
-template <int BITS>
+template <int BITS, class K>
 __global__ void __launch_bounds__(RS_THREADS)
-k_radix_hist(const uint64_t* __restrict__ keys, int64_t n, int shift, uint32_t* __restrict__ hist, uint32_t nblocks) {
+k_radix_hist(const K* __restrict__ keys, int64_t n, int shift, uint32_t* __restrict__ hist, uint32_t nblocks) {
     constexpr uint32_t ND = 1u << BITS;
     __shared__ uint32_t h[ND];
     for (uint32_t d = threadIdx.x; d < ND; d += RS_THREADS) h[d] = 0;
@@ -189,9 +189,9 @@ k_radix_hist(const uint64_t* __restrict__ keys, int64_t n, int shift, uint32_t* 
     for (uint32_t d = threadIdx.x; d < ND; d += RS_THREADS) hist[(size_t)d * nblocks + blockIdx.x] = h[d];
 }
 
-template <int BITS>
+template <int BITS, class K>
 __global__ void __launch_bounds__(RS_THREADS)
-k_radix_scatter(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ vals, uint64_t* __restrict__ keys_out,
+k_radix_scatter(const K* __restrict__ keys, const uint32_t* __restrict__ vals, K* __restrict__ keys_out,
                 uint32_t* __restrict__ vals_out, int64_t n, int shift, const uint32_t* __restrict__ hist_scanned,
                 uint32_t nblocks) {
     constexpr uint32_t ND = 1u << BITS;
@@ -201,7 +201,7 @@ k_radix_scatter(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ 
     __syncthreads();
     uint32_t* wh = wh_s + (size_t)w * ND;
     int64_t tb = (int64_t)blockIdx.x * RS_TILE;
-    uint64_t k[RS_ITEMS];
+    K k[RS_ITEMS];
     uint32_t v[RS_ITEMS];
 #pragma unroll
     for (int it = 0; it < RS_ITEMS; ++it) {
@@ -252,26 +252,29 @@ k_radix_scatter(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ 
 static inline size_t radix_hist_words(int64_t n) { return ((size_t)1 << RS_MAX_BITS) * (size_t)((n + RS_TILE - 1) / RS_TILE) + 256; }
 static inline int64_t radix_scan_words(int64_t n) { return scan_scratch_words((int64_t)radix_hist_words(n)); }
 
-template <int BITS>
-static void radix_pass(const uint64_t* ki, const uint32_t* vi, uint64_t* ko, uint32_t* vo, int64_t n, int shift, uint32_t* hist,
+template <int BITS, class K>
+static void radix_pass(const K* ki, const uint32_t* vi, K* ko, uint32_t* vo, int64_t n, int shift, uint32_t* hist,
                        uint32_t* scan_scratch, cudaStream_t st) {
     const uint32_t nblocks = (uint32_t)((n + RS_TILE - 1) / RS_TILE);
     constexpr size_t smem = (size_t)RS_WARPS * (1u << BITS) * 4;      // 11 bits: 64 KB, opted in per device by radix_sort_init()
-    k_radix_hist<BITS><<<nblocks, RS_THREADS, 0, st>>>(ki, n, shift, hist, nblocks);
+    k_radix_hist<BITS, K><<<nblocks, RS_THREADS, 0, st>>>(ki, n, shift, hist, nblocks);
     ++g_launches;
     exclusive_scan_u32(hist, hist, (int64_t)(1u << BITS) * nblocks, scan_scratch, nullptr, st);
-    k_radix_scatter<BITS><<<nblocks, RS_THREADS, smem, st>>>(ki, vi, ko, vo, n, shift, hist, nblocks);
+    k_radix_scatter<BITS, K><<<nblocks, RS_THREADS, smem, st>>>(ki, vi, ko, vo, n, shift, hist, nblocks);
     ++g_launches;
 }
 
 // once per device: the 11-bit scatter needs more dynamic shared memory than the default limit
 static cudaError_t radix_sort_init() {
-    return cudaFuncSetAttribute(k_radix_scatter<RS_MAX_BITS>, cudaFuncAttributeMaxDynamicSharedMemorySize, RS_WARPS * (1 << RS_MAX_BITS) * 4);
+    cudaError_t e = cudaFuncSetAttribute(k_radix_scatter<RS_MAX_BITS, uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, RS_WARPS * (1 << RS_MAX_BITS) * 4);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(k_radix_scatter<RS_MAX_BITS, uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, RS_WARPS * (1 << RS_MAX_BITS) * 4);
 }
 
 // Stable sort of (keys, vals) on key bits [lo_bit, lo_bit + nbits), in ceil(nbits / 11) passes of equal digit width (>= 8).
 // Ping-pongs between (k0,v0) and (k1,v1); returns 0 if the result is in (k0,v0), 1 if in (k1,v1).
-static int radix_sort_bits(uint64_t* k0, uint32_t* v0, uint64_t* k1, uint32_t* v1, int64_t n, int lo_bit, int nbits, uint32_t* hist,
+template <class K>
+static int radix_sort_bits(K* k0, uint32_t* v0, K* k1, uint32_t* v1, int64_t n, int lo_bit, int nbits, uint32_t* hist,
                            uint32_t* scan_scratch, cudaStream_t st) {
     if (n <= 1 || nbits <= 0) return 0;
     const int npass = (nbits + RS_MAX_BITS - 1) / RS_MAX_BITS;
@@ -279,8 +282,8 @@ static int radix_sort_bits(uint64_t* k0, uint32_t* v0, uint64_t* k1, uint32_t* v
     if (width < 8) width = 8;
     int cur = 0;
     for (int done = 0; done < nbits; done += width) {
-        uint64_t* ki = cur ? k1 : k0; uint32_t* vi = cur ? v1 : v0;
-        uint64_t* ko = cur ? k0 : k1; uint32_t* vo = cur ? v0 : v1;
+        K* ki = cur ? k1 : k0; uint32_t* vi = cur ? v1 : v0;
+        K* ko = cur ? k0 : k1; uint32_t* vo = cur ? v0 : v1;
         const int shift = lo_bit + done;
         switch (width) {
             case 8:  radix_pass<8>(ki, vi, ko, vo, n, shift, hist, scan_scratch, st); break;
