@@ -5,6 +5,7 @@
 //       -> K1 read prep (CIGAR walk, QC gate, locus range, stored window)                         smc_pileup.cuh
 //       -> K2b (read x 32-locus tile) events, radix sort by tile                                  smc_sort.cuh
 //       -> K3a k_gather: lane = locus, base/quality gather, read tallies, fragment merge smc_pileup.cuh
+//          (bases and qualities expanded per chunk into one 16-bit word per stored base first)     smc_upload.cuh
 //       -> K3b k_merge: per-barcode posterior (calProb), prediction index, consensus    smc_pileup.cuh
 //       -> K4 FP64 statistics: PI, ALT, filters, Fisher                                smc_stats.cuh
 //   -> D2H
@@ -80,10 +81,9 @@ enum SmallWord {
     SW_N_MULTI = 10,         // reads of fragments of >= 3 reads (k_place_reads)
     SW_N_UMI = 12,           // distinct barcodes (k_frag_scan)
     SW_PIPE_BLOCKED = 16,    // [SMC_PIPE_MAX]: first unit that has to wait for chunk c + 1
-    SW_PACK_TOTALS = 40,     // [5]: bytes / words of packed bases, qualities, CIGARs, compact qualities, compact bases
+    SW_PACK_TOTALS = 40,     // [6]: bytes / words of packed bases, qualities, CIGARs, compact qualities, compact bases; bq[] words
     SW_SPILL_COUNT = 48,     // k_merge spill records handed out
-    SW_CHUNK_READS = 64,     // [SMC_PIPE_MAX + 2]: first read completed by each upload chunk (compact qualities)
-    SW_CHUNK_READS_SEQ = 96  // the same for the compact bases
+    SW_CHUNK_FIRST = 64      // [SMC_PIPE_MAX]: k_chunk_need's first read per upload chunk
 };
 
 // stage events of ctx->ev; the SMC_TIMELINE line prints the first seven, in this order
@@ -106,20 +106,22 @@ struct smc_ctx {
     cudaStream_t st_copy = nullptr;
     cudaEvent_t ev_link = nullptr, ev_tmp = nullptr, ev_tmp2 = nullptr, ev_chunk[SMC_PIPE_MAX]{};
     int pipe_n = 0;                             // > 1: the chunk events of the current batch are pending / recorded
-    uint32_t pipe_seq_chunk = 0, pipe_qual_chunk = 0;   // bytes of bases / qualities per chunk
     DevBuf d_pipe_need{bufs};
     bool packed_seq = false, packed_qual = false, packed_cigar = false;   // offsets were NULL: computed on the device
     uint32_t pipe_end[SMC_PIPE_MAX]{};          // launch c of the pileup kernels covers units [pipe_end[c-1], pipe_end[c])
     // resident inputs
     int64_t n_reads = 0, n_loci = 0;
     int64_t seq_bytes = 0, qual_bytes = 0, n_cigar_words = 0;
-    DevBuf d_ref_id{bufs}, d_pos{bufs}, d_flag{bufs}, d_mapq{bufs}, d_nm{bufs}, d_lseq{bufs}, d_seq_off{bufs}, d_qual_off{bufs},
-        d_cig_off{bufs}, d_ncig{bufs}, d_umi{bufs}, d_frag{bufs}, d_seq{bufs}, d_qual{bufs}, d_cigar{bufs}, d_store_lo{bufs}, d_store_len{bufs};
+    DevBuf d_ref_id{bufs}, d_pos{bufs}, d_flag{bufs}, d_mapq{bufs}, d_nm{bufs}, d_lseq{bufs}, d_cig_off{bufs}, d_ncig{bufs}, d_umi{bufs},
+        d_frag{bufs}, d_cigar{bufs}, d_store_lo{bufs}, d_store_len{bufs};
     bool has_store = false;                     // reads carry a stored window (smc_reads_soa::store_lo / store_len)
-    int qual_bits = 8;                          // 4 / 2: compact qualities were uploaded (d_qual_packed) and are expanded into d_qual
-    DevBuf d_qual_packed{bufs}, d_qual_poff{bufs}, d_qual_lut{bufs}, d_stage{bufs}, d_spill{bufs}, d_seq_packed{bufs}, d_seq_poff{bufs},
-        d_exc_read{bufs}, d_exc_pos{bufs}, d_exc_nib{bufs};
-    int seq_bits = 4; int64_t n_seq_exc = 0;    // 2: compact bases were uploaded (d_seq_packed) and are expanded into d_seq
+    // Bases and qualities as uploaded (d_seq_up / d_qual_up, any encoding; byte offsets per read in d_seq_poff / d_qual_poff,
+    // narrowed from the caller's d_seq_off / d_qual_off when it gives them) are expanded into the one array the kernels read:
+    // bq[], quality | BAM nibble << 8 per stored base, d_bq_off the word of each read's first stored base
+    int qual_bits = 8, seq_bits = 4; int64_t n_seq_exc = 0;
+    DevBuf d_seq_up{bufs}, d_qual_up{bufs}, d_seq_off{bufs}, d_qual_off{bufs}, d_seq_poff{bufs}, d_qual_poff{bufs}, d_qual_lut{bufs},
+        d_exc_read{bufs}, d_exc_pos{bufs}, d_exc_nib{bufs}, d_bq{bufs}, d_bq_off{bufs}, d_stage{bufs}, d_spill{bufs};
+    uint32_t bq_cap = 0;                        // words of d_bq the current batch may fill
     uint32_t spill_cap = 0;                     // records in the k_merge spill pool (grows x4 on GF_SPILL_FULL)
     DevBuf d_loci_ref{bufs}, d_loci_pos{bufs}, d_loci_base{bufs}, d_loci_key{bufs};
     DevBuf d_keep_idx{bufs}, d_keep_off{bufs}, d_keep_umi{bufs};
@@ -534,13 +536,10 @@ static int pipe_chunks_for(const smc_reads_soa* R) {
 
 static int qual_bits_of(const smc_reads_soa* R) { return (R->qual_bits == 4 || R->qual_bits == 2) ? R->qual_bits : 8; }
 static int seq_bits_of(const smc_reads_soa* R) { return R->seq_bits == 2 ? 2 : 4; }
-// expanded payloads: a read stores (len + 1) / 2 bytes of 4-bit bases for (len + 3) / 4 bytes of 2-bit ones, and never more
-// qualities than two per byte of 4-bit bases; up to 3 bytes of padding per read
-static int64_t expanded_seq_bytes(const smc_reads_soa* R) {
-    return seq_bits_of(R) == 4 ? R->seq_bytes : 2 * R->seq_bytes + 4 * R->n_reads + 16;
-}
-static int64_t expanded_qual_bytes(const smc_reads_soa* R) {
-    return qual_bits_of(R) == 8 ? R->qual_bytes : 2 * (seq_bits_of(R) == 4 ? R->seq_bytes : 2 * R->seq_bytes) + 4 * R->n_reads + 16;
+// words of bq[] a batch may need: a read stores (len + 1) / 2 bytes of 4-bit bases or (len + 3) / 4 bytes of 2-bit ones, and is
+// padded to a multiple of four words
+static int64_t bq_capacity(const smc_reads_soa* R) {
+    return (seq_bits_of(R) == 4 ? 2 : 4) * R->seq_bytes + 4 * R->n_reads + 16;
 }
 
 // Every argument check of an upload.  It runs before anything is queued, so a rejected batch leaves the context as it was.
@@ -562,7 +561,7 @@ static int check_upload(const smc_reads_soa* R, const smc_loci* Lc, std::string&
         err = "smc_upload: ref_id_bits must be 0, 8 or 32 and umi_bits 0, 32 or 64"; return SMC_E_ARG;
     }
     if ((R->store_lo == nullptr) != (R->store_len == nullptr)) { err = "smc_upload: store_lo and store_len must be given together"; return SMC_E_ARG; }
-    if (expanded_seq_bytes(R) >= (1ll << 32) || expanded_qual_bytes(R) >= (1ll << 32)) {
+    if (bq_capacity(R) >= (1ll << 32)) {
         err = "smc_upload: the expanded bases / qualities of the batch exceed 4 GiB; split the batch"; return SMC_E_LIMIT;
     }
     return SMC_OK;
@@ -624,22 +623,21 @@ static int pack_offsets(smc_ctx* ctx, int64_t n, int kind, int qbits, uint32_t* 
 // k_unpack grid (grid-stride over the reads): 8 blocks of 256 threads on each of the 148 SMs of a B200
 static constexpr unsigned UNPACK_GRID = 148u * 8u;
 
-// Compact bases / qualities -> the expanded d_seq / d_qual, for the reads of upload chunk c: d_small words
-// SW_CHUNK_READS_SEQ + c, + c + 1 (bases) and SW_CHUNK_READS + c, + c + 1 (qualities) hold its first read and its end.
-static void expand_compact(smc_ctx* ctx, int c, unsigned grid) {
-    uint32_t* small = ctx->d_small.as<uint32_t>();
+// Uploaded bases / qualities -> bq[], for the reads expanded with upload chunk c (k_chunk_need; a one-chunk upload: all reads).
+static void expand_payload(smc_ctx* ctx, int c, unsigned grid) {
+    const int G = ctx->pipe_n > 1 ? ctx->pipe_n : 1;
+    const uint32_t* first = G > 1 ? ctx->d_small.as<uint32_t>() + SW_CHUNK_FIRST : nullptr;
+    const int64_t n = ctx->n_reads;
     const int32_t* store_len = ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr;
-    if (ctx->seq_bits == 2) {           // compact bases -> nibbles, then the exceptions
-        LAUNCH(k_unpack<2>, grid, 256, 0, small + SW_CHUNK_READS_SEQ + c, ctx->d_seq_poff.as<uint32_t>(), ctx->d_seq_off.as<int64_t>(),
-               ctx->d_lseq.as<int32_t>(), store_len, nullptr, ctx->d_seq_packed.as<uint8_t>(), ctx->d_seq.as<uint8_t>());
-        LAUNCH(k_patch_seq, nblk(ctx->n_seq_exc, 256), 256, 0, small + SW_CHUNK_READS_SEQ + c, ctx->n_seq_exc, ctx->d_exc_read.as<uint32_t>(),
-               ctx->d_exc_pos.as<uint32_t>(), ctx->d_exc_nib.as<uint8_t>(), ctx->d_seq_off.as<int64_t>(), ctx->d_seq.as<uint8_t>());
-    }
-    if (ctx->qual_bits != 8) {          // compact qualities -> bytes
-        auto unpack = ctx->qual_bits == 2 ? k_unpack<0> : k_unpack<1>;
-        LAUNCH(unpack, grid, 256, 0, small + SW_CHUNK_READS + c, ctx->d_qual_poff.as<uint32_t>(), ctx->d_qual_off.as<int64_t>(),
-               ctx->d_lseq.as<int32_t>(), store_len, ctx->d_qual_lut.as<uint8_t>(), ctx->d_qual_packed.as<uint8_t>(), ctx->d_qual.as<uint8_t>());
-    }
+    const bool b2 = ctx->seq_bits == 2;
+    auto unpack = ctx->qual_bits == 2 ? (b2 ? k_unpack<2, 2> : k_unpack<2, 4>) : ctx->qual_bits == 4 ? (b2 ? k_unpack<4, 2> : k_unpack<4, 4>)
+                                      : (b2 ? k_unpack<8, 2> : k_unpack<8, 4>);
+    LAUNCH(unpack, grid, 256, 0, first, c, G, n, ctx->d_seq_poff.as<uint32_t>(), ctx->d_qual_poff.as<uint32_t>(), ctx->d_bq_off.as<uint32_t>(),
+           ctx->bq_cap, ctx->d_lseq.as<int32_t>(), store_len, ctx->d_qual_lut.as<uint8_t>(), ctx->d_seq_up.as<uint8_t>(),
+           ctx->d_qual_up.as<uint8_t>(), ctx->d_bq.as<uint16_t>());
+    if (b2)                             // the bases of 2-bit uploads that are not A / C / G / T
+        LAUNCH(k_patch_seq, nblk(ctx->n_seq_exc, 256), 256, 0, first, c, G, n, ctx->n_seq_exc, ctx->d_exc_read.as<uint32_t>(),
+               ctx->d_exc_pos.as<uint32_t>(), ctx->d_exc_nib.as<uint8_t>(), ctx->d_bq_off.as<uint32_t>(), ctx->bq_cap, ctx->d_bq.as<uint16_t>());
 }
 
 // pipelined = false: everything on ctx->st, synchronised on return (smc_upload).
@@ -691,42 +689,33 @@ static int queue_upload(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc
     for (int k = 0; k < n_narrow; ++k) widen(ctx, ctx->d_stage.as<uint8_t>() + narrow[k].stage_off, narrow[k].bytes, n, narrow[k].dst->p);
     const int qbits = qual_bits_of(R), sbits = seq_bits_of(R);
     ctx->qual_bits = qbits; ctx->seq_bits = sbits; ctx->n_seq_exc = sbits == 2 ? R->n_seq_exc : 0;
-    // offsets: uploaded, or -- NULL = payload packed in read order -- computed here from l_seq / n_cigar (saves 24 B per read of PCIe)
+    // offsets: uploaded, or -- NULL = payload packed in read order -- computed here from l_seq / n_cigar (saves 24 B per read of
+    // PCIe).  Bases and qualities: 32-bit byte offsets into the uploaded arrays (the caller's 64-bit ones are narrowed below).
     ctx->packed_seq = !R->seq_off; ctx->packed_qual = !R->qual_off; ctx->packed_cigar = !R->cigar_off;
-    const int64_t* host_off[3] = {R->seq_off, R->qual_off, R->cigar_off};
-    DevBuf* dev_off[3] = {&ctx->d_seq_off, &ctx->d_qual_off, &ctx->d_cig_off};
-    for (int kind = 0; kind < 3; ++kind) {
-        if (host_off[kind]) { CK(up.copy(*dev_off[kind], host_off[kind], (size_t)n * 8)); continue; }
-        CK(dev_off[kind]->ensure(nz * 8));
-        CK(ctx->d_v0.ensure(nz * 4));
-        // compact payloads are expanded into a device-only layout with every read on a word boundary (k_unpack)
-        const int layout = (kind == 0 && sbits == 2) ? 5 : (kind == 1 && qbits != 8) ? 6 : kind;
-        if (const int rc = pack_offsets(ctx, n, layout, 8, ctx->d_v0.as<uint32_t>(), kind)) return rc;
-        widen(ctx, ctx->d_v0.p, 4, n, dev_off[kind]->p);
+    CK(ctx->d_seq_poff.ensure(nz * 4)); CK(ctx->d_qual_poff.ensure(nz * 4));
+    if (R->seq_off) CK(up.copy(ctx->d_seq_off, R->seq_off, (size_t)n * 8));
+    else if (const int rc = pack_offsets(ctx, n, sbits == 2 ? 4 : 0, 8, ctx->d_seq_poff.as<uint32_t>(), sbits == 2 ? 4 : 0)) return rc;
+    if (R->qual_off) CK(up.copy(ctx->d_qual_off, R->qual_off, (size_t)n * 8));
+    else if (const int rc = pack_offsets(ctx, n, qbits == 8 ? 1 : 3, qbits, ctx->d_qual_poff.as<uint32_t>(), qbits == 8 ? 1 : 3)) return rc;
+    if (R->cigar_off) CK(up.copy(ctx->d_cig_off, R->cigar_off, (size_t)n * 8));
+    else {
+        CK(ctx->d_cig_off.ensure(nz * 8)); CK(ctx->d_v0.ensure(nz * 4));
+        if (const int rc = pack_offsets(ctx, n, 2, 8, ctx->d_v0.as<uint32_t>(), 2)) return rc;
+        widen(ctx, ctx->d_v0.p, 4, n, ctx->d_cig_off.p);
     }
-    if (qbits != 8) {          // byte offsets of the compact qualities inside the uploaded array
-        CK(ctx->d_qual_poff.ensure(nz * 4));
-        if (const int rc = pack_offsets(ctx, n, 3, qbits, ctx->d_qual_poff.as<uint32_t>(), 3)) return rc;
+    // the device layout: every read on a multiple of four bq[] words
+    ctx->bq_cap = (uint32_t)bq_capacity(R);
+    CK(ctx->d_bq_off.ensure(nz * 4)); CK(ctx->d_bq.ensure((size_t)ctx->bq_cap * 2));
+    if (const int rc = pack_offsets(ctx, n, 5, 8, ctx->d_bq_off.as<uint32_t>(), 5)) return rc;
+    if (qbits != 8) {
         CK(ctx->d_qual_lut.ensure(16));
         CK(cudaMemcpyAsync(ctx->d_qual_lut.p, R->qual_lut, qbits == 4 ? 16 : 4, cudaMemcpyHostToDevice, ctx->st));
     }
-    if (sbits == 2) {          // byte offsets of the compact bases inside the uploaded array, and their exceptions
-        CK(ctx->d_seq_poff.ensure(nz * 4));
-        if (const int rc = pack_offsets(ctx, n, 4, 2, ctx->d_seq_poff.as<uint32_t>(), 4)) return rc;
+    if (sbits == 2) {          // the exceptions of the compact bases
         CK(up.copy(ctx->d_exc_read, R->seq_exc_read, (size_t)R->n_seq_exc * 4)); CK(up.copy(ctx->d_exc_pos, R->seq_exc_pos, (size_t)R->n_seq_exc * 4));
         CK(up.copy(ctx->d_exc_nib, R->seq_exc_nib, (size_t)R->n_seq_exc));
     }
-    DevBuf& seq_up = sbits == 4 ? ctx->d_seq : ctx->d_seq_packed;              // where the caller's seq[] bytes land
-    if (sbits == 2) CK(ctx->d_seq.ensure((size_t)expanded_seq_bytes(R) + 16));
-    DevBuf& qual_up = qbits == 8 ? ctx->d_qual : ctx->d_qual_packed;           // where the caller's qual[] bytes land
-    if (qbits != 8) CK(ctx->d_qual.ensure((size_t)expanded_qual_bytes(R) + 16));
-    if (G == 1) {
-        CK(up.copy(seq_up, R->seq, (size_t)R->seq_bytes)); CK(up.copy(qual_up, R->qual, (size_t)R->qual_bytes));
-        const uint32_t whole[2] = {0u, (uint32_t)n};                            // the one chunk: reads [0, n)
-        if (sbits == 2) CK(cudaMemcpyAsync(ctx->d_small.as<uint32_t>() + SW_CHUNK_READS_SEQ, whole, 8, cudaMemcpyHostToDevice, ctx->st));
-        if (qbits != 8) CK(cudaMemcpyAsync(ctx->d_small.as<uint32_t>() + SW_CHUNK_READS, whole, 8, cudaMemcpyHostToDevice, ctx->st));
-        expand_compact(ctx, 0, std::min<unsigned>(nblk(n, 256) + 1u, UNPACK_GRID));
-    }
+    if (G == 1) { CK(up.copy(ctx->d_seq_up, R->seq, (size_t)R->seq_bytes)); CK(up.copy(ctx->d_qual_up, R->qual, (size_t)R->qual_bytes)); }
     CK(up.copy(ctx->d_cigar, R->cigar, (size_t)R->n_cigar_words * 4));
     CK(up.copy(ctx->d_loci_ref, Lc->ref_id, (size_t)nl * 4)); CK(up.copy(ctx->d_loci_pos, Lc->pos0, (size_t)nl * 4));
     CK(up.copy(ctx->d_loci_base, Lc->ref_base, (size_t)nl));
@@ -737,6 +726,13 @@ static int queue_upload(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc
         CK(up.copy(ctx->d_k0, K->locus, (size_t)K->n_loci * 8));              // d_k0 doubles as the staging buffer of the masked-locus list
     }
     CK(up.hand_over());
+    {
+        auto narrow = k_widen<int64_t, uint32_t>;
+        if (R->seq_off) LAUNCH(narrow, nblk(n, 256), 256, 0, ctx->d_seq_off.as<int64_t>(), n, ctx->d_seq_poff.as<uint32_t>());
+        if (R->qual_off) LAUNCH(narrow, nblk(n, 256), 256, 0, ctx->d_qual_off.as<int64_t>(), n, ctx->d_qual_poff.as<uint32_t>());
+    }
+    ctx->n_reads = n; ctx->n_loci = nl;
+    if (G == 1) expand_payload(ctx, 0, std::min<unsigned>(nblk(n, 256) + 1u, UNPACK_GRID));
     if (ctx->has_keep) {
         CK(ctx->d_keep_idx.ensure((size_t)(nl ? nl : 1) * 4));
         LAUNCH(k_fill_i32, nblk(nl, 256), 256, 0, ctx->d_keep_idx.as<int32_t>(), nl, -1);
@@ -744,7 +740,6 @@ static int queue_upload(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc
     }
     CK(ctx->d_loci_key.ensure((size_t)(nl ? nl : 1) * 8));
     LAUNCH(k_loci_keys, nblk(nl, 256), 256, 0, ctx->d_loci_ref.as<int32_t>(), ctx->d_loci_pos.as<int32_t>(), nl, ctx->d_loci_key.as<uint64_t>());
-    ctx->n_reads = n; ctx->n_loci = nl;
     ctx->seq_bytes = R->seq_bytes; ctx->qual_bytes = R->qual_bytes; ctx->n_cigar_words = R->n_cigar_words;
     ctx->tm = smc_timings{};
     ctx->tm.n_reads = n; ctx->tm.n_loci = nl;
@@ -756,20 +751,21 @@ static int queue_upload(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc
         }
     } else {
         // the chunks follow the scalars on the link; everything up to the first pileup launch needs the scalars only
-        CK(up.ensure(seq_up, (size_t)R->seq_bytes + 16)); CK(up.ensure(qual_up, (size_t)R->qual_bytes + 16));
+        CK(up.ensure(ctx->d_seq_up, (size_t)R->seq_bytes + 16)); CK(up.ensure(ctx->d_qual_up, (size_t)R->qual_bytes + 16));
         auto chunk_bytes = [&](int64_t total) { int64_t c = (total + G - 1) / G; c = (c + 255) & ~255ll; return (uint32_t)std::max<int64_t>(c, 256); };
-        ctx->pipe_seq_chunk = chunk_bytes(R->seq_bytes); ctx->pipe_qual_chunk = chunk_bytes(R->qual_bytes);
-        if (qbits != 8)            // which reads each chunk completes (the compact payload is in read order)
-            LAUNCH(k_chunk_reads, 1, 32, 0, ctx->d_qual_poff.as<uint32_t>(), n, (uint32_t)R->qual_bytes, ctx->pipe_qual_chunk, G,
-                   ctx->d_small.as<uint32_t>() + SW_CHUNK_READS);
-        if (sbits == 2)
-            LAUNCH(k_chunk_reads, 1, 32, 0, ctx->d_seq_poff.as<uint32_t>(), n, (uint32_t)R->seq_bytes, ctx->pipe_seq_chunk, G,
-                   ctx->d_small.as<uint32_t>() + SW_CHUNK_READS_SEQ);
+        const uint32_t seq_chunk = chunk_bytes(R->seq_bytes), qual_chunk = chunk_bytes(R->qual_bytes);
+        // which reads each chunk lets k_unpack expand (k_read_prep turns it into the chunk every read's units wait for)
+        uint32_t none[SMC_PIPE_MAX];
+        for (int c = 0; c < SMC_PIPE_MAX; ++c) none[c] = (uint32_t)n;
+        CK(cudaMemcpyAsync(ctx->d_small.as<uint32_t>() + SW_CHUNK_FIRST, none, sizeof(none), cudaMemcpyHostToDevice, ctx->st));
+        LAUNCH(k_chunk_need, nblk(n, 256), 256, 0, ctx->d_seq_poff.as<uint32_t>(), ctx->d_qual_poff.as<uint32_t>(), ctx->d_lseq.as<int32_t>(),
+               ctx->has_store ? ctx->d_store_len.as<int32_t>() : nullptr, n, sbits, qbits, seq_chunk, qual_chunk, G,
+               ctx->d_small.as<uint32_t>() + SW_CHUNK_FIRST);
         for (int c = 0; c < G; ++c) {
-            const int64_t s0 = std::min<int64_t>(R->seq_bytes, (int64_t)c * ctx->pipe_seq_chunk), s1 = std::min<int64_t>(R->seq_bytes, (int64_t)(c + 1) * ctx->pipe_seq_chunk);
-            const int64_t q0 = std::min<int64_t>(R->qual_bytes, (int64_t)c * ctx->pipe_qual_chunk), q1 = std::min<int64_t>(R->qual_bytes, (int64_t)(c + 1) * ctx->pipe_qual_chunk);
-            CK(up.copy(seq_up.as<uint8_t>() + s0, R->seq + s0, (size_t)(s1 - s0)));
-            CK(up.copy(qual_up.as<uint8_t>() + q0, R->qual + q0, (size_t)(q1 - q0)));
+            const int64_t s0 = std::min<int64_t>(R->seq_bytes, (int64_t)c * seq_chunk), s1 = std::min<int64_t>(R->seq_bytes, (int64_t)(c + 1) * seq_chunk);
+            const int64_t q0 = std::min<int64_t>(R->qual_bytes, (int64_t)c * qual_chunk), q1 = std::min<int64_t>(R->qual_bytes, (int64_t)(c + 1) * qual_chunk);
+            CK(up.copy(ctx->d_seq_up.as<uint8_t>() + s0, R->seq + s0, (size_t)(s1 - s0)));
+            CK(up.copy(ctx->d_qual_up.as<uint8_t>() + q0, R->qual + q0, (size_t)(q1 - q0)));
             CK(cudaEventRecord(ctx->ev_chunk[c], ctx->st_copy));
         }
         CK(cudaEventRecord(ctx->ev[EV_COPY_END], ctx->st_copy));
@@ -870,7 +866,7 @@ static int read_prep(smc_ctx* ctx, const uint32_t* inv) {
     P.n_reads = n; P.inv = inv; P.urank = ctx->d_urank.as<uint32_t>(); P.frank = ctx->d_frank.as<uint32_t>();
     P.ref_id = ctx->d_ref_id.as<int32_t>(); P.pos = ctx->d_pos.as<int32_t>(); P.flag = ctx->d_flag.as<uint16_t>();
     P.mapq = ctx->d_mapq.as<uint8_t>(); P.nm = ctx->d_nm.as<int32_t>(); P.l_seq = ctx->d_lseq.as<int32_t>();
-    P.seq_off = ctx->d_seq_off.as<int64_t>(); P.qual_off = ctx->d_qual_off.as<int64_t>(); P.cigar_off = ctx->d_cig_off.as<int64_t>();
+    P.bq_off = ctx->d_bq_off.as<uint32_t>(); P.cigar_off = ctx->d_cig_off.as<int64_t>();
     P.n_cigar = ctx->d_ncig.as<uint16_t>(); P.cigar = ctx->d_cigar.as<uint32_t>();
     if (ctx->has_store) { P.store_lo = ctx->d_store_lo.as<int32_t>(); P.store_len = ctx->d_store_len.as<int32_t>(); }
     P.loci_key = ctx->d_loci_key.as<uint64_t>(); P.n_loci = ctx->n_loci;
@@ -878,19 +874,16 @@ static int read_prep(smc_ctx* ctx, const uint32_t* inv) {
     P.recs = ctx->d_recs.as<ReadRec>(); P.grec = ctx->d_grec.as<GRec>(); P.gflags = small + SW_GFLAGS;
     if (ctx->pipe_n > 1) {
         CK(ctx->d_pipe_need.ensure((size_t)n));
-        P.pipe_need = ctx->d_pipe_need.as<uint8_t>(); P.pipe_n = (uint32_t)ctx->pipe_n;
-        P.pipe_seq_chunk = ctx->pipe_seq_chunk; P.pipe_qual_chunk = ctx->pipe_qual_chunk;
-        if (ctx->qual_bits != 8) { P.qual_poff = ctx->d_qual_poff.as<uint32_t>(); P.qual_bits = ctx->qual_bits; }
-        if (ctx->seq_bits == 2) P.seq_poff = ctx->d_seq_poff.as<uint32_t>();
+        P.pipe_need = ctx->d_pipe_need.as<uint8_t>(); P.pipe_n = (uint32_t)ctx->pipe_n; P.chunk_first = small + SW_CHUNK_FIRST;
     }
     CK(cudaEventRecord(ctx->ev[EV_READ_PREP_BEGIN], ctx->st));
     LAUNCH(k_read_prep, nblk(n, 256), 256, 0, P);
     CK(cudaEventRecord(ctx->ev[EV_READ_PREP_DONE], ctx->st));
-    ctx->tm.read_prep_bytes = n * (int64_t)(4 + 4 + 2 + 1 + 4 + 4 + 8 + 8 + 8 + 2 + (ctx->has_store ? 8 : 0) + 4 + sizeof(ReadRec) + sizeof(GRec)) + 4 * ctx->n_cigar_words;
+    ctx->tm.read_prep_bytes = n * (int64_t)(4 + 4 + 2 + 1 + 4 + 4 + 4 + 8 + 2 + (ctx->has_store ? 8 : 0) + 4 + sizeof(ReadRec) + sizeof(GRec)) + 4 * ctx->n_cigar_words;
     return SMC_OK;
 }
 
-// The input checks only the device can make, from d_small words 0 .. SW_PACK_TOTALS + 4 as the read sort, k_read_prep and the
+// The input checks only the device can make, from d_small words 0 .. SW_PACK_TOTALS + 5 as the read sort, k_read_prep and the
 // upload left them (w[i] = word i).
 static int check_device_inputs(smc_ctx* ctx, const uint32_t* w) {
     const uint32_t gflags = w[SW_GFLAGS];
@@ -906,6 +899,10 @@ static int check_device_inputs(smc_ctx* ctx, const uint32_t* w) {
     if ((ctx->packed_seq && (int64_t)tot[ctx->seq_bits == 2 ? 4 : 0] != ctx->seq_bytes) || (ctx->packed_qual && (int64_t)tot[ctx->qual_bits != 8 ? 3 : 1] != ctx->qual_bytes) ||
         (ctx->packed_cigar && (int64_t)tot[2] != ctx->n_cigar_words)) {
         ctx->err = "packed payload (NULL offsets): seq_bytes / qual_bytes / n_cigar_words do not match the sums of (len+1)/2, len, n_cigar (len = store_len or l_seq)";
+        return SMC_E_ARG;
+    }
+    if (tot[5] > ctx->bq_cap) {             // only a caller's offsets can get here: the packed sizes bound the words
+        ctx->err = "the reads' bases (l_seq or store_len) need more room than seq_bytes provides";
         return SMC_E_ARG;
     }
     return SMC_OK;
@@ -930,7 +927,7 @@ static int expand_tile_events(smc_ctx* ctx) {
 static int tile_events(smc_ctx* ctx) {
     if (ctx->ne_cap < 4 * ctx->n_reads + 4096) ctx->ne_cap = 4 * ctx->n_reads + 4096;
     if (const int rc = expand_tile_events(ctx)) return rc;
-    uint32_t w[SW_PACK_TOTALS + 5];
+    uint32_t w[SW_PACK_TOTALS + 6];
     if (const int rc = read_back(ctx, w, ctx->d_small.p, sizeof(w))) return rc;
     if (const int rc = check_device_inputs(ctx, w)) return rc;
     ctx->tm.n_umi_groups = w[SW_N_UMI];
@@ -1003,7 +1000,7 @@ static DynTab make_dyntab(smc_ctx* ctx) {
     T.dkey = ctx->d_dkey.as<unsigned long long>(); T.dmask = ctx->dyn_cap - 1; T.drep_read = ctx->d_drep_read.as<uint32_t>();
     T.drep_qpos = ctx->d_drep_qpos.as<int32_t>(); T.dlen = ctx->d_dlen.as<int32_t>(); T.dcnt = ctx->d_dcnt.as<int32_t>();
     T.dlimb = ctx->d_dlimb.as<unsigned long long>(); T.diskey = ctx->d_diskey.as<uint8_t>(); T.dcount = small + SW_DYN_COUNT; T.gflags = small + SW_GFLAGS;
-    T.seq = ctx->d_seq.as<uint8_t>(); T.seq_off = ctx->d_seq_off.as<int64_t>();
+    T.bq = ctx->d_bq.as<uint16_t>(); T.bq_off = ctx->d_bq_off.as<uint32_t>();
     T.spill = ctx->d_spill.as<SpillRec>(); T.spill_cap = ctx->spill_cap; T.spill_count = small + SW_SPILL_COUNT;
     return T;
 }
@@ -1025,7 +1022,7 @@ static void fill_kargs(smc_ctx* ctx, KAArgs& A, KBArgs& B, bool list, bool need_
     A.unit_eb = ctx->d_unit_eb.as<uint32_t>(); A.unit_ee = ctx->d_unit_ee.as<uint32_t>(); A.unit_tile = ctx->d_unit_tile.as<uint32_t>();
     A.n_units = ctx->n_units_cap; A.code_mult = ctx->code_mult;
     A.loci_pos = ctx->d_loci_pos.as<int32_t>(); A.n_loci = ctx->n_loci;
-    A.seq = ctx->d_seq.as<uint8_t>(); A.qual = ctx->d_qual.as<uint8_t>(); A.cigar = ctx->d_cigar.as<uint32_t>();
+    A.bq = ctx->d_bq.as<uint16_t>(); A.cigar = ctx->d_cigar.as<uint32_t>();
     A.minBQ = ctx->prm.minBQ; A.primerDist = ctx->prm.primerDist;
     A.codes = ctx->d_codes.as<uint4>(); A.unit_nfrag = ctx->d_unit_nfrag.as<uint32_t>();
     A.frag_first = list ? ctx->d_frag_first.as<uint32_t>() : nullptr;
@@ -1048,7 +1045,7 @@ static void fill_kargs(smc_ctx* ctx, KAArgs& A, KBArgs& B, bool list, bool need_
 }
 
 // k_gather + k_merge over units [0, n_units_cap): one pair, or for a chunked upload one pair per range [pipe_end[c-1],
-// pipe_end[c]) that starts once chunk c is in (after expanding its compact payload when `expand`).  `gather_done`, unless null,
+// pipe_end[c]) that starts once chunk c is in (after expanding its reads' bases and qualities when `expand`).  `gather_done`, unless null,
 // is recorded between the kernels of the one pair, or after the last pair of a chunked run.
 template <bool LIST>
 static int launch_pileup(smc_ctx* ctx, KAArgs& A, KBArgs& B, bool chunked, bool expand, cudaEvent_t gather_done) {
@@ -1057,7 +1054,7 @@ static int launch_pileup(smc_ctx* ctx, KAArgs& A, KBArgs& B, bool chunked, bool 
     for (int c = 0; c < (chunked ? ctx->pipe_n : 1); ++c) {
         if (chunked) {
             CK(cudaStreamWaitEvent(ctx->st, ctx->ev_chunk[c], 0));
-            if (expand) expand_compact(ctx, c, UNPACK_GRID);
+            if (expand) expand_payload(ctx, c, UNPACK_GRID);
         }
         const uint32_t u1 = chunked ? ctx->pipe_end[c] : ctx->n_units_cap;
         if (u1 <= u0) continue;

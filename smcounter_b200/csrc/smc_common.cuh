@@ -23,8 +23,8 @@ struct __align__(16) ReadRec {
                          // other reads: leftSP (low 16) | query_alignment_length (high 16)
     uint32_t meta;       // bit0 passes MQ+mismatch gate, bit1 reverse, bit2 read2, bit3 single ref-consuming M run; bits 8.. n_cigar
     // word 4-7
-    uint32_t seq_off;    // byte offset into seq[]
-    uint32_t qual_off;   // byte offset into qual[]
+    uint32_t bq_off;     // word of query position 0 in bq[] (quality | BAM nibble << 8 per stored base; wrapping 32-bit arithmetic)
+    uint32_t unused;
     int32_t  start;      // 0-based leftmost reference position
     int32_t  hi;
     // word 8-11

@@ -22,13 +22,13 @@
 // ------------------------------------------------------------------------------------------------------------
 
 // The 32 bytes of a read the gather loop needs (the 64-byte ReadRec keeps everything, for the rare paths).  Everything that is
-// the same for all 32 loci of a tile is resolved here, once per read: the byte offsets of query position 0 folded into the
-// payload offsets, and the two "distance to an end" windows of smCounter.py:432-452 as ranges of covered-locus indices.
+// the same for all 32 loci of a tile is resolved here, once per read: the query offset folded into the payload offset, and the
+// two "distance to an end" windows of smCounter.py:432-452 as ranges of covered-locus indices.
 struct __align__(16) GRec {
     int32_t  lo;         // first covered locus index
     uint32_t gspan_fl;   // bits 0-15: simple reads hi - lo, other reads 0 (the gather loop never covers them); bits 16.. GR_* flags
-    uint32_t seq_base;   // the base of reference position p is nibble (p + b) & 1 of seq[seq_base + ((p + b) >> 1)], b = GR_ODD
-    uint32_t qual_base;  // its quality is qual[qual_base + p]                                   (all wrapping 32-bit arithmetic)
+    uint32_t bq_base;    // quality | BAM nibble << 8 of reference position p is bq[bq_base + p]   (wrapping 32-bit arithmetic)
+    uint32_t unused;
     uint32_t le;         // covered loci [lo + (le & 0xffff), lo + (le >> 16)) are within 20 of the barcode end    (:432-452)
     uint32_t ple;        // R2: the same for "within primerDist of the primer end"; empty for R1
     uint32_t urank, frank;
@@ -38,7 +38,6 @@ static_assert(sizeof(GRec) == 32, "GRec must be 32 bytes");
 #define GR_REVERSE (1u << 17)
 #define GR_READ2   (1u << 18)
 #define GR_SIMPLE  (1u << 19)
-#define GR_ODD     (1u << 20)    // b: parity of leftSP - start
 
 struct PrepArgs {
     int64_t n_reads;
@@ -46,15 +45,13 @@ struct PrepArgs {
     const uint32_t* urank;        // per srank
     const uint32_t* frank;
     const int32_t* ref_id; const int32_t* pos; const uint16_t* flag; const uint8_t* mapq; const int32_t* nm;
-    const int32_t* l_seq; const int64_t* seq_off; const int64_t* qual_off; const int64_t* cigar_off;
+    const int32_t* l_seq; const uint32_t* bq_off; const int64_t* cigar_off;   // bq_off: word of the stored window's first base in bq[]
     const int32_t* store_lo; const int32_t* store_len;     // optional stored window of the read's bases / qualities (nullptr: whole read)
     const uint16_t* n_cigar; const uint32_t* cigar;
     const uint64_t* loci_key; int64_t n_loci;
     int minMQ; int primerDist; double mismatchThr;
     ReadRec* recs; GRec* grec; uint32_t* gflags;
-    uint8_t* pipe_need; uint32_t pipe_n, pipe_seq_chunk, pipe_qual_chunk;     // pipelined upload only (else pipe_need == nullptr)
-    const uint32_t* qual_poff; int qual_bits;                                 // compact qualities: their byte offsets in the uploaded array
-    const uint32_t* seq_poff;                                                 // compact (2-bit) bases: likewise
+    uint8_t* pipe_need; uint32_t pipe_n; const uint32_t* chunk_first;       // pipelined upload only (else pipe_need == nullptr)
 };
 
 #define GF_DYN_FULL   1u
@@ -106,15 +103,16 @@ __global__ void __launch_bounds__(256) k_read_prep(PrepArgs A) {
     rec.start = start; rec.lo = (int32_t)lo; rec.hi = (int32_t)hi;
     const bool rev = fl & 0x10u, r2 = fl & 0x80u;
     rec.meta = (ok ? RM_OK : 0u) | (rev ? RM_REVERSE : 0u) | (r2 ? RM_READ2 : 0u) | (simple ? RM_SIMPLE : 0u) | (ncig << 8);
-    // Stored window: bases [slo, slo + slen) of the read are in seq[] / qual[] (slo even).  The record keeps the offset of the
-    // read's (virtual) base 0, so that every later access is offset + query position in wrapping 32-bit arithmetic.
+    // Stored window: bases [slo, slo + slen) of the read are in bq[] (slo even: the uploaded 4-bit bases start on a byte).  The
+    // record keeps the offset of the read's (virtual) base 0, so that every later access is offset + query position in wrapping
+    // 32-bit arithmetic.
     const int32_t slo = A.store_lo ? A.store_lo[r] : 0, slen = A.store_len ? A.store_len[r] : lseq;
     if (slo < 0 || (slo & 1) || slen < 0 || slo + slen > lseq || (!simple && (slo != 0 || slen != lseq))) { atomicOr(A.gflags, GF_BAD_STORE); lo = hi = 0; }
     else if (simple && hi > lo) {          // every target base of the read must be stored: query position = p + leftSP - start
         const int32_t q0 = (int32_t)(uint32_t)A.loci_key[lo] + leftSP - start, q1 = (int32_t)(uint32_t)A.loci_key[hi - 1] + leftSP - start;
         if (q0 < slo || q1 >= slo + slen) { atomicOr(A.gflags, GF_BAD_STORE); lo = hi = 0; }
     }
-    rec.seq_off = (uint32_t)A.seq_off[r] - (uint32_t)(slo >> 1); rec.qual_off = (uint32_t)A.qual_off[r] - (uint32_t)slo;
+    rec.bq_off = A.bq_off[r] - (uint32_t)slo; rec.unused = 0u;
     rec.cigar_off = (uint32_t)co;
     rec.urank = A.urank[s]; rec.frank = A.frank[s];
     rec.read_idx = r; rec.gspan = simple ? (uint32_t)(hi - lo) : 0u;
@@ -123,13 +121,12 @@ __global__ void __launch_bounds__(256) k_read_prep(PrepArgs A) {
     GRec g;
     g.lo = (int32_t)lo;
     g.gspan_fl = rec.gspan | (ok ? GR_OK : 0u) | (rev ? GR_REVERSE : 0u) | (r2 ? GR_READ2 : 0u) | (simple ? GR_SIMPLE : 0u);
-    g.seq_base = rec.seq_off; g.qual_base = rec.qual_off; g.le = 0u; g.ple = 0u;
+    g.bq_base = rec.bq_off; g.unused = 0u; g.le = 0u; g.ple = 0u;
     g.urank = rec.urank; g.frank = rec.frank;
     if (simple && hi > lo) {
         // One aligned run: the query position of reference position p is p + qk, qk = leftSP - start.
         const int32_t qk = leftSP - start;
-        g.seq_base = rec.seq_off + (uint32_t)(qk >> 1); g.qual_base = rec.qual_off + (uint32_t)qk;
-        if (qk & 1) g.gspan_fl |= GR_ODD;
+        g.bq_base = rec.bq_off + (uint32_t)qk;
         // d = p - start is the distance from the alignment start, alnlen - d from its end.
         //   R1: distToBcEnd = rev ? alnlen - d : d;   R2: distToBcEnd = rev ? d : alnlen - d, distToPrimerEnd = rev ? alnlen - d : d
         // "<= X from the start" is the position window [start, start + X], "<= X from the end" is [start + alnlen - X, inf);
@@ -159,15 +156,9 @@ __global__ void __launch_bounds__(256) k_read_prep(PrepArgs A) {
         uint4* gd = reinterpret_cast<uint4*>(&A.grec[s]);
         gd[0] = gs[0]; gd[1] = gs[1];
     }
-    if (A.pipe_need) {                                         // last chunk that carries a byte of this read
+    if (A.pipe_need) {                                         // the chunk this read is expanded with (k_unpack)
         uint32_t c = 0;
-        if (slen > 0) {
-            const uint32_t cs = A.seq_poff ? (uint32_t)((A.seq_poff[r] + ((uint32_t)slen + 3u) / 4u - 1u) / A.pipe_seq_chunk)
-                                           : (uint32_t)(((uint32_t)A.seq_off[r] + ((uint32_t)slen + 1u) / 2u - 1u) / A.pipe_seq_chunk);
-            const uint32_t cq = A.qual_poff ? (uint32_t)((A.qual_poff[r] + ((uint32_t)slen * (uint32_t)A.qual_bits + 7u) / 8u - 1u) / A.pipe_qual_chunk)
-                                            : (uint32_t)(((uint32_t)A.qual_off[r] + (uint32_t)slen - 1u) / A.pipe_qual_chunk);
-            c = min(max(cs, cq), A.pipe_n - 1u);
-        }
+        for (uint32_t k = 1; k < A.pipe_n; ++k) if (A.chunk_first[k] <= (uint32_t)r) c = k;
         A.pipe_need[s] = (uint8_t)c;
     }
 }
@@ -201,9 +192,9 @@ k_unit_bounds(const uint32_t* __restrict__ tile_off, const uint32_t* __restrict_
 
 // ------------------------------------------------------------------------------------------------------------
 // Pipelined upload (smc_call_batch): bases and qualities arrive in up to SMC_PIPE_MAX chunks of equal byte size while the
-// read sort / prep / tile sort already run.  k_read_prep records, per read, the chunk that completes its bases AND its
-// qualities (PrepArgs::pipe_need); a unit may start once the latest chunk any of its reads needs is on the device.  Exact
-// for any payload layout; a payload stored in read order (a BAM decode) makes the units become ready front to back.
+// read sort / prep / tile sort already run.  k_read_prep records, per read, the chunk its bq[] words are expanded with
+// (PrepArgs::pipe_need, k_chunk_need); a unit may start once the latest chunk any of its reads needs is expanded.  Right for
+// any payload layout; a payload stored in read order (a BAM decode) makes the units become ready front to back.
 // ------------------------------------------------------------------------------------------------------------
 #define SMC_PIPE_MAX 16
 // first_blocked[c] = smallest unit that has to wait for chunk c + 1 (one warp per unit)
@@ -263,7 +254,8 @@ struct SpillRec { uint32_t e[NSPILL]; int32_t cnt[NSPILL]; double prod[NSPILL]; 
 struct DynTab {
     unsigned long long* dkey; uint32_t dmask; uint32_t* drep_read; int32_t* drep_qpos; int32_t* dlen;
     int32_t* dcnt; unsigned long long* dlimb; uint8_t* diskey; uint32_t* dcount; uint32_t* gflags;
-    const uint8_t* seq; const int64_t* seq_off;      // bases of every read (caller's SoA order): long insertions are compared base by base
+    const uint16_t* bq; const uint32_t* bq_off;      // bq[] and each read's first stored word (caller's SoA order): long insertions are
+                                                     // compared base by base
     SpillRec* spill; uint32_t spill_cap; uint32_t* spill_count;      // k_merge: pool of spill records (one per overflowing lane and barcode)
 };
 
@@ -296,9 +288,9 @@ __device__ __noinline__ uint32_t dyn_lookup(DynTab T, unsigned long long key, ui
 // Insertions longer than 8 bases do not fit the 64-bit key: the key carries a 32-bit hash of the inserted bases and every hit is
 // verified by length (dlen) and base by base against the entry's representative read (drep_read / drep_qpos); two different insertions with
 // equal hashes chain to separate entries, so alleles are never merged (collision free, like the short ones).
-// `my_seq0`: offset of this read's query position 0 in seq[]; the representative's comes from seq_off[] (reads with an
-// insertion are always stored whole).  drep_read doubles as the "entry published" flag (0xffffffff until the creator is done).
-__device__ __noinline__ uint32_t dyn_lookup_long_ins(DynTab T, unsigned long long key, uint32_t rep_read, int rep_qpos, int len, uint32_t my_seq0) {
+// `my_bq0`: word of this read's query position 0 in bq[]; the representative's comes from bq_off[] (reads with an insertion are
+// always stored whole).  drep_read doubles as the "entry published" flag (0xffffffff until the creator is done).
+__device__ __noinline__ uint32_t dyn_lookup_long_ins(DynTab T, unsigned long long key, uint32_t rep_read, int rep_qpos, int len, uint32_t my_bq0) {
     uint32_t h = hash64to32(key) & T.dmask;
     for (uint32_t probe = 0; probe <= T.dmask; ++probe) {
         unsigned long long cur = __ldcg(&T.dkey[h]);
@@ -319,15 +311,12 @@ __device__ __noinline__ uint32_t dyn_lookup_long_ins(DynTab T, unsigned long lon
             while ((rr = *reinterpret_cast<volatile uint32_t*>(&T.drep_read[h])) == 0xffffffffu) { }
             __threadfence();
             const int rq = *reinterpret_cast<volatile int32_t*>(&T.drep_qpos[h]);
-            const uint32_t rs0 = (uint32_t)T.seq_off[rr];
+            const uint32_t rs0 = T.bq_off[rr];
             // the key carries no length (only the hash seed does): an insertion that is a prefix of the entry's, or the entry's
             // plus more bases, must not match; with equal lengths the comparison also stays inside the representative's insertion
             bool eq = *reinterpret_cast<volatile int32_t*>(&T.dlen[h]) == len;
-            for (int t = 1; t <= len && eq; ++t) {
-                const int qa = rep_qpos + t, qb = rq + t;
-                const uint32_t ba = __ldg(T.seq + (uint32_t)(my_seq0 + (uint32_t)(qa >> 1))), bb = __ldg(T.seq + (uint32_t)(rs0 + (uint32_t)(qb >> 1)));
-                eq = ((qa & 1) ? (ba & 15u) : (ba >> 4)) == ((qb & 1) ? (bb & 15u) : (bb >> 4));
-            }
+            for (int t = 1; t <= len && eq; ++t)
+                eq = (__ldg(T.bq + (uint32_t)(my_bq0 + (uint32_t)(rep_qpos + t))) >> 8) == (__ldg(T.bq + (uint32_t)(rs0 + (uint32_t)(rq + t))) >> 8);
             if (eq) return h;
         }
         h = (h + 1) & T.dmask;
@@ -344,7 +333,7 @@ __device__ __noinline__ uint32_t dyn_lookup_long_ins(DynTab T, unsigned long lon
 //   stage    : lane k loads the GRec of event k and turns everything that is the same for all 32 loci into three 32-bit LANE
 //              MASKS (covered / within 20 of the barcode end / within primerDist of the primer end) and a tally class; barcode
 //              and fragment boundaries of the batch become warp-uniform bit masks (ranks of neighbouring events, ballots);
-//   gather   : KA_GATHER events at a time every lane loads the base nibble and the quality of ITS locus (independent loads:
+//   gather   : KA_GATHER events at a time every lane loads the quality | nibble word of ITS locus (independent loads:
 //              ILP + occupancy hide the latency), adds the event to a per-lane CLASS HISTOGRAM in shared memory (one
 //              fire-and-forget shared atomic: 16 classes = strand x {lowQ, not included, R1 x le20, R2 x le20 x ple}, the four
 //              bases as 8-bit fields of one word) and leaves a 16-bit event code (quality, allele slot, covered / included);
@@ -364,16 +353,17 @@ __device__ __noinline__ uint32_t dyn_lookup_long_ins(DynTab T, unsigned long lon
 #ifndef KA_GATHER
 #define KA_GATHER 4
 #endif
-// per-warp shared memory (words): event masks 32 x uint4 | payload bases 32 x uint2 | srank | event codes 32 x 32 x u16 |
+// per-warp shared memory (words): event masks 32 x uint4 | payload bases 32 | srank | event codes 32 x 32 x u16 |
 // fragment-code staging | class histogram 16 x 32 | (LIST) first-read staging
 #define KA_OFF_BASE  128
-#define KA_OFF_SRANK (KA_OFF_BASE + 64)
+#define KA_OFF_SRANK (KA_OFF_BASE + 32)
 #define KA_OFF_EVC   (KA_OFF_SRANK + 32)
 #define KA_OFF_CST   (KA_OFF_EVC + 512)
 #define KA_OFF_HIST  (KA_OFF_CST + 128)
 #define KA_OFF_FST   (KA_OFF_HIST + 512)
 #define KA_WARP_WORDS(LIST) (KA_OFF_FST + ((LIST) ? 256 : 0))
-#define KA_SMEM_BYTES(LIST) (64 + KA_WARPS * KA_WARP_WORDS(LIST) * 4)
+#define KA_LUT_WORDS 36             // the nibble table of k_gather: 17 x uint2, padded to 16 bytes
+#define KA_SMEM_BYTES(LIST) (KA_LUT_WORDS * 4 + KA_WARPS * KA_WARP_WORDS(LIST) * 4)
 
 // event code (internal to k_gather).  Staged codes of plain aligned reads: quality in bits 0-7, bits 8-11 the allele slot
 // (A0 C1 T3 G4, as in the fragment code) or, with EC_DYN, the BAM nibble of an N / IUPAC base; codes returned by slow_event:
@@ -397,7 +387,7 @@ struct KAArgs {
     uint32_t unit0, n_units;      // this launch covers units [unit0, n_units)
     uint32_t code_mult;
     const int32_t* loci_pos; int64_t n_loci;
-    const uint8_t* seq; const uint8_t* qual; const uint32_t* cigar;
+    const uint16_t* bq; const uint32_t* cigar;
     int minBQ, primerDist;
     uint4* codes; uint32_t* unit_nfrag;
     uint32_t* frag_first;         // LIST only: BAM index of the fragment's first passing read, per (slot, lane)
@@ -433,8 +423,7 @@ __device__ __noinline__ uint32_t dyn_base_event(DynTab T, uint32_t nib, uint32_t
 //   inside a deletion     : x = SMC_A_DEL, bq = minBQ (:416-421)
 //   insertion / deletion start (:371-411): x = NF + row; alleleCnt and strand are tallied here
 __device__ __noinline__ uint2 slow_event(DynTab T, const uint32_t* __restrict__ rw, const uint32_t* __restrict__ cigar,
-                                         const uint8_t* __restrict__ seqp, const uint8_t* __restrict__ qualp, int32_t p, int32_t Li,
-                                         int minBQ, int primerDist) {
+                                         const uint16_t* __restrict__ bqp, int32_t p, int32_t Li, int minBQ, int primerDist) {
     const uint32_t meta = __ldg(rw + 3);
     const int32_t start = (int32_t)__ldg(rw + 6), lo = (int32_t)__ldg(rw + 0), hi = (int32_t)__ldg(rw + 7);
     if (!(Li >= lo && Li < hi)) return make_uint2(0u, 0u);
@@ -442,7 +431,7 @@ __device__ __noinline__ uint2 slow_event(DynTab T, const uint32_t* __restrict__ 
     const uint32_t ncig = meta >> 8;
     const uint32_t spa = __ldg(rw + 2);
     const int leftSP = (int)(spa & 0xffffu), alnlen = (int)(spa >> 16);
-    const uint32_t seq_off = __ldg(rw + 4), qual_off = __ldg(rw + 5), cigar_off = __ldg(rw + 11);
+    const uint32_t bq_off = __ldg(rw + 4), cigar_off = __ldg(rw + 11);
     int qpos = 0, indel = 0; bool isdel = false;
     {
         int x = start, y = 0;
@@ -480,9 +469,8 @@ __device__ __noinline__ uint2 slow_event(DynTab T, const uint32_t* __restrict__ 
         const bool inc = (meta & RM_OK);                                       // bq = minBQ passes the quality gate
         return make_uint2(((uint32_t)minBQ & 255u) | EC_COVERED | (inc ? EC_INC : 0u), (uint32_t)SMC_A_DEL);
     }
-    const uint32_t sb = __ldg(seqp + (uint32_t)(seq_off + (uint32_t)(qpos >> 1)));
-    const uint32_t nib = (qpos & 1) ? (sb & 15u) : (sb >> 4);
-    const uint32_t bq = __ldg(qualp + (uint32_t)(qual_off + (uint32_t)qpos));
+    const uint32_t w = __ldg(bqp + (uint32_t)(bq_off + (uint32_t)qpos));
+    const uint32_t nib = w >> 8, bq = w & 255u;
     const bool lowq = (int)bq < minBQ;
     const bool inc = !lowq && (meta & RM_OK);                                  // :378,400,431
     uint32_t code = bq | (nib << EC_NIB_SH) | EC_COVERED | (inc ? EC_INC : 0u);
@@ -502,19 +490,13 @@ __device__ __noinline__ uint2 slow_event(DynTab T, const uint32_t* __restrict__ 
         unsigned long long payload;
         if (len <= 8) {
             unsigned long long nibs = 0;
-            for (int t = 0; t < len; ++t) {
-                const int qq = qpos + 1 + t;
-                const uint32_t b2 = __ldg(seqp + (uint32_t)(seq_off + (uint32_t)(qq >> 1)));
-                nibs |= (unsigned long long)((qq & 1) ? (b2 & 15u) : (b2 >> 4)) << (28 - 4 * t);
-            }
+            for (int t = 0; t < len; ++t)
+                nibs |= (unsigned long long)(__ldg(bqp + (uint32_t)(bq_off + (uint32_t)(qpos + 1 + t))) >> 8) << (28 - 4 * t);
             payload = ((unsigned long long)len << 32) | nibs;
         } else {
             uint32_t hsh = 2166136261u ^ (uint32_t)len;
-            for (int t = 0; t < len; ++t) {
-                const int qq = qpos + 1 + t;
-                const uint32_t b2 = __ldg(seqp + (uint32_t)(seq_off + (uint32_t)(qq >> 1)));
-                hsh = (hsh ^ ((qq & 1) ? (b2 & 15u) : (b2 >> 4))) * 16777619u;
-            }
+            for (int t = 0; t < len; ++t)
+                hsh = (hsh ^ (__ldg(bqp + (uint32_t)(bq_off + (uint32_t)(qpos + 1 + t))) >> 8)) * 16777619u;
             payload = (15ull << 32) | hsh;
         }
         key = dyn_make_key((uint32_t)Li, SMC_K_INS, nib, payload);
@@ -522,7 +504,7 @@ __device__ __noinline__ uint2 slow_event(DynTab T, const uint32_t* __restrict__ 
         len = -indel;
         key = dyn_make_key((uint32_t)Li, SMC_K_DEL, nib, (unsigned long long)len);
     }
-    const uint32_t e = (indel > 8) ? dyn_lookup_long_ins(T, key, __ldg(rw + 10), qpos, len, seq_off) : dyn_lookup(T, key, __ldg(rw + 10), qpos, len);
+    const uint32_t e = (indel > 8) ? dyn_lookup_long_ins(T, key, __ldg(rw + 10), qpos, len, bq_off) : dyn_lookup(T, key, __ldg(rw + 10), qpos, len);
     atomicAdd(&T.dcnt[(size_t)e * SMC_NCNT + SMC_C_ALLELE], 1);
     if (!reverse) atomicAdd(&T.dcnt[(size_t)e * SMC_NCNT + SMC_C_FWD], 1);
     return make_uint2(code, NF + e);
@@ -593,16 +575,20 @@ __device__ __forceinline__ uint32_t slot_field_one(uint32_t aid) { return 1u << 
 template <bool LIST>
 __global__ void __launch_bounds__(KA_WARPS * 32, KA_MINBLOCKS) k_gather_t(const KAArgs A) {
     extern __shared__ __align__(16) uint32_t smem[];
-    uint32_t* lut = smem;                          // nibble -> field increment 1 << 8*field | allele slot << 28 (0: not A/C/G/T)
-    if (threadIdx.x < 16) {
+    // BAM nibble -> {register field increment 1 << 8*field (0: not A/C/G/T), event-code bits of a covered base: allele slot << 8,
+    // or nibble << 8 | EC_DYN; EC_COVERED}; entry 16 (what the gather reads for a lane the read does not cover): {0, 0}
+    uint2* lut = reinterpret_cast<uint2*>(smem);
+    if (threadIdx.x <= 16) {
         const uint32_t n = threadIdx.x;
         const uint32_t f = nib_field(n);
-        lut[n] = nib_is_acgt(n) ? ((1u << (8u * f)) | ((f + (f >> 1)) << 28)) : 0u;
+        lut[n] = n == 16u ? make_uint2(0u, 0u)
+               : nib_is_acgt(n) ? make_uint2(1u << (8u * f), ((f + (f >> 1)) << SC_AID_SH) | EC_COVERED)
+                                : make_uint2(0u, (n << EC_NIB_SH) | EC_DYN | EC_COVERED);
     }
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    uint32_t* ws = smem + 16 + (size_t)w * KA_WARP_WORDS(LIST);
+    uint32_t* ws = smem + KA_LUT_WORDS + (size_t)w * KA_WARP_WORDS(LIST);
     uint4* smask = reinterpret_cast<uint4*>(ws);                      // per event: covered / le20 / ple lane masks, class + flags
-    uint2* sbase = reinterpret_cast<uint2*>(ws + KA_OFF_BASE);        // per event: seq_base, qual_base
+    uint32_t* sbase = ws + KA_OFF_BASE;                               // per event: bq_base
     uint32_t* srank_s = ws + KA_OFF_SRANK;
     uint16_t* evc = reinterpret_cast<uint16_t*>(ws + KA_OFF_EVC);     // 32 x 32 event codes of the batch
     uint32_t* cst = ws + KA_OFF_CST;                                  // fragment-code staging: word [k >> 1][lane], half k & 1
@@ -625,13 +611,11 @@ __global__ void __launch_bounds__(KA_WARPS * 32, KA_MINBLOCKS) k_gather_t(const 
     const uint32_t validmask = __ballot_sync(FULL_MASK, lane_valid);
     const int32_t p = lane_valid ? A.loci_pos[L] : 0;
     const int32_t Li = lane_valid ? (int32_t)L : -1;                  // -1 is never inside a read's [lo, hi)
-    const uint32_t ph0 = (uint32_t)p >> 1, ph1 = ((uint32_t)p + 1u) >> 1, ppar = (uint32_t)p & 1u;
     const uint32_t lanebit = 1u << lane;
     const int32_t tile0 = (int32_t)(tile * 32u);
     const size_t nl = (size_t)A.n_loci;
     const int minBQ = A.minBQ;
-    const uint8_t* __restrict__ seqp = A.seq;
-    const uint8_t* __restrict__ qualp = A.qual;
+    const uint16_t* __restrict__ bqp = A.bq;
 
     uint32_t conc = 0, disc = 0;                                      // 4 x 8-bit fields (A, C, T, G)
     int cvg = 0;
@@ -716,7 +700,7 @@ __global__ void __launch_bounds__(KA_WARPS * 32, KA_MINBLOCKS) k_gather_t(const 
             }
         } else {                                                             // rare: per-event CIGAR walk, out of line
             const uint32_t* rw = reinterpret_cast<const uint32_t*>(&A.recs[srank_s[e]]);
-            const uint2 ev = slow_event(A.T, rw, A.cigar, seqp, qualp, p, Li, minBQ, A.primerDist);
+            const uint2 ev = slow_event(A.T, rw, A.cigar, bqp, p, Li, minBQ, A.primerDist);
             cd = ev.x; mid = ev.y; one = 0;
             if (cd & EC_COVERED) {
                 const uint32_t meta = __ldg(rw + 3);
@@ -724,8 +708,8 @@ __global__ void __launch_bounds__(KA_WARPS * 32, KA_MINBLOCKS) k_gather_t(const 
                 cvg++;
                 if (cd & EC_REGULAR) {
                     if (!(cd & EC_DYN)) {
-                        const uint32_t lv = lut[(cd >> EC_NIB_SH) & 15u];
-                        one = lv & 0x0fffffffu; mid = lv >> 28;
+                        const uint2 lv = lut[(cd >> EC_NIB_SH) & 15u];
+                        one = lv.x; mid = (lv.y >> SC_AID_SH) & 15u;
                         const uint32_t cls = ((meta & RM_REVERSE) ? TC_REVERSE : 0u) |
                                              (lowq ? 0u : !(cd & EC_INC) ? 1u : (meta & RM_READ2) ? 4u + ((cd & EC_LE20) ? 1u : 0u) + ((cd & EC_PLE) ? 2u : 0u)
                                                                                                    : 2u + ((cd & EC_LE20) ? 1u : 0u));
@@ -755,7 +739,7 @@ __global__ void __launch_bounds__(KA_WARPS * 32, KA_MINBLOCKS) k_gather_t(const 
         if (lane < nb) {
             sr = __ldg(&A.ev_read[base + lane]);
             const uint4* src = reinterpret_cast<const uint4*>(&A.grec[sr]);
-            g0 = __ldg(src); g1 = __ldg(src + 1);                            // lo gspan|flags seq_base qual_base | le ple urank frank
+            g0 = __ldg(src); g1 = __ldg(src + 1);                            // lo gspan|flags bq_base unused | le ple urank frank
         }
         uint32_t pur = __shfl_up_sync(FULL_MASK, g1.z, 1), pfr = __shfl_up_sync(FULL_MASK, g1.w, 1);
         if (lane == 0) { pur = carry_ur; pfr = carry_fr; }
@@ -776,7 +760,7 @@ __global__ void __launch_bounds__(KA_WARPS * 32, KA_MINBLOCKS) k_gather_t(const 
         carry_ur = __shfl_sync(FULL_MASK, g1.z, ncons - 1); carry_fr = __shfl_sync(FULL_MASK, g1.w, ncons - 1);
         {
             // what is the same for all 32 loci, as lane masks: covered loci [lo, lo + gspan), the two end-distance windows
-            // (only ever needed for included reads); tally class of the read; parity of its query offset
+            // (only ever needed for included reads); tally class of the read
             const int rel = (int32_t)g0.x - tile0;
             const bool live = lane < ncons;
             const uint32_t okm = (g0.y & GR_OK) ? 0xffffffffu : 0u;
@@ -784,8 +768,8 @@ __global__ void __launch_bounds__(KA_WARPS * 32, KA_MINBLOCKS) k_gather_t(const 
             const uint32_t le = cov & okm & lane_range_mask(rel + (int)(g1.x & 0xffffu), rel + (int)(g1.x >> 16));
             const uint32_t ple = cov & okm & lane_range_mask(rel + (int)(g1.y & 0xffffu), rel + (int)(g1.y >> 16));
             const uint32_t cls = ((g0.y & GR_REVERSE) ? TC_REVERSE : 0u) | (!(g0.y & GR_OK) ? 1u : (g0.y & GR_READ2) ? 4u : 2u);
-            smask[lane] = make_uint4(cov, le, ple, cls | ((g0.y & GR_ODD) ? 16u : 0u) | ((g0.y & GR_OK) ? 32u : 0u));
-            sbase[lane] = make_uint2(g0.z, g0.w);
+            smask[lane] = make_uint4(cov, le, ple, cls | ((g0.y & GR_OK) ? EC_INC : 0u));
+            sbase[lane] = g0.z;
             srank_s[lane] = sr;
         }
         if (since_flush + 32u > 255u) { flush_tallies(A.cnt, nl, L, lane_valid, hist_lane, conc, disc); since_flush = 0; }
@@ -794,37 +778,29 @@ __global__ void __launch_bounds__(KA_WARPS * 32, KA_MINBLOCKS) k_gather_t(const 
         // ---------------- gather + tally (order independent) of the plain aligned reads, KA_GATHER events at a time
 #pragma unroll 1
         for (int g = 0; g < ncons; g += KA_GATHER) {
-            uint32_t sbv[KA_GATHER], bqv[KA_GATHER];
+            uint32_t wv[KA_GATHER];
             uint4 mk[KA_GATHER];
 #pragma unroll
             for (int u = 0; u < KA_GATHER; ++u) {
                 mk[u] = smask[g + u];
-                const uint2 bs = sbase[g + u];
-                sbv[u] = 0; bqv[u] = 0;
-                if (mk[u].x & lanebit) {
-                    sbv[u] = __ldg(seqp + (bs.x + ((mk[u].w & 16u) ? ph1 : ph0)));
-                    bqv[u] = __ldg(qualp + (bs.y + (uint32_t)p));
-                }
+                wv[u] = (mk[u].x & lanebit) ? __ldg(bqp + (sbase[g + u] + (uint32_t)p)) : 16u << 8;    // not covered: lut[16]
             }
 #pragma unroll
             for (int u = 0; u < KA_GATHER; ++u) {
                 const uint32_t fw = mk[u].w;
                 const bool cov = mk[u].x & lanebit;
-                const uint32_t nib = ((ppar ^ (fw >> 4)) & 1u) ? (sbv[u] & 15u) : (sbv[u] >> 4);   // 0 when not covered
-                const uint32_t bq = bqv[u];
-                const uint32_t lv = lut[nib];
-                const uint32_t one = lv & 0x0fffffffu;                               // 0 when not covered or not A/C/G/T
+                const uint32_t bq = wv[u] & 255u;                                    // 0 when not covered
+                const uint2 lv = lut[wv[u] >> 8];
+                const uint32_t one = lv.x;                                           // 0 when not covered or not A/C/G/T
                 const bool lowq = (int)bq < minBQ;
-                const bool inc = cov && !lowq && (fw & 32u);                         // :431
-                const bool dynb = cov && !one;
+                const uint32_t inc = (cov && !lowq) ? (fw & EC_INC) : 0u;           // :431
                 cvg += cov ? 1 : 0;                                                  // :368
                 uint32_t cls = fw & 15u;                                             // :428-459, as one class count
                 if (mk[u].y & lanebit) cls += 1u;
                 if (mk[u].z & lanebit) cls += 2u;
                 if (lowq) cls = fw & TC_REVERSE;
                 atomicAdd(&hist_lane[cls * 32], one);                                // fire and forget; adds 0 for a lane the read does not cover
-                evc[(g + u) * 32 + lane] = (uint16_t)(bq | ((dynb ? nib : (lv >> 28)) << SC_AID_SH) | (cov ? EC_COVERED : 0u) | (dynb ? EC_DYN : 0u) |
-                                                      (inc ? EC_INC : 0u));
+                evc[(g + u) * 32 + lane] = (uint16_t)(bq | lv.y | inc);
             }
         }
         // fragment structure of the batch, one event per lane: which fragments are complete runs of one or two plain
