@@ -126,8 +126,8 @@ typedef struct smc_loci {
 
 /*
  * Optional down-sampling mask (smCounter.py:496-500): for the listed loci only the listed barcodes are used.
- * The selection itself (random.seed(pos); random.sample(bcDict.keys(), ds)) depends on CPython-2 dict order and
- * is made on the host; the device only applies it.
+ * A caller may draw the selection itself (random.seed(pos); random.sample(bcDict.keys(), ds), which depends on CPython-2
+ * dict order) and pass it here, or let the library draw it on the device (smc_set_downsample).
  */
 typedef struct smc_umi_keep {
     int64_t         n_loci;     /* number of masked loci */
@@ -182,6 +182,7 @@ typedef struct smc_umi_keep {
 #define SMC_ST_NEED_DOWNSAMPLE 2u   /* len(bcDict) > ds and no mask given: tallies cover ALL barcodes; re-run with a mask */
 #define SMC_ST_UMI_OVERFLOW    4u   /* a barcode showed > 6 distinct non-ACGT/DEL alleles at this locus (unsupported) */
 #define SMC_ST_BAD_MASK        8u   /* mask given but kept count != ds */
+#define SMC_ST_DOWNSAMPLED    16u   /* the barcodes were drawn on the device (smc_set_downsample(ctx, SMC_DS_DEVICE)) */
 
 /* dynamic allele kinds (dyn_kind) */
 #define SMC_K_BASE 0   /* single non-ACGT base (N or IUPAC): dyn_site = BAM nibble */
@@ -284,6 +285,30 @@ int smc_run_resident(smc_ctx *ctx);
 int smc_download(smc_ctx *ctx, smc_out *out);
 
 int smc_get_timings(smc_ctx *ctx, smc_timings *t);
+
+/*
+ * Down-sampling drawn on the device.  With SMC_DS_DEVICE, smc_run_resident / smc_call_batch draw the reference's sample
+ * (random.seed(str(pos)); random.sample(bcDict.keys(), ds) over CPython-2 dict order, smCounter.py:496-500) for every locus
+ * that would be flagged SMC_ST_NEED_DOWNSAMPLE and run the pileup and the statistics again with it on the resident batch:
+ * no locus keeps that flag, the drawn ones carry SMC_ST_DOWNSAMPLED.  Loci with a caller-given mask keep it.  A batch
+ * without such loci runs exactly as with SMC_DS_FLAG.  In a run that drew, ms_stats and ms_total_device include the draw
+ * and the second pileup.  The mode is sticky per context; SMC_DS_FLAG is the default.
+ */
+#define SMC_DS_FLAG   0   /* flag the loci (SMC_ST_NEED_DOWNSAMPLE), tallies over all barcodes; the caller draws */
+#define SMC_DS_DEVICE 1   /* draw on the device */
+int smc_set_downsample(smc_ctx *ctx, int mode);
+
+/* The Py2 hash(str) of dictionary-coded barcodes (umi codes with the top bit set; the library cannot spell them) for the
+ * following device draws: code[n] strictly ascending.  A draw that meets a dictionary code missing here fails with SMC_E_ARG
+ * naming the code.  n = 0 clears the table. */
+int smc_set_barcode_hashes(smc_ctx *ctx, int64_t n, const uint64_t *code /* ascending */, const int64_t *py2_hash);
+
+/* The device draw on caller-given key sets, independent of any batch (a validation entry point, like smc_fisher_exact): set i
+ * holds the barcode codes codes[off[i] .. off[i+1]) in dict insertion order; random.seed(str(seed_pos1[i]));
+ * random.sample(keys in CPython-2 dict order, k[i]).  out[off[i] + j], j < k[i], receives the insertion index of the j-th drawn
+ * key.  Dictionary codes take their hashes from smc_set_barcode_hashes. */
+int smc_draw_sample(smc_ctx *ctx, int64_t n_sets, const int64_t *off, const uint64_t *codes /* insertion order */,
+                   const int64_t *seed_pos1, const int64_t *k, int64_t *out);
 
 /* For loci flagged SMC_ST_NEED_DOWNSAMPLE (after smc_run_resident / smc_call_batch): list the barcodes of bcDict (those
  * with >= 1 read passing incCond, smCounter.py:467) so that the host can draw the reference's sample (:496-500).

@@ -15,7 +15,8 @@ SMC_OK, SMC_E_CUDA, SMC_E_ARG, SMC_E_LIMIT, SMC_E_OVERFLOW, SMC_E_STATE = 0, -1,
 (C_ALLELE, C_FWD, C_REV, C_LOWQ, C_R1LE, C_R1TOT, C_R2LE, C_R2TOT, C_R2PLE, C_CONCORD, C_DISCORD, C_MT,
  C_STRONG) = range(13)
 (L_CVG, L_ALLFRAG, L_ALLMT, L_USEDFRAG, L_NBC, L_USEDMT, L_MT3, L_MT5, L_MT7, L_MT10, L_KEYMASK, L_STATUS) = range(12)
-ST_ZERO_COVERAGE, ST_NEED_DOWNSAMPLE, ST_UMI_OVERFLOW, ST_BAD_MASK = 1, 2, 4, 8
+ST_ZERO_COVERAGE, ST_NEED_DOWNSAMPLE, ST_UMI_OVERFLOW, ST_BAD_MASK, ST_DOWNSAMPLED = 1, 2, 4, 8, 16
+DS_FLAG, DS_DEVICE = 0, 1
 K_BASE, K_INS, K_DEL = 0, 1, 2
 F_LM, F_LSM, F_DP, F_SB, F_LOWQ, F_R1CP, F_R2CP, F_PRIMERCP = (1 << i for i in range(8))
 F_HPGATE, F_EVALUATED = 1 << 16, 1 << 17
@@ -77,7 +78,7 @@ HP_HOMOPOLYMER, HP_LOWCOMP = 1, 2
 
 EXPORTS = ("smc_version", "smc_ctx_create", "smc_ctx_destroy", "smc_last_error", "smc_call_batch", "smc_upload",
            "smc_run_resident", "smc_download", "smc_get_timings", "smc_list_barcodes", "smc_hp_lowcomp", "smc_fisher_exact", "smc_host_alloc",
-           "smc_host_free")
+           "smc_host_free", "smc_set_downsample", "smc_set_barcode_hashes", "smc_draw_sample")
 
 _lib = None
 
@@ -119,6 +120,12 @@ def load():
     lib.smc_list_barcodes.restype = C.c_int
     lib.smc_hp_lowcomp.argtypes = [_vp, C.POINTER(smc_hp_batch), _vp]
     lib.smc_hp_lowcomp.restype = C.c_int
+    lib.smc_set_downsample.argtypes = [_vp, C.c_int]
+    lib.smc_set_downsample.restype = C.c_int
+    lib.smc_set_barcode_hashes.argtypes = [_vp, C.c_int64, _vp, _vp]
+    lib.smc_set_barcode_hashes.restype = C.c_int
+    lib.smc_draw_sample.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]
+    lib.smc_draw_sample.restype = C.c_int
     _lib = lib
     return lib
 

@@ -164,9 +164,12 @@ class UmiKeep:
 
 
 class GpuCaller:
-    """One context per GPU (not thread-safe per context; ctypes releases the GIL during calls)."""
+    """One context per GPU (not thread-safe per context; ctypes releases the GIL during calls).
 
-    def __init__(self, params: VcParams, device: int = 0):
+    ``device_downsample``: draw the reference's down-sampling sample on the device inside every call (smc_set_downsample), so
+    that no locus comes back flagged ST_NEED_DOWNSAMPLE; dictionary-coded barcodes need their hashes (set_barcode_hashes)."""
+
+    def __init__(self, params: VcParams, device: int = 0, device_downsample: bool = False):
         self.lib = _ffi.load()
         self.params = params
         p = _ffi.smc_params(params.minBQ, params.minMQ, params.mtDepth, params.mtDrop, params.maxMT, params.primerDist,
@@ -177,6 +180,10 @@ class GpuCaller:
             raise RuntimeError("smc_ctx_create failed (%d): %s" % (rc, self.lib.smc_last_error(None).decode()))
         self.h = h
         self._keepalive = None
+        if device_downsample:
+            rc = self.lib.smc_set_downsample(self.h, _ffi.DS_DEVICE)
+            if rc != 0:
+                raise self._err("smc_set_downsample", rc)
 
     def close(self):
         if getattr(self, "h", None):
@@ -292,6 +299,27 @@ class GpuCaller:
             if rc != 0:
                 raise self._err("smc_list_barcodes", rc)
         return off, umi[:total], first[:total]
+
+    def set_barcode_hashes(self, codes, py2_hashes):
+        """The Py2 hash(str) of dictionary-coded barcodes (top bit set) for the following device draws; ``codes`` ascending."""
+        c = np.ascontiguousarray(codes, dtype=np.uint64)
+        h = np.ascontiguousarray(py2_hashes, dtype=np.int64)
+        rc = self.lib.smc_set_barcode_hashes(self.h, len(c), _ffi.ptr(c), _ffi.ptr(h))
+        if rc != 0:
+            raise self._err("smc_set_barcode_hashes", rc)
+
+    def draw_sample(self, off, codes, seed_pos1, k) -> np.ndarray:
+        """random.seed(str(seed_pos1[i])); random.sample(keys in CPython-2 dict order, k[i]) on the device for the key sets
+        codes[off[i]:off[i+1]] (insertion order): out[off[i] + j], j < k[i], is the insertion index of the j-th drawn key."""
+        off = np.ascontiguousarray(off, dtype=np.int64)
+        codes = np.ascontiguousarray(codes, dtype=np.uint64)
+        pos = np.ascontiguousarray(seed_pos1, dtype=np.int64)
+        k = np.ascontiguousarray(k, dtype=np.int64)
+        out = np.full(max(int(off[-1]), 1), -1, dtype=np.int64)
+        rc = self.lib.smc_draw_sample(self.h, len(k), _ffi.ptr(off), _ffi.ptr(codes), _ffi.ptr(pos), _ffi.ptr(k), _ffi.ptr(out))
+        if rc != 0:
+            raise self._err("smc_draw_sample", rc)
+        return out[:int(off[-1])]
 
     def hp_lowcomp(self, hpLen: int, candidates) -> np.ndarray:
         """isHPorLowComp() (smCounter.py:122-177) on the device for ``candidates`` = [(window, pos_in_window, ref, alt)]

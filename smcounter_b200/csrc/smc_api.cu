@@ -8,7 +8,10 @@
 //          (bases and qualities expanded per chunk into one 16-bit word per stored base first)     smc_upload.cuh
 //       -> K3b k_merge: per-barcode posterior (calProb), prediction index, consensus    smc_pileup.cuh
 //       -> K4 FP64 statistics: PI, ALT, filters, Fisher                                smc_stats.cuh
+//       -> (SMC_DS_DEVICE, loci flagged for down-sampling only) listing pass, Py2 draw, K3 + K4 again with the drawn masks
+//                                                                                      smc_downsample.cuh
 //   -> D2H
+#include <algorithm>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -16,6 +19,7 @@
 #include <new>
 #include <mutex>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include <nvtx3/nvToolsExt.h>      // header-only: ranges show up under nsys / ncu --nvtx, cost nothing otherwise
@@ -25,6 +29,7 @@
 #include "smc_pileup.cuh"
 #include "smc_stats.cuh"
 #include "smc_upload.cuh"
+#include "smc_downsample.cuh"
 
 namespace {
 
@@ -80,9 +85,12 @@ enum SmallWord {
     SW_CVG_SUM = 8,          // u64: sum of cvg over the loci (= pileup read-events)
     SW_N_MULTI = 10,         // reads of fragments of >= 3 reads (k_place_reads)
     SW_N_UMI = 12,           // distinct barcodes (k_frag_scan)
+    SW_DS_LOCI = 13,         // loci k_call flagged SMC_ST_NEED_DOWNSAMPLE (device draw on), then u64 at 14: their barcodes
     SW_PIPE_BLOCKED = 16,    // [SMC_PIPE_MAX]: first unit that has to wait for chunk c + 1
     SW_PACK_TOTALS = 40,     // [6]: bytes / words of packed bases, qualities, CIGARs, compact qualities, compact bases; bq[] words
     SW_SPILL_COUNT = 48,     // k_merge spill records handed out
+    SW_DS_MISSING = 50,      // u64: a dictionary-coded barcode of a drawn locus that has no hash (0: none)
+    SW_DS_OR = 52,           // u64: OR of the barcode codes of the drawn loci
     SW_CHUNK_FIRST = 64      // [SMC_PIPE_MAX]: k_chunk_need's first read per upload chunk
 };
 
@@ -150,6 +158,16 @@ struct smc_ctx {
     // barcode listing
     DevBuf d_list_idx{bufs}, d_list_count{bufs}, d_list_off{bufs}, d_list_umi{bufs}, d_list_first{bufs};
     DevBuf d_hp_bases{bufs}, d_hp_meta{bufs}, d_hp_flags{bufs};     // smc_hp_lowcomp
+    // down-sampling drawn on the device (smc_set_downsample): the flagged loci of the last call_stats, the caller's part of the
+    // mask CSR, the keep index from which masks were drawn, the Py2 hashes of dictionary-coded barcodes, and the draw's scratch
+    int ds_mode = SMC_DS_FLAG;
+    int64_t ds_flagged = 0, ds_barcodes = 0;
+    int64_t keep_n = 0, keep_total = 0;
+    int32_t ds_first_drawn = INT32_MAX;
+    int64_t n_bc = 0;
+    DevBuf d_bc_code{bufs}, d_bc_hash{bufs};
+    DevBuf d_ds_flag{bufs}, d_ds_nbc{bufs}, d_ds_locus{bufs}, d_ds_k0{bufs}, d_ds_k1{bufs}, d_ds_v0{bufs}, d_ds_v1{bufs}, d_ds_codes{bufs},
+        d_ds_hash{bufs}, d_ds_scratch{bufs}, d_ds_keep_off{bufs}, d_ds_keep_umi{bufs};
     smc_timings tm{};
     uint32_t chunk = 128;       // tile events per warp unit (A/B on B200, whole step: 96 -> 4.42 ms, 128 -> 4.39, 160 -> 4.39, 256 -> 4.47, 384 -> 4.60)
     const uint32_t* ev_read_sorted = nullptr;   // tile-sorted event -> srank map (lives in d_ev0 or d_ev1)
@@ -720,6 +738,9 @@ static int queue_upload(smc_ctx* ctx, const smc_reads_soa* R, const smc_loci* Lc
     CK(up.copy(ctx->d_loci_ref, Lc->ref_id, (size_t)nl * 4)); CK(up.copy(ctx->d_loci_pos, Lc->pos0, (size_t)nl * 4));
     CK(up.copy(ctx->d_loci_base, Lc->ref_base, (size_t)nl));
     ctx->has_keep = K && K->n_loci > 0;
+    ctx->keep_n = ctx->has_keep ? K->n_loci : 0;
+    ctx->keep_total = ctx->has_keep ? K->off[K->n_loci] : 0;
+    ctx->ds_first_drawn = INT32_MAX;
     if (ctx->has_keep) {
         CK(up.copy(ctx->d_keep_off, K->off, (size_t)(K->n_loci + 1) * 8));
         CK(up.copy(ctx->d_keep_umi, K->umi, (size_t)K->off[K->n_loci] * 8));
@@ -1162,6 +1183,11 @@ static int dyn_rows(smc_ctx* ctx) {
     return SMC_OK;
 }
 
+// ds = maxMT or round(2 * mtDepth) (smCounter.py:486)
+static int ds_of(const smc_ctx* ctx) {
+    return ctx->prm.maxMT > 0 ? ctx->prm.maxMT : (int)std::llround(2.0 * (double)ctx->prm.mtDepth);
+}
+
 // K4: k_call (PI, ALT, filters, Fisher task list), k_fisher, and the sum of cvg.  The round trip after them brings back the task
 // count: a list longer than its buffer is grown and the three kernels run once more.
 static int call_stats(smc_ctx* ctx) {
@@ -1179,7 +1205,12 @@ static int call_stats(smc_ctx* ctx) {
         B.dyn_limb = ctx->d_s_limb.as<unsigned long long>(); B.dyn_iskey = ctx->d_s_iskey.as<uint8_t>(); B.dyn_pi = ctx->d_s_pi.as<double>();
         B.dyn_first = ctx->d_dyn_first.as<uint32_t>();
         B.keep_idx = ctx->has_keep ? ctx->d_keep_idx.as<int32_t>() : nullptr;
-        B.ds = ctx->prm.maxMT > 0 ? ctx->prm.maxMT : (int)std::llround(2.0 * (double)ctx->prm.mtDepth);   // smCounter.py:486
+        B.ds = ds_of(ctx);
+        B.ds_first_drawn = ctx->ds_first_drawn;
+        if (ctx->ds_mode == SMC_DS_DEVICE) {
+            B.ds_count = small + SW_DS_LOCI;
+            CK(cudaMemsetAsync(small + SW_DS_LOCI, 0, 12, ctx->st));
+        }
         B.max_allele = ctx->d_max.as<int32_t>(); B.second_allele = ctx->d_second.as<int32_t>(); B.alt_allele = ctx->d_alt.as<int32_t>();
         B.alt_pi = ctx->d_altpi.as<double>(); B.second_pi = ctx->d_secondpi.as<double>(); B.fl1 = ctx->d_fl1.as<uint32_t>();
         B.fl2 = ctx->d_fl2.as<uint32_t>(); B.biallelic = ctx->d_bial.as<uint8_t>(); B.fisher_p = ctx->d_fp.as<double>();
@@ -1193,18 +1224,154 @@ static int call_stats(smc_ctx* ctx) {
         LAUNCH(k_sum_cvg, std::min<unsigned>(nblk(nl, 256), 592u), 256, 0, ctx->d_loc.as<int32_t>() + (size_t)SMC_L_CVG * nl, nl,
                (unsigned long long*)(small + SW_CVG_SUM));
         CK(cudaEventRecord(ctx->ev[EV_STATS_DONE], ctx->st));
-        uint32_t w[3];                                               // d_small words SW_N_TASKS, SW_CVG_SUM (u64)
-        if (const int rc = read_back(ctx, w, small + SW_N_TASKS, sizeof(w))) return rc;
+        uint32_t w[9];                                               // d_small words SW_N_TASKS, SW_CVG_SUM (u64), .. SW_DS_LOCI, SW_DS_LOCI + 1 (u64)
+        const size_t nw = ctx->ds_mode == SMC_DS_DEVICE ? 9 : 3;
+        if (const int rc = read_back(ctx, w, small + SW_N_TASKS, nw * 4)) return rc;
         CK(cudaGetLastError());
         const uint32_t n_tasks = w[0];
         if (n_tasks <= ctx->task_cap) {
             ctx->tm.n_fisher = n_tasks;
             ctx->tm.n_pileup_events = (int64_t)(w[1] | (uint64_t)w[2] << 32);
+            ctx->ds_flagged = nw == 9 ? w[SW_DS_LOCI - SW_N_TASKS] : 0;
+            ctx->ds_barcodes = nw == 9 ? (int64_t)(w[SW_DS_LOCI + 1 - SW_N_TASKS] | (uint64_t)w[SW_DS_LOCI + 2 - SW_N_TASKS] << 32) : 0;
             return SMC_OK;
         }
         if (attempt == 1) { ctx->err = "Fisher task list overflow"; return SMC_E_OVERFLOW; }
         ctx->task_cap = n_tasks + n_tasks / 4 + 1024;                // grow and redo the (cheap) call kernel
     }
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// Down-sampling drawn on the device (smc_downsample.cuh)
+
+// draw scratch of one k_ds_draw launch: sets beyond it go to further launches (a set alone may exceed it)
+static constexpr int64_t DS_WAVE_WORDS = 1ll << 30;
+
+static int bit_length(uint64_t v) { return v ? 64 - __builtin_clzll(v) : 0; }
+
+// k_ds_draw over the sets [0, nsets) of the device offsets d_off (total keys), in waves whose scratch stays within
+// DS_WAVE_WORDS; host_off are the same offsets on the host, or null (then read back when one wave does not hold them all)
+static int draw_sets(smc_ctx* ctx, const int64_t* d_off, const int64_t* host_off, int64_t nsets, int64_t total, const int64_t* d_pos1,
+                     const int32_t* d_locus, const int64_t* d_k, int64_t ds, const int64_t* d_hash, uint32_t* d_out) {
+    auto at = [](const int64_t* off, int64_t k) { return 16 * (off[k] + k) + (PY2_MT_N + 16) * k; };
+    const int64_t all = 16 * (total + nsets) + (PY2_MT_N + 16) * nsets;
+    std::vector<int64_t> off_h;
+    if (all > DS_WAVE_WORDS && !host_off) {
+        off_h.resize((size_t)nsets + 1);
+        if (const int rc = read_back(ctx, off_h.data(), d_off, off_h.size() * 8)) return rc;
+        host_off = off_h.data();
+    }
+    for (int64_t k0 = 0; k0 < nsets;) {
+        int64_t k1 = nsets, words = all;
+        if (all > DS_WAVE_WORDS) {
+            k1 = k0 + 1;
+            while (k1 < nsets && at(host_off, k1 + 1) - at(host_off, k0) <= DS_WAVE_WORDS) ++k1;
+            words = at(host_off, k1) - at(host_off, k0);
+        }
+        CK(ctx->d_ds_scratch.ensure((size_t)words * 4));
+        LAUNCH(k_ds_draw, nblk(k1 - k0, 64), 64, 0, d_off, k0, k1, d_pos1, d_locus, ctx->d_loci_pos.as<int32_t>(), d_k, ds, d_hash,
+               ctx->d_ds_scratch.as<uint32_t>(), d_out);
+        k0 = k1;
+    }
+    return SMC_OK;
+}
+
+// k_ds_hash over `total` codes; fails with SMC_E_ARG naming a dictionary-coded barcode without a hash.  *code_or: OR of the codes.
+static int hash_barcodes(smc_ctx* ctx, const uint32_t* order, const uint64_t* umi, int64_t total, uint64_t* code_or) {
+    uint32_t* small = ctx->d_small.as<uint32_t>();
+    CK(ctx->d_ds_codes.ensure((size_t)total * 8)); CK(ctx->d_ds_hash.ensure((size_t)total * 8));
+    CK(cudaMemsetAsync(small + SW_DS_MISSING, 0, 16, ctx->st));
+    LAUNCH(k_ds_hash, nblk(total, 256), 256, 0, order, umi, total, ctx->d_bc_code.as<uint64_t>(), ctx->d_bc_hash.as<int64_t>(), ctx->n_bc,
+           ctx->d_ds_codes.as<uint64_t>(), ctx->d_ds_hash.as<int64_t>(), (unsigned long long*)(small + SW_DS_MISSING),
+           (unsigned long long*)(small + SW_DS_OR));
+    uint64_t w[2];
+    if (const int rc = read_back(ctx, w, small + SW_DS_MISSING, sizeof(w))) return rc;
+    CK(cudaGetLastError());
+    if (w[0]) {
+        char code[24];
+        snprintf(code, sizeof(code), "0x%016llx", (unsigned long long)w[0]);
+        ctx->err = std::string("no Py2 hash for the dictionary-coded barcode ") + code + " (smc_set_barcode_hashes)";
+        return SMC_E_ARG;
+    }
+    *code_or = w[1];
+    return SMC_OK;
+}
+
+// The loci call_stats flagged SMC_ST_NEED_DOWNSAMPLE: number them and list their barcodes, order each locus's barcodes by first
+// passing read, hash them, draw ds of them per locus, merge the kept codes (ascending per locus) into the mask CSR behind the
+// caller's masks, and run the pileup and the statistics again on the resident batch.
+static int device_downsample(smc_ctx* ctx) {
+    NvtxRange nvtx_r("smc:downsample");
+    const int64_t nl = ctx->n_loci, nflag = ctx->ds_flagged, T = ctx->ds_barcodes, ds = ds_of(ctx), m = nflag * ds;
+    if (T > 0xffffffffll) { ctx->err = "down-sampling: more than 2^32 barcodes at the flagged loci of one batch; split the batch"; return SMC_E_LIMIT; }
+    const size_t tz = (size_t)(T ? T : 1), wz = (size_t)std::max<int64_t>(std::max<int64_t>(nl, T), 1);
+    CK(ctx->d_ds_flag.ensure((size_t)nl * 4)); CK(ctx->d_ds_nbc.ensure((size_t)nl * 4)); CK(ctx->d_list_idx.ensure((size_t)nl * 4));
+    CK(ctx->d_list_off.ensure((size_t)(nflag + 1) * 8)); CK(ctx->d_ds_locus.ensure((size_t)nflag * 4)); CK(ctx->d_list_count.ensure((size_t)nflag * 4));
+    CK(ctx->d_ds_v0.ensure(wz * 4)); CK(ctx->d_ds_v1.ensure(wz * 4)); CK(ctx->d_ds_k0.ensure(tz * 8)); CK(ctx->d_ds_k1.ensure(tz * 8));
+    CK(ctx->d_list_umi.ensure(tz * 8)); CK(ctx->d_list_first.ensure(tz * 4));
+    CK(ctx->d_hist.ensure(radix_hist_words(T) * 4 + 1024));
+    CK(ctx->d_scan.ensure((size_t)std::max<int64_t>(radix_scan_words(T), scan_scratch_words(nl)) * 4 + 1024));
+    uint32_t *v0 = ctx->d_ds_v0.as<uint32_t>(), *v1 = ctx->d_ds_v1.as<uint32_t>();
+    uint64_t *k0 = ctx->d_ds_k0.as<uint64_t>(), *k1 = ctx->d_ds_k1.as<uint64_t>();
+    int64_t* list_off = ctx->d_list_off.as<int64_t>();
+    int32_t* locus = ctx->d_ds_locus.as<int32_t>();
+    // 1. ordinal and first listed barcode of every flagged locus
+    LAUNCH(k_ds_flags, nblk(nl, 256), 256, 0, ctx->d_loc.as<int32_t>(), nl, ctx->d_ds_flag.as<uint32_t>(), ctx->d_ds_nbc.as<uint32_t>());
+    exclusive_scan_u32(ctx->d_ds_flag.as<uint32_t>(), v0, nl, ctx->d_scan.as<uint32_t>(), nullptr, ctx->st);
+    exclusive_scan_u32(ctx->d_ds_nbc.as<uint32_t>(), v1, nl, ctx->d_scan.as<uint32_t>(), nullptr, ctx->st);
+    LAUNCH(k_ds_list_fill, nblk(nl, 256), 256, 0, ctx->d_ds_flag.as<uint32_t>(), v0, v1, nl, nflag, T, ctx->d_list_idx.as<int32_t>(), list_off, locus);
+    // 2. their barcodes with their first passing reads: the listing pass of the pileup pair
+    CK(cudaMemsetAsync(ctx->d_list_count.p, 0, (size_t)nflag * 4, ctx->st));
+    if (const int rc = ensure_code_storage(ctx, true, true)) return rc;
+    {
+        KAArgs A; KBArgs B;
+        fill_kargs(ctx, A, B, true, true);
+        B.keep_idx = nullptr;
+        B.list_idx = ctx->d_list_idx.as<int32_t>(); B.list_count = ctx->d_list_count.as<uint32_t>();
+        B.list_off = list_off; B.list_umi = ctx->d_list_umi.as<uint64_t>(); B.list_first = ctx->d_list_first.as<uint32_t>(); B.list_cap = T;
+        if (const int rc = launch_pileup<true>(ctx, A, B, false, false, nullptr)) return rc;
+    }
+    // 3. bcDict insertion order: (locus, first passing read); 4. the hashes in that order
+    LAUNCH(k_ds_sort_keys, nblk(T, 256), 256, 0, list_off, nflag, ctx->d_list_first.as<uint32_t>(), T, k0, v0);
+    const int r1 = radix_sort_bits(k0, v0, k1, v1, T, 0, 30 + bit_length((uint64_t)(nflag - 1)), ctx->d_hist.as<uint32_t>(), ctx->d_scan.as<uint32_t>(), ctx->st);
+    uint64_t code_or = 0;
+    if (const int rc = hash_barcodes(ctx, r1 ? v1 : v0, ctx->d_list_umi.as<uint64_t>(), T, &code_or)) return rc;
+    // 5. the draw: insertion indices of the kept barcodes, ds per locus, then their codes in ascending order per locus
+    if (const int rc = draw_sets(ctx, list_off, nullptr, nflag, T, nullptr, locus, nullptr, ds, ctx->d_ds_hash.as<int64_t>(), v0)) return rc;
+    const uint32_t* order = nullptr;
+    uint64_t* code_sorted = ctx->d_ds_codes.as<uint64_t>();
+    if (m > 0) {
+        LAUNCH(k_ds_kept, nblk(m, 256), 256, 0, list_off, m, ds, ctx->d_ds_codes.as<uint64_t>(), k0, v0);
+        const int r2 = radix_sort_bits(k0, v0, k1, v1, m, 0, bit_length(code_or), ctx->d_hist.as<uint32_t>(), ctx->d_scan.as<uint32_t>(), ctx->st);
+        uint64_t* ka = r2 ? k1 : k0; uint32_t* va = r2 ? v1 : v0;
+        LAUNCH(k_ds_group_keys, nblk(m, 256), 256, 0, m, ds, ka, va, code_sorted);
+        const int r3 = radix_sort_bits(ka, va, r2 ? k0 : k1, r2 ? v0 : v1, m, 0, bit_length((uint64_t)(nflag - 1)), ctx->d_hist.as<uint32_t>(),
+                                       ctx->d_scan.as<uint32_t>(), ctx->st);
+        order = r3 ? (r2 ? v0 : v1) : va;
+    }
+    // 6. the mask CSR: the caller's masks first, then the drawn ones
+    const int64_t n_keep = ctx->keep_n + nflag, keep_total = ctx->keep_total + m;
+    CK(ctx->d_ds_keep_off.ensure((size_t)(n_keep + 1) * 8)); CK(ctx->d_ds_keep_umi.ensure((size_t)std::max<int64_t>(keep_total, 1) * 8));
+    if (ctx->keep_n > 0) {
+        CK(cudaMemcpyAsync(ctx->d_ds_keep_off.p, ctx->d_keep_off.p, (size_t)ctx->keep_n * 8, cudaMemcpyDeviceToDevice, ctx->st));
+        CK(cudaMemcpyAsync(ctx->d_ds_keep_umi.p, ctx->d_keep_umi.p, (size_t)ctx->keep_total * 8, cudaMemcpyDeviceToDevice, ctx->st));
+    }
+    if (!ctx->has_keep) {
+        CK(ctx->d_keep_idx.ensure((size_t)nl * 4));
+        LAUNCH(k_fill_i32, nblk(nl, 256), 256, 0, ctx->d_keep_idx.as<int32_t>(), nl, -1);
+    }
+    LAUNCH(k_ds_csr, nblk(std::max<int64_t>(nflag + 1, m), 256), 256, 0, nflag, ds, ctx->keep_n, ctx->keep_total, locus, order, code_sorted,
+           ctx->d_keep_idx.as<int32_t>(), ctx->d_ds_keep_off.as<int64_t>(), ctx->d_ds_keep_umi.as<uint64_t>());
+    std::swap(ctx->d_keep_off.p, ctx->d_ds_keep_off.p); std::swap(ctx->d_keep_off.cap, ctx->d_ds_keep_off.cap);
+    std::swap(ctx->d_keep_umi.p, ctx->d_ds_keep_umi.p); std::swap(ctx->d_keep_umi.cap, ctx->d_ds_keep_umi.cap);
+    ctx->has_keep = true;
+    ctx->ds_first_drawn = (int32_t)ctx->keep_n;
+    ctx->keep_n = n_keep; ctx->keep_total = keep_total;
+    // 7. the batch again, every base and quality already expanded
+    ctx->pipe_n = 0;
+    if (const int rc = pileup(ctx)) return rc;
+    if (const int rc = dyn_rows(ctx)) return rc;
+    return call_stats(ctx);
 }
 
 // smc_timings of the run: the stage times from the events the stages that ran recorded, and the work counts
@@ -1260,6 +1427,8 @@ extern "C" int smc_run_resident(smc_ctx* ctx) {
     CK(cudaEventRecord(ctx->ev[EV_PILEUP_DONE], ctx->st));
     if (const int rc = dyn_rows(ctx)) return rc;
     if (const int rc = call_stats(ctx)) return rc;
+    if (ctx->ds_flagged > 0)
+        if (const int rc = device_downsample(ctx)) return rc;
     record_timings(ctx);
     ctx->ran = true;
     return SMC_OK;
@@ -1419,6 +1588,63 @@ extern "C" int smc_list_barcodes(smc_ctx* ctx, int64_t n, const int64_t* locus, 
     CK(cudaMemcpyAsync(first_read_out, ctx->d_list_first.p, (size_t)total * 4, cudaMemcpyDeviceToHost, ctx->st));
     CK(cudaStreamSynchronize(ctx->st));
     CK(cudaGetLastError());
+    return SMC_OK;
+}
+
+extern "C" int smc_set_downsample(smc_ctx* ctx, int mode) {
+    if (!ctx) return SMC_E_ARG;
+    if (mode != SMC_DS_FLAG && mode != SMC_DS_DEVICE) { ctx->err = "smc_set_downsample: mode must be SMC_DS_FLAG or SMC_DS_DEVICE"; return SMC_E_ARG; }
+    ctx->ds_mode = mode;
+    return SMC_OK;
+}
+
+extern "C" int smc_set_barcode_hashes(smc_ctx* ctx, int64_t n, const uint64_t* code, const int64_t* py2_hash) {
+    if (!ctx) return SMC_E_ARG;
+    if (n < 0 || (n > 0 && (!code || !py2_hash))) { ctx->err = "smc_set_barcode_hashes: bad arguments"; return SMC_E_ARG; }
+    for (int64_t i = 0; i < n; ++i)
+        if (!(code[i] >> 63) || (i > 0 && code[i] <= code[i - 1])) {
+            ctx->err = "smc_set_barcode_hashes: codes must be dictionary codes (top bit set), strictly ascending"; return SMC_E_ARG;
+        }
+    CK(cudaSetDevice(ctx->device));
+    CK(ctx->d_bc_code.ensure((size_t)std::max<int64_t>(n, 1) * 8)); CK(ctx->d_bc_hash.ensure((size_t)std::max<int64_t>(n, 1) * 8));
+    CK(cudaMemcpyAsync(ctx->d_bc_code.p, code, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->st));
+    CK(cudaMemcpyAsync(ctx->d_bc_hash.p, py2_hash, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->st));
+    CK(cudaStreamSynchronize(ctx->st));
+    ctx->n_bc = n;
+    return SMC_OK;
+}
+
+extern "C" int smc_draw_sample(smc_ctx* ctx, int64_t n_sets, const int64_t* off, const uint64_t* codes, const int64_t* seed_pos1,
+                              const int64_t* k, int64_t* out) {
+    if (!ctx) return SMC_E_ARG;
+    if (n_sets < 0 || (n_sets > 0 && (!off || !seed_pos1 || !k || (off[n_sets] > 0 && (!codes || !out))))) {
+        ctx->err = "smc_draw_sample: bad arguments"; return SMC_E_ARG;
+    }
+    if (n_sets == 0) return SMC_OK;
+    for (int64_t i = 0; i < n_sets; ++i)
+        if (off[0] != 0 || off[i + 1] < off[i] || k[i] < 0 || k[i] > off[i + 1] - off[i] || seed_pos1[i] < 0) {
+            ctx->err = "smc_draw_sample: set " + std::to_string(i) + ": off must start at 0 and not decrease, 0 <= k <= set size, seed_pos1 >= 0";
+            return SMC_E_ARG;
+        }
+    const int64_t T = off[n_sets];
+    if (T > 0xffffffffll) { ctx->err = "smc_draw_sample: more than 2^32 keys"; return SMC_E_LIMIT; }
+    CK(cudaSetDevice(ctx->device));
+    const size_t tz = (size_t)(T ? T : 1);
+    CK(ctx->d_list_off.ensure((size_t)(n_sets + 1) * 8)); CK(ctx->d_ds_k0.ensure((size_t)n_sets * 8)); CK(ctx->d_ds_k1.ensure((size_t)n_sets * 8));
+    CK(ctx->d_list_umi.ensure(tz * 8)); CK(ctx->d_ds_v0.ensure(tz * 4));
+    CK(cudaMemcpyAsync(ctx->d_list_off.p, off, (size_t)(n_sets + 1) * 8, cudaMemcpyHostToDevice, ctx->st));
+    CK(cudaMemcpyAsync(ctx->d_ds_k0.p, seed_pos1, (size_t)n_sets * 8, cudaMemcpyHostToDevice, ctx->st));
+    CK(cudaMemcpyAsync(ctx->d_ds_k1.p, k, (size_t)n_sets * 8, cudaMemcpyHostToDevice, ctx->st));
+    CK(cudaMemcpyAsync(ctx->d_list_umi.p, codes, (size_t)T * 8, cudaMemcpyHostToDevice, ctx->st));
+    uint64_t code_or = 0;
+    if (const int rc = hash_barcodes(ctx, nullptr, ctx->d_list_umi.as<uint64_t>(), T, &code_or)) return rc;
+    if (const int rc = draw_sets(ctx, ctx->d_list_off.as<int64_t>(), off, n_sets, T, ctx->d_ds_k0.as<int64_t>(), nullptr,
+                                 ctx->d_ds_k1.as<int64_t>(), 0, ctx->d_ds_hash.as<int64_t>(), ctx->d_ds_v0.as<uint32_t>())) return rc;
+    std::vector<uint32_t> idx(tz);
+    if (const int rc = read_back(ctx, idx.data(), ctx->d_ds_v0.p, (size_t)T * 4)) return rc;
+    CK(cudaGetLastError());
+    for (int64_t i = 0; i < n_sets; ++i)
+        for (int64_t j = 0; j < k[i]; ++j) out[off[i] + j] = idx[(size_t)(off[i] + j)];
     return SMC_OK;
 }
 

@@ -29,11 +29,12 @@ import numpy as np
 from . import repeats, writers
 from .bam import read_bam
 from ._bamio import pack_upload
-from .caller import GpuCaller, PinnedArena, UmiKeep, VcParams
-from .downsample import draw_keep_masks
+from .caller import GpuCaller, PinnedArena, VcParams
+from .downsample import py2_string_hash
 from .fasta import FastaFile
 from .rows import device_hp_flags, emit_rows, headerAll, headerVariants
 from .shard import ReadLocator, plan_batches, plan_shards, split_long_intervals
+from .soa import umi_string
 from .targets import build_loci, intervals_from_bed_lines
 
 parser = None
@@ -125,7 +126,7 @@ def _run_shards(reads, intervals, refs, prm: VcParams, gpus, devices, stage_time
             # (ctypes drops the GIL inside the library), so the PCIe link and the SMs are both kept busy across batches.
             n_ctx = max(1, min(int(os.environ.get("SMC_CTX_PER_GPU", "3")), len(batches)))
             t_create = time.perf_counter()
-            callers = [GpuCaller(prm, devices[g]) for _ in range(n_ctx)]
+            callers = [GpuCaller(prm, devices[g], device_downsample=True) for _ in range(n_ctx)]      # smCounter.py:486-500 on the device
             arenas = [_take_arena() for _ in range(n_ctx)]      # the upload buffers of each context, recycled batch after batch
             free = queue.SimpleQueue()
             for i in range(n_ctx):
@@ -152,11 +153,9 @@ def _run_shards(reads, intervals, refs, prm: VcParams, gpus, devices, stage_time
                     if stage_times is not None:
                         with lock:
                             stage_times["ms_select_pack"] = stage_times.get("ms_select_pack", 0.0) + 1e3 * (t0 - t_pack)
+                    caller.set_barcode_hashes(*_dictionary_hashes(sub.umi, reads.umi_names))
                     res = caller.call(sub, loci)
                     tm = caller.timings()
-                    keep = draw_keep_masks(caller, res, sub, loci, chroms, prm)        # smCounter.py:496-500
-                    if keep is not None:
-                        res = caller.call(sub, loci, keep)
                     hp = device_hp_flags(caller, res, sub, loci, chroms, refs, prm.hpLen)   # isHPorLowComp, smCounter.py:122-177
                     t1 = time.perf_counter()
                     em = emit_rows(res, sub, loci, chroms, refs, prm.hpLen, bed_order, hp_flags=hp, **emit_kw)
@@ -202,6 +201,15 @@ def _run_shards(reads, intervals, refs, prm: VcParams, gpus, devices, stage_time
         if e is not None:
             raise e
     return per_interval
+
+
+def _dictionary_hashes(umi, names):
+    """The batch's dictionary-coded barcodes (top bit set: not spelt by their code) and their Py2 string hashes, for the device
+    draw of the down-sampling sample."""
+    if umi.dtype != np.uint64:
+        return np.zeros(0, np.uint64), np.zeros(0, np.int64)
+    codes = np.unique(umi[umi >= np.uint64(1 << 63)])
+    return codes, np.asarray([py2_string_hash(umi_string(int(c), names)) for c in codes], dtype=np.int64)
 
 
 class _Joined:
