@@ -7,6 +7,7 @@
 //       -> K3a k_gather: lane = locus, base/quality gather, read tallies, fragment merge smc_pileup.cuh
 //          (bases and qualities expanded per chunk into one 16-bit word per stored base first)     smc_upload.cuh
 //       -> K3b k_merge: per-barcode posterior (calProb), prediction index, consensus    smc_pileup.cuh
+//          (k_merge_deferred: the barcodes whose calProb takes the general form)
 //       -> K4 FP64 statistics: PI, ALT, filters, Fisher                                smc_stats.cuh
 //       -> (SMC_DS_DEVICE, loci flagged for down-sampling only) listing pass, Py2 draw, K3 + K4 again with the drawn masks
 //                                                                                      smc_downsample.cuh
@@ -88,7 +89,7 @@ enum SmallWord {
     SW_DS_LOCI = 13,         // loci k_call flagged SMC_ST_NEED_DOWNSAMPLE (device draw on), then u64 at 14: their barcodes
     SW_PIPE_BLOCKED = 16,    // [SMC_PIPE_MAX]: first unit that has to wait for chunk c + 1
     SW_PACK_TOTALS = 40,     // [6]: bytes / words of packed bases, qualities, CIGARs, compact qualities, compact bases; bq[] words
-    SW_SPILL_COUNT = 48,     // k_merge spill records handed out
+    SW_DEFER_COUNT = 48,     // deferred-barcode records k_merge appended
     SW_DS_MISSING = 50,      // u64: a dictionary-coded barcode of a drawn locus that has no hash (0: none)
     SW_DS_OR = 52,           // u64: OR of the barcode codes of the drawn loci
     SW_CHUNK_FIRST = 64      // [SMC_PIPE_MAX]: k_chunk_need's first read per upload chunk
@@ -128,9 +129,9 @@ struct smc_ctx {
     // bq[], quality | BAM nibble << 8 per stored base, d_bq_off the word of each read's first stored base
     int qual_bits = 8, seq_bits = 4; int64_t n_seq_exc = 0;
     DevBuf d_seq_up{bufs}, d_qual_up{bufs}, d_seq_off{bufs}, d_qual_off{bufs}, d_seq_poff{bufs}, d_qual_poff{bufs}, d_qual_lut{bufs},
-        d_exc_read{bufs}, d_exc_pos{bufs}, d_exc_nib{bufs}, d_bq{bufs}, d_bq_off{bufs}, d_stage{bufs}, d_spill{bufs};
+        d_exc_read{bufs}, d_exc_pos{bufs}, d_exc_nib{bufs}, d_bq{bufs}, d_bq_off{bufs}, d_stage{bufs}, d_defer{bufs};
     uint32_t bq_cap = 0;                        // words of d_bq the current batch may fill
-    uint32_t spill_cap = 0;                     // records in the k_merge spill pool (grows x4 on GF_SPILL_FULL)
+    uint32_t defer_cap = 0;                     // records in the deferred-barcode list of k_merge (grows x4 on GF_DEFER_FULL)
     DevBuf d_loci_ref{bufs}, d_loci_pos{bufs}, d_loci_base{bufs}, d_loci_key{bufs};
     DevBuf d_keep_idx{bufs}, d_keep_off{bufs}, d_keep_umi{bufs};
     bool has_keep = false, uploaded = false, ran = false;
@@ -1022,7 +1023,6 @@ static DynTab make_dyntab(smc_ctx* ctx) {
     T.drep_qpos = ctx->d_drep_qpos.as<int32_t>(); T.dlen = ctx->d_dlen.as<int32_t>(); T.dcnt = ctx->d_dcnt.as<int32_t>();
     T.dlimb = ctx->d_dlimb.as<unsigned long long>(); T.diskey = ctx->d_diskey.as<uint8_t>(); T.dcount = small + SW_DYN_COUNT; T.gflags = small + SW_GFLAGS;
     T.bq = ctx->d_bq.as<uint16_t>(); T.bq_off = ctx->d_bq_off.as<uint32_t>();
-    T.spill = ctx->d_spill.as<SpillRec>(); T.spill_cap = ctx->spill_cap; T.spill_count = small + SW_SPILL_COUNT;
     return T;
 }
 
@@ -1063,11 +1063,13 @@ static void fill_kargs(smc_ctx* ctx, KAArgs& A, KBArgs& B, bool list, bool need_
     B.loc = ctx->d_loc.as<int32_t>(); B.cnt = ctx->d_cnt.as<int32_t>(); B.limb = ctx->d_limb.as<unsigned long long>();
     B.T = A.T;
     B.list_idx = nullptr;
+    B.defer = ctx->d_defer.as<uint4>(); B.defer_cap = ctx->defer_cap; B.defer_count = ctx->d_small.as<uint32_t>() + SW_DEFER_COUNT;
 }
 
 // k_gather + k_merge over units [0, n_units_cap): one pair, or for a chunked upload one pair per range [pipe_end[c-1],
-// pipe_end[c]) that starts once chunk c is in (after expanding its reads' bases and qualities when `expand`).  `gather_done`, unless null,
-// is recorded between the kernels of the one pair, or after the last pair of a chunked run.
+// pipe_end[c]) that starts once chunk c is in (after expanding its reads' bases and qualities when `expand`); then
+// k_merge_deferred over the barcodes the k_merge launches deferred (the list's count is cleared by the caller).
+// `gather_done`, unless null, is recorded between the kernels of the one pair, or after the last pair of a chunked run.
 template <bool LIST>
 static int launch_pileup(smc_ctx* ctx, KAArgs& A, KBArgs& B, bool chunked, bool expand, cudaEvent_t gather_done) {
     if (chunked) ctx->tm.pipe_launches = 0;
@@ -1087,12 +1089,21 @@ static int launch_pileup(smc_ctx* ctx, KAArgs& A, KBArgs& B, bool chunked, bool 
         if (chunked) ++ctx->tm.pipe_launches;
     }
     if (gather_done && chunked) CK(cudaEventRecord(gather_done, ctx->st));
+    // the record count is only known on the device: at most one wave of threads, each walks the list with a grid stride
+    LAUNCH(k_merge_deferred, std::min<unsigned>(nblk(ctx->defer_cap, KD_THREADS), 148u * 8u), KD_THREADS, 0, B);
     return SMC_OK;
 }
 
+// Initial length of the deferred-barcode list of k_merge: one record per 32 tile events, never below 1024.  The batches of cfg2
+// (6.9 - 10.4 M tile events) defer 14.7 k - 25.6 k (barcode, locus) pairs, about one per 400 tile events; a batch that
+// defers more runs its pileup again with the list grown x4, and the context keeps the longer list.
+static uint32_t defer_cap_for(int64_t n_tile_events) {
+    return (uint32_t)std::min<int64_t>(std::max<int64_t>(1024, n_tile_events / 32), 1ll << 24);
+}
+
 // K3: the pileup, into per-locus accumulators and a dynamic-allele table cleared for it.  The round trip after it brings back
-// the overflow flags: a pileup that overflowed the dynamic-allele table, the fragment-code storage or the spill pool runs again
-// with the one that overflowed grown.
+// the overflow flags: a pileup that overflowed the dynamic-allele table, the fragment-code storage or the deferred-barcode list
+// runs again with the one that overflowed grown.
 static int pileup(smc_ctx* ctx) {
     NvtxRange nvtx_r("smc:pileup");
     const size_t nlz = (size_t)(ctx->n_loci ? ctx->n_loci : 1);
@@ -1112,6 +1123,12 @@ static int pileup(smc_ctx* ctx) {
         }
         ctx->dyn_cap = want;
     }
+    if (const char* ev = ctx->defer_cap == 0 ? getenv("SMC_SPILL_CAP0") : nullptr) {     // test hook: start small to exercise the regrowth path
+        const long v = atol(ev);
+        if (v >= 1 && v <= (1l << 24)) ctx->defer_cap = (uint32_t)v;
+    } else {
+        ctx->defer_cap = std::max(ctx->defer_cap, defer_cap_for(ctx->n_tile_events));
+    }
     for (int attempt = 0;; ++attempt) {
         const uint32_t cap = ctx->dyn_cap;
         CK(ctx->d_dkey.ensure((size_t)cap * 8)); CK(ctx->d_drep_read.ensure((size_t)cap * 4)); CK(ctx->d_drep_qpos.ensure((size_t)cap * 4));
@@ -1126,12 +1143,8 @@ static int pileup(smc_ctx* ctx) {
         CK(cudaMemsetAsync(ctx->d_cnt.p, 0, nlz * SMC_NFIXED * SMC_NCNT * 4, ctx->st));
         CK(cudaMemsetAsync(ctx->d_limb.p, 0, nlz * SMC_NFIXED * 3 * 8, ctx->st));
         CK(cudaMemsetAsync(small + SW_GFLAGS, 0, 24, ctx->st));     // gflags, dyn count, n_tasks, cvg sum
-        if (ctx->spill_cap == 0) {
-            ctx->spill_cap = 1024;
-            if (const char* ev = getenv("SMC_SPILL_CAP0")) { long v = atol(ev); if (v >= 1 && v <= (1l << 24)) ctx->spill_cap = (uint32_t)v; }   // test hook
-        }
-        CK(ctx->d_spill.ensure((size_t)ctx->spill_cap * sizeof(SpillRec)));
-        CK(cudaMemsetAsync(small + SW_SPILL_COUNT, 0, 4, ctx->st));
+        CK(ctx->d_defer.ensure((size_t)ctx->defer_cap * sizeof(uint4)));
+        CK(cudaMemsetAsync(small + SW_DEFER_COUNT, 0, 4, ctx->st));
         if (ctx->n_tile_events > 0) {
             if (const int rc = ensure_code_storage(ctx, false, ctx->has_keep)) return rc;
             KAArgs A; KBArgs B;
@@ -1144,8 +1157,8 @@ static int pileup(smc_ctx* ctx) {
         if (const int rc = read_back(ctx, w, small + SW_GFLAGS, sizeof(w))) return rc;
         CK(cudaGetLastError());
         const uint32_t gflags = w[0];
-        if (!(gflags & (GF_DYN_FULL | GF_CODE_FULL | GF_SPILL_FULL))) { ctx->n_dyn = w[1]; return SMC_OK; }
-        if (gflags & GF_SPILL_FULL) ctx->spill_cap = ctx->spill_cap >= (1u << 24) ? ctx->spill_cap : ctx->spill_cap * 4;
+        if (!(gflags & (GF_DYN_FULL | GF_CODE_FULL | GF_DEFER_FULL))) { ctx->n_dyn = w[1]; return SMC_OK; }
+        if (gflags & GF_DEFER_FULL) ctx->defer_cap = ctx->defer_cap >= (1u << 26) ? ctx->defer_cap : ctx->defer_cap * 4;
         if (attempt == 5) { ctx->err = "dynamic allele table / fragment code storage overflow"; return SMC_E_OVERFLOW; }
         if (gflags & GF_CODE_FULL) ctx->code_mult = 3;             // worst-case layout: always fits
         if (gflags & GF_DYN_FULL) {
@@ -1322,6 +1335,7 @@ static int device_downsample(smc_ctx* ctx) {
     LAUNCH(k_ds_list_fill, nblk(nl, 256), 256, 0, ctx->d_ds_flag.as<uint32_t>(), v0, v1, nl, nflag, T, ctx->d_list_idx.as<int32_t>(), list_off, locus);
     // 2. their barcodes with their first passing reads: the listing pass of the pileup pair
     CK(cudaMemsetAsync(ctx->d_list_count.p, 0, (size_t)nflag * 4, ctx->st));
+    CK(cudaMemsetAsync(ctx->d_small.as<uint32_t>() + SW_DEFER_COUNT, 0, 4, ctx->st));
     if (const int rc = ensure_code_storage(ctx, true, true)) return rc;
     {
         KAArgs A; KBArgs B;

@@ -11,7 +11,8 @@
 //   k_gather  (K3a)  smCounter.py:368-479   pileup of every read event: base / quality gather, read-level tallies, fragment
 //                    merge.  No FP64, few registers, high occupancy: this is where all the DRAM / L2 latency of the path is.
 //   k_merge   (K3b)  smCounter.py:26-98, 482-532   per-barcode posterior (calProb), prediction index, consensus counters.
-//                    FP64 and 128-bit fixed point; its only input is the coalesced stream of fragment codes.
+//                    FP64 and 128-bit fixed point; its only input is the coalesced stream of fragment codes.  The rare
+//                    barcodes whose calProb takes the general form go to k_merge_deferred, one thread per barcode and locus.
 #pragma once
 #include "smc_common.cuh"
 
@@ -58,7 +59,7 @@ struct PrepArgs {
 #define GF_BAD_READ   2u     // l_seq / clip length beyond the 16-bit record fields
 #define GF_CODE_FULL  4u     // a unit ran out of fragment-code storage (host retries with the worst-case layout)
 #define GF_BAD_STORE  8u     // stored window (store_lo / store_len) malformed or not covering every target base of the read
-#define GF_SPILL_FULL 16u    // k_merge ran out of spill records (host retries with a larger pool)
+#define GF_DEFER_FULL 16u    // k_merge ran out of deferred-barcode records (host retries with a longer list)
 #define GF_FRAG_UMI   32u    // a frag_id carries reads of two barcodes (k_umi_slots)
 
 __global__ void __launch_bounds__(256) k_read_prep(PrepArgs A) {
@@ -244,11 +245,8 @@ static inline uint64_t code_slots_total(uint64_t ne, uint64_t n_units, uint32_t 
 }
 
 #define NF SMC_NFIXED
-#define NDYN 6             // dynamic alleles (indel starts, N / IUPAC bases) of one barcode at one locus that live in shared memory
-#define NSLOT (NF + NDYN)  // per-barcode allele slots in shared memory: 5 fixed + NDYN dynamic
-#define NSPILL 21          // further dynamic alleles of the barcode live in a spill record in global memory (5 + 6 + 21 = the 32
-                           // slots of the lane's allele bit mask; a barcode beyond that raises SMC_ST_UMI_OVERFLOW)
-struct SpillRec { uint32_t e[NSPILL]; int32_t cnt[NSPILL]; double prod[NSPILL]; };
+#define NDYN 27            // dynamic alleles (indel starts, N / IUPAC bases) of one barcode at one locus: 5 fixed + 27 = the 32
+                           // slots of the allele bit mask; a barcode beyond that raises SMC_ST_UMI_OVERFLOW
 
 // The dynamic-allele table, passed BY VALUE to the out-of-line helpers.
 struct DynTab {
@@ -256,7 +254,6 @@ struct DynTab {
     int32_t* dcnt; unsigned long long* dlimb; uint8_t* diskey; uint32_t* dcount; uint32_t* gflags;
     const uint16_t* bq; const uint32_t* bq_off;      // bq[] and each read's first stored word (caller's SoA order): long insertions are
                                                      // compared base by base
-    SpillRec* spill; uint32_t spill_cap; uint32_t* spill_count;      // k_merge: pool of spill records (one per overflowing lane and barcode)
 };
 
 // BAM nibble of A, C, G, T (1, 2, 4, 8) -> field A0 C1 T2 G3 of the packed register counters / allele slot A0 C1 T3 G4
@@ -896,16 +893,21 @@ __global__ void __launch_bounds__(KA_WARPS * 32, KA_MINBLOCKS) k_gather_t(const 
 #define KB_WARPS 4
 #endif
 #ifndef KB_MINBLOCKS
-#define KB_MINBLOCKS 5
+#define KB_MINBLOCKS 7    // B200, cfg2: 5 / 6 / 7 / 8 blocks of 4 warps 1.070 / 0.984 / 0.954 / 0.961 ms; 8 warps x 3 / 4 blocks 1.003 / 0.974
 #endif
 #define KB_FC_WORDS    (NF * 32)                // MTCnt | strongMTCnt << 16 per fixed allele and lane
 #define KB_LIMB_WORDS  (NF * 4 * 32)            // 128-bit fixed-point PI accumulator per fixed allele and lane
-#define KB_UCNT_WORDS  (NSLOT * 32)
-#define KB_UPROD_WORDS (NSLOT * 64)
-#define KB_UDYN_WORDS  (NDYN * 32)              // dynamic-allele row of slot NF + k of the open barcode, per lane
-#define KB_WARP_WORDS  (KB_FC_WORDS + KB_LIMB_WORDS + KB_UCNT_WORDS + KB_UPROD_WORDS + KB_UDYN_WORDS)
-#define KB_TAB_BYTES   4128                     // {p, 1 - p} of a fragment: entry 0 = not 'Paired' (0.1), entry 1 + quality = 'Paired' (257 x double2)
+#define KB_WARP_WORDS  (KB_FC_WORDS + KB_LIMB_WORDS)
+#define KB_TAB_BYTES   2064                     // 1 - p of a fragment: entry 0 = not 'Paired' (p = 0.1), entry 1 + quality = 'Paired' (257 doubles, padded to 16 B)
 #define KB_SMEM_BYTES  (KB_TAB_BYTES + KB_WARPS * KB_WARP_WORDS * 4)
+#define KD_THREADS     128                      // k_merge_deferred
+
+// A barcode whose calProb takes the general form (several alleles, a DEL or dynamic allele, or more fragments than the prior
+// table holds) is left by k_merge to k_merge_deferred, in a record of the list KBArgs::defer:
+//   {unit, the barcode's first fragment code in the unit, extension rows of the unit before that code, lane | DR_* bits}.
+// Such pairs are rare (cfg2: one per ~400 tile events); k_merge keeps neither their per-allele products nor their dynamic-allele
+// slots, which keeps its registers and shared memory to what the single-allele barcodes need.
+#define DR_STATUS_ONLY (1u << 8)     // a barcode outside the call (masked out, or n <= mtDrop): replayed only for SMC_ST_UMI_OVERFLOW
 
 struct KBArgs {
     const uint4* codes; const uint32_t* unit_nfrag; const uint32_t* frag_first; const uint32_t* umi_urank;
@@ -921,6 +923,7 @@ struct KBArgs {
     DynTab T;
     // optional: list the barcodes of bcDict for flagged loci (down-sampling support)
     const int32_t* list_idx; uint32_t* list_count; const int64_t* list_off; uint64_t* list_umi; uint32_t* list_first; int64_t list_cap;
+    uint4* defer; uint32_t defer_cap; uint32_t* defer_count;      // deferred barcodes (GF_DEFER_FULL when the list is full)
 };
 
 // A non-negative double < 2^20 as a 128-bit fixed-point integer with LSB 2^-PI_FIX_LSB (= 2^-80), truncated: the integer part
@@ -948,32 +951,33 @@ __device__ __forceinline__ void split_limbs(unsigned long long lo, unsigned long
     a1 = ((lo >> 44) | (hi << 20)) & M44;
     a2 = hi >> 24;
 }
+// a 128-bit PI term or sum -> adds its limbs to the global accumulator l[0], l[stride], l[2 * stride]
+__device__ __forceinline__ void add_limbs(unsigned long long* l, size_t stride, unsigned long long lo, unsigned long long hi) {
+    unsigned long long a0, a1, a2;
+    split_limbs(lo, hi, a0, a1, a2);
+    if (a0) atomicAdd(l, a0);
+    if (a1) atomicAdd(l + stride, a1);
+    if (a2) atomicAdd(l + 2 * stride, a2);
+}
 
 // per-lane flags of the open barcode
 #define LF_UMI_SEEN  (1u << 0)    // a read of the barcode covers the locus
 #define LF_UMI_BC    (1u << 1)    // the barcode is in bcDict (a read passed incCond)
+#define LF_DEFER     (1u << 2)    // a fragment showed a second allele or a dynamic one: k_merge_deferred finishes the barcode
 
 struct MergeState {
     // locus-level
     int allFrag, allMT, usedFrag, nBC, usedMT, mt3, mt5, mt7, mt10;
-    uint32_t keymask, status;
+    uint32_t keymask;
     unsigned long long pad_lo, pad_hi;      // PI terms that go to all of A, C, G, T (single-allele barcodes, see umi_finalize)
     uint32_t flags;                         // LF_*
-    // barcode-level
-    int n; uint32_t exist; double Q, rightP; uint32_t last_aid; int ndyn;      // the rows of the dynamic slots live in shared memory (UDYN) ...
-    SpillRec* sp;                           // ... and, from the 7th dynamic allele of the barcode on, in this spill record (else nullptr)
+    // barcode-level: until LF_DEFER the barcode has shown one allele, so its product over fragments is rightP and its count n
+    int n; uint32_t exist; double rightP; uint32_t last_aid;
     uint32_t first_read;                    // BAM index of the barcode's first passing read at this locus (listing only)
 };
 
 #define FCW(a)      fc[(a) * 32 + lane]
 #define LIMB(a)     limb[(a) * 32 + lane]
-#define UCNT(s)     ucnt[(s) * 32 + lane]
-#define UPROD(s)    uprod[(s) * 32 + lane]
-#define UDYN(k)     (reinterpret_cast<uint32_t*>(uprod + NSLOT * 32)[(k) * 32 + lane])
-// the same three per-slot arrays with the spill record behind them (`sp` in scope; never touched for slots in shared memory)
-#define XCNT(s)     (*((s) < NSLOT ? &UCNT(s) : &sp->cnt[(s) - NSLOT]))
-#define XPROD(s)    (*((s) < NSLOT ? &UPROD(s) : &sp->prod[(s) - NSLOT]))
-#define XDYN(k)     (*((k) < NDYN ? &UDYN(k) : &sp->e[(k) - NDYN]))
 
 // MTCnt / strongMTCnt of an allele that may be dynamic; add = 1 (MTCnt) or 0x10001 (both)
 __device__ __forceinline__ void bump_mt(int32_t* dcnt, int* fc, int lane, uint32_t aid, uint32_t add) {
@@ -985,53 +989,53 @@ __device__ __forceinline__ void bump_mt(int32_t* dcnt, int* fc, int lane, uint32
     }
 }
 
-// first use of the per-barcode shared-memory arrays: a barcode that has shown a single allele so far keeps its state in
-// registers only (its product over fragments IS rightP, its count IS n)
-__device__ __forceinline__ void umi_materialize(int lane, int* ucnt, double* uprod, uint32_t exist, int n, double rightP) {
-    const int s0 = __ffs(exist) - 1;
-    UCNT(s0) = n; UPROD(s0) = rightP;
+// A deferred barcode at one locus, as k_merge_deferred rebuilds it (one thread, local memory): allele slots 0 .. NF - 1 are
+// the fixed alleles, slot NF + k the barcode's k-th dynamic allele (its row of the dynamic-allele table is dyn[k]).
+struct UmiState {
+    int n; uint32_t exist; double Q, rightP; uint32_t last_aid; int ndyn; uint32_t status;
+    int cnt[NF + NDYN]; double prod[NF + NDYN]; uint32_t dyn[NDYN];
+};
+
+// While a barcode shows one allele, its count is n and its product over fragments rightP; its slot is filled when a second
+// allele joins, or before umi_general.
+__device__ __forceinline__ void umi_fill_single(UmiState& U) {
+    const int s0 = __ffs(U.exist) - 1;
+    U.cnt[s0] = U.n; U.prod[s0] = U.rightP;
 }
 
-// one fragment of bcDict joins the open barcode (the per-fragment part of calProb, smCounter.py:56-77)
-__device__ __forceinline__ void fragment_join(DynTab T, double p, double q1, uint32_t aid, int lane, int* ucnt, double* uprod, MergeState& S) {
+// one fragment of bcDict joins the barcode (the per-fragment part of calProb, smCounter.py:56-77)
+__device__ __forceinline__ void fragment_join(double p, double q1, uint32_t aid, UmiState& U) {
     int slot = (int)aid;
-    SpillRec* sp = S.sp;
     if (aid >= NF) {
         const uint32_t e = aid - NF;
         int k = 0;
-        while (k < S.ndyn && XDYN(k) != e) ++k;
-        if (k == S.ndyn) {
-            if (k >= NDYN && !sp) {                                   // 7th dynamic allele of this barcode: take a spill record
-                const uint32_t r = atomicAdd(T.spill_count, 1u);
-                if (r >= T.spill_cap) atomicOr(T.gflags, GF_SPILL_FULL);
-                sp = S.sp = T.spill + (r < T.spill_cap ? r : 0u);
-            }
-            if (k < NDYN + NSPILL) { XDYN(k) = e; S.ndyn = k + 1; }
-            else { S.status |= SMC_ST_UMI_OVERFLOW; k = 0; }
+        while (k < U.ndyn && U.dyn[k] != e) ++k;
+        if (k == U.ndyn) {
+            if (k < NDYN) { U.dyn[k] = e; U.ndyn = k + 1; }
+            else { U.status |= SMC_ST_UMI_OVERFLOW; k = 0; }
         }
         slot = NF + k;
     }
     const uint32_t bit = 1u << slot;
-    if (S.exist == 0) S.exist = bit;
+    if (U.exist == 0) U.exist = bit;
     else {
-        const bool multi = (S.exist & (S.exist - 1u)) != 0u;
-        if (multi || S.exist != bit) {
-            if (!multi) umi_materialize(lane, ucnt, uprod, S.exist, S.n, S.rightP);
-            if (!(S.exist & bit)) { S.exist |= bit; XCNT(slot) = 0; XPROD(slot) = S.Q; }
-            uint32_t m = S.exist;
+        const bool multi = (U.exist & (U.exist - 1u)) != 0u;
+        if (multi || U.exist != bit) {
+            if (!multi) umi_fill_single(U);
+            if (!(U.exist & bit)) { U.exist |= bit; U.cnt[slot] = 0; U.prod[slot] = U.Q; }
+            uint32_t m = U.exist;
             while (m) {                                                  // :70-74
                 int s = __ffs(m) - 1; m &= m - 1;
-                XPROD(s) = __dmul_rn(XPROD(s), s == slot ? q1 : p);
+                U.prod[s] = __dmul_rn(U.prod[s], s == slot ? q1 : p);
             }
-            XCNT(slot) += 1;
+            U.cnt[slot] += 1;
         }
     }
-    S.Q = __dmul_rn(S.Q, p);
-    S.rightP = __dmul_rn(S.rightP, q1);                              // :77
-    S.n += 1;
-    S.last_aid = aid;
+    U.Q = __dmul_rn(U.Q, p);
+    U.rightP = __dmul_rn(U.rightP, q1);                              // :77
+    U.n += 1;
+    U.last_aid = aid;
 }
-
 
 // PCR prior outside the host-built table (barcodes with > pcr_nmax fragments or > 6 distinct alleles): device pow()
 __device__ __noinline__ double pcr_slow(int cnt, double denom) {
@@ -1076,21 +1080,30 @@ __device__ __forceinline__ double neg_log10_1m_small(double p) {
     return (s * q) * 0.43429448190325182765;             // 1 / ln(10)
 }
 
+// MTCnt / strongMTCnt of an allele that may be dynamic, straight to the per-locus accumulators
+__device__ __forceinline__ void bump_mt_global(int32_t* cnt, size_t nl, int64_t L, int32_t* dcnt, uint32_t aid, bool strong) {
+    int32_t* row = aid < NF ? cnt + (size_t)aid * SMC_NCNT * nl + L : dcnt + (size_t)(aid - NF) * SMC_NCNT;
+    const size_t stride = aid < NF ? nl : 1;
+    atomicAdd(&row[SMC_C_MT * stride], 1);
+    if (strong) atomicAdd(&row[SMC_C_STRONG * stride], 1);
+}
+
 // calProb + consensus for a barcode that shows several alleles, a DEL / dynamic allele, or more fragments than the prior
-// table holds (smCounter.py:26-98, 506-523) -- the general form; the per-barcode arrays are in shared memory.
-// Returns the finalDict keys it touched among the fixed alleles.
-__device__ __noinline__ uint32_t umi_general(DynTab T, const double* __restrict__ pcrtab, int pcr_nmax, double smt, int lane, int n,
-                                             uint32_t exist, double rightP, int ndyn, uint32_t last_aid,
-                                             int* fc, ulonglong2* limb, int* ucnt, double* uprod, SpillRec* sp) {
-    uint32_t keymask = 0;
+// table holds (smCounter.py:26-98, 506-523) -- the general form, for the barcode U at locus L; its PI terms and MT counts go
+// to the per-locus accumulators with atomics.  Returns the finalDict keys it touched among the fixed alleles.
+__device__ __noinline__ uint32_t umi_general(DynTab T, const double* __restrict__ pcrtab, int pcr_nmax, double smt,
+                                             int32_t* cnt, unsigned long long* limb, size_t nl, int64_t L, UmiState& U) {
+    const int n = U.n, ndyn = U.ndyn;
+    const double rightP = U.rightP;
+    uint32_t exist = U.exist, keymask = 0;
     // canonical order of the dynamic slots = ascending allele key (insertion sort of the slot rows; a slot whose exist bit is
     // clear -- its fragments were all deleted again -- travels with its bit)
     for (int i = 1; i < ndyn; ++i)
-        for (int j = i; j > 0 && __ldcg(&T.dkey[XDYN(j - 1)]) > __ldcg(&T.dkey[XDYN(j)]); --j) {
+        for (int j = i; j > 0 && __ldcg(&T.dkey[U.dyn[j - 1]]) > __ldcg(&T.dkey[U.dyn[j]]); --j) {
             const int a = NF + j - 1, b = NF + j;
-            const uint32_t tu = XDYN(j - 1); XDYN(j - 1) = XDYN(j); XDYN(j) = tu;
-            const int tc = XCNT(a); XCNT(a) = XCNT(b); XCNT(b) = tc;
-            const double tp = XPROD(a); XPROD(a) = XPROD(b); XPROD(b) = tp;
+            const uint32_t tu = U.dyn[j - 1]; U.dyn[j - 1] = U.dyn[j]; U.dyn[j] = tu;
+            const int tc = U.cnt[a]; U.cnt[a] = U.cnt[b]; U.cnt[b] = tc;
+            const double tp = U.prod[a]; U.prod[a] = U.prod[b]; U.prod[b] = tp;
             const uint32_t ba = (exist >> a) & 1u, bb = (exist >> b) & 1u;
             exist = (exist & ~((1u << a) | (1u << b))) | (bb << a) | (ba << b);
         }
@@ -1111,7 +1124,7 @@ __device__ __noinline__ uint32_t umi_general(DynTab T, const double* __restrict_
     double tpad = rightP;                                         // :88-91
     for (uint32_t m = exist; m; m &= m - 1) {
         const int s = __ffs(m) - 1;
-        const int c = XCNT(s);
+        const int c = U.cnt[s];
         const double v = tab ? __ldg(trow + c) : pcr_slow(c, denom);
         tpad = __dmul_rn(tpad, v);
         if (v < m1) { m2 = m1; m1 = v; arg1 = s; } else if (v < m2) m2 = v;
@@ -1121,12 +1134,12 @@ __device__ __noinline__ uint32_t umi_general(DynTab T, const double* __restrict_
     for (uint32_t m = exist; m; m &= m - 1) {
         const int s = __ffs(m) - 1;
         const double minp = (s == arg1) ? m2 : m1;                // min over the OTHER members of uniq
-        XPROD(s) = __dadd_rn(__dmul_rn(PCR_NO_ERROR, XPROD(s)), __dmul_rn(rightP, minp));
+        U.prod[s] = __dadd_rn(__dmul_rn(PCR_NO_ERROR, U.prod[s]), __dmul_rn(rightP, minp));
     }
     double sumP = 0.0;                                            // :93, in canonical slot order
     for (uint32_t m = uniq; m; m &= m - 1) {
         const int s = __ffs(m) - 1;
-        sumP = __dadd_rn(sumP, ((exist >> s) & 1u) ? XPROD(s) : tpad);
+        sumP = __dadd_rn(sumP, ((exist >> s) & 1u) ? U.prod[s] : tpad);
     }
     // ---- posterior -> -log10(1-p) (:96, :509-510), PI accumulation (:512), consensus (:514-523).
     // One loop over the members of uniq in slot order; the pads share one value (computed at the first pad).
@@ -1139,32 +1152,26 @@ __device__ __noinline__ uint32_t umi_general(DynTab T, const double* __restrict_
         double l; unsigned long long lo, hi;
         if (is_pad && have_pad) { l = l_pad; lo = plo; hi = phi; }
         else {
-            l = neg_log10_1m(sumP <= 0.0 ? 0.0 : (is_pad ? tpad : XPROD(s)) / sumP);
+            l = neg_log10_1m(sumP <= 0.0 ? 0.0 : (is_pad ? tpad : U.prod[s]) / sumP);
             pi_fixed128(l, lo, hi);
             if (is_pad) { have_pad = true; l_pad = l; plo = lo; phi = hi; }
         }
         if (s < NF) {
-            ulonglong2 v = LIMB(s);
-            add128(v.x, v.y, lo, hi);
-            LIMB(s) = v;
+            add_limbs(limb + (size_t)s * 3 * nl + L, nl, lo, hi);
             keymask |= 1u << s;
         } else {
-            const uint32_t e = XDYN(s - NF);
-            unsigned long long a0, a1, a2;
-            split_limbs(lo, hi, a0, a1, a2);
-            if (a0) atomicAdd(&T.dlimb[(size_t)e * 3 + 0], a0);
-            if (a1) atomicAdd(&T.dlimb[(size_t)e * 3 + 1], a1);
-            if (a2) atomicAdd(&T.dlimb[(size_t)e * 3 + 2], a2);
+            const uint32_t e = U.dyn[s - NF];
+            add_limbs(T.dlimb + (size_t)e * 3, 1, lo, hi);
             T.diskey[e] = 1;
         }
         if (l > best) { best = l; nbest = 1; cons = s; }
         else if (l == best) nbest++;
     }
     if (nbest == 1) {                                             // :515-519
-        const uint32_t aid = cons < NF ? (uint32_t)cons : NF + XDYN(cons - NF);
-        bump_mt(T.dcnt, fc, lane, aid, best > smt ? 0x10001u : 1u);
+        const uint32_t aid = cons < NF ? (uint32_t)cons : NF + U.dyn[cons - NF];
+        bump_mt_global(cnt, nl, L, T.dcnt, aid, best > smt);
     } else if (n == 1) {                                          // :521-523
-        bump_mt(T.dcnt, fc, lane, last_aid, 1u);
+        bump_mt_global(cnt, nl, L, T.dcnt, U.last_aid, false);
     }
     return keymask;
 }
@@ -1191,10 +1198,11 @@ __device__ __noinline__ bool umi_mask_and_list(MaskListArgs A, int ki, int li, u
     return used;
 }
 
-// calProb + the per-barcode part of vc() (smCounter.py:26-98, 506-532) for the lane's locus.
+// calProb + the per-barcode part of vc() (smCounter.py:26-98, 506-532) for the lane's locus; the general form of calProb is
+// deferred: `rec` is the record k_merge_deferred gets for it.
 template <bool LIST>
-__device__ __forceinline__ void umi_finalize(const KBArgs& A, int lane, int ki, int li, uint32_t umi_slot, int* fc, ulonglong2* limb,
-                                             int* ucnt, double* uprod, MergeState& S) {
+__device__ __forceinline__ void umi_finalize(const KBArgs& A, int lane, int ki, int li, uint32_t umi_slot, uint4 rec, int* fc, ulonglong2* limb,
+                                             MergeState& S) {
     if (S.flags & LF_UMI_SEEN) S.allMT++;
     bool used = S.flags & LF_UMI_BC;
     if (used) {
@@ -1210,12 +1218,11 @@ __device__ __forceinline__ void umi_finalize(const KBArgs& A, int lane, int ki, 
         const int n = S.n;
         S.usedMT++; S.usedFrag += n;
         S.mt3 += n >= 3; S.mt5 += n >= 5; S.mt7 += n >= 7; S.mt10 += n >= 10;
-        const bool multi = (S.exist & (S.exist - 1u)) != 0u;
         const uint32_t ACGT = (1u << SMC_A_A) | (1u << SMC_A_T) | (1u << SMC_A_G) | (1u << SMC_A_C);
         if (n <= A.mtDrop) {                              // :28-32 -> four zeros, a 4-way tie (:514-523)
             S.keymask |= ACGT;
             if (n == 1) bump_mt(A.T.dcnt, fc, lane, S.last_aid, 1u);
-        } else if (!multi && (S.exist & ACGT) && n <= A.pcr_nmax) {
+        } else if (!(S.flags & LF_DEFER) && (S.exist & ACGT) && n <= A.pcr_nmax) {
             // ---- fast path: every fragment of the barcode shows the same base a0 in {A,C,G,T}; uniq = {A,C,G,T} (:49-54).
             // Same operations in the same order as umi_general (prodP[a0] == rightP, one present allele, three pads
             // sharing one value), with all intermediates in registers.
@@ -1248,29 +1255,28 @@ __device__ __forceinline__ void umi_finalize(const KBArgs& A, int lane, int ki, 
             if (l_e > l_pad) FCW(a0) += (l_e > A.smt) ? 0x10001 : 1;
             else if (n == 1) FCW(a0) += 1;
         } else {
-            if (!multi) umi_materialize(lane, ucnt, uprod, S.exist, n, S.rightP);
-            S.keymask |= umi_general(A.T, A.pcrtab, A.pcr_nmax, A.smt, lane, n, S.exist, S.rightP, S.ndyn,
-                                     S.last_aid, fc, limb, ucnt, uprod, S.sp);
+            rec.w &= ~DR_STATUS_ONLY;
         }
     }
-    S.n = 0; S.exist = 0; S.Q = 1.0; S.rightP = 1.0; S.ndyn = 0; S.flags = 0; S.first_read = 0xffffffffu; S.sp = nullptr;
+    // the general form, or a deferred barcode outside the call that may hold more dynamic alleles than its slots
+    if (!(rec.w & DR_STATUS_ONLY) || ((S.flags & LF_DEFER) && S.n > NDYN)) {
+        const uint32_t r = atomicAdd(A.defer_count, 1u);
+        if (r < A.defer_cap) A.defer[r] = rec;
+        else atomicOr(A.T.gflags, GF_DEFER_FULL);
+    }
+    S.n = 0; S.exist = 0; S.rightP = 1.0; S.flags = 0; S.first_read = 0xffffffffu;
 }
 
 template <bool LIST>
 __global__ void __launch_bounds__(KB_WARPS * 32, KB_MINBLOCKS) k_merge_t(const KBArgs A) {
     extern __shared__ __align__(16) uint32_t smem[];
-    double2* pq_s = reinterpret_cast<double2*>(smem);        // fragment probability (smCounter.py:65-68) and its complement (:72, :77)
-    for (int i = threadIdx.x; i < 257; i += KB_WARPS * 32) {
-        const double pf = i == 0 ? 0.1 : __ldg(&A.bqtab[i - 1]);
-        pq_s[i] = make_double2(pf, 1.0 - pf);
-    }
+    double* q_s = reinterpret_cast<double*>(smem);           // complement of the fragment probability (smCounter.py:65-68, :77)
+    for (int i = threadIdx.x; i < 257; i += KB_WARPS * 32) q_s[i] = 1.0 - (i == 0 ? 0.1 : __ldg(&A.bqtab[i - 1]));
     __syncthreads();
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
     uint32_t* ws = smem + KB_TAB_BYTES / 4 + (size_t)w * KB_WARP_WORDS;
     int* fc = (int*)ws;
     ulonglong2* limb = (ulonglong2*)(ws + KB_FC_WORDS);
-    int* ucnt = (int*)(ws + KB_FC_WORDS + KB_LIMB_WORDS);
-    double* uprod = (double*)(ws + KB_FC_WORDS + KB_LIMB_WORDS + KB_UCNT_WORDS);
 
     const uint32_t unit = A.unit0 + blockIdx.x * KB_WARPS + w;
     if (unit >= A.n_units) return;
@@ -1291,12 +1297,13 @@ __global__ void __launch_bounds__(KB_WARPS * 32, KB_MINBLOCKS) k_merge_t(const K
 
     MergeState S;
     S.allFrag = S.allMT = S.usedFrag = S.nBC = S.usedMT = S.mt3 = S.mt5 = S.mt7 = S.mt10 = 0;
-    S.keymask = 0; S.status = 0; S.pad_lo = S.pad_hi = 0;
+    S.keymask = 0; S.pad_lo = S.pad_hi = 0;
     S.flags = 0;
-    S.n = 0; S.exist = 0; S.Q = 1.0; S.rightP = 1.0; S.last_aid = 0; S.ndyn = 0; S.sp = nullptr;
+    S.n = 0; S.exist = 0; S.rightP = 1.0; S.last_aid = 0;
     S.first_read = 0xffffffffu;
 
-    uint32_t umi_slot = eb;                                        // warp uniform: umi_urank[] slot of the open barcode
+    // warp uniform: umi_urank[] slot, first fragment code and the extension rows before it of the open barcode; rows read
+    uint32_t umi_slot = eb, umi_f = 0, umi_x = 0, nx = 0;
     const uint4* cp = A.codes + (so >> 3) * 32 + lane;
     const uint32_t* extp = reinterpret_cast<const uint32_t*>(A.codes) + (so + cap) * 16 + lane;   // extension rows, downward
     const uint32_t* ffp = LIST ? A.frag_first + so * 32 + lane : nullptr;
@@ -1312,9 +1319,12 @@ __global__ void __launch_bounds__(KB_WARPS * 32, KB_MINBLOCKS) k_merge_t(const K
         }
         const uint32_t cd = f < F ? (v.x & 0xffffu) : FC_UMIFIRST;
         v.x = __funnelshift_r(v.x, v.y, 16); v.y = __funnelshift_r(v.y, v.z, 16); v.z = __funnelshift_r(v.z, v.w, 16); v.w >>= 16;
-        if ((cd & FC_UMIFIRST) && f != 0u) {                           // warp uniform: the previous barcode is complete
-            umi_finalize<LIST>(A, lane, ki, li, umi_slot, fc, limb, ucnt, uprod, S);
-            ++umi_slot;
+        if (cd & FC_UMIFIRST) {                                        // warp uniform
+            if (f != 0u) {                                             // the previous barcode is complete
+                umi_finalize<LIST>(A, lane, ki, li, umi_slot, make_uint4(unit, umi_f, umi_x, (uint32_t)lane | DR_STATUS_ONLY), fc, limb, S);
+                ++umi_slot;
+            }
+            umi_f = f; umi_x = nx;
         }
         const uint32_t st = (cd >> FC_ST_SH) & 3u;
         S.allFrag += st ? 1 : 0;                                       // :463-464
@@ -1322,24 +1332,21 @@ __global__ void __launch_bounds__(KB_WARPS * 32, KB_MINBLOCKS) k_merge_t(const K
         if (LIST) { S.first_read = min(S.first_read, f < F ? __ldg(ffp) : 0xffffffffu); ffp += 32; }
         uint32_t aid = (cd >> FC_AID_SH) & 7u;
         if (cd & FC_EXT) {                                             // warp uniform
-            extp -= 32;
+            extp -= 32; ++nx;
             const uint32_t e = __ldg(extp);
             if (aid == FC_AID_DYN) aid = NF + e;
         }
-        const double2 pq = pq_s[((cd >> 13) & 1u) * ((cd & 0xffu) + 1u)];                // smCounter.py:65-68 (a valid entry for any code)
+        const double q = q_s[((cd >> 13) & 1u) * ((cd & 0xffu) + 1u)];                  // smCounter.py:65-68 (a valid entry for any code)
         const bool join = st == 3u;
-        // Nine rows out of ten no lane's barcode shows a second allele or a dynamic one: the fragment joins a single-allele
-        // barcode (fragment_join reduces to two products and a count), done without a divergent branch -- a fragment that
-        // is not in bcDict multiplies by exactly 1.0.
+        // The fragment joins a barcode that has shown one allele so far (fragment_join reduces to a product and a count),
+        // branch free -- a fragment that is not in bcDict multiplies by exactly 1.0.  A second allele or a dynamic one defers
+        // the barcode to k_merge_deferred; from then on only its count and last allele matter here.
         const uint32_t bit = 1u << (aid & 31u);
-        const bool rare = join && (aid >= NF || (S.exist & ~bit) != 0u);
-        if (!__any_sync(FULL_MASK, rare)) {
-            S.Q = __dmul_rn(S.Q, join ? pq.x : 1.0);
-            S.rightP = __dmul_rn(S.rightP, join ? pq.y : 1.0);                        // :77
-            S.n += join ? 1 : 0;
-            S.exist |= join ? bit : 0u;
-            S.last_aid = join ? aid : S.last_aid;
-        } else if (join) fragment_join(A.T, pq.x, pq.y, aid, lane, ucnt, uprod, S);
+        S.flags |= (join && (aid >= NF || (S.exist & ~bit) != 0u)) ? LF_DEFER : 0u;
+        S.rightP = __dmul_rn(S.rightP, join ? q : 1.0);                                  // :77
+        S.n += join ? 1 : 0;
+        S.exist |= join ? bit : 0u;
+        S.last_aid = join ? aid : S.last_aid;
     }
     // ---- flush the lane's locus to the per-locus accumulators ([field][locus] layout: coalesced across lanes)
     if (lane_valid) {
@@ -1351,11 +1358,7 @@ __global__ void __launch_bounds__(KB_WARPS * 32, KB_MINBLOCKS) k_merge_t(const K
             if (mv >> 16) atomicAdd(&A.cnt[((size_t)a * SMC_NCNT + SMC_C_STRONG) * nl + L], (int)(mv >> 16));
             ulonglong2 v2 = LIMB(a);
             if (a != SMC_A_DEL) add128(v2.x, v2.y, S.pad_lo, S.pad_hi);
-            unsigned long long a0, a1, a2;
-            split_limbs(v2.x, v2.y, a0, a1, a2);
-            if (a0) atomicAdd(&A.limb[((size_t)a * 3 + 0) * nl + L], a0);
-            if (a1) atomicAdd(&A.limb[((size_t)a * 3 + 1) * nl + L], a1);
-            if (a2) atomicAdd(&A.limb[((size_t)a * 3 + 2) * nl + L], a2);
+            add_limbs(A.limb + (size_t)a * 3 * nl + L, nl, v2.x, v2.y);
         }
         int32_t* loc = A.loc;
         if (S.allFrag) atomicAdd(&loc[SMC_L_ALLFRAG * nl + L], S.allFrag);
@@ -1368,6 +1371,47 @@ __global__ void __launch_bounds__(KB_WARPS * 32, KB_MINBLOCKS) k_merge_t(const K
         if (S.mt7) atomicAdd(&loc[SMC_L_MT7 * nl + L], S.mt7);
         if (S.mt10) atomicAdd(&loc[SMC_L_MT10 * nl + L], S.mt10);
         if (S.keymask) atomicOr(&loc[SMC_L_KEYMASK * nl + L], (int)S.keymask);
-        if (S.status) atomicOr(&loc[SMC_L_STATUS * nl + L], (int)S.status);
+    }
+}
+
+// The barcodes k_merge deferred, one thread per record: the barcode's fragments at the lane's locus run through the general
+// fragment_join again, from its first fragment code to the next barcode's, and umi_general finishes it.  Every fragment takes
+// the same operations in the same order as it would have inside k_merge; the results go to the same accumulators with atomics
+// (integers and 128-bit fixed point, so where and when they are added does not change them).
+__global__ void __launch_bounds__(KD_THREADS) k_merge_deferred(const KBArgs A) {
+    const uint32_t nrec = min(*A.defer_count, A.defer_cap);
+    const size_t nl = (size_t)A.n_loci;
+    for (uint32_t r = blockIdx.x * KD_THREADS + threadIdx.x; r < nrec; r += gridDim.x * KD_THREADS) {
+        const uint4 rec = A.defer[r];
+        const uint32_t unit = rec.x, lane = rec.w & 31u;
+        const uint32_t F = A.unit_nfrag[unit], eb = A.unit_eb[unit], ee = A.unit_ee[unit];
+        const uint64_t so = unit_slot_base(eb, unit, A.code_mult);
+        const uint32_t cap = unit_slot_cap(ee - eb, A.code_mult);
+        const int64_t L = (int64_t)A.unit_tile[unit] * 32 + lane;
+        const uint16_t* cp = reinterpret_cast<const uint16_t*>(A.codes) + so * 32 + lane * 8;      // code f: cp[(f >> 3) * 256 + (f & 7)]
+        const uint32_t* extp = reinterpret_cast<const uint32_t*>(A.codes) + (so + cap) * 16 + lane - (size_t)rec.z * 32;
+        UmiState U;
+        U.n = 0; U.exist = 0; U.Q = 1.0; U.rightP = 1.0; U.last_aid = 0; U.ndyn = 0; U.status = 0;
+#pragma unroll 1
+        for (uint32_t f = rec.y; f < F; ++f) {
+            const uint32_t cd = __ldg(cp + (f >> 3) * 256 + (f & 7u));
+            if ((cd & FC_UMIFIRST) && f != rec.y) break;
+            uint32_t aid = (cd >> FC_AID_SH) & 7u;
+            if (cd & FC_EXT) {
+                extp -= 32;
+                const uint32_t e = __ldg(extp);
+                if (aid == FC_AID_DYN) aid = NF + e;
+            }
+            if (((cd >> FC_ST_SH) & 3u) == 3u) {
+                const uint32_t i = ((cd >> 13) & 1u) * ((cd & 0xffu) + 1u);                   // as k_merge's table
+                const double pf = i == 0 ? 0.1 : __ldg(&A.bqtab[i - 1]);
+                fragment_join(pf, 1.0 - pf, aid, U);
+            }
+        }
+        if (U.status) atomicOr(&A.loc[SMC_L_STATUS * nl + L], (int)U.status);
+        if (rec.w & DR_STATUS_ONLY) continue;
+        if (U.exist && !(U.exist & (U.exist - 1u))) umi_fill_single(U);      // a DEL, or more fragments than the prior table holds
+        const uint32_t keymask = umi_general(A.T, A.pcrtab, A.pcr_nmax, A.smt, A.cnt, A.limb, nl, L, U);
+        if (keymask) atomicOr(&A.loc[SMC_L_KEYMASK * nl + L], (int)keymask);
     }
 }
