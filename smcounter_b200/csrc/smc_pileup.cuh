@@ -342,10 +342,10 @@ __device__ __noinline__ uint32_t dyn_lookup_long_ins(DynTab T, unsigned long lon
 // non-ACGT bases, pairs on a deletion or a dynamic allele.
 // ============================================================================================================
 #ifndef KA_WARPS
-#define KA_WARPS 8
+#define KA_WARPS 4
 #endif
 #ifndef KA_MINBLOCKS
-#define KA_MINBLOCKS 3
+#define KA_MINBLOCKS 7    // B200, cfg2: 4 warps x 6 / 7 / 8 blocks 1.335 / 1.251 / 1.552 ms; 8 warps x 3 / 4 blocks 1.362 / 1.591
 #endif
 #ifndef KA_GATHER
 #define KA_GATHER 4
