@@ -24,6 +24,8 @@
 
 #include <stdint.h>
 
+#include "smc_bamio.h"
+
 #ifdef __cplusplus
 extern "C" {
 #endif
@@ -37,6 +39,8 @@ extern "C" {
 #define SMC_E_LIMIT      -3   /* input exceeds a documented batch limit (split the batch) */
 #define SMC_E_OVERFLOW   -4   /* an internal table overflowed even after regrowth */
 #define SMC_E_STATE      -5   /* call order violated (e.g. run before upload) */
+#define SMC_E_INFLATE    -6   /* smc_decode_bam: a BGZF block the device inflater rejects (decode that file on the host) */
+#define SMC_E_BUDGET     -7   /* smc_decode_bam: the inflated stream does not fit the device (decode that file on the host) */
 
 /* Parameters of vc() that reach the device (reference smCounter.py:274, CLI :619-633). */
 typedef struct smc_params {
@@ -360,6 +364,29 @@ int smc_fisher_exact(smc_ctx *ctx, int64_t n, const int32_t *tables, double *p_o
  * kernels (pageable memory is staged by the driver at a fraction of the link rate).  Not tied to a context. */
 int  smc_host_alloc(int64_t bytes, void **out);
 void smc_host_free(void *p);
+
+/*
+ * BAM decode on the GPU: the same smc_bam_reads, element for element, as smc_bam_decode of include/smc_bamio.h gives for the
+ * same file, intervals and trim setting.  Inputs are what smc_bam_plan / smc_bam_read_blocks give: the block table, the
+ * compressed bytes (readable 64 bytes past comp_bytes; pinned memory copies fastest), the stream's length and its first record;
+ * n_ref is the header's reference count.  The device inflates the blocks, finds the record boundaries, decodes the fields,
+ * numbers the fragments and the dictionary barcodes and copies the kept reads into one arena that comes back in one copy.
+ * The arrays of *out are host memory owned by the context (not page-locked: locking a fresh arena costs far more than the one
+ * copy into it), valid until the next smc_decode_bam on it or smc_ctx_destroy.  SMC_E_INFLATE / SMC_E_BUDGET: the host decoder can decode this file (a block the device inflater does not
+ * take; a stream that does not fit the free device memory, or of 4 GiB or more).  SMC_E_ARG with the host decoder's message:
+ * truncated or malformed records.  SMC_BAM_TIMING=1 prints one stderr line per stage (CUDA events).
+ */
+int smc_decode_bam(smc_ctx *ctx, const smc_bgzf_block *blocks, int64_t n_blocks, const uint8_t *comp, int64_t comp_bytes,
+                   int64_t raw_bytes, int64_t first_record, int32_t n_ref, int64_t n_intervals, const int32_t *iv_ref,
+                   const int32_t *iv_start, const int32_t *iv_end, int32_t trim, smc_bam_reads *out);
+/* barcode string of dictionary id i of the last smc_decode_bam (the counterpart of smc_bam_dict_umi) */
+const char *smc_decoded_dict_umi(smc_ctx *ctx, int64_t i);
+
+/* The device inflater on caller-given raw DEFLATE streams (a validation entry point): stream i is in[in_off[i], +in_len[i])
+ * (readable 64 bytes further) and must inflate to exactly out_len[i] bytes at out + out_off[i]; status[i] = 0, or -1 where
+ * smc_bam_inflate_raw would return -1.  Bytes of out outside the streams' slices come back unchanged. */
+int smc_inflate_device(smc_ctx *ctx, int64_t n, const uint8_t *in, int64_t in_bytes, const int64_t *in_off, const int64_t *in_len,
+                       uint8_t *out, int64_t out_bytes, const int64_t *out_off, const int64_t *out_len, int32_t *status);
 
 #ifdef __cplusplus
 }

@@ -82,6 +82,37 @@ const char *smc_bam_dict_umi(smc_bam *h, int64_t i);                      /* bar
  * hands the block to zlib). */
 int         smc_bam_inflate_raw(const uint8_t *in, int64_t in_len, uint8_t *out, int64_t out_len);
 
+/* ---- The compressed blocks of a decode, for a decoder elsewhere (the GPU decoder of include/smc_b200.h: smc_decode_bam).
+ * Plan, then read: smc_bam_plan works out which compressed byte ranges the decode needs (with intervals and an index, the
+ * index chunks exactly as smc_bam_decode chooses them; otherwise the whole file) and their total size; the caller allocates
+ * comp_bytes + 64 bytes and smc_bam_read_blocks reads the ranges into it
+ * (threaded pread, the 64 bytes of slack zeroed) and lists their BGZF blocks.  Inflating block i and storing its bytes
+ * [lo, hi) at uoff of the stream gives, for every i, exactly the stream smc_bam_decode walks; its first record is at
+ * first_record (the header's length for a whole file, 0 for index chunks).  Index errors are -3 with smc_bam_decode's
+ * messages.  Both need a handle opened header-only; the block table stays valid until smc_bam_close(). */
+typedef struct smc_bgzf_block {
+    int64_t  coff;      /* deflate payload at buf + coff ... */
+    int64_t  clen;      /* ... of clen bytes */
+    int64_t  uoff;      /* where [lo, hi) of the inflated block goes in the stream */
+    uint32_t isize;     /* inflated size of the block */
+    uint32_t lo, hi;
+    uint32_t reserved;
+} smc_bgzf_block;
+
+typedef struct smc_bgzf_plan {
+    int64_t               n_blocks;
+    const smc_bgzf_block *blocks;
+    int64_t               comp_bytes;
+    int64_t               raw_bytes;     /* length of the inflated stream */
+    int64_t               first_record;
+} smc_bgzf_plan;
+
+/* header-only open without an index (smc_bam_open_indexed is header-only already); smc_bam_decode on it reads the whole file */
+int         smc_bam_open_header(const char *path, int threads, smc_bam **out);
+int         smc_bam_plan(smc_bam *h, int64_t n_intervals, const int32_t *iv_ref, const int32_t *iv_start, const int32_t *iv_end,
+                         int64_t *comp_bytes);
+int         smc_bam_read_blocks(smc_bam *h, uint8_t *buf, smc_bgzf_plan *out);
+
 #ifdef __cplusplus
 }
 #endif

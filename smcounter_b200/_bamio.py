@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libsmc_bamio.so")
 EXPORTS = ("smc_bam_set_trim", "smc_bam_open", "smc_bam_open_indexed", "smc_bam_close", "smc_bam_last_error", "smc_bam_n_refs", "smc_bam_ref_name", "smc_bam_ref_length",
            "smc_bam_decode", "smc_bam_dict_umi", "smc_bam_inflate_raw", "smc_rows_emit", "smc_rows_free", "smc_soa_qual_hist", "smc_soa_ref_end", "smc_soa_order_stats", "smc_soa_pack_begin", "smc_soa_pack_fill",
-           "smc_soa_pack_end")
+           "smc_soa_pack_end", "smc_bam_open_header", "smc_bam_plan", "smc_bam_read_blocks")
 _vp = C.c_void_p
 
 
@@ -21,6 +21,16 @@ class smc_bam_reads(C.Structure):
                 ("seq_off", _vp), ("qual_off", _vp), ("cigar_off", _vp), ("n_cigar", _vp), ("umi", _vp), ("frag_id", _vp),
                 ("seq", _vp), ("seq_bytes", C.c_int64), ("qual", _vp), ("qual_bytes", C.c_int64), ("cigar", _vp),
                 ("n_cigar_words", C.c_int64), ("n_dict_umis", C.c_int64), ("store_lo", _vp), ("store_len", _vp), ("qual_hist", _vp)]
+
+
+class smc_bgzf_block(C.Structure):
+    _fields_ = [("coff", C.c_int64), ("clen", C.c_int64), ("uoff", C.c_int64), ("isize", C.c_uint32), ("lo", C.c_uint32), ("hi", C.c_uint32),
+                ("reserved", C.c_uint32)]
+
+
+class smc_bgzf_plan(C.Structure):
+    _fields_ = [("n_blocks", C.c_int64), ("blocks", C.POINTER(smc_bgzf_block)), ("comp_bytes", C.c_int64), ("raw_bytes", C.c_int64),
+                ("first_record", C.c_int64)]
 
 
 class smc_rows_in(C.Structure):               # include/smc_rows.h
@@ -93,6 +103,12 @@ def load():
     lib.smc_bam_dict_umi.restype = C.c_char_p
     lib.smc_bam_inflate_raw.argtypes = [_vp, C.c_int64, _vp, C.c_int64]
     lib.smc_bam_inflate_raw.restype = C.c_int
+    lib.smc_bam_open_header.argtypes = [C.c_char_p, C.c_int, C.POINTER(_vp)]
+    lib.smc_bam_open_header.restype = C.c_int
+    lib.smc_bam_plan.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, C.POINTER(C.c_int64)]
+    lib.smc_bam_plan.restype = C.c_int
+    lib.smc_bam_read_blocks.argtypes = [_vp, _vp, C.POINTER(smc_bgzf_plan)]
+    lib.smc_bam_read_blocks.restype = C.c_int
     lib.smc_rows_emit.argtypes = [C.POINTER(smc_rows_in), C.POINTER(smc_rows_out)]
     lib.smc_rows_emit.restype = C.c_int
     lib.smc_rows_free.argtypes = [C.POINTER(smc_rows_out)]
@@ -148,57 +164,156 @@ def _raise(rc, msg):
     raise (IOError if rc == E_INDEX else ValueError)(msg.decode())
 
 
-def read_bam_native(path: str, intervals=None, threads: int = 0, trim: bool = False, index: str | None = None) -> ReadsSoA:
-    """``index``: path of the BAM's .bai; with intervals, only the index chunks they need are read and inflated."""
-    lib = load()
+def _open(lib, path, threads, index, header_only=False):
     h = _vp()
     if index is not None:
         rc = lib.smc_bam_open_indexed(os.fsencode(path), os.fsencode(index), int(threads), C.byref(h))
+    elif header_only:
+        rc = lib.smc_bam_open_header(os.fsencode(path), int(threads), C.byref(h))
     else:
         rc = lib.smc_bam_open(os.fsencode(path), int(threads), C.byref(h))
     if rc != 0:
         _raise(rc, lib.smc_bam_last_error(None))
+    return h
+
+
+def _intervals(lib, h, intervals):
+    """(chroms, n_iv, (iv_ref, iv_start, iv_end), trim allowed) as smc_bam_decode takes them"""
+    chroms = [lib.smc_bam_ref_name(h, i).decode() for i in range(lib.smc_bam_n_refs(h))]
+    cidx = {c: i for i, c in enumerate(chroms)}
+    ivs = [(cidx[c], s, e) for (c, s, e) in (intervals or ()) if c in cidx and e > s]
+    if intervals is not None and not ivs:
+        return chroms, 1, (np.asarray([-1], np.int32), np.zeros(1, np.int32), np.zeros(1, np.int32)), False   # nothing can match
+    args = tuple(np.asarray([v[k] for v in ivs], dtype=np.int32) for k in range(3))
+    return chroms, len(ivs), args, bool(ivs)
+
+
+def _soa(out, chroms, owner, dict_umi):
+    """ReadsSoA over the arrays of an smc_bam_reads (views kept alive by ``owner``); dict_umi(i) = barcode of dictionary id i"""
+    n = out.n_reads
+    A = lambda ptr, count, dtype: _arr(ptr, count, dtype, owner)
+    names = {(1 << 63) | i: dict_umi(i).decode() for i in range(out.n_dict_umis)}
+    # 2-bit packed codes decode to their barcode on demand (soa.umi_string); only the dictionary-coded ones need a name
+    soa = ReadsSoA(
+        ref_id=A(out.ref_id, n, np.int32), pos=A(out.pos, n, np.int32), flag=A(out.flag, n, np.uint16),
+        mapq=A(out.mapq, n, np.uint8), nm=A(out.nm, n, np.int32), l_seq=A(out.l_seq, n, np.int32),
+        seq_off=A(out.seq_off, n, np.int64), qual_off=A(out.qual_off, n, np.int64), cigar_off=A(out.cigar_off, n, np.int64),
+        n_cigar=A(out.n_cigar, n, np.uint16), umi=A(out.umi, n, np.uint64), frag_id=A(out.frag_id, n, np.uint32),
+        seq=A(out.seq, out.seq_bytes, np.uint8), qual=A(out.qual, out.qual_bytes, np.uint8),
+        cigar=A(out.cigar, out.n_cigar_words, np.uint32), chroms=chroms, umi_names=names, packed=True,
+        store_lo=A(out.store_lo, n, np.int32) if out.store_lo else None,
+        store_len=A(out.store_len, n, np.int32) if out.store_len else None)
+    if out.qual_hist:                   # counted during the decode: the upload codebook needs no pass of its own
+        soa.__dict__["_qual_hist"] = np.frombuffer((C.c_uint64 * 256).from_address(out.qual_hist), dtype=np.uint64).copy()
+    return soa
+
+
+def read_bam_native(path: str, intervals=None, threads: int = 0, trim: bool = False, index: str | None = None) -> ReadsSoA:
+    """``index``: path of the BAM's .bai; with intervals, only the index chunks they need are read and inflated."""
+    lib = load()
+    h = _open(lib, path, threads, index)
     owner = _Handle(lib, h)
     ok = False
     try:
-        chroms = [lib.smc_bam_ref_name(h, i).decode() for i in range(lib.smc_bam_n_refs(h))]
-        cidx = {c: i for i, c in enumerate(chroms)}
-        ivs = [(cidx[c], s, e) for (c, s, e) in (intervals or ()) if c in cidx and e > s]
-        iv_ref = np.asarray([v[0] for v in ivs], dtype=np.int32)
-        iv_s = np.asarray([v[1] for v in ivs], dtype=np.int32)
-        iv_e = np.asarray([v[2] for v in ivs], dtype=np.int32)
+        chroms, n_iv, args, can_trim = _intervals(lib, h, intervals)
         out = smc_bam_reads()
-        if intervals is not None and not ivs:
-            n_iv, args = 1, (np.asarray([-1], np.int32), np.zeros(1, np.int32), np.zeros(1, np.int32))   # nothing can match
-        else:
-            n_iv, args = len(ivs), (iv_ref, iv_s, iv_e)
-        lib.smc_bam_set_trim(h, 1 if (trim and ivs) else 0)
+        lib.smc_bam_set_trim(h, 1 if (trim and can_trim) else 0)
         rc = lib.smc_bam_decode(h, n_iv, args[0].ctypes.data, args[1].ctypes.data, args[2].ctypes.data, C.byref(out))
         if rc != 0:
             _raise(rc, lib.smc_bam_last_error(h))
-        n = out.n_reads
-        A = lambda ptr, count, dtype: _arr(ptr, count, dtype, owner)
-        umi = A(out.umi, n, np.uint64)
-        names = {}
-        for i in range(out.n_dict_umis):
-            names[(1 << 63) | i] = lib.smc_bam_dict_umi(h, i).decode()
-        # 2-bit packed codes decode to their barcode on demand (soa.umi_string); only the dictionary-coded ones need a name
-        soa = ReadsSoA(
-            ref_id=A(out.ref_id, n, np.int32), pos=A(out.pos, n, np.int32), flag=A(out.flag, n, np.uint16),
-            mapq=A(out.mapq, n, np.uint8), nm=A(out.nm, n, np.int32), l_seq=A(out.l_seq, n, np.int32),
-            seq_off=A(out.seq_off, n, np.int64), qual_off=A(out.qual_off, n, np.int64), cigar_off=A(out.cigar_off, n, np.int64),
-            n_cigar=A(out.n_cigar, n, np.uint16), umi=umi, frag_id=A(out.frag_id, n, np.uint32),
-            seq=A(out.seq, out.seq_bytes, np.uint8), qual=A(out.qual, out.qual_bytes, np.uint8),
-            cigar=A(out.cigar, out.n_cigar_words, np.uint32), chroms=chroms, umi_names=names, packed=True,
-            store_lo=A(out.store_lo, n, np.int32) if out.store_lo else None,
-            store_len=A(out.store_len, n, np.int32) if out.store_len else None)
-        if out.qual_hist:                   # counted during the decode: the upload codebook needs no pass of its own
-            soa.__dict__["_qual_hist"] = np.frombuffer((C.c_uint64 * 256).from_address(out.qual_hist), dtype=np.uint64).copy()
+        soa = _soa(out, chroms, owner, lambda i: lib.smc_bam_dict_umi(h, i))
+        soa.__dict__["_bam_decoder"] = "host"
         ok = True
         return soa
     finally:
         if not ok:
             owner.close()
+
+
+class _Context:
+    """Owns the smc_ctx of a GPU decode; destroyed when the last array that views its output arena is gone."""
+
+    def __init__(self, lib, ctx):
+        self.lib, self.ctx = lib, ctx
+
+    def close(self):
+        if self.ctx:
+            self.lib.smc_ctx_destroy(self.ctx)
+            self.ctx = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def plan_blocks(path: str, intervals=None, threads: int = 0, index: str | None = None):
+    """The compressed blocks a decode of ``path`` needs (smc_bam_plan + smc_bam_read_blocks): (compressed bytes as a uint8 array
+    with 64 bytes of zero slack, [(coff, clen, uoff, isize, lo, hi)], inflated length, first record).  Plain memory: for tests."""
+    lib = load()
+    h = _open(lib, path, threads, index, header_only=True)
+    try:
+        _chroms, n_iv, args, _ = _intervals(lib, h, intervals) if intervals is not None else (None, 0, (None,) * 3, False)
+        comp = C.c_int64()
+        rc = lib.smc_bam_plan(h, n_iv, *[a.ctypes.data if a is not None else None for a in args], C.byref(comp))
+        if rc != 0:
+            _raise(rc, lib.smc_bam_last_error(h))
+        buf = np.empty(comp.value + 64, np.uint8)
+        plan = smc_bgzf_plan()
+        rc = lib.smc_bam_read_blocks(h, buf.ctypes.data, C.byref(plan))
+        if rc != 0:
+            _raise(rc, lib.smc_bam_last_error(h))
+        blocks = [(b.coff, b.clen, b.uoff, b.isize, b.lo, b.hi) for b in plan.blocks[:plan.n_blocks]]
+        return buf, blocks, plan.raw_bytes, plan.first_record
+    finally:
+        lib.smc_bam_close(h)
+
+
+def read_bam_device(path: str, intervals=None, device: int = 0, threads: int = 0, trim: bool = False, index: str | None = None) -> ReadsSoA:
+    """``read_bam_native`` with the decode on GPU ``device`` (include/smc_b200.h: smc_decode_bam): the host reads the compressed
+    blocks the decode needs, the GPU inflates and decodes them.  The same arrays as the host decoder.  A file the GPU cannot
+    take (a block its inflater rejects, a stream larger than its memory) is decoded on the host instead, with one warning line."""
+    from . import _ffi
+    lib, fl = load(), _ffi.load()
+    h = _open(lib, path, threads, index, header_only=True)
+    ctx = _vp()
+    try:
+        chroms, n_iv, args, can_trim = _intervals(lib, h, intervals)
+        comp = C.c_int64()
+        rc = lib.smc_bam_plan(h, n_iv, args[0].ctypes.data, args[1].ctypes.data, args[2].ctypes.data, C.byref(comp))
+        if rc != 0:
+            _raise(rc, lib.smc_bam_last_error(h))
+        # ordinary memory: page-locking a buffer of the file's size costs more than the one copy to the GPU it would speed up
+        buf = np.empty(comp.value + 64, np.uint8)
+        plan = smc_bgzf_plan()
+        rc = lib.smc_bam_read_blocks(h, buf.ctypes.data, C.byref(plan))
+        if rc != 0:
+            _raise(rc, lib.smc_bam_last_error(h))
+        rc = fl.smc_ctx_create(int(device), C.byref(_ffi.smc_params()), C.byref(ctx))
+        if rc != 0:
+            raise RuntimeError("smc_ctx_create failed (%d): %s" % (rc, fl.smc_last_error(None).decode()))
+        out = smc_bam_reads()
+        rc = fl.smc_decode_bam(ctx, C.cast(plan.blocks, _vp), plan.n_blocks, buf.ctypes.data, plan.comp_bytes, plan.raw_bytes, plan.first_record,
+                               len(chroms), n_iv, args[0].ctypes.data, args[1].ctypes.data, args[2].ctypes.data,
+                               1 if (trim and can_trim) else 0, C.byref(out))
+        if rc in (_ffi.SMC_E_INFLATE, _ffi.SMC_E_BUDGET):
+            print("warning: %s: decoding %s on the host" % (fl.smc_last_error(ctx).decode(), path))
+        elif rc == _ffi.SMC_E_ARG:
+            raise ValueError(fl.smc_last_error(ctx).decode())
+        elif rc != 0:
+            raise RuntimeError("smc_decode_bam failed (%d): %s" % (rc, fl.smc_last_error(ctx).decode()))
+        else:
+            owner = _Context(fl, ctx)
+            ctx = None
+            soa = _soa(out, chroms, owner, lambda i: fl.smc_decoded_dict_umi(owner.ctx, i))
+            soa.__dict__["_bam_decoder"] = "device"
+            return soa
+    finally:
+        if ctx:
+            fl.smc_ctx_destroy(ctx)
+        lib.smc_bam_close(h)
+    return read_bam_native(path, intervals, threads, trim, index)
 
 
 # ------------------------------------------------------------------------------------------------------------

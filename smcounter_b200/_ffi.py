@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libsmc_b200.so")
 
 SMC_NFIXED, SMC_NCNT, SMC_NLOC = 5, 13, 12
-SMC_OK, SMC_E_CUDA, SMC_E_ARG, SMC_E_LIMIT, SMC_E_OVERFLOW, SMC_E_STATE = 0, -1, -2, -3, -4, -5
+SMC_OK, SMC_E_CUDA, SMC_E_ARG, SMC_E_LIMIT, SMC_E_OVERFLOW, SMC_E_STATE, SMC_E_INFLATE, SMC_E_BUDGET = 0, -1, -2, -3, -4, -5, -6, -7
 (C_ALLELE, C_FWD, C_REV, C_LOWQ, C_R1LE, C_R1TOT, C_R2LE, C_R2TOT, C_R2PLE, C_CONCORD, C_DISCORD, C_MT,
  C_STRONG) = range(13)
 (L_CVG, L_ALLFRAG, L_ALLMT, L_USEDFRAG, L_NBC, L_USEDMT, L_MT3, L_MT5, L_MT7, L_MT10, L_KEYMASK, L_STATUS) = range(12)
@@ -78,7 +78,8 @@ HP_HOMOPOLYMER, HP_LOWCOMP = 1, 2
 
 EXPORTS = ("smc_version", "smc_ctx_create", "smc_ctx_destroy", "smc_last_error", "smc_call_batch", "smc_upload",
            "smc_run_resident", "smc_download", "smc_get_timings", "smc_list_barcodes", "smc_hp_lowcomp", "smc_fisher_exact", "smc_host_alloc",
-           "smc_host_free", "smc_set_downsample", "smc_set_barcode_hashes", "smc_draw_sample")
+           "smc_host_free", "smc_set_downsample", "smc_set_barcode_hashes", "smc_draw_sample", "smc_decode_bam", "smc_decoded_dict_umi",
+           "smc_inflate_device")
 
 _lib = None
 
@@ -126,6 +127,12 @@ def load():
     lib.smc_set_barcode_hashes.restype = C.c_int
     lib.smc_draw_sample.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]
     lib.smc_draw_sample.restype = C.c_int
+    lib.smc_decode_bam.argtypes = [_vp, _vp, C.c_int64, _vp, C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_int64, _vp, _vp, _vp, C.c_int32, _vp]
+    lib.smc_decode_bam.restype = C.c_int
+    lib.smc_decoded_dict_umi.argtypes = [_vp, C.c_int64]
+    lib.smc_decoded_dict_umi.restype = C.c_char_p
+    lib.smc_inflate_device.argtypes = [_vp, C.c_int64, _vp, C.c_int64, _vp, _vp, _vp, C.c_int64, _vp, _vp, _vp]
+    lib.smc_inflate_device.restype = C.c_int
     _lib = lib
     return lib
 

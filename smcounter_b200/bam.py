@@ -369,15 +369,20 @@ def read_chunks(path: str, chunks, index_path: str) -> bytes:
     return b"".join(out)
 
 
-def read_bam(path: str, intervals=None, native: bool | None = None, threads: int = 0, trim: bool = False) -> ReadsSoA:
+def read_bam(path: str, intervals=None, native: bool | None = None, threads: int = 0, trim: bool = False, device: int | None = None) -> ReadsSoA:
     """Decode ``path`` into a ReadsSoA (BAM order).  ``intervals`` = [(chrom, start, end)]: keep only reads whose
     reference span touches a target interval (the only reads a pileup over those targets can see).  With intervals and a
     .bai beside the BAM that is not older than it (``find_index``), only the index chunks the intervals need are read and
     inflated; the result is the same as that of a whole-file decode.
 
     ``native``: True = require libsmc_bamio.so, False = Python walker, None = native when built.
-    ``trim``: store only each read's target window (ReadsSoA.store_lo / store_len): what the calling path uploads."""
+    ``trim``: store only each read's target window (ReadsSoA.store_lo / store_len): what the calling path uploads.
+    ``device``: None = decode on the host; a GPU index = inflate and decode on that GPU (libsmc_b200: smc_decode_bam), with the
+    same result; a file the GPU cannot take is decoded on the host with a warning line."""
     index = find_index(path) if intervals else None
+    if device is not None:
+        from . import _bamio
+        return _bamio.read_bam_device(path, intervals, int(device), threads, trim, index=index)
     if native is not False:
         try:
             from . import _bamio

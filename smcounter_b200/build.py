@@ -9,7 +9,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libsmc_b200.so")
 SOURCES = ["smc_api.cu"]
-HEADERS = ["smc_common.cuh", "smc_sort.cuh", "smc_pileup.cuh", "smc_stats.cuh", "smc_upload.cuh", "smc_downsample.cuh", "smc_py2rand.h", os.path.join("..", "..", "include", "smc_b200.h")]
+HEADERS = ["smc_common.cuh", "smc_sort.cuh", "smc_pileup.cuh", "smc_stats.cuh", "smc_upload.cuh", "smc_downsample.cuh", "smc_py2rand.h", "smc_bgzf.cuh",
+           "smc_inflate.h", "smc_bamrec.h", os.path.join("..", "..", "include", "smc_b200.h"), os.path.join("..", "..", "include", "smc_bamio.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-fmad=false",                 # FP64 parity: no FMA contraction anywhere in the statistics
               "-shared", "-Xcompiler", "-fPIC"]
@@ -33,7 +34,7 @@ SOA_HDR = os.path.join(HERE, "..", "include", "smc_soa.h")
 
 def build_bamio(force: bool = False) -> str:
     """Host-side BAM decoder (C++17, zlib, threads) -> libsmc_bamio.so."""
-    if not force and os.path.exists(BAMIO_OUT) and os.path.getmtime(BAMIO_OUT) >= max(os.path.getmtime(f) for f in (BAMIO_SRC, BAMIO_HDR, ROWS_SRC, ROWS_HDR, SOA_SRC, SOA_HDR, os.path.join(CSRC, "smc_inflate.h"), os.path.join(CSRC, "smc_host.h"))):
+    if not force and os.path.exists(BAMIO_OUT) and os.path.getmtime(BAMIO_OUT) >= max(os.path.getmtime(f) for f in (BAMIO_SRC, BAMIO_HDR, ROWS_SRC, ROWS_HDR, SOA_SRC, SOA_HDR, os.path.join(CSRC, "smc_inflate.h"), os.path.join(CSRC, "smc_bamrec.h"), os.path.join(CSRC, "smc_host.h"))):
         return BAMIO_OUT
     cmd = [os.environ.get("CXX", "g++"), "-O2", "-std=c++17", "-shared", "-fPIC", "-pthread", "-o", BAMIO_OUT, BAMIO_SRC, ROWS_SRC, SOA_SRC, "-lz"]
     r = subprocess.run(cmd, capture_output=True, text=True)

@@ -31,6 +31,7 @@
 #include "smc_stats.cuh"
 #include "smc_upload.cuh"
 #include "smc_downsample.cuh"
+#include "smc_bgzf.cuh"
 
 namespace {
 
@@ -169,6 +170,15 @@ struct smc_ctx {
     DevBuf d_bc_code{bufs}, d_bc_hash{bufs};
     DevBuf d_ds_flag{bufs}, d_ds_nbc{bufs}, d_ds_locus{bufs}, d_ds_k0{bufs}, d_ds_k1{bufs}, d_ds_v0{bufs}, d_ds_v1{bufs}, d_ds_codes{bufs},
         d_ds_hash{bufs}, d_ds_scratch{bufs}, d_ds_keep_off{bufs}, d_ds_keep_umi{bufs};
+    // BAM decode (smc_decode_bam): device passes, and the decoded arrays in one pinned host arena owned by the context
+    DevBuf d_bz_comp{bufs}, d_bz_jobs{bufs}, d_bz_raw{bufs}, d_bz_scratch{bufs}, d_bz_status{bufs}, d_bz_walk{bufs}, d_bz_base{bufs},
+        d_bz_offs{bufs}, d_bz_info{bufs}, d_bz_cnt{bufs}, d_bz_k0{bufs}, d_bz_k1{bufs}, d_bz_v0{bufs}, d_bz_v1{bufs}, d_bz_first{bufs},
+        d_bz_isfirst{bufs}, d_bz_dfirst{bufs}, d_bz_disfirst{bufs}, d_bz_hist{bufs}, d_bz_scan{bufs}, d_bz_tg{bufs}, d_bz_out{bufs},
+        d_bz_dict{bufs}, d_bz_small{bufs};
+    void* h_bz_out = nullptr; size_t h_bz_cap = 0;
+    int n_sm = 148;                             // multiprocessors of the device (smc_ctx_create)
+    std::vector<std::string> bz_dict;
+    uint64_t* bz_qual_hist = nullptr;
     smc_timings tm{};
     uint32_t chunk = 128;       // tile events per warp unit (A/B on B200, whole step: 96 -> 4.42 ms, 128 -> 4.39, 160 -> 4.39, 256 -> 4.47, 384 -> 4.60)
     const uint32_t* ev_read_sorted = nullptr;   // tile-sorted event -> srank map (lives in d_ev0 or d_ev1)
@@ -473,6 +483,7 @@ extern "C" int smc_ctx_create(int device, const smc_params* params, smc_ctx** ou
     };
     if ((e = cudaSetDevice(device)) != cudaSuccess) return fail("cudaSetDevice", e);
     if ((e = cudaStreamCreateWithFlags(&ctx->st, cudaStreamNonBlocking)) != cudaSuccess) return fail("cudaStreamCreate", e);
+    if ((e = cudaDeviceGetAttribute(&ctx->n_sm, cudaDevAttrMultiProcessorCount, device)) != cudaSuccess) return fail("cudaDeviceGetAttribute", e);
     for (DevBuf* b : ctx->bufs) b->st = ctx->st;
     {   // keep freed scratch in the pool for the next batch / context of this process
         cudaMemPool_t pool;
@@ -538,6 +549,7 @@ extern "C" void smc_ctx_destroy(smc_ctx* ctx) {
     }
     if (ctx->st_copy) cudaStreamDestroy(ctx->st_copy);
     if (ctx->st) cudaStreamDestroy(ctx->st);
+    free(ctx->h_bz_out);
     delete ctx;
 }
 
@@ -1713,5 +1725,313 @@ extern "C" int smc_hp_lowcomp(smc_ctx* ctx, const smc_hp_batch* Bt, uint8_t* fla
     CK(cudaMemcpyAsync(flags_out, ctx->d_hp_flags.p, (size_t)n, cudaMemcpyDeviceToHost, ctx->st));
     CK(cudaStreamSynchronize(ctx->st));
     CK(cudaGetLastError());
+    return SMC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// BAM decode on the device (include/smc_b200.h: smc_decode_bam)
+// ------------------------------------------------------------------------------------------------------------
+// Device bytes a decode may need: the compressed and inflated streams, the scratch of partly kept blocks, about 200 bytes of
+// per-record tables (at most one record per 36 stream bytes) and the output, which is no larger than the stream plus 64 bytes
+// per record
+static int64_t bam_decode_bytes(int64_t comp, int64_t raw, int64_t scratch) {
+    const int64_t nrec = raw / 36 + 1;
+    return comp + 64 + 2 * raw + scratch + nrec * 264 + ((int64_t)1 << 24);
+}
+
+static int bam_rewalk(smc_ctx* ctx, const uint8_t* raw, int64_t size, int64_t first, const BgzfJob* jobs, int64_t nb, int32_t nref,
+                      int64_t t, int64_t start, std::vector<int64_t>& wk) {
+    int64_t* d = ctx->d_bz_walk.as<int64_t>();
+    CK(cudaMemcpyAsync(d + t, &start, 8, cudaMemcpyHostToDevice, ctx->st));
+    k_walk<<<1, 1, 0, ctx->st>>>(raw, size, first, jobs, nb, t, t + 1, nref, 0, d, nullptr, nullptr);
+    ++g_launches;
+    for (int k = 0; k < 4; ++k) CK(cudaMemcpyAsync(&wk[(size_t)k * nb + t], d + (size_t)k * nb + t, 8, cudaMemcpyDeviceToHost, ctx->st));
+    CK(cudaStreamSynchronize(ctx->st));
+    return SMC_OK;
+}
+
+extern "C" int smc_decode_bam(smc_ctx* ctx, const smc_bgzf_block* blocks, int64_t n_blocks, const uint8_t* comp, int64_t comp_bytes,
+                              int64_t raw_bytes, int64_t first_record, int32_t n_ref, int64_t n_iv, const int32_t* iv_ref,
+                              const int32_t* iv_start, const int32_t* iv_end, int32_t trim, smc_bam_reads* out) {
+    if (!ctx) return SMC_E_ARG;
+    if (!out || n_blocks < 0 || comp_bytes < 0 || raw_bytes < 0 || n_ref < 0 || first_record < 0 || (n_blocks > 0 && (!blocks || !comp)) ||
+        (n_iv > 0 && (!iv_ref || !iv_start || !iv_end))) {
+        ctx->err = "smc_decode_bam: bad argument"; return SMC_E_ARG;
+    }
+    NvtxRange nv("smc_decode_bam");
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->st;
+    const bool timing = getenv("SMC_BAM_TIMING") != nullptr;
+    constexpr int NEV = 10;
+    cudaEvent_t ev[NEV];
+    for (auto& e : ev) CK(cudaEventCreate(&e));
+    struct EvFree { cudaEvent_t* e; ~EvFree() { for (int k = 0; k < NEV; ++k) cudaEventDestroy(e[k]); } } ev_free{ev};
+    // the block table: validated against the streams, and the scratch offset of every block that is only partly kept
+    std::vector<BgzfJob> jobs((size_t)n_blocks);
+    int64_t scratch = 0, uoff = 0;
+    for (int64_t i = 0; i < n_blocks; ++i) {
+        const smc_bgzf_block& b = blocks[i];
+        if (b.coff < 0 || b.clen < 0 || b.coff + b.clen > comp_bytes || b.lo > b.hi || b.hi > b.isize || b.uoff != uoff) {
+            ctx->err = "smc_decode_bam: block " + std::to_string(i) + " does not fit the compressed or the inflated stream"; return SMC_E_ARG;
+        }
+        const bool whole = b.lo == 0 && b.hi == b.isize;
+        jobs[(size_t)i] = BgzfJob{b.coff, b.clen, b.uoff, whole ? 0 : scratch, b.isize, b.lo, b.hi, whole ? 1u : 0u};
+        if (!whole) scratch += b.isize;
+        uoff += b.hi - b.lo;
+    }
+    if (uoff != raw_bytes || first_record > raw_bytes) { ctx->err = "smc_decode_bam: the blocks do not add up to raw_bytes"; return SMC_E_ARG; }
+    {   // what the device can hold: streams of up to 4 GiB (32-bit scans) that fit the free memory
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        int64_t budget = (int64_t)free_b;
+        if (const char* ev_b = getenv("SMC_BAM_DEVICE_BUDGET")) budget = std::min<int64_t>(budget, atoll(ev_b));
+        const int64_t need = bam_decode_bytes(comp_bytes, raw_bytes, scratch);
+        if (raw_bytes >= ((int64_t)1 << 32) || need > budget) {
+            ctx->err = "smc_decode_bam: the inflated stream (" + std::to_string(raw_bytes) + " bytes, about " + std::to_string(need >> 20) +
+                       " MiB of device memory) exceeds the device budget (" + std::to_string(budget >> 20) + " MiB, streams < 4 GiB)";
+            return SMC_E_BUDGET;
+        }
+    }
+    const int64_t nb = n_blocks;
+    CK(ctx->d_bz_comp.ensure((size_t)comp_bytes + 64));
+    CK(ctx->d_bz_jobs.ensure(sizeof(BgzfJob) * (size_t)(nb + 1)));
+    CK(ctx->d_bz_raw.ensure((size_t)raw_bytes + 64));
+    CK(ctx->d_bz_scratch.ensure((size_t)scratch + 64));
+    CK(ctx->d_bz_status.ensure(4 * (size_t)(nb + 1)));
+    CK(ctx->d_bz_walk.ensure(32 * (size_t)(nb + 1)));
+    CK(ctx->d_bz_base.ensure(8 * (size_t)(nb + 1)));
+    CK(ctx->d_bz_small.ensure(256));
+    uint8_t* raw = ctx->d_bz_raw.as<uint8_t>();
+    BgzfJob* d_jobs = ctx->d_bz_jobs.as<BgzfJob>();
+    uint32_t* small = ctx->d_bz_small.as<uint32_t>();             // [0, 1] bad record (u64), 2 any_dict, 4.. scan totals
+    CK(cudaEventRecord(ev[0], st));
+    if (comp_bytes) CK(cudaMemcpyAsync(ctx->d_bz_comp.p, comp, (size_t)comp_bytes + 64, cudaMemcpyHostToDevice, st));
+    if (nb) CK(cudaMemcpyAsync(d_jobs, jobs.data(), sizeof(BgzfJob) * (size_t)nb, cudaMemcpyHostToDevice, st));
+    CK(cudaEventRecord(ev[1], st));
+    // ---- inflate
+    LAUNCH(k_inflate, nblk(nb, INFLATE_WARPS), INFLATE_WARPS * 32, 0, ctx->d_bz_comp.as<uint8_t>(), d_jobs, nb, raw,
+           ctx->d_bz_scratch.as<uint8_t>(), ctx->d_bz_status.as<int32_t>(), 1);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ev[2], st));
+    // ---- record boundaries
+    int64_t* d_wk = ctx->d_bz_walk.as<int64_t>();
+    LAUNCH(k_walk, nblk(nb, 128), 128, 0, raw, raw_bytes, first_record, d_jobs, nb, (int64_t)0, nb, n_ref, 1, d_wk, (int64_t*)nullptr,
+           (const int64_t*)nullptr);
+    std::vector<int32_t> status((size_t)nb);
+    std::vector<int64_t> wk(4 * (size_t)nb);
+    if (nb) {
+        CK(cudaMemcpyAsync(status.data(), ctx->d_bz_status.p, 4 * (size_t)nb, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(wk.data(), d_wk, 32 * (size_t)nb, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaStreamSynchronize(st));
+    for (int64_t i = 0; i < nb; ++i)
+        if (status[(size_t)i] != 0) {
+            ctx->err = "smc_decode_bam: the device inflater rejects BGZF block " + std::to_string(i) + " (compressed offset " +
+                       std::to_string(blocks[i].coff) + ")";
+            return SMC_E_INFLATE;
+        }
+    // every range must start where the previous one ended (the first at the first record): by induction the chain is then the
+    // true one; a range that does not is walked again from there
+    std::vector<int64_t> base((size_t)nb + 1, 0);
+    {
+        int64_t expect = first_record;
+        for (int64_t t = 0; t < nb; ++t) {
+            if (wk[(size_t)t] != expect) { const int rc = bam_rewalk(ctx, raw, raw_bytes, first_record, d_jobs, nb, n_ref, t, expect, wk); if (rc) return rc; }
+            if (wk[(size_t)(3 * nb + t)] >= 0) { ctx->err = "truncated BAM record at offset " + std::to_string(wk[(size_t)(3 * nb + t)]); return SMC_E_ARG; }
+            expect = wk[(size_t)(nb + t)];
+            base[(size_t)t + 1] = base[(size_t)t] + wk[(size_t)(2 * nb + t)];
+        }
+    }
+    const int64_t nrec = base[(size_t)nb];
+    CK(ctx->d_bz_offs.ensure(8 * (size_t)(nrec + 1)));
+    if (nb) CK(cudaMemcpyAsync(ctx->d_bz_base.p, base.data(), 8 * (size_t)nb, cudaMemcpyHostToDevice, st));
+    LAUNCH(k_walk, nblk(nb, 128), 128, 0, raw, raw_bytes, first_record, d_jobs, nb, (int64_t)0, nb, n_ref, 0, d_wk, ctx->d_bz_offs.as<int64_t>(),
+           ctx->d_bz_base.as<int64_t>());
+    CK(cudaEventRecord(ev[3], st));
+    // ---- fields
+    const smc_rec::Targets tg((size_t)n_ref, n_iv, iv_ref, iv_start, iv_end);
+    const size_t ntg = tg.st.size();
+    std::vector<int64_t> tgv(tg.off.begin(), tg.off.end());
+    tgv.insert(tgv.end(), tg.st.begin(), tg.st.end());
+    tgv.insert(tgv.end(), tg.en.begin(), tg.en.end());
+    CK(ctx->d_bz_tg.ensure(8 * tgv.size()));
+    CK(cudaMemcpyAsync(ctx->d_bz_tg.p, tgv.data(), 8 * tgv.size(), cudaMemcpyHostToDevice, st));
+    const int64_t* d_tg = ctx->d_bz_tg.as<int64_t>();
+    CK(ctx->d_bz_info.ensure(sizeof(BamRec) * (size_t)(nrec + 1)));
+    CK(ctx->d_bz_cnt.ensure(4 * 4 * (size_t)(nrec + 1)));
+    CK(ctx->d_bz_k0.ensure(8 * (size_t)(nrec + 1))); CK(ctx->d_bz_k1.ensure(8 * (size_t)(nrec + 1)));
+    CK(ctx->d_bz_v0.ensure(4 * (size_t)(nrec + 1))); CK(ctx->d_bz_v1.ensure(4 * (size_t)(nrec + 1)));
+    CK(ctx->d_bz_first.ensure(4 * (size_t)(nrec + 1))); CK(ctx->d_bz_isfirst.ensure(4 * (size_t)(nrec + 1)));
+    CK(ctx->d_bz_hist.ensure(4 * radix_hist_words(nrec)));
+    CK(ctx->d_bz_scan.ensure(4 * (size_t)std::max<int64_t>(radix_scan_words(nrec), scan_scratch_words(4 * nrec))));
+    const BamRec* info = ctx->d_bz_info.as<BamRec>();
+    const int64_t* offs = ctx->d_bz_offs.as<int64_t>();
+    uint32_t* cnt = ctx->d_bz_cnt.as<uint32_t>();
+    CK(cudaMemsetAsync(small, 0xff, 8, st));
+    CK(cudaMemsetAsync(small + 2, 0, 64, st));
+    const int has_tg = n_iv > 0 ? 1 : 0, do_trim = trim && n_iv > 0 ? 1 : 0;
+    LAUNCH(k_fields, nblk(nrec, 256), 256, 0, raw, raw_bytes, offs, nrec, n_ref, d_tg, d_tg + n_ref + 1, d_tg + n_ref + 1 + ntg, has_tg, do_trim,
+           ctx->d_bz_info.as<BamRec>(), cnt, ctx->d_bz_k0.as<uint64_t>(), ctx->d_bz_v0.as<uint32_t>(), reinterpret_cast<unsigned long long*>(small),
+           small + 2);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ev[4], st));
+    // ---- identities: records sorted stably by identity hash, the first of each identity verified on the name bytes, ids by a
+    // scan over "is a first record" in record order; then the same for the barcodes that need the dictionary
+    auto number = [&](uint32_t* first, uint32_t* isfirst, int bc_only, uint32_t* total) {
+        const int r = radix_sort_bits<uint64_t>(ctx->d_bz_k0.as<uint64_t>(), ctx->d_bz_v0.as<uint32_t>(), ctx->d_bz_k1.as<uint64_t>(),
+                                                ctx->d_bz_v1.as<uint32_t>(), nrec, 0, 64, ctx->d_bz_hist.as<uint32_t>(), ctx->d_bz_scan.as<uint32_t>(), st);
+        cudaMemsetAsync(isfirst, 0, 4 * (size_t)(nrec + 1), st);
+        LAUNCH(k_first, nblk(nrec, 256), 256, 0, r ? ctx->d_bz_k1.as<uint64_t>() : ctx->d_bz_k0.as<uint64_t>(),
+               r ? ctx->d_bz_v1.as<uint32_t>() : ctx->d_bz_v0.as<uint32_t>(), nrec, raw, offs, info, bc_only, first, isfirst);
+        exclusive_scan_u32(isfirst, first == ctx->d_bz_first.as<uint32_t>() ? ctx->d_bz_k1.as<uint32_t>() : ctx->d_bz_v1.as<uint32_t>(), nrec,
+                           ctx->d_bz_scan.as<uint32_t>(), total, st);
+    };
+    // frag ids land in d_bz_k1 (viewed as u32) once the identity sort no longer needs it; dictionary ids in d_bz_v1
+    number(ctx->d_bz_first.as<uint32_t>(), ctx->d_bz_isfirst.as<uint32_t>(), 0, small + 4);
+    uint32_t any_dict = 0;
+    CK(cudaMemcpyAsync(&any_dict, small + 2, 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    uint32_t* fid = ctx->d_bz_k1.as<uint32_t>();
+    uint32_t* dfirst = nullptr; uint32_t* did = nullptr; uint32_t* disfirst = nullptr;
+    if (any_dict) {
+        // the identity ids move out of d_bz_k1 before the dictionary sort reuses it
+        CK(ctx->d_bz_disfirst.ensure(4 * (size_t)(nrec + 1)));
+        CK(cudaMemcpyAsync(ctx->d_bz_isfirst.p, fid, 4 * (size_t)nrec, cudaMemcpyDeviceToDevice, st));
+        fid = ctx->d_bz_isfirst.as<uint32_t>();
+        CK(ctx->d_bz_dfirst.ensure(4 * (size_t)(nrec + 1)));
+        LAUNCH(k_dict_keys, nblk(nrec, 256), 256, 0, raw, offs, nrec, info, ctx->d_bz_k0.as<uint64_t>(), ctx->d_bz_v0.as<uint32_t>());
+        dfirst = ctx->d_bz_dfirst.as<uint32_t>(); disfirst = ctx->d_bz_disfirst.as<uint32_t>();
+        number(dfirst, disfirst, 1, small + 5);
+        did = ctx->d_bz_v1.as<uint32_t>();
+    }
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ev[5], st));
+    // ---- offsets: output slots and payload offsets (scans of the four counts), their totals, then the output arena
+    for (int k = 0; k < 4; ++k) exclusive_scan_u32(cnt + (size_t)k * nrec, cnt + (size_t)k * nrec, nrec, ctx->d_bz_scan.as<uint32_t>(), small + 6 + k, st);
+    CK(cudaEventRecord(ev[6], st));
+    uint32_t tot[6] = {0, 0, 0, 0, 0, 0};                 // identities, dictionary barcodes, kept reads, seq bytes, quality bytes, CIGAR words
+    unsigned long long bad = 0;
+    CK(cudaMemcpyAsync(tot, small + 4, sizeof(tot), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&bad, small, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (bad != ~0ull) { ctx->err = "malformed BAM record (field lengths exceed block_size)"; return SMC_E_ARG; }
+    const int64_t n = tot[2], ndict = any_dict ? tot[1] : 0;
+    // the arena: every output array 256-byte aligned, in one device buffer and one pinned host buffer (one copy back)
+    size_t at = 0;
+    auto carve = [&](size_t bytes) { const size_t o = at; at += (bytes + 255) & ~(size_t)255; return o; };
+    const size_t o_ref = carve(4 * n), o_pos = carve(4 * n), o_nm = carve(4 * n), o_lseq = carve(4 * n), o_slo = carve(do_trim ? 4 * n : 0),
+                 o_slen = carve(do_trim ? 4 * n : 0), o_frag = carve(4 * n), o_flag = carve(2 * n), o_ncig = carve(2 * n), o_mapq = carve(n),
+                 o_soff = carve(8 * n), o_qoff = carve(8 * n), o_coff = carve(8 * n), o_umi = carve(8 * n), o_cig = carve(4 * (size_t)tot[5]),
+                 o_seq = carve(tot[3]), o_qual = carve(tot[4]), o_hist = carve(256 * 8);
+    CK(ctx->d_bz_out.ensure(at));
+    // Ordinary host memory: a decode is one copy back, and page-locking the arena cost 250-290 ms for a 100-interval panel on a
+    // B200 host (profiles/bam_decode_gpu_b200.jsonl) against about 12 ms for the copy itself
+    if (ctx->h_bz_cap < at) {
+        free(ctx->h_bz_out);
+        ctx->h_bz_out = malloc(at ? at : 1);
+        if (!ctx->h_bz_out) { ctx->h_bz_cap = 0; ctx->err = "smc_decode_bam: out of host memory for the decoded arrays"; return SMC_E_CUDA; }
+        ctx->h_bz_cap = at;
+    }
+    CK(cudaEventRecord(ev[7], st));           // ev[6] .. ev[7]: the totals' round trip and the output arena's allocation (host)
+    uint8_t* D = ctx->d_bz_out.as<uint8_t>();
+    uint8_t* H = static_cast<uint8_t*>(ctx->h_bz_out);
+    BamOut o;
+    o.ref_id = (int32_t*)(D + o_ref); o.pos = (int32_t*)(D + o_pos); o.nm = (int32_t*)(D + o_nm); o.l_seq = (int32_t*)(D + o_lseq);
+    o.store_lo = (int32_t*)(D + o_slo); o.store_len = (int32_t*)(D + o_slen); o.frag_id = (uint32_t*)(D + o_frag);
+    o.flag = (uint16_t*)(D + o_flag); o.n_cigar = (uint16_t*)(D + o_ncig); o.mapq = D + o_mapq; o.seq_off = (int64_t*)(D + o_soff);
+    o.qual_off = (int64_t*)(D + o_qoff); o.cigar_off = (int64_t*)(D + o_coff); o.umi = (uint64_t*)(D + o_umi); o.cigar = D + o_cig;
+    o.seq = D + o_seq; o.qual = D + o_qual; o.qual_hist = (unsigned long long*)(D + o_hist);
+    o.n = n; o.seq_bytes = tot[3]; o.qual_bytes = tot[4]; o.cigar_words = tot[5];
+    CK(cudaMemsetAsync(o.qual_hist, 0, 256 * 8, st));
+    if (ndict) {
+        CK(ctx->d_bz_dict.ensure((size_t)ndict * (BAM_DICT_STRIDE + 4)));
+        LAUNCH(k_dict_strings, nblk(nrec, 256), 256, 0, raw, offs, nrec, info, disfirst, did, ctx->d_bz_dict.as<uint8_t>(),
+               reinterpret_cast<uint32_t*>(ctx->d_bz_dict.as<uint8_t>() + (size_t)ndict * BAM_DICT_STRIDE));
+    }
+    LAUNCH(k_copy, (unsigned)std::min<int64_t>(nblk(nrec, COPY_WARPS), (int64_t)ctx->n_sm * 32), COPY_WARPS * 32, 0, raw, offs, nrec, info, cnt, ctx->d_bz_first.as<uint32_t>(), fid, dfirst, did, do_trim, o);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ev[8], st));
+    CK(cudaMemcpyAsync(H, D, at, cudaMemcpyDeviceToHost, st));
+    std::vector<uint8_t> dict;
+    if (ndict) {
+        dict.resize((size_t)ndict * (BAM_DICT_STRIDE + 4));
+        CK(cudaMemcpyAsync(dict.data(), ctx->d_bz_dict.p, dict.size(), cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaEventRecord(ev[9], st));
+    CK(cudaStreamSynchronize(st));
+    ctx->bz_dict.clear();
+    for (int64_t k = 0; k < ndict; ++k) {
+        uint32_t len;
+        memcpy(&len, &dict[(size_t)ndict * BAM_DICT_STRIDE + 4 * (size_t)k], 4);
+        ctx->bz_dict.emplace_back(reinterpret_cast<const char*>(&dict[(size_t)k * BAM_DICT_STRIDE]), len);
+    }
+    if (timing) {
+        static const char* stage[NEV - 1] = {"H2D compressed", "inflate", "record boundaries", "fields + hash", "fragment identities",
+                                             "offsets", "totals + output arena (host)", "copy", "D2H"};
+        for (int k = 0; k < NEV - 1; ++k) {
+            float ms = 0.f;
+            cudaEventElapsedTime(&ms, ev[k], ev[k + 1]);
+            fprintf(stderr, "[smc_b200] bam decode %s: %.3f ms\n", stage[k], ms);
+        }
+        float ms = 0.f;
+        cudaEventElapsedTime(&ms, ev[0], ev[NEV - 1]);
+        fprintf(stderr, "[smc_b200] bam decode total: %.3f ms (%lld blocks, %lld compressed bytes, %lld inflated, %lld records, %lld kept)\n", ms,
+                (long long)nb, (long long)comp_bytes, (long long)raw_bytes, (long long)nrec, (long long)n);
+    }
+    *out = smc_bam_reads{};
+    out->n_reads = n;
+    out->ref_id = (const int32_t*)(H + o_ref); out->pos = (const int32_t*)(H + o_pos); out->flag = (const uint16_t*)(H + o_flag);
+    out->mapq = H + o_mapq; out->nm = (const int32_t*)(H + o_nm); out->l_seq = (const int32_t*)(H + o_lseq);
+    out->seq_off = (const int64_t*)(H + o_soff); out->qual_off = (const int64_t*)(H + o_qoff); out->cigar_off = (const int64_t*)(H + o_coff);
+    out->n_cigar = (const uint16_t*)(H + o_ncig); out->umi = (const uint64_t*)(H + o_umi); out->frag_id = (const uint32_t*)(H + o_frag);
+    out->seq = H + o_seq; out->seq_bytes = tot[3]; out->qual = H + o_qual; out->qual_bytes = tot[4];
+    out->cigar = (const uint32_t*)(H + o_cig); out->n_cigar_words = tot[5]; out->n_dict_umis = ndict;
+    out->store_lo = do_trim ? (const int32_t*)(H + o_slo) : nullptr; out->store_len = do_trim ? (const int32_t*)(H + o_slen) : nullptr;
+    out->qual_hist = (const uint64_t*)(H + o_hist);
+    // the results are in the pinned arena: the device side of the decode goes back to the pool (a context that keeps the arrays
+    // alive for the rest of a run holds no device memory for them)
+    for (DevBuf* b : {&ctx->d_bz_comp, &ctx->d_bz_jobs, &ctx->d_bz_raw, &ctx->d_bz_scratch, &ctx->d_bz_status, &ctx->d_bz_walk, &ctx->d_bz_base,
+                      &ctx->d_bz_offs, &ctx->d_bz_info, &ctx->d_bz_cnt, &ctx->d_bz_k0, &ctx->d_bz_k1, &ctx->d_bz_v0, &ctx->d_bz_v1, &ctx->d_bz_first,
+                      &ctx->d_bz_isfirst, &ctx->d_bz_dfirst, &ctx->d_bz_disfirst, &ctx->d_bz_hist, &ctx->d_bz_scan, &ctx->d_bz_tg, &ctx->d_bz_out,
+                      &ctx->d_bz_dict, &ctx->d_bz_small})
+        b->release();
+    return SMC_OK;
+}
+
+extern "C" const char* smc_decoded_dict_umi(smc_ctx* ctx, int64_t i) {
+    return (ctx && i >= 0 && i < (int64_t)ctx->bz_dict.size()) ? ctx->bz_dict[(size_t)i].c_str() : "";
+}
+
+// caller-given raw DEFLATE streams through the device inflater (a validation entry point, like smc_fisher_exact)
+extern "C" int smc_inflate_device(smc_ctx* ctx, int64_t n, const uint8_t* in, int64_t in_bytes, const int64_t* in_off, const int64_t* in_len,
+                                  uint8_t* out, int64_t out_bytes, const int64_t* out_off, const int64_t* out_len, int32_t* status) {
+    if (!ctx) return SMC_E_ARG;
+    if (n < 0 || in_bytes < 0 || out_bytes < 0 || (n > 0 && (!in || !in_off || !in_len || !out || !out_off || !out_len || !status))) {
+        ctx->err = "smc_inflate_device: bad argument"; return SMC_E_ARG;
+    }
+    std::vector<BgzfJob> jobs((size_t)n);
+    for (int64_t i = 0; i < n; ++i) {
+        if (in_off[i] < 0 || in_len[i] < 0 || in_off[i] + in_len[i] + 64 > in_bytes || out_off[i] < 0 || out_len[i] < 0 ||
+            out_len[i] > 0xffffffffll || out_off[i] + out_len[i] > out_bytes) {
+            ctx->err = "smc_inflate_device: stream " + std::to_string(i) + " does not fit its buffers"; return SMC_E_ARG;
+        }
+        jobs[(size_t)i] = BgzfJob{in_off[i], in_len[i], out_off[i], 0, (uint32_t)out_len[i], 0u, (uint32_t)out_len[i], 1u};
+    }
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->st;
+    CK(ctx->d_bz_comp.ensure((size_t)in_bytes + 1));
+    CK(ctx->d_bz_raw.ensure((size_t)out_bytes + 1));
+    CK(ctx->d_bz_jobs.ensure(sizeof(BgzfJob) * (size_t)(n + 1)));
+    CK(ctx->d_bz_status.ensure(4 * (size_t)(n + 1)));
+    if (n == 0) return SMC_OK;
+    CK(cudaMemcpyAsync(ctx->d_bz_comp.p, in, (size_t)in_bytes, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ctx->d_bz_raw.p, out, (size_t)out_bytes, cudaMemcpyHostToDevice, st));     // whatever lies between the outputs stays
+    CK(cudaMemcpyAsync(ctx->d_bz_jobs.p, jobs.data(), sizeof(BgzfJob) * (size_t)n, cudaMemcpyHostToDevice, st));
+    LAUNCH(k_inflate, nblk(n, INFLATE_WARPS), INFLATE_WARPS * 32, 0, ctx->d_bz_comp.as<uint8_t>(), ctx->d_bz_jobs.as<BgzfJob>(), n,
+           ctx->d_bz_raw.as<uint8_t>(), (uint8_t*)nullptr, ctx->d_bz_status.as<int32_t>(), 0);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(out, ctx->d_bz_raw.p, (size_t)out_bytes, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(status, ctx->d_bz_status.p, 4 * (size_t)n, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
     return SMC_OK;
 }

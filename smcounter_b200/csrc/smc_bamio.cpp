@@ -17,11 +17,15 @@
 #include <vector>
 
 #include "../../include/smc_bamio.h"
+#include "smc_bamrec.h"
 #include "smc_host.h"
 #include "smc_inflate.h"
 
 using smc_host::for_each_thread;
 using smc_host::for_ranges;
+using smc_rec::rd16;
+using smc_rec::rd32;
+using smc_rec::rdi32;
 
 namespace {
 thread_local std::string g_open_error;
@@ -30,10 +34,6 @@ thread_local std::string g_open_error;
 smc_host::PhaseTimer phase_timer() { return smc_host::PhaseTimer("SMC_BAM_TIMING", "smc_bamio"); }
 
 int out_of_memory(std::string& err, const char* what) { err = std::string("out of memory for ") + what; return -1; }
-
-inline uint16_t rd16(const uint8_t* p) { uint16_t v; memcpy(&v, p, 2); return v; }
-inline uint32_t rd32(const uint8_t* p) { uint32_t v; memcpy(&v, p, 4); return v; }
-inline int32_t rdi32(const uint8_t* p) { int32_t v; memcpy(&v, p, 4); return v; }
 
 // one BGZF block: its deflate payload at coff, and the bytes [lo, hi) of its isize inflated ones that go to uoff of the stream
 struct Block { size_t coff, clen; size_t uoff; uint32_t isize, lo, hi; };
@@ -87,11 +87,20 @@ struct smc_bam {
     uint64_t qual_hist[256] = {0};              // how often every phred value occurs among the stored qualities
     int trim = 0;
     bool decoded = false;
-    // opened through an index (smc_bam_open_indexed): raw holds only the header until smc_bam_decode reads the chunks it needs
-    bool indexed = false;
-    std::string path, index_path;
+    // opened header-only (smc_bam_open_indexed, smc_bam_open_header): raw holds only the header until smc_bam_decode reads the
+    // chunks it needs, or the whole file (no index, or no intervals)
+    bool lazy = false;
+    std::string path, index_path;               // index_path empty: no index
     size_t file_size = 0;
     std::vector<BaiRef> bai;
+    // smc_bam_plan / smc_bam_read_blocks: the compressed byte ranges to read (file offset, end, offset in the caller's buffer),
+    // their chunks (empty: the whole file) and, once read, the blocks
+    struct Range { size_t cbeg, cend, buf; };
+    std::vector<Range> plan_ranges;
+    std::vector<BaiChunk> plan_chunks;
+    size_t plan_comp = 0;
+    bool planned = false, plan_whole = false;
+    std::vector<smc_bgzf_block> plan_blocks;
 };
 
 // the BGZF header at seg[off] (seg has n bytes): 0 and its BSIZE (the block's size - 1, from the BC subfield) and XLEN;
@@ -161,14 +170,14 @@ static int inflate_blocks(const uint8_t* src, const std::vector<Block>& blocks, 
     return 0;
 }
 
-static int inflate_all(const Buf<uint8_t>& file, int threads, Buf<uint8_t>& out, std::string& err) {
-    std::vector<Block> blocks;
-    size_t off = 0, uoff = 0;
-    const size_t n = file.size();
+// the blocks of a whole BGZF file of n bytes at data, back to back in the inflated stream; uoff = the stream's length
+static int file_blocks(const uint8_t* data, size_t n, std::vector<Block>& blocks, size_t& uoff, std::string& err) {
+    size_t off = 0;
+    uoff = 0;
     while (off < n) {
         Block b;
         size_t nxt = 0;
-        const int rc = bgzf_block(file.data(), n, off, b, nxt);
+        const int rc = bgzf_block(data, n, off, b, nxt);
         if (rc == 1) { err = "not a BGZF block at offset " + std::to_string(off); return -1; }
         if (rc == 2) { err = "truncated or malformed BGZF block at offset " + std::to_string(off); return -1; }
         b.uoff = uoff;
@@ -176,6 +185,13 @@ static int inflate_all(const Buf<uint8_t>& file, int threads, Buf<uint8_t>& out,
         blocks.push_back(b);
         off = nxt;
     }
+    return 0;
+}
+
+static int inflate_all(const Buf<uint8_t>& file, int threads, Buf<uint8_t>& out, std::string& err) {
+    std::vector<Block> blocks;
+    size_t uoff = 0;
+    if (file_blocks(file.data(), file.size(), blocks, uoff, err) != 0) return -1;
     if (!out.resize(uoff)) return out_of_memory(err, "the inflated BAM");
     return inflate_blocks(file.data(), blocks, threads, out, err);
 }
@@ -323,16 +339,17 @@ static int parse_bai(const std::string& ipath, size_t n_ref_bam, std::vector<Bai
     return 0;
 }
 
-extern "C" int smc_bam_open_indexed(const char* path, const char* index_path, int threads, smc_bam** out) {
-    if (!path || !index_path || !out) { g_open_error = "smc_bam_open_indexed: null argument"; return -2; }
+// a handle that holds only the header: the BGZF blocks from offset 0, inflated one at a time until the header text and the
+// reference list are complete (h->first_record: the header's length in the inflated stream); nullptr and g_open_error on failure
+static smc_bam* open_header(const char* path, int threads) {
     auto pt = phase_timer();
     threads = smc_host::n_threads(threads);
     const int fd = open(path, O_RDONLY);
-    if (fd < 0) { g_open_error = std::string("smc_bam_open: cannot open ") + path; return -1; }
+    if (fd < 0) { g_open_error = std::string("smc_bam_open: cannot open ") + path; return nullptr; }
     struct stat st;
     const size_t size = fstat(fd, &st) == 0 && st.st_size > 0 ? (size_t)st.st_size : 0;
     smc_bam* h = new smc_bam();
-    h->threads = threads; h->indexed = true; h->path = path; h->index_path = index_path; h->file_size = size;
+    h->threads = threads; h->lazy = true; h->path = path; h->file_size = size;
     // the header: BGZF blocks from offset 0, one at a time, until the header text and the reference list are complete
     std::vector<uint8_t> comp((size_t(1) << 16) + 64, 0), hdr;
     size_t off = 0, comp_read = 0;
@@ -357,9 +374,26 @@ extern "C" int smc_bam_open_indexed(const char* path, const char* index_path, in
         off += nxt;
     }
     close(fd);
-    if (st_hdr != 0) { delete h; return -1; }
+    if (st_hdr != 0) { delete h; return nullptr; }
     pt.lap("header blocks");
     timing_bytes("header", comp_read, hdr.size());
+    return h;
+}
+
+extern "C" int smc_bam_open_header(const char* path, int threads, smc_bam** out) {
+    if (!path || !out) { g_open_error = "smc_bam_open_header: null argument"; return -2; }
+    smc_bam* h = open_header(path, threads);
+    if (!h) return -1;
+    *out = h;
+    return 0;
+}
+
+extern "C" int smc_bam_open_indexed(const char* path, const char* index_path, int threads, smc_bam** out) {
+    if (!path || !index_path || !out) { g_open_error = "smc_bam_open_indexed: null argument"; return -2; }
+    auto pt = phase_timer();
+    smc_bam* h = open_header(path, threads);
+    if (!h) return -1;
+    h->index_path = index_path;
     const int rc = parse_bai(h->index_path, h->ref_names.size(), h->bai, g_open_error);
     if (rc != 0) { delete h; return rc; }
     pt.lap("index parse");
@@ -379,10 +413,11 @@ static void reg2bins(int64_t beg, int64_t end, std::vector<uint32_t>& out) {
     for (int64_t k = 4681 + (beg >> 14); k <= 4681 + (end >> 14); ++k) out.push_back((uint32_t)k);
 }
 
-// h->raw = the records of the index chunks that the intervals need, in file order.  A chunk [beg, end) covers whole records,
-// so the concatenated slices are a valid record chain; chunks that share a BGZF block are merged, which adds only whole records
-// in between (dropped by the interval filter like any other) and inflates every block once.
-static int load_chunks(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, const int32_t* iv_start, const int32_t* iv_end) {
+// The index chunks that the intervals need, in file order (h->plan_chunks), and their compressed byte ranges (h->plan_ranges,
+// back to back from buffer offset 0; h->plan_comp bytes in all).  A chunk [beg, end) covers whole records, so the concatenated
+// slices are a valid record chain; chunks that share a BGZF block are merged, which adds only whole records in between (dropped
+// by the interval filter like any other) and inflates every block once.
+static int chunk_ranges(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, const int32_t* iv_start, const int32_t* iv_end) {
     auto pt = phase_timer();
     const std::string who = "BAM index " + h->index_path + ": ";
     auto chunk_error = [&](const BaiChunk& c, const std::string& what) {
@@ -407,7 +442,8 @@ static int load_chunks(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, const in
         }
     }
     std::sort(ch.begin(), ch.end(), [](const BaiChunk& a, const BaiChunk& b) { return a.beg < b.beg || (a.beg == b.beg && a.end < b.end); });
-    std::vector<BaiChunk> merged;
+    std::vector<BaiChunk>& merged = h->plan_chunks;
+    merged.clear();
     for (const BaiChunk& c : ch) {
         if (!merged.empty() && (c.beg >> 16) <= (merged.back().end >> 16)) merged.back().end = std::max(merged.back().end, c.end);
         else merged.push_back(c);
@@ -417,8 +453,7 @@ static int load_chunks(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, const in
     // of that block when the end is at its offset 0)
     const int fd = open(h->path.c_str(), O_RDONLY);
     if (fd < 0) { h->err = "smc_bam_decode: cannot open " + h->path; return -1; }
-    struct Range { size_t cbeg, cend, buf; };
-    std::vector<Range> ranges;
+    h->plan_ranges.clear();
     size_t total = 0;
     int rc = 0;
     for (const BaiChunk& c : merged) {
@@ -440,26 +475,40 @@ static int load_chunks(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, const in
         }
         if (stop > h->file_size || cbeg >= h->file_size) { rc = chunk_error(c, "points past the end of " + h->path); break; }
         if (cbeg >= stop) { rc = chunk_error(c, "is malformed"); break; }
-        ranges.push_back({cbeg, stop, total});
+        h->plan_ranges.push_back({cbeg, stop, total});
         total += stop - cbeg;
     }
-    Buf<uint8_t> comp;
-    if (rc == 0 && !comp.resize(total, 64)) rc = out_of_memory(h->err, "the compressed chunks");
-    if (rc == 0) {
-        std::vector<std::array<size_t, 3>> pieces;
-        for (const Range& g : ranges) add_pieces(pieces, g.cbeg, g.buf, g.cend - g.cbeg);
-        if (!pread_pieces(fd, comp.p, pieces, h->threads)) { h->err = "smc_bam_decode: short read of " + h->path; rc = -1; }
-    }
     close(fd);
-    if (rc != 0) return rc;
-    pt.lap("index: chunk reads");
-    // the blocks of every range, each with the slice of its inflated bytes that the chunk covers
-    std::vector<Block> blocks;
-    size_t uoff = 0;
-    for (size_t g = 0; g < ranges.size(); ++g) {
-        const Range& R = ranges[g];
-        const BaiChunk& c = merged[g];
-        const uint8_t* seg = comp.p + R.buf;
+    h->plan_comp = total;
+    return rc;
+}
+
+// read the planned ranges into buf (plan_comp bytes, readable and zeroed 64 bytes past them)
+static int read_ranges(smc_bam* h, uint8_t* buf) {
+    const int fd = open(h->path.c_str(), O_RDONLY);
+    if (fd < 0) { h->err = "smc_bam_decode: cannot open " + h->path; return -1; }
+    std::vector<std::array<size_t, 3>> pieces;
+    for (const auto& g : h->plan_ranges) add_pieces(pieces, g.cbeg, g.buf, g.cend - g.cbeg);
+    const bool ok = pread_pieces(fd, buf, pieces, h->threads);
+    close(fd);
+    memset(buf + h->plan_comp, 0, 64);
+    if (!ok) { h->err = "smc_bam_decode: short read of " + h->path; return -1; }
+    return 0;
+}
+
+// the blocks of every planned chunk range read into comp, each with the slice of its inflated bytes that the chunk covers;
+// uoff = the length of the concatenated slices
+static int chunk_blocks(smc_bam* h, const uint8_t* comp, std::vector<Block>& blocks, size_t& uoff) {
+    const std::string who = "BAM index " + h->index_path + ": ";
+    auto chunk_error = [&](const BaiChunk& c, const std::string& what) {
+        h->err = who + "chunk [" + std::to_string(c.beg) + ", " + std::to_string(c.end) + ") " + what;
+        return -3;
+    };
+    uoff = 0;
+    for (size_t g = 0; g < h->plan_ranges.size(); ++g) {
+        const auto& R = h->plan_ranges[g];
+        const BaiChunk& c = h->plan_chunks[g];
+        const uint8_t* seg = comp + R.buf;
         const size_t n = R.cend - R.cbeg;
         for (size_t off = 0; off < n;) {
             Block b;
@@ -477,11 +526,77 @@ static int load_chunks(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, const in
             off = nxt;
         }
     }
+    return 0;
+}
+
+// h->raw = the records of the index chunks that the intervals need, in file order
+static int load_chunks(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, const int32_t* iv_start, const int32_t* iv_end) {
+    int rc = chunk_ranges(h, n_iv, iv_ref, iv_start, iv_end);
+    if (rc != 0) return rc;
+    auto pt = phase_timer();
+    Buf<uint8_t> comp;
+    if (!comp.resize(h->plan_comp, 64)) return out_of_memory(h->err, "the compressed chunks");
+    if ((rc = read_ranges(h, comp.p)) != 0) return rc;
+    pt.lap("index: chunk reads");
+    std::vector<Block> blocks;
+    size_t uoff = 0;
+    if ((rc = chunk_blocks(h, comp.p, blocks, uoff)) != 0) return rc;
     if (!h->raw.resize(uoff)) return out_of_memory(h->err, "the inflated chunks");
     if (inflate_blocks(comp.data(), blocks, h->threads, h->raw, h->err) != 0) return -1;
     h->first_record = 0;
     pt.lap("index: chunk inflate");
-    timing_bytes("index chunks", total, uoff);
+    timing_bytes("index chunks", h->plan_comp, uoff);
+    return 0;
+}
+
+// ---- the blocks of a decode without inflating them (a decoder elsewhere inflates them: include/smc_b200.h smc_decode_bam)
+extern "C" int smc_bam_plan(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, const int32_t* iv_start, const int32_t* iv_end, int64_t* comp_bytes) {
+    if (!h || !comp_bytes || (n_iv > 0 && (!iv_ref || !iv_start || !iv_end))) { if (h) h->err = "smc_bam_plan: null argument"; return -2; }
+    if (!h->lazy || h->planned) { h->err = "smc_bam_plan: needs a handle opened header-only (smc_bam_open_header / _indexed), planned once"; return -2; }
+    h->planned = true;
+    h->plan_ranges.clear(); h->plan_chunks.clear(); h->plan_comp = 0;
+    try {
+        if (n_iv > 0 && !h->index_path.empty()) {
+            const int rc = chunk_ranges(h, n_iv, iv_ref, iv_start, iv_end);
+            if (rc != 0) return rc;
+        } else {
+            h->plan_ranges.push_back({0, h->file_size, 0});
+            h->plan_comp = h->file_size;
+            h->plan_whole = true;
+        }
+    } catch (const std::bad_alloc&) {
+        return out_of_memory(h->err, "the plan");
+    }
+    *comp_bytes = (int64_t)h->plan_comp;
+    return 0;
+}
+
+extern "C" int smc_bam_read_blocks(smc_bam* h, uint8_t* buf, smc_bgzf_plan* out) {
+    if (!h || !buf || !out) { if (h) h->err = "smc_bam_read_blocks: null argument"; return -2; }
+    if (!h->planned) { h->err = "smc_bam_read_blocks: smc_bam_plan first"; return -2; }
+    auto pt = phase_timer();
+    int rc = read_ranges(h, buf);
+    if (rc != 0) return rc;
+    pt.lap("read compressed blocks");
+    std::vector<Block> blocks;
+    size_t uoff = 0;
+    try {
+        rc = h->plan_whole ? file_blocks(buf, h->plan_comp, blocks, uoff, h->err) : chunk_blocks(h, buf, blocks, uoff);
+        if (rc != 0) return rc;
+        h->plan_blocks.resize(blocks.size());
+        for (size_t i = 0; i < blocks.size(); ++i) {
+            const Block& b = blocks[i];
+            h->plan_blocks[i] = smc_bgzf_block{(int64_t)b.coff, (int64_t)b.clen, (int64_t)b.uoff, b.isize, b.lo, b.hi, 0u};
+        }
+    } catch (const std::bad_alloc&) {
+        return out_of_memory(h->err, "the block table");
+    }
+    pt.lap("block table");
+    out->n_blocks = (int64_t)blocks.size();
+    out->blocks = h->plan_blocks.data();
+    out->comp_bytes = (int64_t)h->plan_comp;
+    out->raw_bytes = (int64_t)uoff;
+    out->first_record = h->plan_whole ? (int64_t)h->first_record : 0;
     return 0;
 }
 
@@ -496,43 +611,6 @@ extern "C" int smc_bam_n_refs(smc_bam* h) { return h ? (int)h->ref_names.size() 
 extern "C" const char* smc_bam_ref_name(smc_bam* h, int i) { return (h && i >= 0 && i < (int)h->ref_names.size()) ? h->ref_names[i].c_str() : ""; }
 extern "C" int64_t smc_bam_ref_length(smc_bam* h, int i) { return (h && i >= 0 && i < (int)h->ref_lens.size()) ? h->ref_lens[i] : -1; }
 extern "C" const char* smc_bam_dict_umi(smc_bam* h, int64_t i) { return (h && i >= 0 && i < (int64_t)h->dict_umis.size()) ? h->dict_umis[(size_t)i].c_str() : ""; }
-
-// value of the first NM tag in [p, end), 0 when absent (smCounter.py:329-334)
-static int32_t first_nm(const uint8_t* p, const uint8_t* end) {
-    while (p + 3 <= end) {
-        const uint8_t t0 = p[0], t1 = p[1], ty = p[2];
-        p += 3;
-        size_t sz = 0;
-        switch (ty) {
-            case 'A': case 'c': case 'C': sz = 1; break;
-            case 's': case 'S': sz = 2; break;
-            case 'i': case 'I': case 'f': sz = 4; break;
-            case 'Z': case 'H': { const void* q = memchr(p, 0, (size_t)(end - p)); if (!q) return 0; p = (const uint8_t*)q + 1; continue; }
-            case 'B': {
-                if (p + 5 > end) return 0;
-                const uint8_t sub = p[0];
-                const int32_t cnt = rdi32(p + 1);
-                const size_t es = (sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : 4;
-                p += 5 + (size_t)cnt * es;
-                continue;
-            }
-            default: return 0;
-        }
-        if (p + sz > end) return 0;
-        if (t0 == 'N' && t1 == 'M' && ty != 'A' && ty != 'f') {
-            switch (ty) {
-                case 'c': return (int8_t)p[0];
-                case 'C': return p[0];
-                case 's': { int16_t v; memcpy(&v, p, 2); return v; }
-                case 'S': return rd16(p);
-                case 'i': return rdi32(p);
-                default:  return (int32_t)rd32(p);
-            }
-        }
-        p += sz;
-    }
-    return 0;
-}
 
 // ------------------------------------------------------------------------------------------------------------
 // Record decode (smc_bam_decode), four passes, each a function below:
@@ -553,52 +631,18 @@ struct RecInfo {
     uint64_t code;                 // packed barcode, 0 = needs the dictionary
 };
 
-inline uint64_t mix64(uint64_t x) { x ^= x >> 32; x *= 0xd6e8feb86659fd93ull; x ^= x >> 32; x *= 0xd6e8feb86659fd93ull; x ^= x >> 32; return x; }
-inline void hash_bytes(const uint8_t* p, size_t n, uint64_t& a, uint64_t& b) {
-    while (n >= 8) { uint64_t w; memcpy(&w, p, 8); a = mix64(a ^ w); b = (b + w) * 0x9e3779b97f4a7c15ull; b ^= b >> 29; p += 8; n -= 8; }
-    uint64_t w = 0; memcpy(&w, p, n);
-    a = mix64(a ^ w ^ ((uint64_t)n << 56)); b = (b + w + n) * 0x9e3779b97f4a7c15ull; b ^= b >> 29;
-}
-
 template <class F> void parallel_for(size_t n, int threads, F&& f) {       // f(begin, end, thread); one thread per 4096 items at most
     for_ranges(n, (int)std::max<size_t>(1, std::min<size_t>((size_t)threads, (n + 4095) / 4096)), f);
 }
 
-// The target intervals of every reference, sorted and merged where they overlap.  Intervals that only touch ([a, b) and
-// [b, c)) stay apart: a read without reference length at b touches neither, and merging them would make it touch [a, c).
-struct Targets {
-    std::vector<std::vector<std::pair<int64_t, int64_t>>> by_ref;
-
-    Targets(size_t nref, int64_t n_iv, const int32_t* iv_ref, const int32_t* iv_start, const int32_t* iv_end) : by_ref(nref) {
-        for (int64_t k = 0; k < n_iv; ++k)
-            if (iv_ref[k] >= 0 && (size_t)iv_ref[k] < nref && iv_end[k] > iv_start[k]) by_ref[(size_t)iv_ref[k]].push_back({iv_start[k], iv_end[k]});
-        for (auto& v : by_ref) {
-            std::sort(v.begin(), v.end());
-            size_t m = 0;
-            for (const auto& pr : v) {
-                if (m > 0 && pr.first < v[m - 1].second) v[m - 1].second = std::max(v[m - 1].second, pr.second);
-                else v[m++] = pr;
-            }
-            v.resize(m);
-        }
-    }
-    // the intervals that the read [s, e) touches (start < e and end > s): [first, last), empty when the read touches no target.
-    // Starts and ends both ascend, so each bound is one binary search.
-    using It = std::vector<std::pair<int64_t, int64_t>>::const_iterator;
-    std::pair<It, It> touched(int32_t rid, int64_t s, int64_t e) const {
-        const auto& v = by_ref[(size_t)rid];
-        return {std::partition_point(v.begin(), v.end(), [&](const std::pair<int64_t, int64_t>& iv) { return iv.second <= s; }),
-                std::partition_point(v.begin(), v.end(), [&](const std::pair<int64_t, int64_t>& iv) { return iv.first < e; })};
-    }
-};
 }  // namespace
 
 // h->raw = the records to decode.  A handle opened through an index holds only the header so far: the records come from the
 // index chunks the intervals need, or from the whole file when there are no intervals.
 static int load_records(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, const int32_t* iv_start, const int32_t* iv_end) {
-    if (!h->indexed) return 0;
-    h->indexed = false;
-    if (n_iv > 0) return load_chunks(h, n_iv, iv_ref, iv_start, iv_end);
+    if (!h->lazy) return 0;
+    h->lazy = false;
+    if (n_iv > 0 && !h->index_path.empty()) return load_chunks(h, n_iv, iv_ref, iv_start, iv_end);
     auto pt = phase_timer();
     Buf<uint8_t> file;
     if (read_whole_file(h->path.c_str(), h->threads, file, h->err) != 0 || inflate_all(file, h->threads, h->raw, h->err) != 0) return -1;
@@ -613,19 +657,6 @@ static int load_records(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, const i
 // range's walk ends exactly where the next range started -- by induction from the known first record the chain is then
 // the true one.  Anything else (including a malformed record) falls back to the plain serial walk and its error report.
 static int record_offsets(const uint8_t* r, size_t begin, size_t size, size_t nref, int threads, std::vector<size_t>& offs, std::string& err) {
-    auto plausible = [&](size_t p) -> size_t {                // 0 = no; else offset of the next record
-        if (p + 36 > size) return 0;
-        const int32_t bs = rdi32(&r[p]);
-        if (bs < 32 || p + 4 + (size_t)bs > size) return 0;
-        const uint8_t* b = &r[p + 4];
-        const int32_t refID = rdi32(b), pos = rdi32(b + 4), l_seq = rdi32(b + 16), nref_id = rdi32(b + 20), npos = rdi32(b + 24);
-        const uint32_t l_rn = b[8], n_cig = rd16(b + 12);
-        if (refID < -1 || refID >= (int32_t)nref || pos < -1 || nref_id < -1 || nref_id >= (int32_t)nref || npos < -1) return 0;
-        if (l_rn < 1 || l_seq < 0) return 0;
-        const size_t need = 32 + (size_t)l_rn + 4 * (size_t)n_cig + ((size_t)l_seq + 1) / 2 + (size_t)l_seq;
-        if (need > (size_t)bs || b[32 + l_rn - 1] != 0) return 0;
-        return p + 4 + (size_t)bs;
-    };
     const size_t span = size > begin ? size - begin : 0;
     const int T = (int)std::max<size_t>(1, std::min<size_t>((size_t)threads, span / (4u << 20)));
     bool ok = T > 1;
@@ -637,15 +668,8 @@ static int record_offsets(const uint8_t* r, size_t begin, size_t size, size_t nr
             const size_t lo = begin + span * (size_t)t / T, hi = t + 1 == T ? size : begin + span * (size_t)(t + 1) / T;
             size_t p = lo;
             if (t > 0) {                                         // first plausible chain of three at or after lo
-                for (;; ++p) {
+                for (; !smc_rec::plausible_chain(r, p, size, nref); ++p)
                     if (p + 4 > hi + (1u << 20) || p + 4 > size) { good[t] = 0; return; }
-                    size_t q = plausible(p);
-                    if (!q) continue;
-                    size_t q2 = q + 4 <= size ? plausible(q) : (q == size ? q : 0);
-                    if (!q2) continue;
-                    if (q2 != size && q2 + 4 <= size && !plausible(q2)) continue;
-                    break;
-                }
             }
             first[t] = p;
             part[t].reserve((hi - lo) / 200 + 16);
@@ -680,7 +704,7 @@ static int record_offsets(const uint8_t* r, size_t begin, size_t size, size_t nr
 
 // ---- pass 2: per record the fields, the interval filter (tg: null without intervals), the stored window (trim), the barcode
 // code and the identity hash; n_kept = the reads kept
-static int record_fields(const uint8_t* r, const std::vector<size_t>& offs, size_t nref, const Targets* tg, bool trim, int threads,
+static int record_fields(const uint8_t* r, const std::vector<size_t>& offs, size_t nref, const smc_rec::Targets* tg, bool trim, int threads,
                          Buf<RecInfo>& info, size_t& n_kept, std::string& err) {
     const size_t nrec = offs.size();
     if (!info.resize(nrec)) return out_of_memory(err, "the record table");   // pass 2 writes keep for every record, the rest for kept ones
@@ -711,46 +735,18 @@ static int record_fields(const uint8_t* r, const std::vector<size_t>& offs, size
             if ((flag & 0x4) || refID < 0 || (size_t)refID >= nref) continue;
             R.store_lo = 0; R.store_len = (uint32_t)l_seq;
             if (tg) {
-                int64_t reflen = 0;
-                int n_run = 0; bool plain = true;                      // one aligned run, nothing but soft clips around it
-                for (uint16_t k = 0; k < n_cig; ++k) {
-                    const uint32_t cw = rd32(cig + 4 * k), op = cw & 15u;
-                    if (op == 0 || op == 2 || op == 3 || op == 7 || op == 8) reflen += cw >> 4;
-                    if (op == 0 || op == 7 || op == 8) ++n_run; else if (op != 4) plain = false;
-                }
-                const int64_t s0 = pos, e0 = (int64_t)pos + reflen;
-                const auto iv = tg->touched(refID, s0, e0);
-                if (iv.first >= iv.second) continue;
-                if (trim && plain && n_run == 1) {
-                    // query bases from the first to the last target position of the read (include/smc_b200.h: store_lo / store_len)
-                    const int64_t p_lo = std::max(s0, iv.first->first), p_hi = std::min(e0, (iv.second - 1)->second) - 1;
-                    const int64_t left_sp = (n_cig > 0 && (rd32(cig) & 15u) == 4) ? (int64_t)(rd32(cig) >> 4) : 0;
-                    const int64_t q_lo = (p_lo - s0 + left_sp) & ~1ll, q_hi = p_hi - s0 + left_sp + 1;
-                    if (q_lo >= 0 && q_hi <= l_seq && q_hi >= q_lo) { R.store_lo = (uint32_t)q_lo; R.store_len = (uint32_t)(q_hi - q_lo); }
-                }
+                bool plain = false;
+                const int64_t s0 = pos, e0 = (int64_t)pos + smc_rec::cigar_span(cig, n_cig, plain);
+                const size_t o = tg->off[(size_t)refID];
+                size_t a, e;
+                smc_rec::touched(tg->st.data() + o, tg->en.data() + o, tg->off[(size_t)refID + 1] - o, s0, e0, a, e);
+                if (a >= e) continue;
+                if (trim && plain) smc_rec::trim_window(s0, e0, tg->st[o + a], tg->en[o + e - 1], cig, n_cig, l_seq, R.store_lo, R.store_len);
             }
-            // identity: BC = parts[-2], readid = ':'.join(parts[:-2])   (smCounter.py:319-325)
-            const size_t qn = l_rn ? (size_t)l_rn - 1 : 0;
-            long c1 = -1, c2 = -1;                  // last and second-to-last ':'
-            for (long k = (long)qn - 1; k >= 0; --k)
-                if (qname[k] == ':') { if (c1 < 0) c1 = k; else { c2 = k; break; } }
-            if (c1 < 0) { R.bc_off = 0; R.bc_len = 0; R.rid_len = 0; }          // fewer than 2 fields: parts[-2] would raise in Python
-            else if (c2 < 0) { R.bc_off = 0; R.bc_len = (uint32_t)c1; R.rid_len = 0; }
-            else { R.bc_off = (uint32_t)(c2 + 1); R.bc_len = (uint32_t)(c1 - c2 - 1); R.rid_len = (uint32_t)c2; }
-            uint64_t code = 1;
-            bool packable = R.bc_len <= 31;
-            if (packable)
-                for (uint32_t k = 0; k < R.bc_len; ++k) {
-                    const char ch = qname[R.bc_off + k];
-                    const int v = ch == 'A' ? 0 : ch == 'C' ? 1 : ch == 'G' ? 2 : ch == 'T' ? 3 : -1;
-                    if (v < 0) { packable = false; break; }
-                    code = (code << 2) | (uint64_t)v;
-                }
-            R.code = packable ? code : 0;
-            uint64_t h1 = 0x243f6a8885a308d3ull ^ R.bc_len, h2 = 0x13198a2e03707344ull + R.rid_len;
-            hash_bytes(reinterpret_cast<const uint8_t*>(qname) + R.bc_off, R.bc_len, h1, h2);
-            hash_bytes(reinterpret_cast<const uint8_t*>(qname), R.rid_len, h1, h2);
-            R.h1 = h1; R.h2 = h2;
+            const uint8_t* qn8 = reinterpret_cast<const uint8_t*>(qname);
+            smc_rec::split_qname(qn8, l_rn ? (size_t)l_rn - 1 : 0, R.bc_off, R.bc_len, R.rid_len);
+            R.code = smc_rec::barcode_code(qn8 + R.bc_off, R.bc_len);
+            smc_rec::identity_hash(qn8, R.bc_off, R.bc_len, R.rid_len, R.h1, R.h2);
             R.keep = 1;
             ++kept_here;
         }
@@ -915,7 +911,7 @@ static void copy_records(smc_bam* h, const uint8_t* r, const std::vector<size_t>
             const uint8_t* sq = cig + 4 * (size_t)n_cig;
             const uint8_t* ql = sq + ((size_t)l_seq + 1) / 2;
             h->ref_id[o] = rdi32(b); h->pos[o] = rdi32(b + 4); h->flag[o] = rd16(b + 14); h->mapq[o] = b[9];
-            h->nm[o] = first_nm(ql + l_seq, rec_end); h->l_seq[o] = l_seq; h->n_cigar[o] = n_cig;
+            h->nm[o] = smc_rec::first_nm(ql + l_seq, rec_end); h->l_seq[o] = l_seq; h->n_cigar[o] = n_cig;
             const size_t w_lo = info[i].store_lo, w_len = info[i].store_len;
             if (trim) { h->store_lo[o] = (int32_t)w_lo; h->store_len[o] = (int32_t)w_len; }
             if (w_len) memcpy(&h->seq[(size_t)h->seq_off[o]], sq + w_lo / 2, (w_len + 1) / 2);
@@ -954,7 +950,7 @@ extern "C" int smc_bam_decode(smc_bam* h, int64_t n_iv, const int32_t* iv_ref, c
         const int rc = load_records(h, n_iv, iv_ref, iv_start, iv_end);
         if (rc != 0) { h->decoded = true; return rc; }
         const size_t nref = h->ref_names.size();
-        const Targets targets(nref, n_iv, iv_ref, iv_start, iv_end);
+        const smc_rec::Targets targets(nref, n_iv, iv_ref, iv_start, iv_end);
         const bool trim = h->trim && n_iv > 0;
         const uint8_t* r = h->raw.data();
         auto pt = phase_timer();

@@ -9,20 +9,30 @@
 #include <cstdint>
 #include <cstring>
 
+// Compiled for the device as well (smc_bgzf.cuh): SMC_HD marks the routines __host__ __device__ under nvcc and is empty under
+// a host compiler, so the host build is the same code either way.
+#ifndef SMC_HD
+#ifdef __CUDACC__
+#define SMC_HD __host__ __device__
+#else
+#define SMC_HD
+#endif
+#endif
+
 namespace smc_inflate_detail {
 
 constexpr int LIT_BITS = 10, DIST_BITS = 8, PRE_BITS = 7;
 constexpr int LIT_TABLE = 2048, DIST_TABLE = 1024;           // primary + worst-case secondary tables (zlib's ENOUGH: 1332 / 400)
 // entry: bits 0-7 code length, bits 8-15 op, bits 16-31 value
 constexpr uint32_t OP_LITERAL = 0, OP_BASE = 16 /* | extra bits: a length or a distance */, OP_END = 32, OP_LINK = 64 /* | sub bits */, OP_BAD = 128;
-inline uint32_t entry(uint32_t op, uint32_t bits, uint32_t val) { return bits | (op << 8) | (val << 16); }
+SMC_HD inline uint32_t entry(uint32_t op, uint32_t bits, uint32_t val) { return bits | (op << 8) | (val << 16); }
 
 struct Tables {
     uint32_t lit[LIT_TABLE];
     uint32_t dist[DIST_TABLE];
 };
 
-inline uint32_t reverse_bits(uint32_t code, int len) {
+SMC_HD inline uint32_t reverse_bits(uint32_t code, int len) {
     uint32_t r = 0;
     for (int i = 0; i < len; ++i) { r = (r << 1) | (code & 1u); code >>= 1; }
     return r;
@@ -31,7 +41,7 @@ inline uint32_t reverse_bits(uint32_t code, int len) {
 // Canonical Huffman table over `n` symbols with code lengths lens[] (0 = unused).  kind: 0 literal/length alphabet, 1 distance
 // alphabet, 2 code-length alphabet (values are the symbols themselves).  Returns the entries used, or -1 for an over-subscribed
 // code, or an incomplete one other than the single-code cases RFC 1951 allows.
-inline int build_table(const uint8_t* lens, int n, int root, int kind, uint32_t* table, int table_cap) {
+SMC_HD inline int build_table(const uint8_t* lens, int n, int root, int kind, uint32_t* table, int table_cap) {
     static const uint16_t len_base[29] = {3, 4, 5, 6, 7, 8, 9, 10, 11, 13, 15, 17, 19, 23, 27, 31, 35, 43, 51, 59, 67, 83, 99, 115, 131, 163, 195, 227, 258};
     static const uint8_t len_extra[29] = {0, 0, 0, 0, 0, 0, 0, 0, 1, 1, 1, 1, 2, 2, 2, 2, 3, 3, 3, 3, 4, 4, 4, 4, 5, 5, 5, 5, 0};
     static const uint16_t dist_base[30] = {1, 2, 3, 4, 5, 7, 9, 13, 17, 25, 33, 49, 65, 97, 129, 193, 257, 385, 513, 769, 1025, 1537, 2049, 3073, 4097, 6145,
@@ -97,7 +107,8 @@ inline int build_table(const uint8_t* lens, int n, int root, int kind, uint32_t*
 
 // Inflates one raw DEFLATE stream of exactly out_len bytes.  `in` must be readable up to in + in_len + 64 (the bit buffer is
 // refilled eight bytes at a time and may run a few refills past a truncated stream before the end checks stop it).  Returns 0, or -1 if the stream is malformed, does not end where it should, or does not produce out_len bytes.
-inline int smc_inflate_raw(const uint8_t* in, size_t in_len, uint8_t* out, size_t out_len) {
+// T: the decode tables (12 KiB), wherever the caller keeps them (the device decoder: shared memory).
+SMC_HD inline int smc_inflate_raw_t(const uint8_t* in, size_t in_len, uint8_t* out, size_t out_len, smc_inflate_detail::Tables& T) {
     using namespace smc_inflate_detail;
     const uint8_t* const in_end = in + in_len;
     uint8_t* const out_start = out;
@@ -113,7 +124,6 @@ inline int smc_inflate_raw(const uint8_t* in, size_t in_len, uint8_t* out, size_
         bitsleft |= 56u;                                                          \
     } while (0)
 #define SMC_TAKE(nb) (bitbuf >>= (nb), bitsleft -= (nb))
-    Tables T;
     static const uint8_t pre_order[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
     for (;;) {
         if (in > in_end + 8) return -1;
@@ -171,8 +181,8 @@ inline int smc_inflate_raw(const uint8_t* in, size_t in_len, uint8_t* out, size_
                     while (rep--) lens[i++] = (uint8_t)val;
                 }
                 if (lens[256] == 0) return -1;                              // no end-of-block code
-                // the distance lengths follow the literal / length ones: move them to a fixed place
-                memmove(lens + 288, lens + nlit, (size_t)ndist);
+                // the distance lengths follow the literal / length ones: move them to a fixed place (288 >= nlit: back to front)
+                for (int k = ndist - 1; k >= 0; --k) lens[288 + k] = lens[nlit + k];
                 for (int k = nlit; k < 288; ++k) lens[k] = 0;
             }
             if (build_table(lens, nlit, LIT_BITS, 0, T.lit, LIT_TABLE) < 0) return -1;
@@ -246,6 +256,11 @@ inline int smc_inflate_raw(const uint8_t* in, size_t in_len, uint8_t* out, size_
     const uint8_t* used = in - (bitsleft >> 3);
     if (out != out_end || used > in_end) return -1;
     return 0;
+}
+
+SMC_HD inline int smc_inflate_raw(const uint8_t* in, size_t in_len, uint8_t* out, size_t out_len) {
+    smc_inflate_detail::Tables T;
+    return smc_inflate_raw_t(in, in_len, out, out_len, T);
 }
 
 #endif

@@ -66,6 +66,7 @@ def argParseInit():
     parser.add_argument('--logFile', default=None, help='log file')
     parser.add_argument('--paramFile', default=None, help='optional parameter file that contains the above paramters. if specified, this must be the only parameter, except for --logFile.')
     parser.add_argument('--gpus', type=int, default=1, help='number of B200 GPUs to shard the target over (BED intervals, balanced by depth)')
+    parser.add_argument('--bamDecoder', choices=('host', 'gpu'), default='host', help='where the BAM is inflated and decoded: host (default, threaded C++) or gpu (the first GPU of the run; the same reads)')
     parser.add_argument('--fisherLegacy', type=int, default=0, help='1: two-sided Fisher p-values as scipy <= 1.6 computed them (epsilon = 1 - 1e-4, the scipy of the 2017 reference run); 0 (default): scipy >= 1.7')
 
 
@@ -325,7 +326,8 @@ def main(args):
         bed_lines = fh.readlines()
     intervals = intervals_from_bed_lines(bed_lines)
     refs = FastaFile(args.refGenome)
-    reads = read_bam(args.bamFile, intervals, threads=max(1, args.nCPU), trim=True)      # only the target windows cross PCIe
+    reads = read_bam(args.bamFile, intervals, threads=max(1, args.nCPU), trim=True,      # only the target windows cross PCIe
+                     device=0 if getattr(args, 'bamDecoder', 'host') == 'gpu' else None)
     prm = VcParams(mtDepth=args.mtDepth, rpb=args.rpb, minBQ=args.minBQ, minMQ=args.minMQ, hpLen=args.hpLen,
                    mismatchThr=args.mismatchThr, mtDrop=args.mtDrop, maxMT=args.maxMT, primerDist=args.primerDist,
                    fisherLegacy=args.fisherLegacy)
